@@ -4,14 +4,15 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]                 our CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W] the reference's CPU path on host cores
     python bench.py --workload sweep [--gpus N]                         BASELINE.json configs[4] only
+    python bench.py --dump-outputs DIR ...                              also save what the last timed step returned
 
 A step = one pass of the hot path over one batch of synthetic KITTI-shaped frames (BASELINE.json configs[1]:
 256 frames of 352x1216, 64-beam pattern, ~5 % density; outputs filled depth + distance channel + validity mask).
 Weak scaling: every rank processes its own batch of 256 frames per step; `value` = total frames of all ranks /
-max-over-ranks device time.  The K-step block is repeated until the timed region has lasted >= 1 s; the median
-block is reported.  After the timed region 64 frames of the timed run's own outputs are compared with the CPU
-oracle, bit for bit (`parity_checked`).  `e2e` is the drop-in call `tools.DT_complete_batch(x)` with pageable numpy
-arrays in and out (tools.py:13-35); `e2e_pinned` is the C ABI with pinned buffers and all three outputs.
+max-over-ranks device time of exactly K timed steps between two CUDA events.  After the timed region 64 frames of
+the timed run's own outputs are compared with the CPU oracle, bit for bit (`parity_checked`).  `e2e` is the drop-in
+call `tools.DT_complete_batch(x)` with pageable numpy arrays in and out (tools.py:13-35); `e2e_pinned` is the C ABI
+with pinned buffers and all three outputs.
 The same line carries `sweep`: BASELINE.json configs[4] (8192 frames sharded over the ranks, fill + per-frame
 metrics on the GPU, one NCCL sum all-reduce of the totals inside the timed region; strong scaling).
 Prints ONE JSON line on rank 0.
@@ -46,6 +47,27 @@ def measured_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+DUMP_BYTES = 60_000_000      # --dump-outputs stays below 64 MB
+
+
+def dump_outputs(path: str, out: dict, B: int, H: int, W: int):
+    """What one step returned to its caller (DTFillEngine.fill: depth, dt, mask, counts) as DIR/<name>.npy in float32 or
+    float64: depth, dt and mask of a fixed, seeded sample of the batch's frames (11 of 256 KITTI frames fit the budget),
+    counts [B,2] of every frame, and frame_index, the sampled frames' positions in the batch."""
+    import torch
+    n = min(B, DUMP_BYTES // (12 * H * W))
+    sel = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    tsel = torch.from_numpy(sel).to(out["depth"].device)
+    arrays = {"frame_index": sel.astype(np.float64),
+              "depth": out["depth"][tsel].cpu().numpy(),
+              "dt": out["dt"][tsel].cpu().numpy(),
+              "mask": out["mask"][tsel].cpu().numpy().astype(np.float32),
+              "counts": out["counts"].cpu().numpy().astype(np.float64)}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -469,9 +491,8 @@ def run_ours(args, rank, world, local_rank):
     no = len(outs)
     K = args.steps
 
-    def timed_blocks(depth, min_seconds):
-        """Blocks of exactly K steps between two events on the launching stream (max over ranks per block), repeated
-        until the timed region has lasted min_seconds; clocks are sampled over the whole region."""
+    def timed_steps(depth):
+        """Exactly K steps between two events on the launching stream (max over ranks); clocks are sampled over them."""
         eng.handle.set_pipeline_depth(depth)
         for i in range(args.warmup):
             eng.fill(x, src_thr=src_thr, out=outs[i % no])
@@ -480,41 +501,37 @@ def run_ours(args, rank, world, local_rank):
         sampler_ = ClockSampler(local_rank)
         barrier()
         sampler_.start()
-        blocks, total = [], 0.0
-        while total < min_seconds * 1e3 and len(blocks) < 2000:
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for i in range(K):
-                eng.fill(x, src_thr=src_thr, out=outs[i % no])
-            eng.flush()                                   # every step's outputs are complete at e1
-            e1.record()
-            barrier()
-            ms_ = e0.elapsed_time(e1)
-            if dist is not None:
-                t_ = torch.tensor([ms_], dtype=torch.float64, device=dev)
-                dist.all_reduce(t_, op=dist.ReduceOp.MAX)
-                ms_ = float(t_.item())
-            blocks.append(ms_)
-            total += ms_
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for i in range(K):
+            eng.fill(x, src_thr=src_thr, out=outs[i % no])
+        eng.flush()                                   # every step's outputs are complete at e1
+        e1.record()
+        barrier()
+        ms_ = e0.elapsed_time(e1)
+        if dist is not None:
+            t_ = torch.tensor([ms_], dtype=torch.float64, device=dev)
+            dist.all_reduce(t_, op=dist.ReduceOp.MAX)
+            ms_ = float(t_.item())
         clocks_ = sampler_.stop()
         bad_, _ = eng.status()
         assert bad_ == -1, f"unexpected bad frame {bad_}"
-        return blocks, launches_, clocks_
+        return ms_, launches_, clocks_
 
-    blocks_strict, launches_per_step, clocks_strict = timed_blocks(1, min(args.min_seconds, 0.3))
+    ms_strict, launches_per_step, clocks_strict = timed_steps(1)
     if args.pipeline > 1:
-        blocks, launches_per_step, clocks = timed_blocks(args.pipeline, args.min_seconds)
+        ms, launches_per_step, clocks = timed_steps(args.pipeline)
     else:
-        blocks, clocks = blocks_strict, clocks_strict
-    ms = statistics.median(blocks)
-    ms_strict = statistics.median(blocks_strict)
+        ms, clocks = ms_strict, clocks_strict
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs[(K - 1) % no], B, H, W)     # the last timed step wrote this output set
     ms_per_step = ms / K
     value = world * B * K / (ms * 1e-3)
-    strict = {"value": world * B * K / (ms_strict * 1e-3), "ms_per_step": ms_strict / K, "blocks": len(blocks_strict),
-              "what": "same K-step blocks with strict stream order between steps (pipeline depth 1, the API default)"}
+    strict = {"value": world * B * K / (ms_strict * 1e-3), "ms_per_step": ms_strict / K,
+              "what": "same K steps with strict stream order between steps (pipeline depth 1, the API default)"}
 
     # ---- parity at the benchmarked configuration: 64 frames of the timed run's own outputs against the oracle ----
-    # (the last block wrote output set (K-1) % no last; every step has the same input)
+    # (the last timed step wrote output set (K-1) % no; every step has the same input)
     sel = np.unique(np.linspace(0, B - 1, min(B, args.parity_frames)).astype(int))
     want = O.dt_fill(frames_np[sel], src_thr=src_thr)
     last = outs[(K - 1) % no]
@@ -675,7 +692,7 @@ def run_ours(args, rank, world, local_rank):
         "algorithmic_bytes": ALG_BYTES_PER_PX * px_step, "peak_source": peak_src,
         "strict_frac": ALG_BYTES_PER_PX * px_step / (ms_strict / K * 1e-3) / 1e9 / peak,
         "what": "whole fused path of one step (k1_mask_rows + k1b_scan_compact + k2_chamfer + k3_sky [+ k2_chamfer_wide "
-                f"no-op]): {ALG_BYTES_PER_PX} B/px x {px_step} px per step / step time (median K-step block); dominant "
+                f"no-op]): {ALG_BYTES_PER_PX} B/px x {px_step} px per step / step time (K timed steps); dominant "
                 "kernel k2_chamfer; kernel_ms = CUDA events between the launches of separate, strictly ordered steps",
         "kernel_ms": kt, "kernel_share": {k: (v / ktot if ktot else None) for k, v in kt.items()},
         "dominant_kernel": {"name": "k2_chamfer", "ms": kt.get("k2_chamfer"),
@@ -719,17 +736,15 @@ def run_ours(args, rank, world, local_rank):
                    "frames_per_step_per_gpu": B,
                    "pipeline": (f"{args.pipeline} batches in flight (dtfill_set_pipeline_depth): K1/K1b of step n+1 "
                                 f"overlap K2 of step n; {no} output sets rotate; all outputs complete at the end "
-                                "of every timed block") if args.pipeline > 1 else "strict stream order between steps",
-                   "timing": f"blocks of {K} steps between CUDA events (max over ranks), repeated until the timed region "
-                             "has lasted min_seconds; value = median block"},
-        "timed_region_s": sum(blocks) * 1e-3, "blocks": len(blocks),
-        "block_ms": {"median": ms, "min": min(blocks), "max": max(blocks)},
+                                "of the timed steps") if args.pipeline > 1 else "strict stream order between steps",
+                   "timing": f"{K} steps between two CUDA events (max over ranks)"},
+        "timed_region_s": ms * 1e-3,
         "strict": strict, "parity_checked": int(len(sel)),
         "parity_what": f"{len(sel)} frames of the timed run's own outputs (depth, dt, mask; lbl in a second pass in the "
                        "same mode) bit-identical to oracle/dtfill_oracle.c, on every rank",
         "roofline": roofline, "cpu_baseline": cpu,
         "e2e": e2e, "e2e_pinned": e2e_pinned, "sweep": sweep,
-        "gpu_launches": launches_per_step * K * len(blocks), "gpu_launches_per_step": launches_per_step,
+        "gpu_launches": launches_per_step * K, "gpu_launches_per_step": launches_per_step,
         "clocks": clocks, "clocks_strict": clocks_strict,
     }
     emit(line)
@@ -760,7 +775,7 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps (one batch per GPU each)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="frames per GPU and step (default: the workload's)")
@@ -770,12 +785,14 @@ def main():
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--pipeline", type=int, default=4, choices=[1, 2, 3, 4],
                     help="batches in flight in the device-resident timing (1 = strict stream order)")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="least duration of the timed region")
+    ap.add_argument("--min-seconds", type=float, default=1.0, help="least duration of the timed sweep region")
     ap.add_argument("--parity-frames", type=int, default=64)
     ap.add_argument("--sweep-frames", type=int, default=8192)
     ap.add_argument("--sweep-batch", type=int, default=256)
     ap.add_argument("--band-cap", type=int, default=None, help="override the band planner target (row steps)")
     ap.add_argument("--subbatches", type=int, default=None, help="override the number of sub-batch streams")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (a seeded sample of frames, rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))

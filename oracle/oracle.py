@@ -12,8 +12,8 @@ Three layers, each a restatement of reference lines (file:line relative to /root
   used as the "reference CPU path" timing arm when ``cv2`` is importable on the box.
 * ``result_kitti`` / ``result_nyu`` -- numpy restatement of evaluation.py:82-123 and evaluation.py:196-239.
 
-Parity pin: no tests/golden vectors exist in the reference; the pin is the live reference run in the build
-container (tests/test_oracle_vs_reference.py) and the fixtures it produced (tests/golden/).
+Parity pin: the reference ships no test vectors; the pin is the reference's own output on seeded inputs, stored under
+tests/golden/ by tests/golden/make_golden.py (tests/test_oracle_golden.py, tests/test_oracle_vs_reference.py).
 """
 from __future__ import annotations
 

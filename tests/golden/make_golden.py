@@ -1,13 +1,14 @@
-"""Generates tests/golden/*.npz by running the REFERENCE itself in the build container.
+"""Generates tests/golden/*.npz by running the REFERENCE itself (a checkout named by $DTFILL_REFERENCE).
 
-The reference (/root/reference, read-only) ships no tests or golden vectors, so the pin is its own output on
+The reference ships no tests or golden vectors, so the pin is its own output on
 seeded synthetic inputs:  solution_DeepNet/tools.py (imported with a stub `tensorflow` module and the `cv2` it
 forgot to import injected), the two functions of solution_DeepNet/eval_NYU.py:114-133 (AST-extracted, that
 script builds a TF model at import), evaluation.py's Result / Result_NYU, live cv2 4.13.0, and the DT-pooling lines of net.py:71-123 / demo.py:65-149
 (AST-extracted, run on tests/golden/tf_numpy_shim.py: TensorFlow itself is absent).
-/root/reference does not exist on the GPU box, which is why the vectors are committed.
+The vectors are committed so that the tests need no reference checkout.
 
-    python tests/golden/make_golden.py [pool]   (from the repo root; needs /root/reference and cv2)
+    python tests/golden/make_golden.py [pool]   (from the repo root; needs a reference checkout and cv2)
+    python tests/golden/make_golden.py cv2      (cv2_masks.npz alone; needs cv2 only)
 """
 import ast
 import hashlib
@@ -118,6 +119,34 @@ def write_pool_golden():
     np.savez_compressed(os.path.join(OUT, "dt_pool.npz"), **pool)
 
 
+def random_masks():
+    """Inputs of cv2_masks.npz: 300 uint8 masks of 1..40 x 1..60 pixels (0 = source), densities 1 % .. 90 %."""
+    rng = np.random.default_rng(0)
+    masks = []
+    for _ in range(300):
+        H, W = int(rng.integers(1, 41)), int(rng.integers(1, 61))
+        dens = rng.choice([0.01, 0.05, 0.2, 0.5, 0.9])
+        masks.append((rng.random((H, W)) >= dens).astype(np.uint8))
+    return masks
+
+
+def write_cv2_golden():
+    """cv2.distanceTransformWithLabels(DIST_L1, 5, DIST_LABEL_PIXEL) -- the call at tools.py:9 -- on random_masks(),
+    concatenated as flat arrays with the shape of every mask; needs only cv2."""
+    import cv2
+    masks = random_masks()
+    dts, lbls = [], []
+    for m in masks:
+        dt, lbl = cv2.distanceTransformWithLabels(m, cv2.DIST_L1, 5, labelType=cv2.DIST_LABEL_PIXEL)
+        assert dt.dtype == np.float32 and np.array_equal(dt, np.rint(dt)) and lbl.max() < 2 ** 15
+        dts.append(dt.ravel())
+        lbls.append(lbl.ravel())
+    np.savez_compressed(os.path.join(OUT, "cv2_masks.npz"), cv2_version=np.array(cv2.__version__),
+                        shapes=np.array([m.shape for m in masks], np.int32),
+                        mask=np.concatenate([m.ravel() for m in masks]),
+                        dt_u16=np.concatenate(dts).astype(np.uint16), lbl_i16=np.concatenate(lbls).astype(np.int16))
+
+
 def main():
     from distancetransform_depthcompletion_b200 import synth
     tools, evaluation, nyu_nearest_point, nyu_distance_transform, cv2 = load_reference()
@@ -200,6 +229,7 @@ def main():
         met[f"nyu_s{seed}"] = np.array([R.mse, R.rmse, R.mae, R.irmse, R.imae, R.delta1, R.delta2, R.delta3])
     np.savez_compressed(os.path.join(OUT, "metrics.npz"), **met)
     write_pool_golden()
+    write_cv2_golden()
     for f in sorted(os.listdir(OUT)):
         if f.endswith(".npz"):
             print(f, os.path.getsize(os.path.join(OUT, f)))
@@ -208,5 +238,7 @@ def main():
 if __name__ == "__main__":
     if sys.argv[1:] == ["pool"]:          # only dt_pool.npz (the other fixtures stay byte-identical in git)
         write_pool_golden()
+    elif sys.argv[1:] == ["cv2"]:         # only cv2_masks.npz (needs cv2, not the reference checkout)
+        write_cv2_golden()
     else:
         main()

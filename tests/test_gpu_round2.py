@@ -256,7 +256,7 @@ def test_allreduce_sums_two_ranks_equal_one_rank(handle, torch_mod):
     (eval.py:212-232, 252-259)."""
     torch = torch_mod
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     import torch.multiprocessing as mp
     from distancetransform_depthcompletion_b200.engine import DTFillEngine
     with socket.socket() as s:

@@ -1,14 +1,9 @@
 """KITTI outlier filter (SURVEY.md section 8 f-2, data_read.py:103-128)."""
-import ast
-import os
-
 import numpy as np
 import pytest
 
 from distancetransform_depthcompletion_b200 import data_read, synth
 from oracle import oracle as O
-
-REF = os.environ.get("DTFILL_REFERENCE", "/root/reference")
 
 
 def _frames():
@@ -23,31 +18,6 @@ def _frames():
     signed[::7, ::5] = np.float32(-5.0)                                                   # negative neighbours
     return [x, synth.kitti_frame(3, beam_step=4), x[:9, :13].copy(), x[200:203, :].copy(), x[:, 600:602].copy(),
             dense, signed, x[:, 1:1216].copy()]
-
-
-@pytest.mark.skipif(not (os.path.isdir(REF) and O.have_cv2()), reason="reference checkout or cv2 absent")
-def test_port_matches_the_reference_function():
-    """The port in oracle.py against the reference's own def, AST-extracted from data_read.py (that module imports
-    matplotlib/h5py/skimage at the top and cannot be imported here)."""
-    import cv2
-
-    class NP:                       # numpy with the np.float alias the 2019 code uses
-        float = np.float64
-
-        def __getattr__(self, k):
-            return getattr(np, k)
-
-    ns = {"np": NP(), "cv2": cv2}
-    tree = ast.parse(open(os.path.join(REF, "data_read.py")).read())
-    for node in tree.body:
-        if isinstance(node, ast.FunctionDef) and node.name == "outlier_removal":
-            exec(compile(ast.Module([node], []), "data_read.py", "exec"), ns)
-    for f in _frames():
-        if min(f.shape) < 2:
-            continue
-        want = ns["outlier_removal"](f[None, :, :, None])
-        got = O.cv2_port_outlier_removal(f[None, :, :, None])
-        assert want.dtype == np.float32 and np.array_equal(want, got)
 
 
 @pytest.mark.gpu
