@@ -15,10 +15,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # DTFILL_LIB: another build of the same library (kernel experiments); the product is the in-tree libdtfill.so
 LIB_PATH = os.environ.get("DTFILL_LIB") or os.path.join(_HERE, "libdtfill.so")
 
-E_ARG, E_CUDA, E_INDEX, E_NOMEM = -1, -2, -3, -4
+E_ARG, E_CUDA, E_INDEX, E_NOMEM, E_DATA = -1, -2, -3, -4, -5
 METRICS_KITTI, METRICS_NYU = 0, 1
 METRIC_COLS = 9
-ABI_VERSION = 5          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
+ABI_VERSION = 6          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
 METRIC_NAMES = ("mse", "rmse", "mae", "irmse", "imae", "delta1", "delta2", "delta3", "count")
 
 _c_float_p = ctypes.POINTER(ctypes.c_float)
@@ -87,6 +87,9 @@ def load() -> ctypes.CDLL:
         L.dtfill_outlier_removal.argtypes = [vp, vp, ci, ci, ci, ci, vp, ci]
         L.dtfill_dt_pool_demo.argtypes = [vp, vp, ci, ci, ci, ci, ci, ci, vp, ci]
         L.dtfill_edt.argtypes = [vp, vp, ci, ci, ci, ci, cf, vp, vp, ci]
+        L.dtfill_png_decode.argtypes = [vp, vp, vp, ci, ci, ci, ci, vp, vp, ci, ctypes.POINTER(ci)]
+        L.dtfill_run_png.argtypes = [vp, vp, vp, ci, ci, ci, ci, ci, cf, cf, vp, vp, vp, vp, vp, vp, ci, ctypes.POINTER(ci)]
+        L.dtfill_debug_png_decode_host.argtypes = [vp, ctypes.c_long, ci, ci, vp]
         L.dtfill_host_alloc.argtypes = [ctypes.POINTER(vp), ctypes.c_size_t]
         L.dtfill_host_free.argtypes = [vp]
         L.dtfill_host_free.restype = None
@@ -96,7 +99,8 @@ def load() -> ctypes.CDLL:
                      "dtfill_kernel_times", "dtfill_metrics_ex", "dtfill_nccl_unique_id", "dtfill_comm_create",
                      "dtfill_comm_destroy", "dtfill_allreduce_sums", "dtfill_set_stage_threads", "dtfill_debug_set_skip",
                      "dtfill_run_eval_async", "dtfill_eval_totals", "dtfill_edt", "dtfill_set_sparse_upload",
-                     "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo"):
+                     "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo", "dtfill_png_decode",
+                     "dtfill_run_png", "dtfill_debug_png_decode_host"):
             getattr(L, name).restype = ci
         _lib = L
         return L
@@ -112,7 +116,7 @@ def _check(rc: int, what: str):
     msg = last_error()
     if rc == E_INDEX:
         raise IndexError(msg)
-    if rc == E_ARG:
+    if rc in (E_ARG, E_DATA):
         raise ValueError(f"{what}: {msg}")
     if rc == E_NOMEM:
         raise MemoryError(f"{what}: {msg}")
@@ -221,6 +225,49 @@ class Handle:
             return res
         _check(rc, "dtfill_run_u16")
         return res
+
+    def png_decode(self, data: np.ndarray, offsets: np.ndarray, H: int, W: int, out=None):
+        """16-bit grayscale PNG files packed back to back in data (uint8), file b = data[offsets[b]:offsets[b+1]] ->
+        (samples uint16 [B,H,W], status int32 [B]).  Raises ValueError naming the first failed frame and the reason
+        (the other frames are still decoded; a failed frame's samples are zero)."""
+        data, offsets = _png_args(data, offsets)
+        B = offsets.size - 1
+        out = np.empty((B, H, W), np.uint16) if out is None else out
+        assert out.dtype == np.uint16 and out.shape == (B, H, W) and out.flags.c_contiguous
+        status = np.empty(B, np.int32)
+        bad = ctypes.c_int(-1)
+        _check(self._L.dtfill_png_decode(self._h, _ptr(data), _ptr(offsets), 0, B, int(H), int(W), _ptr(out),
+                                         _ptr(status), 0, ctypes.byref(bad)), "dtfill_png_decode")
+        return out, status
+
+    def run_host_png(self, data: np.ndarray, offsets: np.ndarray, H_in: int, W: int, crop_top: int, src_thr: float,
+                     val_thr: float, want_lidar=False, want_counts=True, out=None):
+        """PNG files (as png_decode) decoded on the device and filled like run_host_u16, the samples never leaving the
+        device.  Outputs as run_host_u16; a decode failure raises ValueError, an IndexError is reported in the dict."""
+        data, offsets = _png_args(data, offsets)
+        B = offsets.size - 1
+        H = H_in - int(crop_top)
+        out = out or {}
+        lidar = (out.get("lidar") if out.get("lidar") is not None else np.empty((B, H, W), np.float32)) if want_lidar else None
+        depth = out.get("depth") if out.get("depth") is not None else np.empty((B, H, W), np.float32)
+        counts = np.empty((B, 2), np.int32) if want_counts else None
+        bad = ctypes.c_int(-1)
+        rc = self._L.dtfill_run_png(self._h, _ptr(data), _ptr(offsets), 0, B, int(H_in), int(W), int(crop_top),
+                                    float(src_thr), float(val_thr), _ptr(lidar), _ptr(depth), None, None, None,
+                                    _ptr(counts), 0, ctypes.byref(bad))
+        res = dict(lidar=lidar, depth=depth, counts=counts, first_bad=bad.value)
+        if rc == E_INDEX:
+            res["index_error"] = last_error()
+            return res
+        _check(rc, "dtfill_run_png")
+        return res
+
+    def png_decode_device_async(self, data_ptr: int, offsets_ptr: int, B: int, H: int, W: int, out_ptr: int,
+                                status_ptr: int):
+        """Device files and offsets -> device samples and status, enqueued on the handle's stream only."""
+        bad = ctypes.c_int(-1)
+        _check(self._L.dtfill_png_decode(self._h, _ptr(data_ptr), _ptr(offsets_ptr), 1, int(B), int(H), int(W),
+                                         _ptr(out_ptr), _ptr(status_ptr), 1, ctypes.byref(bad)), "dtfill_png_decode")
 
     # ---- device path (raw pointers, e.g. torch tensors' data_ptr()) ------------------------------------
     def run_device_u16_async(self, in_ptr: int, B: int, H_in: int, W: int, crop_top: int, src_thr: float,
@@ -394,6 +441,31 @@ class Handle:
 
 
 NCCL_ID_BYTES = 128
+
+PNG_STATUS = ("ok", "bad signature", "unsupported IHDR", "size differs from the batch's",
+              "broken or truncated chunk structure, or no IDAT", "bad zlib header", "invalid DEFLATE data",
+              "decompressed size differs from H*(1+2W)", "filter type > 4", "Adler-32 mismatch")
+
+
+def _png_args(data, offsets):
+    data = np.ascontiguousarray(data, dtype=np.uint8).reshape(-1)
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64).reshape(-1)
+    if offsets.size < 2:
+        raise ValueError("PNG decode: offsets must hold B + 1 >= 2 entries")
+    if offsets[0] < 0 or offsets[-1] > data.size or np.any(np.diff(offsets) < 0):
+        raise ValueError("PNG decode: offsets must be non-decreasing and lie within the data")
+    return data, offsets
+
+
+def png_decode_host(png: bytes, H: int, W: int):
+    """Test hook: the decode of one file run serially on the CPU (no GPU) -> (status, samples uint16 [H,W])."""
+    png = bytes(png)
+    buf = np.frombuffer(png or b"\0", np.uint8)
+    out = np.empty((H, W), np.uint16)
+    st = load().dtfill_debug_png_decode_host(_ptr(buf), len(png), int(H), int(W), _ptr(out))
+    if st < 0:
+        raise ValueError("dtfill_debug_png_decode_host: bad arguments")
+    return st, out
 
 
 def nccl_unique_id() -> bytes:

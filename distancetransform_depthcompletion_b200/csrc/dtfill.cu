@@ -372,6 +372,9 @@ struct dtfill_ctx {
     PinBuf pin_in, pin_depth, pin_dt, pin_lbl, pin_mask, pin_lidar, pin_sparse;
     Buf sparse_dev;                   // (index, value) pairs of a sparse upload, per slice
     Buf mx_terms, mx_counts, mx_leaf_start, mx_leaf_sum;     // dtfill_metrics in numpy's summation order (k4x_*)
+    // PNG decode (k8_png_*): uploaded files + offsets, filtered bytes per frame, decoded samples (dtfill_run_png), status
+    Buf png_data, png_scratch, png_samples, png_status;
+    PinBuf pin_png, pin_png_status;   // pinned staging of host file bytes / of the per-frame status
     bool metrics_exact = true;        // dtfill_metrics / _ex reproduce np.mean's pairwise sums bit for bit
     bool sparse_upload = true;        // pageable float32 inputs are compacted on the host instead of mirrored (see CopyPool)
     size_t last_h2d_bytes = 0, last_d2h_bytes = 0;   // bytes the last synchronous host call moved over the link
@@ -801,7 +804,7 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
     h->cur_status_early = nsub == 1 && !(h->debug_skip & 2);     // slices share the words: their copy follows the last slice
     void* dense_pin = hio ? hio->in_pin : nullptr;      // pinned mirror of a pageable input (allocated late on the sparse path)
     auto copy_in = [&](cudaStream_t st, int b0, int nb) -> int {
-        if (!hio) return 0;
+        if (!hio || !hio->in) return 0;
         const size_t frame_bytes = h->in_u16 ? (size_t)h->in_H * W * 2 : (size_t)H * W * 4;
         const char* src = (const char*)hio->in + b0 * frame_bytes;
         if (hio->sparse_pin) {     // pageable float32 input: compact the slice on the host, rebuild it on the device
@@ -1055,14 +1058,16 @@ void dtfill_destroy(dtfill_t* h) {
     }
     Buf* bufs[] = {&h->in_dev, &h->depth_dev, &h->dt_dev, &h->lbl_dev, &h->mask_dev, &h->counts_out_dev, &h->lidar_out_dev,
                    &h->gt_dev, &h->partial, &h->per_frame, &h->sums, &h->edt_rows, &h->edt_stack, &h->sparse_dev,
-                   &h->mx_terms, &h->mx_counts, &h->mx_leaf_start, &h->mx_leaf_sum};
+                   &h->mx_terms, &h->mx_counts, &h->mx_leaf_start, &h->mx_leaf_sum, &h->png_data, &h->png_scratch,
+                   &h->png_samples, &h->png_status};
     for (Buf* b : bufs)
         if (b->p) cudaFree(b->p);
     for (void* q : h->retired) cudaFree(q);
     if (h->counts_host) cudaFreeHost(h->counts_host);
     delete h->pool_in;
     delete h->pool_out;
-    for (PinBuf* b : {&h->pin_in, &h->pin_depth, &h->pin_dt, &h->pin_lbl, &h->pin_mask, &h->pin_lidar, &h->pin_sparse})
+    for (PinBuf* b : {&h->pin_in, &h->pin_depth, &h->pin_dt, &h->pin_lbl, &h->pin_mask, &h->pin_lidar, &h->pin_sparse, &h->pin_png,
+                      &h->pin_png_status})
         if (b->p) cudaFreeHost(b->p);
     if (h->status_ring) cudaFreeHost(h->status_ring);
     if (h->status_dev) cudaFree(h->status_dev);
@@ -1160,13 +1165,15 @@ struct InputScope {
 // dtfill_run / dtfill_run_u16: buffers on either side, synchronous.  u16: `in` holds uint16 samples [B,in_H,W].
 int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, int in_crop, int B, int H, int W,
              float src_thr, float val_thr, float* out_lidar, float* out_depth, float* out_dt, int32_t* out_lbl,
-             uint8_t* out_mask, int32_t* out_counts, int out_is_device, int* first_bad_frame) {
+             uint8_t* out_mask, int32_t* out_counts, int out_is_device, int* first_bad_frame, bool in_resident = false) {
     CU(cudaSetDevice(h->device));
     const size_t npx = (size_t)B * H * W;
     const size_t in_bytes = u16 ? (size_t)B * in_H * W * 2 : npx * 4;
     int rc;
     const void* in_d = in;
-    const bool pipelined = !in_is_device && !out_is_device;     // both sides on the host: copies are sliced
+    // outputs on the host: copies are sliced.  in_resident: the input is a device buffer the library itself just produced
+    // (dtfill_run_png), so only the outputs go through the slices
+    const bool pipelined = !out_is_device && (!in_is_device || in_resident);
     if (!in_is_device) {
         if ((rc = ensure(h, h->in_dev, in_bytes))) return rc;
         if (!pipelined) CU(cudaMemcpyAsync(h->in_dev.p, in, in_bytes, cudaMemcpyHostToDevice, h->stream));
@@ -1187,10 +1194,10 @@ int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, 
     h->last_h2d_bytes = h->last_d2h_bytes = 0;
     if (pipelined) {
         HostIO hio;
-        hio.in = in; hio.lidar = out_lidar; hio.depth = out_depth; hio.dt = out_dt; hio.lbl = out_lbl; hio.mask = out_mask;
+        hio.in = in_resident ? nullptr : in; hio.lidar = out_lidar; hio.depth = out_depth; hio.dt = out_dt; hio.lbl = out_lbl; hio.mask = out_mask;
         // pageable buffers go through pinned mirrors (DTFILL_STAGE_THREADS=0 / dtfill_set_stage_threads(h, 0): never)
         if (h->stage_threads != 0) {
-            const bool pin_i = is_pageable(in);
+            const bool pin_i = !in_resident && is_pageable(in);
             const bool pin_d = is_pageable(out_depth), pin_t = out_dt && is_pageable(out_dt);
             const bool pin_l = out_lbl && is_pageable(out_lbl), pin_m = out_mask && is_pageable(out_mask);
             const bool pin_x = out_lidar && is_pageable(out_lidar);
@@ -1290,6 +1297,200 @@ int dtfill_run_u16_async(dtfill_t* h, const uint16_t* in_dev, int B, int H_in, i
     InputScope scope(h, true, H_in, crop_top, out_lidar_dev);
     return enqueue(h, in_dev, B, H_in - crop_top, W, src_thr, val_thr, out_depth_dev, out_dt_dev, out_lbl_dev, out_mask_dev,
                    out_counts_dev);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// 16-bit grayscale PNG files -> uint16 samples (k8_png_inflate, k8_png_unfilter; see dtfill_k8_png.cuh)
+// ------------------------------------------------------------------------------------------------------------
+namespace {
+
+const char* png_reason(int st) {
+    switch (st) {
+        case png::ST_SIGNATURE: return "bad PNG signature";
+        case png::ST_IHDR: return "unsupported IHDR (only non-interlaced 16-bit grayscale PNGs are supported)";
+        case png::ST_SIZE: return "image size differs from the batch's";
+        case png::ST_CHUNKS: return "broken or truncated chunk structure, or no IDAT";
+        case png::ST_ZLIB: return "bad zlib header";
+        case png::ST_DEFLATE: return "invalid DEFLATE data";
+        case png::ST_LENGTH: return "decompressed size differs from H*(1+2W)";
+        case png::ST_FILTER: return "row filter type > 4";
+        case png::ST_ADLER: return "Adler-32 mismatch";
+        default: return "unknown status";
+    }
+}
+
+int png_args(const char* who, dtfill_t* h, const void* data, const int64_t* offsets, const void* out, int B, int H, int W) {
+    if (!h || !data || !offsets || !out) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, data, offsets or output");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H, W must be positive");
+    // the Adler-32 sums of k8_png_inflate are exact in 64 bits below this size
+    if ((int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28))
+        return fail(DTFILL_E_ARG, std::string(who) + ": frame too large (H * (1 + 2 W) < 2^28 bytes)");
+    return 0;
+}
+
+// First failed frame of a host copy of the per-frame status: DTFILL_E_DATA with the frame and the reason, or 0.
+int png_verdict(const int32_t* st, int B, int* first_bad_frame) {
+    for (int b = 0; b < B; ++b)
+        if (st[b] != png::ST_OK) {
+            if (first_bad_frame) *first_bad_frame = b;
+            return fail(DTFILL_E_DATA, "frame " + std::to_string(b) + ": " + png_reason(st[b]) + " (status " +
+                                           std::to_string(st[b]) + ")");
+        }
+    return 0;
+}
+
+// Enqueue the decode of B files on the handle's stream: samples into out_dev [B,H,W], status into status_dev [B].  Host
+// files go up in one copy through a pinned staging buffer (bytes, then the offsets rebased to 0); the caller waits for
+// the call before the buffer is used again.
+int png_enqueue(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H, int W,
+                uint16_t* out_dev, int32_t* status_dev) {
+    int rc;
+    const uint8_t* d_data = data;
+    const int64_t* d_off = offsets;
+    if (!in_is_device) {
+        const int64_t o0 = offsets[0];
+        if (o0 < 0) return fail(DTFILL_E_ARG, "dtfill_png_decode: offsets[0] < 0");
+        for (int b = 0; b < B; ++b)
+            if (offsets[b + 1] < offsets[b]) return fail(DTFILL_E_ARG, "dtfill_png_decode: offsets decrease at file " + std::to_string(b));
+        const size_t nbytes = (size_t)(offsets[B] - o0);
+        const size_t off_at = (nbytes + 15) & ~(size_t)15;
+        const size_t total = off_at + (size_t)(B + 1) * 8;
+        if ((rc = ensure_pinned(h->pin_png, total))) return rc;
+        if ((rc = ensure(h, h->png_data, total))) return rc;
+        uint8_t* pin = (uint8_t*)h->pin_png.p;
+        memcpy(pin, data + o0, nbytes);
+        int64_t* po = (int64_t*)(pin + off_at);
+        for (int b = 0; b <= B; ++b) po[b] = offsets[b] - o0;
+        CU(cudaMemcpyAsync(h->png_data.p, pin, total, cudaMemcpyHostToDevice, h->stream));
+        h->last_h2d_bytes = total;
+        d_data = (const uint8_t*)h->png_data.p;
+        d_off = (const int64_t*)((uint8_t*)h->png_data.p + off_at);
+    }
+    const size_t fbytes = (size_t)H * (1 + 2 * (size_t)W);
+    if ((rc = ensure(h, h->png_scratch, (size_t)B * fbytes))) return rc;
+    const int grid = (B + png::K8_WARPS - 1) / png::K8_WARPS;
+    uint8_t* scr = (uint8_t*)h->png_scratch.p;
+    png::k8_png_inflate<<<grid, 32 * png::K8_WARPS, 0, h->stream>>>(d_data, d_off, B, H, W, scr, status_dev);
+    png::k8_png_unfilter<<<grid, 32 * png::K8_WARPS, 0, h->stream>>>(scr, B, H, W, out_dev, status_dev);
+    CU(cudaGetLastError());
+    return 0;
+}
+
+int png_status_host(dtfill_t* h, int B, int32_t** out) {
+    int rc = ensure_pinned(h->pin_png_status, (size_t)B * 4);
+    if (rc) return rc;
+    *out = (int32_t*)h->pin_png_status.p;
+    return 0;
+}
+
+}  // namespace
+
+int dtfill_png_decode(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H, int W,
+                      uint16_t* out, int32_t* out_status, int out_is_device, int* first_bad_frame) {
+    if (first_bad_frame) *first_bad_frame = -1;
+    int rc = png_args("dtfill_png_decode", h, data, offsets, out, B, H, W);
+    if (rc) return rc;
+    if (out_is_device && !out_status) return fail(DTFILL_E_ARG, "dtfill_png_decode: out_status is required with device outputs");
+    CU(cudaSetDevice(h->device));
+    uint16_t* od = out;
+    int32_t* os = out_status;
+    if (!out_is_device) {
+        if ((rc = ensure(h, h->png_samples, (size_t)B * H * W * 2))) return rc;
+        if ((rc = ensure(h, h->png_status, (size_t)B * 4))) return rc;
+        od = (uint16_t*)h->png_samples.p;
+        os = (int32_t*)h->png_status.p;
+    }
+    if ((rc = png_enqueue(h, data, offsets, in_is_device, B, H, W, od, os))) return rc;
+    if (in_is_device && out_is_device) return 0;
+    int32_t* st_host = nullptr;
+    if ((rc = png_status_host(h, B, &st_host))) return rc;
+    if (!out_is_device) CU(cudaMemcpyAsync(out, od, (size_t)B * H * W * 2, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(st_host, os, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    if (!out_is_device && out_status) memcpy(out_status, st_host, (size_t)B * 4);
+    return png_verdict(st_host, B, first_bad_frame);
+}
+
+int dtfill_run_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H_in, int W,
+                   int crop_top, float src_thr, float val_thr, float* out_lidar, float* out_depth, float* out_dt,
+                   int32_t* out_lbl, uint8_t* out_mask, int32_t* out_counts, int out_is_device, int* first_bad_frame) {
+    if (first_bad_frame) *first_bad_frame = -1;
+    int rc = png_args("dtfill_run_png", h, data, offsets, out_depth, B, H_in, W);
+    if (rc) return rc;
+    if ((rc = check_u16_args("dtfill_run_png", h, data, out_depth, B, H_in, W, crop_top))) return rc;
+    CU(cudaSetDevice(h->device));
+    if ((rc = ensure(h, h->png_samples, (size_t)B * H_in * W * 2))) return rc;
+    if ((rc = ensure(h, h->png_status, (size_t)B * 4))) return rc;
+    int32_t* st_host = nullptr;
+    if ((rc = png_status_host(h, B, &st_host))) return rc;
+    uint16_t* samples = (uint16_t*)h->png_samples.p;
+    if ((rc = png_enqueue(h, data, offsets, in_is_device, B, H_in, W, samples, (int32_t*)h->png_status.p))) return rc;
+    CU(cudaMemcpyAsync(st_host, h->png_status.p, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream));
+    const size_t h2d = in_is_device ? 0 : h->last_h2d_bytes;
+    // the fill of dtfill_run_u16 on the decoded samples; it ends with a synchronisation, so st_host is final afterwards
+    rc = run_sync(h, samples, 1, true, H_in, crop_top, B, H_in - crop_top, W, src_thr, val_thr, out_lidar, out_depth, out_dt,
+                  out_lbl, out_mask, out_counts, out_is_device, first_bad_frame, true);
+    h->last_h2d_bytes += h2d;
+    if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
+    const int rd = png_verdict(st_host, B, first_bad_frame);     // a decode failure wins over IndexError
+    return rd ? rd : rc;
+}
+
+int dtfill_debug_png_decode_host(const uint8_t* f, long nbytes, int H, int W, uint16_t* out) {
+    using namespace png;
+    if (!f || !out || nbytes < 0 || H <= 0 || W <= 0 || (int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28)) return -1;
+    const uint32_t total = (uint32_t)H * (uint32_t)(1 + 2 * W);
+    std::vector<uint8_t> scr(total);
+    std::vector<uint16_t> llut(1 << LBITS), dlut(1 << DBITS);
+    uint16_t lsym[288], dsym[32], lcount[16], dcount[16];
+    uint32_t qlen[QCAP], qarg[QCAP];
+    uint8_t lit[LITCAP], lens[19 + 320];
+    Huff lh{llut.data(), lcount, lsym, LBITS}, dh{dlut.data(), dcount, dsym, DBITS};
+    Queue q{qlen, qarg, lit, 0, 0};
+    Inflate s{};
+    int64_t first = 0;
+    int st = check_structure(f, nbytes, H, W, &first);
+    if (st == ST_OK) {
+        idat_open(s.b.in, f, first);
+        s.total = total;
+        st = zlib_header(s);
+    }
+    uint32_t p = 0;
+    while (st == ST_OK) {
+        st = inflate_tokens(s, lh, dh, lens, q);
+        for (int i = 0; i < q.n; ++i) {
+            const uint32_t len = qlen[i], arg = qarg[i];
+            if (arg & LIT_RUN) memcpy(&scr[p], lit + (arg & 0xffff), len);
+            else for (uint32_t j = 0; j < len; ++j) scr[p + j] = scr[p - arg + j];
+            p += len;
+        }
+        if (s.state == 3) break;
+    }
+    if (st == ST_OK) st = finish(s);
+    if (st == ST_OK) {
+        uint32_t a = 1, bsum = 0;
+        for (uint32_t i = 0; i < total; ++i) { a = (a + scr[i]) % ADLER_MOD; bsum = (bsum + a) % ADLER_MOD; }
+        if (((bsum << 16) | a) != s.adler) st = ST_ADLER;
+    }
+    const size_t stride = 1 + 2 * (size_t)W;
+    if (st == ST_OK)
+        for (int r = 0; r < H; ++r)
+            if (scr[r * stride] > 4) { st = ST_FILTER; break; }
+    if (st != ST_OK) {
+        memset(out, 0, (size_t)H * W * 2);
+        return st;
+    }
+    for (int r = 0; r < H; ++r) {
+        const uint8_t* row = &scr[r * stride];
+        const int ft = row[0];
+        uint16_t* o = out + (size_t)r * W;
+        const uint16_t* up = r ? o - W : nullptr;
+        for (int c = 0; c < W; ++c) {
+            const uint32_t a = c ? o[c - 1] : 0, b = up ? up[c] : 0, cc = (up && c) ? up[c - 1] : 0;
+            o[c] = (uint16_t)unfilter_sample(ft, row[1 + 2 * c], row[2 + 2 * c], a, b, cc);
+        }
+    }
+    return ST_OK;
 }
 
 namespace {

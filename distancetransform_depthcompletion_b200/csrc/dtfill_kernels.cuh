@@ -17,6 +17,8 @@
 //   K5  k5_dt_pool_*      one level of the CNN input stage's DT pooling (net.py:71-123)
 //   K6  k6_outlier_removal  KITTI outlier filter (data_read.py:103-128)
 //   K7  k7_edt_*          exact Euclidean feature transform (extension, SURVEY.md 8 f-4): column pass + parabola row pass
+//   K8  k8_png_*          16-bit grayscale PNG files -> uint16 samples (inflate, then row unfilter), the step before K1
+//                         of the uint16 entry (data_read.py:215 reads the files with PIL)
 // One header per kernel (dtfill_k*.cuh); dtfill_common.cuh holds the key format, the structs and the helpers.
 //
 // Key format of the fast path (SURVEY.md section 7 H1): dist:11 | order:4 | label:17.  "order" is the position
@@ -37,3 +39,4 @@
 #include "dtfill_k5_pool.cuh"
 #include "dtfill_k6_outlier.cuh"
 #include "dtfill_k7_edt.cuh"
+#include "dtfill_k8_png.cuh"

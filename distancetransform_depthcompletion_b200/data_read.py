@@ -1,11 +1,14 @@
-"""Drop-in for the one compute function of the reference's data_read.py that sits next to the hot path:
+"""Drop-ins for the compute of the reference's data_read.py that sits next to the hot path:
 
     outlier_removal(lidar)        data_read.py:103-128   (SURVEY.md section 8 f-2)
+    read_depth_pngs(files)        data_read.py:215 / :223 `np.array(Image.open(f))`, a batch of files at once
 
-numpy in, numpy out; the 7 x 7 diamond filter runs on the GPU (kernel k6_outlier_removal).  The file IO of
-data_read.py (PNG / h5 readers) is out of scope.
+numpy in, numpy out; the 7 x 7 diamond filter runs on the GPU (kernel k6_outlier_removal), the PNG files are decoded on
+the GPU (kernels k8_png_inflate, k8_png_unfilter).  The h5 reader of NYU is out of scope.
 """
 from __future__ import annotations
+
+import struct
 
 import numpy as np
 
@@ -21,3 +24,34 @@ def outlier_removal(lidar, device: int | None = None):
     if sparse_lidar.dtype != np.float32:
         raise TypeError(f"outlier_removal: dtype {sparse_lidar.dtype} not supported by the CUDA path (float32 only)")
     return _lib.get_handle(device).outlier_removal(np.ascontiguousarray(sparse_lidar)[None])[0]
+
+
+def _file_bytes(f) -> bytes:
+    if isinstance(f, (bytes, bytearray, memoryview)):
+        return bytes(f)
+    with open(f, "rb") as fh:
+        return fh.read()
+
+
+def pack_png_files(files):
+    """Files (paths or bytes) -> (data uint8, offsets int64 [B+1], H, W), the size read from the first file's IHDR."""
+    blobs = [_file_bytes(f) for f in files]
+    if not blobs:
+        raise ValueError("read_depth_pngs: no files")
+    head = blobs[0]
+    if len(head) < 24 or head[:8] != b"\x89PNG\r\n\x1a\n" or head[12:16] != b"IHDR":
+        raise ValueError("read_depth_pngs: file 0 is not a PNG file")
+    W, H = struct.unpack(">II", head[16:24])
+    offsets = np.zeros(len(blobs) + 1, np.int64)
+    np.cumsum([len(b) for b in blobs], out=offsets[1:])
+    return np.frombuffer(b"".join(blobs), np.uint8), offsets, int(H), int(W)
+
+
+def read_depth_pngs(files, device: int | None = None) -> np.ndarray:
+    """The reference's `np.array(Image.open(f))` of 16-bit grayscale PNGs (KITTI depth maps and ground truth,
+    data_read.py:215, :223) for a batch of files, decoded on the GPU: uint16 [B,H,W].  files: paths or the files' bytes,
+    all of the size the first file's IHDR gives.  Raises ValueError naming the first file that is not an intact 16-bit
+    grayscale PNG of that size."""
+    data, offsets, H, W = pack_png_files(files)
+    out = _lib.output_empty((offsets.size - 1, H, W), np.uint16)
+    return _lib.get_handle(device).png_decode(data, offsets, H, W, out=out)[0]

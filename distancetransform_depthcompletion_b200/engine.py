@@ -126,6 +126,25 @@ class DTFillEngine:
         self._hold(png, lidar, depth, dt, mask, lbl, counts)
         return dict(lidar=lidar, depth=depth, dt=dt, mask=mask, lbl=lbl, counts=counts)
 
+    def decode_png(self, data_u8, offsets_i64, H: int, W: int):
+        """16-bit grayscale PNG files on the device: data_u8 uint8 CUDA tensor of the files back to back, offsets_i64
+        int64 CUDA tensor [B+1] (file b = data_u8[offsets[b]:offsets[b+1]]) -> (samples uint16 [B,H,W], status int32 [B]:
+        0 ok, else the code of include/dtfill.h dtfill_png_decode, named by _lib.PNG_STATUS; a failed frame's samples are
+        zero), enqueued on torch's current stream.  The samples are what fill_png() takes."""
+        torch = self.torch
+        assert data_u8.is_cuda and data_u8.dtype == torch.uint8 and data_u8.is_contiguous()
+        assert offsets_i64.is_cuda and offsets_i64.dtype == torch.int64 and offsets_i64.is_contiguous()
+        B = offsets_i64.numel() - 1
+        assert B >= 1
+        dev = data_u8.device
+        samples = torch.empty((B, H, W), dtype=torch.uint16, device=dev)
+        status = torch.empty((B,), dtype=torch.int32, device=dev)
+        self._bind_stream()
+        self.handle.png_decode_device_async(data_u8.data_ptr(), offsets_i64.data_ptr(), B, H, W, samples.data_ptr(),
+                                            status.data_ptr())
+        self._hold(data_u8, offsets_i64, samples, status)
+        return samples, status
+
     def flush(self):
         """Pipelined mode: torch's current stream waits for every fill still in flight."""
         self._bind_stream()

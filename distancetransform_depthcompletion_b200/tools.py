@@ -3,6 +3,9 @@ backed by the sm_100a kernels behind libdtfill.so.  numpy in, numpy out.
 
     nearest_point(refined_lidar)      -> (dt float32 [H,W], lbl int32 [H,W])      tools.py:7-10
     DT_complete_batch(lidar_batch)    -> float32 [B,352,1216,1]                     tools.py:13-35
+
+and, for the uint16 samples of KITTI's depth PNGs or the PNG files themselves, DT_complete_batch_png and
+DT_complete_batch_png_files (loader + crop + fill in one call).
 """
 from __future__ import annotations
 
@@ -152,6 +155,35 @@ def DT_complete_batch_png(depth_png_batch, crop_top: int = 96, device: int | Non
         raise ValueError(f"cannot reshape array of size {H * W} into shape ({_H},{_W})")            # tools.py:25-27
     r = _lib.get_handle(device).run_host_u16(np.ascontiguousarray(png), crop_top, KITTI_SRC_THR, VALID_THR,
                                              want_lidar=True)
+    if "index_error" in r:
+        raise IndexError(r["index_error"])                                                          # tools.py:26
+    return r["lidar"].reshape(B, H, W, 1), r["depth"].reshape(B, _H, _W, 1)
+
+
+def DT_complete_batch_png_files(files, crop_top: int = 96, device: int | None = None):
+    """DT_complete_batch_png on the PNG files themselves (paths or bytes), decoded on the GPU:
+
+        depth_png = np.array(Image.open(f), dtype=int)      data_read.py:215, per file
+        ... DT_complete_batch_png(depth_png batch)
+
+    Only the compressed files cross the PCIe link; the decoded samples never leave the device.  Same shapes, checks
+    and exceptions as DT_complete_batch_png, plus ValueError for a file that is not an intact 16-bit grayscale PNG of
+    the first file's size."""
+    from .data_read import pack_png_files
+    files = list(files)
+    if not files:
+        e = np.expand_dims(np.asarray([]), axis=-1).astype(np.float32)
+        return e, e
+    data, offsets, Hin, W = pack_png_files(files)
+    B = len(files)
+    H = Hin - int(crop_top)
+    if crop_top < 0 or H <= 0:
+        raise ValueError(f"DT_complete_batch_png_files: crop_top {crop_top} leaves no rows of {Hin}")
+    if H * W != _H * _W:
+        raise ValueError(f"cannot reshape array of size {H * W} into shape ({_H},{_W})")            # tools.py:25-27
+    out = {"lidar": _lib.output_empty((B, H, W), np.float32), "depth": _lib.output_empty((B, H, W), np.float32)}
+    r = _lib.get_handle(device).run_host_png(data, offsets, Hin, W, crop_top, KITTI_SRC_THR, VALID_THR, want_lidar=True,
+                                             want_counts=False, out=out)
     if "index_error" in r:
         raise IndexError(r["index_error"])                                                          # tools.py:26
     return r["lidar"].reshape(B, H, W, 1), r["depth"].reshape(B, _H, _W, 1)

@@ -26,14 +26,15 @@
 extern "C" {
 #endif
 
-#define DTFILL_ABI_VERSION 5      /* 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
+#define DTFILL_ABI_VERSION 6      /* 6: PNG decode (dtfill_png_decode, dtfill_run_png, DTFILL_E_DATA); 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
 
 enum {
     DTFILL_OK = 0,
     DTFILL_E_ARG = -1,        /* bad argument (NULL pointer, non-positive size, unsupported size)            */
     DTFILL_E_CUDA = -2,       /* a CUDA runtime call failed; message has the CUDA error string               */
     DTFILL_E_INDEX = -3,      /* numpy's IndexError: a frame's labels index outside its list of valid depths */
-    DTFILL_E_NOMEM = -4
+    DTFILL_E_NOMEM = -4,
+    DTFILL_E_DATA = -5        /* a file is not a supported or intact 16-bit grayscale PNG                     */
 };
 
 enum { DTFILL_METRICS_KITTI = 0, DTFILL_METRICS_NYU = 1 };
@@ -107,6 +108,35 @@ int dtfill_run_u16_async(dtfill_t* h, const uint16_t* in_dev, int B, int H_in, i
                          float src_thr, float val_thr,
                          float* out_lidar_dev, float* out_depth_dev, float* out_dt_dev, int32_t* out_lbl_dev,
                          uint8_t* out_mask_dev, int32_t* out_counts_dev);
+
+/*
+ * The step in front of dtfill_run_u16: KITTI depth PNG files (data_read.py:215 `Image.open(f)`) decoded on the device
+ * (kernels k8_png_inflate, k8_png_unfilter; dtfill_k8_png.cuh).  Only non-interlaced 16-bit grayscale PNGs are supported
+ * (any row filters, any DEFLATE content, the zlib stream split over any IDAT chunks, ancillary chunks skipped); chunk
+ * CRC-32s are not checked, the zlib stream's Adler-32 is.  Per-frame status codes (int32):
+ *   0 ok, 1 bad signature, 2 unsupported IHDR, 3 size differs from (H, W), 4 broken or truncated chunk structure or no
+ *   IDAT, 5 bad zlib header, 6 invalid DEFLATE data (including running out of input), 7 decompressed size != H*(1+2W),
+ *   8 filter type > 4, 9 Adler-32 mismatch.
+ * A failed frame's samples are zero.  H * (1 + 2 W) < 2^28.
+ *
+ * dtfill_png_decode: B files packed back to back in `data`; file b is data[offsets[b], offsets[b+1]) (offsets int64
+ * [B+1], on the same side as data).  Writes uint16 [B,H,W] native-endian samples and out_status int32 [B] (nullable when
+ * the outputs are host pointers).  Enqueue-only when input and outputs are all device pointers; otherwise the call
+ * waits and returns DTFILL_E_DATA with *first_bad_frame when a frame failed (the other frames are still written).
+ */
+int dtfill_png_decode(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H, int W,
+                      uint16_t* out, int32_t* out_status, int out_is_device, int* first_bad_frame);
+
+/* Decode into the handle's workspace, then exactly the dtfill_run_u16 path (crop_top, thresholds, outputs, IndexError):
+ * the decoded samples never leave the device.  Synchronous.  A decode failure (DTFILL_E_DATA, first failed frame) wins
+ * over IndexError. */
+int dtfill_run_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H_in, int W,
+                   int crop_top, float src_thr, float val_thr, float* out_lidar, float* out_depth, float* out_dt,
+                   int32_t* out_lbl, uint8_t* out_mask, int32_t* out_counts, int out_is_device, int* first_bad_frame);
+
+/* Host-only test hook (no handle, no GPU), like dtfill_debug_compact: the same decode of one file of nbytes, run serially
+ * on the CPU.  Returns the status code above (samples of a failed file are zero), or -1 for bad arguments. */
+int dtfill_debug_png_decode_host(const uint8_t* png, long nbytes, int H, int W, uint16_t* out);
 
 /* Synchronise and report the outcome of EVERY dtfill_run_async / dtfill_run_u16_async since the previous dtfill_status:
  * DTFILL_OK, or DTFILL_E_INDEX with *first_bad_frame = the smallest frame index (within its call) that any of those
