@@ -18,7 +18,7 @@ LIB_PATH = os.environ.get("DTFILL_LIB") or os.path.join(_HERE, "libdtfill.so")
 E_ARG, E_CUDA, E_INDEX, E_NOMEM, E_DATA = -1, -2, -3, -4, -5
 METRICS_KITTI, METRICS_NYU = 0, 1
 METRIC_COLS = 9
-ABI_VERSION = 6          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
+ABI_VERSION = 7          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
 METRIC_NAMES = ("mse", "rmse", "mae", "irmse", "imae", "delta1", "delta2", "delta3", "count")
 
 _c_float_p = ctypes.POINTER(ctypes.c_float)
@@ -90,6 +90,16 @@ def load() -> ctypes.CDLL:
         L.dtfill_png_decode.argtypes = [vp, vp, vp, ci, ci, ci, ci, vp, vp, ci, ctypes.POINTER(ci)]
         L.dtfill_run_png.argtypes = [vp, vp, vp, ci, ci, ci, ci, ci, cf, cf, vp, vp, vp, vp, vp, vp, ci, ctypes.POINTER(ci)]
         L.dtfill_debug_png_decode_host.argtypes = [vp, ctypes.c_long, ci, ci, vp]
+        i64 = ctypes.c_int64
+        L.dtfill_png_encode_bound.argtypes = [ci, ci]
+        L.dtfill_png_encode_bound.restype = i64
+        L.dtfill_png_encode.argtypes = [vp, vp, ci, ci, ci, ci, vp, i64, vp, ci]
+        L.dtfill_png_encode_depth.argtypes = [vp, vp, ci, ci, ci, ci, vp, i64, vp, ci]
+        L.dtfill_run_png_to_png.argtypes = [vp, vp, vp, ci, ci, ci, ci, ci, cf, cf, vp, i64, vp, ci, ctypes.POINTER(ci)]
+        L.dtfill_debug_png_encode_host.argtypes = [vp, ci, ci, vp, ctypes.c_long]
+        L.dtfill_debug_png_encode_host.restype = ctypes.c_long
+        L.dtfill_debug_depth_samples_host.argtypes = [vp, ctypes.c_long, vp]
+        L.dtfill_debug_depth_samples_host.restype = ci
         L.dtfill_host_alloc.argtypes = [ctypes.POINTER(vp), ctypes.c_size_t]
         L.dtfill_host_free.argtypes = [vp]
         L.dtfill_host_free.restype = None
@@ -100,7 +110,8 @@ def load() -> ctypes.CDLL:
                      "dtfill_comm_destroy", "dtfill_allreduce_sums", "dtfill_set_stage_threads", "dtfill_debug_set_skip",
                      "dtfill_run_eval_async", "dtfill_eval_totals", "dtfill_edt", "dtfill_set_sparse_upload",
                      "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo", "dtfill_png_decode",
-                     "dtfill_run_png", "dtfill_debug_png_decode_host"):
+                     "dtfill_run_png", "dtfill_debug_png_decode_host", "dtfill_png_encode", "dtfill_png_encode_depth",
+                     "dtfill_run_png_to_png"):
             getattr(L, name).restype = ci
         _lib = L
         return L
@@ -268,6 +279,58 @@ class Handle:
         bad = ctypes.c_int(-1)
         _check(self._L.dtfill_png_decode(self._h, _ptr(data_ptr), _ptr(offsets_ptr), 1, int(B), int(H), int(W),
                                          _ptr(out_ptr), _ptr(status_ptr), 1, ctypes.byref(bad)), "dtfill_png_decode")
+
+    def png_encode(self, samples: np.ndarray) -> list:
+        """uint16 samples [B,H,W] -> B 16-bit grayscale PNG files (list of bytes), encoded on the device."""
+        return self._png_encode(samples, np.uint16, "dtfill_png_encode")
+
+    def png_encode_depth(self, depth: np.ndarray) -> list:
+        """float32 depth in metres [B,H,W] -> B 16-bit grayscale PNG files (list of bytes), encoded on the device with
+        sample = clip(nan_to_num(fl32(d * 256), nan=0, posinf=65535), 0, 65535) truncated toward zero, which is
+        (d * 256).astype(np.uint16) for d in [0, 65535/256] and the identity on d = k/256."""
+        return self._png_encode(depth, np.float32, "dtfill_png_encode_depth")
+
+    def _png_encode(self, x, dtype, fn):
+        x = np.ascontiguousarray(x)
+        assert x.dtype == dtype and x.ndim == 3, (x.dtype, x.shape)
+        B, H, W = x.shape
+        cap = B * png_encode_bound(H, W)
+        # pageable and untouched beyond offsets[B]: only the bytes of the files are copied into it
+        out = np.empty(cap, np.uint8)
+        offsets = np.empty(B + 1, np.int64)
+        _check(getattr(self._L, fn)(self._h, _ptr(x), 0, B, H, W, _ptr(out), cap, _ptr(offsets), 0), fn)
+        return _split_files(out, offsets)
+
+    def run_host_png_to_png(self, data: np.ndarray, offsets: np.ndarray, H_in: int, W: int, crop_top: int,
+                            src_thr: float, val_thr: float):
+        """PNG files (as png_decode) decoded, filled like run_host_png and the filled depth encoded, all on the device ->
+        dict(files=list of bytes, first_bad).  A decode failure raises ValueError; an IndexError is reported in the dict
+        under "index_error" (the files of all frames are still returned)."""
+        data, offsets = _png_args(data, offsets)
+        B = offsets.size - 1
+        H = H_in - int(crop_top)
+        cap = B * png_encode_bound(H, W)
+        out = np.empty(cap, np.uint8)
+        out_off = np.empty(B + 1, np.int64)
+        bad = ctypes.c_int(-1)
+        rc = self._L.dtfill_run_png_to_png(self._h, _ptr(data), _ptr(offsets), 0, B, int(H_in), int(W), int(crop_top),
+                                           float(src_thr), float(val_thr), _ptr(out), cap, _ptr(out_off), 0,
+                                           ctypes.byref(bad))
+        res = dict(first_bad=bad.value)
+        if rc == E_INDEX:
+            res["index_error"] = last_error()
+        else:
+            _check(rc, "dtfill_run_png_to_png")
+        res["files"] = _split_files(out, out_off)
+        return res
+
+    def png_encode_device_async(self, in_ptr: int, is_float: bool, B: int, H: int, W: int, out_ptr: int,
+                                capacity: int, offsets_ptr: int):
+        """Device frames (uint16, or float32 depth when is_float) -> device files + offsets [B+1], enqueued on the
+        handle's stream only."""
+        fn = "dtfill_png_encode_depth" if is_float else "dtfill_png_encode"
+        _check(getattr(self._L, fn)(self._h, _ptr(in_ptr), 1, int(B), int(H), int(W), _ptr(out_ptr), int(capacity),
+                                    _ptr(offsets_ptr), 1), fn)
 
     # ---- device path (raw pointers, e.g. torch tensors' data_ptr()) ------------------------------------
     def run_device_u16_async(self, in_ptr: int, B: int, H_in: int, W: int, crop_top: int, src_thr: float,
@@ -467,6 +530,40 @@ def png_decode_host(png: bytes, H: int, W: int):
         raise ValueError("dtfill_debug_png_decode_host: bad arguments")
     return st, out
 
+
+def png_encode_bound(H: int, W: int) -> int:
+    """Worst-case bytes of one encoded file of H x W samples (include/dtfill.h dtfill_png_encode_bound)."""
+    n = load().dtfill_png_encode_bound(int(H), int(W))
+    if n < 0:
+        raise ValueError(f"PNG encode: unsupported size {H} x {W} (H * (1 + 2 W) < 2^28)")
+    return n
+
+
+def _split_files(buf: np.ndarray, offsets: np.ndarray) -> list:
+    return [buf[offsets[b]:offsets[b + 1]].tobytes() for b in range(offsets.size - 1)]
+
+
+def png_encode_host(samples) -> bytes:
+    """Test hook: the encoder run serially on the CPU (no GPU): uint16 [H,W] -> the PNG file the device writes."""
+    x = np.ascontiguousarray(samples)
+    if x.dtype != np.uint16 or x.ndim != 2:
+        raise TypeError(f"png_encode_host: uint16 [H,W] expected, got {x.dtype} {x.shape}")
+    H, W = x.shape
+    cap = png_encode_bound(H, W)
+    out = np.empty(cap, np.uint8)
+    n = load().dtfill_debug_png_encode_host(_ptr(x), H, W, _ptr(out), cap)
+    if n < 0:
+        raise ValueError("dtfill_debug_png_encode_host: bad arguments")
+    return out[:n].tobytes()
+
+
+def depth_samples_host(depth) -> np.ndarray:
+    """Test hook: the depth -> sample rule of png_encode_depth run on the CPU: float32 array -> uint16 array."""
+    x = np.ascontiguousarray(depth, dtype=np.float32)
+    out = np.empty(x.shape, np.uint16)
+    if load().dtfill_debug_depth_samples_host(_ptr(x), x.size, _ptr(out)) != 0:
+        raise ValueError("dtfill_debug_depth_samples_host: bad arguments")
+    return out
 
 def nccl_unique_id() -> bytes:
     buf = ctypes.create_string_buffer(NCCL_ID_BYTES)

@@ -375,6 +375,10 @@ struct dtfill_ctx {
     // PNG decode (k8_png_*): uploaded files + offsets, filtered bytes per frame, decoded samples (dtfill_run_png), status
     Buf png_data, png_scratch, png_samples, png_status;
     PinBuf pin_png, pin_png_status;   // pinned staging of host file bytes / of the per-frame status
+    // PNG encode (k9_png_*): uploaded input, filtered bytes, row Adler-32s, segment chunks and sizes, packed files and
+    // their offsets (host outputs), filled depth of dtfill_run_png_to_png
+    Buf enc_in, enc_filt, enc_adler, enc_slots, enc_seg, enc_out, enc_off, enc_depth;
+    PinBuf pin_enc_off;
     bool metrics_exact = true;        // dtfill_metrics / _ex reproduce np.mean's pairwise sums bit for bit
     bool sparse_upload = true;        // pageable float32 inputs are compacted on the host instead of mirrored (see CopyPool)
     size_t last_h2d_bytes = 0, last_d2h_bytes = 0;   // bytes the last synchronous host call moved over the link
@@ -1059,7 +1063,8 @@ void dtfill_destroy(dtfill_t* h) {
     Buf* bufs[] = {&h->in_dev, &h->depth_dev, &h->dt_dev, &h->lbl_dev, &h->mask_dev, &h->counts_out_dev, &h->lidar_out_dev,
                    &h->gt_dev, &h->partial, &h->per_frame, &h->sums, &h->edt_rows, &h->edt_stack, &h->sparse_dev,
                    &h->mx_terms, &h->mx_counts, &h->mx_leaf_start, &h->mx_leaf_sum, &h->png_data, &h->png_scratch,
-                   &h->png_samples, &h->png_status};
+                   &h->png_samples, &h->png_status, &h->enc_in, &h->enc_filt, &h->enc_adler, &h->enc_slots, &h->enc_seg,
+                   &h->enc_out, &h->enc_off, &h->enc_depth};
     for (Buf* b : bufs)
         if (b->p) cudaFree(b->p);
     for (void* q : h->retired) cudaFree(q);
@@ -1067,7 +1072,7 @@ void dtfill_destroy(dtfill_t* h) {
     delete h->pool_in;
     delete h->pool_out;
     for (PinBuf* b : {&h->pin_in, &h->pin_depth, &h->pin_dt, &h->pin_lbl, &h->pin_mask, &h->pin_lidar, &h->pin_sparse, &h->pin_png,
-                      &h->pin_png_status})
+                      &h->pin_png_status, &h->pin_enc_off})
         if (b->p) cudaFreeHost(b->p);
     if (h->status_ring) cudaFreeHost(h->status_ring);
     if (h->status_dev) cudaFree(h->status_dev);
@@ -1491,6 +1496,250 @@ int dtfill_debug_png_decode_host(const uint8_t* f, long nbytes, int H, int W, ui
         }
     }
     return ST_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// uint16 samples / float32 depth -> 16-bit grayscale PNG files (k9_png_*; see dtfill_k9_png_encode.cuh)
+// ------------------------------------------------------------------------------------------------------------
+namespace {
+
+int png_encode_args(const char* who, dtfill_t* h, const void* in, const void* out, const int64_t* out_offsets, int B,
+                    int H, int W, int64_t out_capacity) {
+    if (!h || !in || !out || !out_offsets) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, input, out or out_offsets");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H, W must be positive");
+    if ((int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28))
+        return fail(DTFILL_E_ARG, std::string(who) + ": frame too large (H * (1 + 2 W) < 2^28 bytes)");
+    const int64_t need = (int64_t)B * png::encode_bound(H, W);
+    if (out_capacity < need)
+        return fail(DTFILL_E_ARG, std::string(who) + ": out_capacity " + std::to_string(out_capacity) + " < B * bound = " +
+                                      std::to_string(need));
+    return 0;
+}
+
+// Enqueue the encode of B device frames (uint16, or float32 depth when is_float) on the handle's stream: the files
+// back to back into out_dev, their offsets into off_dev [B+1].
+int png_encode_enqueue(dtfill_t* h, const void* in_dev, bool is_float, int B, int H, int W, uint8_t* out_dev,
+                       int64_t* off_dev) {
+    using namespace png;
+    int rc;
+    const int64_t stride = 1 + 2 * (int64_t)W, fbytes = (int64_t)H * stride;
+    const int nseg = segments(H);
+    // a slot holds the chunk header, the larger of the stored form and what the coded form writes before it gives up
+    // (at most one batch of tokens, 124 bytes, past the stored size), and the CRC
+    const int64_t slot = (8 + stored_bytes((int64_t)(H < SEG_ROWS ? H : SEG_ROWS) * stride) + 256 + 15) & ~(int64_t)15;
+    if ((rc = ensure(h, h->enc_filt, (size_t)B * fbytes))) return rc;
+    if ((rc = ensure(h, h->enc_adler, (size_t)B * H * 4))) return rc;
+    if ((rc = ensure(h, h->enc_slots, (size_t)B * nseg * slot))) return rc;
+    if ((rc = ensure(h, h->enc_seg, (size_t)B * nseg * 4))) return rc;
+    uint8_t* filt = (uint8_t*)h->enc_filt.p;
+    uint32_t* adler = (uint32_t*)h->enc_adler.p;
+    uint8_t* slots = (uint8_t*)h->enc_slots.p;
+    uint32_t* seg = (uint32_t*)h->enc_seg.p;
+    const int64_t rows = (int64_t)B * H;
+    const unsigned fgrid = (unsigned)((rows + K9_WARPS - 1) / K9_WARPS);
+    if (is_float)
+        k9_png_filter<float><<<fgrid, 32 * K9_WARPS, 0, h->stream>>>((const float*)in_dev, B, H, W, filt, adler);
+    else
+        k9_png_filter<uint16_t><<<fgrid, 32 * K9_WARPS, 0, h->stream>>>((const uint16_t*)in_dev, B, H, W, filt, adler);
+    const size_t smem = 256 * 4 + K9_WARPS * sizeof(DeflateSmem);
+    CU(cudaFuncSetAttribute(k9_png_deflate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const unsigned dgrid = (unsigned)(((int64_t)B * nseg + K9_WARPS - 1) / K9_WARPS);
+    k9_png_deflate<<<dgrid, 32 * K9_WARPS, smem, h->stream>>>(filt, B, H, W, slots, slot, seg);
+    k9_png_offsets<<<1, 1024, 0, h->stream>>>(seg, B, nseg, off_dev);
+    k9_png_pack<<<(unsigned)((int64_t)B * (nseg + 2)), 256, 0, h->stream>>>(slots, slot, seg, adler, B, H, W, off_dev, out_dev);
+    CU(cudaGetLastError());
+    return 0;
+}
+
+// dtfill_png_encode / dtfill_png_encode_depth
+int png_encode_call(const char* who, dtfill_t* h, const void* in, bool is_float, int in_is_device, int B, int H, int W,
+                    uint8_t* out, int64_t out_capacity, int64_t* out_offsets, int out_is_device) {
+    int rc = png_encode_args(who, h, in, out, out_offsets, B, H, W, out_capacity);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    h->last_h2d_bytes = h->last_d2h_bytes = 0;
+    const void* in_d = in;
+    if (!in_is_device) {
+        const size_t in_bytes = (size_t)B * H * W * (is_float ? 4 : 2);
+        if ((rc = ensure(h, h->enc_in, in_bytes))) return rc;
+        CU(cudaMemcpyAsync(h->enc_in.p, in, in_bytes, cudaMemcpyHostToDevice, h->stream));
+        h->last_h2d_bytes = in_bytes;
+        in_d = h->enc_in.p;
+    }
+    uint8_t* out_d = out;
+    int64_t* off_d = out_offsets;
+    if (!out_is_device) {
+        if ((rc = ensure(h, h->enc_out, (size_t)B * png::encode_bound(H, W)))) return rc;
+        if ((rc = ensure(h, h->enc_off, (size_t)(B + 1) * 8))) return rc;
+        out_d = (uint8_t*)h->enc_out.p;
+        off_d = (int64_t*)h->enc_off.p;
+    }
+    if ((rc = png_encode_enqueue(h, in_d, is_float, B, H, W, out_d, off_d))) return rc;
+    if (in_is_device && out_is_device) return 0;
+    if (out_is_device) {
+        CU(cudaStreamSynchronize(h->stream));
+        return 0;
+    }
+    // offsets first, then exactly offsets[B] bytes of files
+    if ((rc = ensure_pinned(h->pin_enc_off, (size_t)(B + 1) * 8))) return rc;
+    int64_t* off_h = (int64_t*)h->pin_enc_off.p;
+    CU(cudaMemcpyAsync(off_h, off_d, (size_t)(B + 1) * 8, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    memcpy(out_offsets, off_h, (size_t)(B + 1) * 8);
+    CU(cudaMemcpyAsync(out, out_d, (size_t)off_h[B], cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    h->last_d2h_bytes = (size_t)(B + 1) * 8 + (size_t)off_h[B];
+    return 0;
+}
+
+// The deflate of segment f[s0, s1) run serially: the candidates, parse, codes and fallback of k9_png_deflate.  Writes
+// the segment's compressed bytes to out (capacity >= 2 (s1 - s0) + 64) and returns their number.
+int64_t png_deflate_segment_host(const uint8_t* f, int64_t s0, int64_t s1, int64_t stride, bool final_seg, uint8_t* out,
+                                 uint32_t* head) {
+    using namespace png;
+    for (int i = 0; i < HSIZE; ++i) head[i] = NO_POS;
+    memset(out, 0, (size_t)(2 * (s1 - s0) + 64));
+    uint64_t bitpos = 0;
+    auto put = [&](uint32_t v, int n) {
+        for (int i = 0; i < n; ++i, ++bitpos)
+            if ((v >> i) & 1) out[bitpos >> 3] |= (uint8_t)(1u << (bitpos & 7));
+    };
+    put(2, 3);                                      // BFINAL 0, BTYPE 01
+    const int64_t hash_end = s1 - 2;
+    int64_t hashed = s0;
+    for (int64_t p = s0; p < s1;) {
+        for (; hashed < p; ++hashed)
+            if (hashed < hash_end) head[hash3(f + hashed)] = (uint32_t)hashed;
+        const uint32_t qh = p < hash_end ? head[hash3(f + p)] : NO_POS;
+        const int maxlen = (int)((s1 - p) < MAX_MATCH ? s1 - p : MAX_MATCH);
+        int best_len = 0;
+        int64_t best_d = 0;
+        if (maxlen >= 3) {
+            const int64_t dist[4] = {1, 2, stride, qh != NO_POS ? p - (int64_t)qh : 0};
+            for (int c = 0; c < 4; ++c) {
+                if (!(dist[c] > 0 && dist[c] <= p && dist[c] <= WINDOW)) continue;
+                const int n = match_len(f, p, dist[c], maxlen);
+                if (n >= 3 && (n > best_len || (n == best_len && dist[c] < best_d))) { best_len = n; best_d = dist[c]; }
+            }
+        }
+        uint32_t bits;
+        const int nb = token_bits((uint32_t)best_len, best_len ? (uint32_t)best_d : f[p], &bits);
+        put(bits, nb);
+        p += best_len ? best_len : 1;
+    }
+    put(0, 7);                                      // end of block
+    put(final_seg ? 1 : 0, 3);                      // empty stored block
+    bitpos = (bitpos + 7) & ~(uint64_t)7;
+    put(0xffff0000u, 32);
+    const int64_t nbytes = (int64_t)(bitpos >> 3);
+    if (nbytes <= stored_bytes(s1 - s0)) return nbytes;
+    return write_stored(f, s0, s1, final_seg, out, 0, 1);
+}
+
+}  // namespace
+
+int64_t dtfill_png_encode_bound(int H, int W) {
+    if (H <= 0 || W <= 0 || (int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28)) return DTFILL_E_ARG;
+    return png::encode_bound(H, W);
+}
+
+int dtfill_png_encode(dtfill_t* h, const uint16_t* in, int in_is_device, int B, int H, int W, uint8_t* out,
+                      int64_t out_capacity, int64_t* out_offsets, int out_is_device) {
+    return png_encode_call("dtfill_png_encode", h, in, false, in_is_device, B, H, W, out, out_capacity, out_offsets,
+                           out_is_device);
+}
+
+int dtfill_png_encode_depth(dtfill_t* h, const float* in, int in_is_device, int B, int H, int W, uint8_t* out,
+                            int64_t out_capacity, int64_t* out_offsets, int out_is_device) {
+    return png_encode_call("dtfill_png_encode_depth", h, in, true, in_is_device, B, H, W, out, out_capacity, out_offsets,
+                           out_is_device);
+}
+
+int dtfill_run_png_to_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H_in,
+                          int W, int crop_top, float src_thr, float val_thr, uint8_t* out, int64_t out_capacity,
+                          int64_t* out_offsets, int out_is_device, int* first_bad_frame) {
+    if (first_bad_frame) *first_bad_frame = -1;
+    if (!h || !data || !offsets) return fail(DTFILL_E_ARG, "dtfill_run_png_to_png: NULL handle, data or offsets");
+    if (B <= 0 || H_in <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_run_png_to_png: B, H_in, W must be positive");
+    if (crop_top < 0 || crop_top >= H_in) return fail(DTFILL_E_ARG, "dtfill_run_png_to_png: crop_top must lie in [0, H_in)");
+    const int H = H_in - crop_top;
+    int rc = png_encode_args("dtfill_run_png_to_png", h, data, out, out_offsets, B, H, W, out_capacity);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    if ((rc = ensure(h, h->enc_depth, (size_t)B * H * W * 4))) return rc;
+    float* depth = (float*)h->enc_depth.p;
+    const int run = dtfill_run_png(h, data, offsets, in_is_device, B, H_in, W, crop_top, src_thr, val_thr, nullptr, depth,
+                                   nullptr, nullptr, nullptr, nullptr, 1, first_bad_frame);
+    if (run != 0 && run != DTFILL_E_INDEX && run != DTFILL_E_DATA) return run;
+    const std::string verdict = g_err;
+    const size_t h2d = h->last_h2d_bytes;
+    if ((rc = png_encode_call("dtfill_run_png_to_png", h, depth, true, 1, B, H, W, out, out_capacity, out_offsets,
+                              out_is_device)))
+        return rc;
+    if (out_is_device) CU(cudaStreamSynchronize(h->stream));
+    h->last_h2d_bytes = h2d;
+    if (run) g_err = verdict;
+    return run;
+}
+
+int dtfill_debug_depth_samples_host(const float* depth, long n, uint16_t* out) {
+    if (!depth || !out || n < 0) return -1;
+    for (long i = 0; i < n; ++i) out[i] = (uint16_t)png::depth_sample(depth[i]);
+    return 0;
+}
+
+long dtfill_debug_png_encode_host(const uint16_t* samples, int H, int W, uint8_t* out, long capacity) {
+    using namespace png;
+    if (!samples || !out || H <= 0 || W <= 0 || (int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28)) return -1;
+    if (capacity < encode_bound(H, W)) return -1;
+    const int64_t stride = 1 + 2 * (int64_t)W;
+    std::vector<uint8_t> filt((size_t)H * stride);
+    for (int r = 0; r < H; ++r) {
+        const uint16_t* x = samples + (size_t)r * W;
+        const uint16_t* up = r ? x - W : nullptr;
+        auto sample = [&](int ft, int c) {
+            return filter_sample(ft, x[c], c ? x[c - 1] : 0, up ? up[c] : 0, (up && c) ? up[c - 1] : 0);
+        };
+        int best = 0;
+        unsigned long long best_cost = 0;
+        for (int ft = 0; ft < 5; ++ft) {
+            unsigned long long cost = 0;
+            for (int c = 0; c < W; ++c) {
+                const uint32_t y = sample(ft, c);
+                cost += msad(y >> 8) + msad(y & 255);
+            }
+            if (ft == 0 || cost < best_cost) { best = ft; best_cost = cost; }
+        }
+        uint8_t* o = &filt[(size_t)r * stride];
+        o[0] = (uint8_t)best;
+        for (int c = 0; c < W; ++c) {
+            const uint32_t y = sample(best, c);
+            o[1 + 2 * c] = (uint8_t)(y >> 8);
+            o[2 + 2 * c] = (uint8_t)y;
+        }
+    }
+    uint32_t tab[256];
+    for (uint32_t i = 0; i < 256; ++i) tab[i] = crc_table_entry(i);
+    uint32_t a = 1, bsum = 0;
+    for (uint8_t v : filt) { a = (a + v) % ADLER_MOD; bsum = (bsum + a) % ADLER_MOD; }
+    std::vector<uint32_t> head(HSIZE);
+    std::vector<uint8_t> seg;
+    write_head(out, tab, H, W);
+    int64_t pos = HEAD_BYTES;
+    const int nseg = segments(H);
+    for (int s = 0; s < nseg; ++s) {
+        int64_t s0, s1;
+        segment_range(s, H, stride, &s0, &s1);
+        seg.resize((size_t)(2 * (s1 - s0) + 64));
+        const int64_t n = png_deflate_segment_host(filt.data(), s0, s1, stride, s == nseg - 1, seg.data(), head.data());
+        put_be32(out + pos, (uint32_t)n);
+        put_be32(out + pos + 4, T_IDAT);
+        memcpy(out + pos + 8, seg.data(), (size_t)n);
+        put_be32(out + pos + 8 + n, crc32_bytes(tab, 0, out + pos + 4, n + 4));
+        pos += 12 + n;
+    }
+    write_tail(out + pos, tab, (bsum << 16) | a);
+    return (long)(pos + TAIL_BYTES);
 }
 
 namespace {

@@ -19,6 +19,8 @@
 //   K7  k7_edt_*          exact Euclidean feature transform (extension, SURVEY.md 8 f-4): column pass + parabola row pass
 //   K8  k8_png_*          16-bit grayscale PNG files -> uint16 samples (inflate, then row unfilter), the step before K1
 //                         of the uint16 entry (data_read.py:215 reads the files with PIL)
+//   K9  k9_png_*          uint16 samples or float32 depth -> 16-bit grayscale PNG files (row filter, deflate per segment,
+//                         offsets, pack), so that filled maps leave the device compressed
 // One header per kernel (dtfill_k*.cuh); dtfill_common.cuh holds the key format, the structs and the helpers.
 //
 // Key format of the fast path (SURVEY.md section 7 H1): dist:11 | order:4 | label:17.  "order" is the position
@@ -40,3 +42,4 @@
 #include "dtfill_k6_outlier.cuh"
 #include "dtfill_k7_edt.cuh"
 #include "dtfill_k8_png.cuh"
+#include "dtfill_k9_png_encode.cuh"

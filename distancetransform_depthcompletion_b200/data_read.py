@@ -2,9 +2,10 @@
 
     outlier_removal(lidar)        data_read.py:103-128   (SURVEY.md section 8 f-2)
     read_depth_pngs(files)        data_read.py:215 / :223 `np.array(Image.open(f))`, a batch of files at once
+    write_depth_pngs(batch)       its mirror: uint16 samples or depth in metres -> 16-bit grayscale PNG files
 
 numpy in, numpy out; the 7 x 7 diamond filter runs on the GPU (kernel k6_outlier_removal), the PNG files are decoded on
-the GPU (kernels k8_png_inflate, k8_png_unfilter).  The h5 reader of NYU is out of scope.
+the GPU (kernels k8_png_inflate, k8_png_unfilter) and encoded there (kernels k9_png_*).  The h5 reader of NYU is out of scope.
 """
 from __future__ import annotations
 
@@ -55,3 +56,32 @@ def read_depth_pngs(files, device: int | None = None) -> np.ndarray:
     data, offsets, H, W = pack_png_files(files)
     out = _lib.output_empty((offsets.size - 1, H, W), np.uint16)
     return _lib.get_handle(device).png_decode(data, offsets, H, W, out=out)[0]
+
+
+def write_depth_pngs(batch, paths=None, device: int | None = None) -> list:
+    """The mirror of read_depth_pngs: a batch of depth maps encoded on the GPU as 16-bit grayscale PNG files (KITTI's
+    depth format).  batch: uint16 samples [B,H,W], or float32 depth in metres [B,H,W] / [B,H,W,1], whose samples are
+
+        sample = clip(nan_to_num(fl32(d * 256), nan=0, posinf=65535), 0, 65535) truncated toward zero,
+
+    which equals (d * 256).astype(np.uint16) for every d in [0, 65535/256] (the usual way KITTI predictions are
+    written) and is the identity on depths read from such files (d = k/256).  Returns the files' bytes; with ``paths``
+    (one per frame) it also writes them.  Other dtypes raise TypeError, other shapes ValueError."""
+    x = np.asarray(batch)
+    if x.dtype not in (np.uint16, np.float32):
+        raise TypeError(f"write_depth_pngs: uint16 samples or float32 depth expected, got {x.dtype}")
+    if x.ndim == 4 and x.shape[-1] == 1 and x.dtype == np.float32:
+        x = x[..., 0]
+    if x.ndim != 3 or 0 in x.shape:
+        raise ValueError(f"write_depth_pngs: expected [B,H,W] (or float32 [B,H,W,1]), got shape {np.shape(batch)}")
+    if paths is not None:
+        paths = list(paths)
+        if len(paths) != x.shape[0]:
+            raise ValueError(f"write_depth_pngs: {len(paths)} paths for {x.shape[0]} frames")
+    h = _lib.get_handle(device)
+    x = np.ascontiguousarray(x)
+    files = h.png_encode(x) if x.dtype == np.uint16 else h.png_encode_depth(x)
+    for p, f in zip(paths or (), files):
+        with open(p, "wb") as fh:
+            fh.write(f)
+    return files

@@ -145,6 +145,27 @@ class DTFillEngine:
         self._hold(data_u8, offsets_i64, samples, status)
         return samples, status
 
+    def encode_png(self, t):
+        """t: uint16 samples or float32 depth in metres, CUDA tensor [B,H,W] -> (data uint8 CUDA tensor [B * bound],
+        offsets int64 CUDA tensor [B+1]): B 16-bit grayscale PNG files back to back, file b = data[offsets[b]:
+        offsets[b+1]] (the layout decode_png takes), enqueued on torch's current stream.  Depth becomes
+        sample = clip(nan_to_num(fl32(d * 256), nan=0, posinf=65535), 0, 65535) truncated toward zero.  In pipelined
+        mode the fills in flight are joined into the stream first (no host synchronisation), so the output of fill() /
+        fill_png() can be passed straight in."""
+        torch = self.torch
+        assert t.is_cuda and t.dtype in (torch.uint16, torch.float32) and t.is_contiguous() and t.dim() == 3
+        B, H, W = t.shape
+        bound = _lib.png_encode_bound(H, W)
+        data = torch.empty((B * bound,), dtype=torch.uint8, device=t.device)
+        offsets = torch.empty((B + 1,), dtype=torch.int64, device=t.device)
+        self._bind_stream()
+        if self.pipeline_depth > 1:
+            self.handle.flush()
+        self.handle.png_encode_device_async(t.data_ptr(), t.dtype == torch.float32, B, H, W, data.data_ptr(), B * bound,
+                                            offsets.data_ptr())
+        self._hold(t, data, offsets)
+        return data, offsets
+
     def flush(self):
         """Pipelined mode: torch's current stream waits for every fill still in flight."""
         self._bind_stream()

@@ -5,7 +5,8 @@ backed by the sm_100a kernels behind libdtfill.so.  numpy in, numpy out.
     DT_complete_batch(lidar_batch)    -> float32 [B,352,1216,1]                     tools.py:13-35
 
 and, for the uint16 samples of KITTI's depth PNGs or the PNG files themselves, DT_complete_batch_png and
-DT_complete_batch_png_files (loader + crop + fill in one call).
+DT_complete_batch_png_files (loader + crop + fill in one call), and DT_complete_batch_png_files_to_png (files in, the
+refined frames as PNG files out).
 """
 from __future__ import annotations
 
@@ -187,3 +188,25 @@ def DT_complete_batch_png_files(files, crop_top: int = 96, device: int | None = 
     if "index_error" in r:
         raise IndexError(r["index_error"])                                                          # tools.py:26
     return r["lidar"].reshape(B, H, W, 1), r["depth"].reshape(B, _H, _W, 1)
+
+
+def DT_complete_batch_png_files_to_png(files, crop_top: int = 96, device: int | None = None) -> list:
+    """DT_complete_batch_png_files with the refined frames written as 16-bit grayscale PNG files (KITTI's depth format,
+    sample = depth * 256), all on the GPU: only compressed bytes cross the PCIe link in either direction.  Returns one
+    file (bytes) per input file; each decodes to (DT_complete_batch_png_files(files)[1][..., 0] * 256).astype(np.uint16).
+    The depth -> sample rule is that of data_read.write_depth_pngs.  Same checks and exceptions as
+    DT_complete_batch_png_files: ValueError for a size or a broken file (naming the frame), IndexError (tools.py:26)."""
+    from .data_read import pack_png_files
+    files = list(files)
+    if not files:
+        return []
+    data, offsets, Hin, W = pack_png_files(files)
+    H = Hin - int(crop_top)
+    if crop_top < 0 or H <= 0:
+        raise ValueError(f"DT_complete_batch_png_files_to_png: crop_top {crop_top} leaves no rows of {Hin}")
+    if H * W != _H * _W:
+        raise ValueError(f"cannot reshape array of size {H * W} into shape ({_H},{_W})")            # tools.py:25-27
+    r = _lib.get_handle(device).run_host_png_to_png(data, offsets, Hin, W, crop_top, KITTI_SRC_THR, VALID_THR)
+    if "index_error" in r:
+        raise IndexError(r["index_error"])                                                          # tools.py:26
+    return r["files"]

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DTFILL_ABI_VERSION 6      /* 6: PNG decode (dtfill_png_decode, dtfill_run_png, DTFILL_E_DATA); 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
+#define DTFILL_ABI_VERSION 7      /* 7: PNG encode (dtfill_png_encode, dtfill_png_encode_depth, dtfill_run_png_to_png); 6: PNG decode (dtfill_png_decode, dtfill_run_png, DTFILL_E_DATA); 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
 
 enum {
     DTFILL_OK = 0,
@@ -137,6 +137,46 @@ int dtfill_run_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int
 /* Host-only test hook (no handle, no GPU), like dtfill_debug_compact: the same decode of one file of nbytes, run serially
  * on the CPU.  Returns the status code above (samples of a failed file are zero), or -1 for bad arguments. */
 int dtfill_debug_png_decode_host(const uint8_t* png, long nbytes, int H, int W, uint16_t* out);
+
+/*
+ * The way out, the mirror of dtfill_png_decode: frames encoded on the device as 16-bit grayscale PNG files (kernels
+ * k9_png_filter, k9_png_deflate, k9_png_offsets, k9_png_pack; dtfill_k9_png_encode.cuh), so that only compressed bytes
+ * cross the link.  Every file is colour type 0, bit depth 16, non-interlaced: signature, IHDR, an IDAT holding the zlib
+ * header, one IDAT per 16 rows (fixed-Huffman DEFLATE blocks, or stored blocks where those would be larger, ending
+ * byte-aligned), an IDAT holding the Adler-32, IEND.  Rows are filtered with libpng's heuristic (least sum of absolute
+ * signed differences, ties to the lowest filter type).  The bytes are a pure function of the samples: the host hook
+ * below writes identical files.  H * (1 + 2 W) < 2^28.
+ *
+ * dtfill_png_encode_bound: worst-case bytes of one file (every segment stored, plus all chunk overhead); DTFILL_E_ARG
+ * for an unsupported size.
+ * dtfill_png_encode: uint16 samples [B,H,W] -> B files back to back in out; out_offsets int64 [B+1] (file b =
+ * out[off[b], off[b+1])), the layout dtfill_png_decode takes.  out_capacity must be >= B * dtfill_png_encode_bound(H, W)
+ * (else DTFILL_E_ARG and nothing is written).  Enqueue-only when input and outputs are all device pointers; otherwise
+ * the call waits and copies only offsets[B] bytes device -> host.
+ * dtfill_png_encode_depth: float32 depth in metres [B,H,W]; each sample is
+ *     sample = clip(nan_to_num(fl32(d * 256), nan=0, posinf=65535), 0, 65535) truncated toward zero,
+ * applied inside k9_png_filter (no uint16 copy exists).  For d in [0, 65535/256] this is (d * 256).astype(np.uint16),
+ * the usual way KITTI depth is written; on d = k/256 (a frame decoded from a PNG) it is the identity.
+ */
+int64_t dtfill_png_encode_bound(int H, int W);
+int dtfill_png_encode(dtfill_t* h, const uint16_t* in, int in_is_device, int B, int H, int W,
+                      uint8_t* out, int64_t out_capacity, int64_t* out_offsets, int out_is_device);
+int dtfill_png_encode_depth(dtfill_t* h, const float* in, int in_is_device, int B, int H, int W,
+                            uint8_t* out, int64_t out_capacity, int64_t* out_offsets, int out_is_device);
+
+/* dtfill_run_png, then the filled depth encoded as by dtfill_png_encode_depth: PNG files in, PNG files of
+ * H = H_in - crop_top rows out.  The decoded samples and the float32 depth never leave the device.  Synchronous.
+ * DTFILL_E_DATA (first failed frame) wins over DTFILL_E_INDEX; with either, the files of all frames are still written. */
+int dtfill_run_png_to_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H_in,
+                          int W, int crop_top, float src_thr, float val_thr, uint8_t* out, int64_t out_capacity,
+                          int64_t* out_offsets, int out_is_device, int* first_bad_frame);
+
+/* Host-only test hook (no handle, no GPU): the same encoder run serially on the CPU.  capacity >= the bound.  Returns the
+ * file size, or -1 for bad arguments. */
+long dtfill_debug_png_encode_host(const uint16_t* samples, int H, int W, uint8_t* out, long capacity);
+/* Host-only test hook: the depth -> sample rule of dtfill_png_encode_depth (the function k9_png_filter runs) on n floats.
+ * Returns 0, or -1 for bad arguments. */
+int dtfill_debug_depth_samples_host(const float* depth, long n, uint16_t* out);
 
 /* Synchronise and report the outcome of EVERY dtfill_run_async / dtfill_run_u16_async since the previous dtfill_status:
  * DTFILL_OK, or DTFILL_E_INDEX with *first_bad_frame = the smallest frame index (within its call) that any of those
