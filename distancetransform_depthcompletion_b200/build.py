@@ -38,7 +38,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     """Compile csrc/*.cu for sm_100a into libdtfill.so next to this file; returns the path."""
     if not force and not needs_build():
         return LIB_PATH
-    extra = os.environ.get("DTFILL_NVCC_EXTRA", "").split()        # experiments: -D switches of the kernels
+    extra = os.environ.get("DTFILL_NVCC_EXTRA", "").split()        # instrumented builds: -DDTFILL_TRACE, -DDTFILL_PLANNER_CLOCKS
     cmd = [_nvcc(), *NVCC_FLAGS, *extra, "-I", INCLUDE, "-I", CSRC, "-o", LIB_PATH] + [os.path.join(CSRC, s) for s in SOURCES]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")

@@ -311,8 +311,6 @@ struct Lane {
     cudaStream_t side[MAX_SUB] = {};     // narrow tiles run next to the full-width tasks of the same sub-batch
     cudaEvent_t side_fork[MAX_SUB] = {}, side_join[MAX_SUB] = {};
     cudaStream_t pipe = nullptr;         // pipelined mode: the stream this lane's calls run on
-    cudaStream_t pipe_front = nullptr;   // pipelined mode: low-priority stream of the first stage (k1_mask_rows)
-    cudaEvent_t front_done = nullptr;
     cudaEvent_t done = nullptr;          // ... and the end of its last call
     bool pending = false;                // done not yet waited for by the handle's stream
     int last_launches = 0;
@@ -392,18 +390,12 @@ struct dtfill_ctx {
     unsigned long long* trace_dev = nullptr;   // [TRACE_CALLS][4 kernels][4]
     static const int TRACE_CALLS = 256;
 #endif
-    bool prio_split = false;          // pipelined mode: first stage on a low-priority stream, the rest on a high-priority one
     int debug_skip = 0;               // tuning only (dtfill_debug_set_skip): bit 0 K1, 1 K1b, 2 K2, 3 k3_sky are not launched
-    bool tiles2d = true;
-    int max_col_tiles = 4;
     int sky_min = -1;             // source-free top rows go to k3_sky when there are at least this many; 0: never;
                                   // -1: automatic = 8 (measured in strict order on KITTI-64 frames: one frame 0.209 ->
                                   // 0.137 ms, 16 frames 0.222 -> 0.165, 256 frames 0.551 -> 0.536; the launch costs
                                   // 2 % on frames without such rows, 256 NYU frames 0.603 -> 0.616)
     int nsub = -1;                // -1: automatic
-    bool sky_split = true;        // strict order: k3_sky beside the narrow tiles (DTFILL_SKY_SPLIT=0: behind them)
-    bool narrow_main = true;      // the half-width scan instance on the call's own stream, the full-width one on the side
-                                  // stream (DTFILL_NARROW_MAIN=0: the other way round; strict step of 256 KITTI frames 0.536 -> 0.519)
     int band_cap = -1;            // -1: automatic (see enqueue); 0: never split frames; >0: task cost target in row steps
     cudaEvent_t ev[DTFILL_NUM_KERNELS + 1] = {};
 };
@@ -540,9 +532,11 @@ static float source_cut(float thr) {
     return ordered_to_float(hi);
 }
 
+constexpr int MAX_COL_TILES = 4;      // planner: at most this many half-width tiles side by side in a band
+
 // Enqueue the path for frames [b0, b0+nb) of the batch on stream s; all pointers are device pointers to the whole
 // batch, the workspace is sliced per frame so sub-batches never share anything but the status words.
-int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, cudaStream_t s_front, const Plan& plan, int b0, int nb, int Btot, const void* in, int H, int W,
+int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0, int nb, int Btot, const void* in, int H, int W,
                   float src_thr, float val_thr, float* out_depth, float* out_dt, int32_t* out_lbl, uint8_t* out_mask,
                   int32_t* out_counts, int scratch_units_per_frame, int sub_index, int* launches) {
     const int WW = (W + 31) / 32;
@@ -558,15 +552,15 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, cudaStream_t s_front, co
     fp.force_wide = plan.ppl == 0;
     fp.scratch_units_per_frame = scratch_units_per_frame;
     fp.wide_ppl = plan.ppl ? plan.ppl : 1;
-    fp.narrow_ppl = (h->tiles2d && plan.ppl) ? plan.narrow : 0;
+    fp.narrow_ppl = plan.ppl ? plan.narrow : 0;
     fp.frame0 = b0;
     fp.sky_min = h->sky_min >= 0 ? h->sky_min : 8;
     // strict order with two scan instances: k3_sky follows the full-width instance on the side stream (see the planner)
     // -- while the scan leaves SMs idle: measured on KITTI frames, 4 / 16 / 32 / 64 frames per call -4 / -10 / -9 / -2 %,
     // 128 / 256 frames +4 / +2 % (the wide instance then takes registers from the narrow tiles)
-    fp.sky_split = (h->sky_split && !h->cur_pipelined && !h->profiling && h->tiles2d && plan.ppl && plan.narrow &&
-                    h->narrow_main && fp.sky_min > 0 && W <= SKY_MAX_W && (long)Btot * H * W <= 28000000L) ? 1 : 0;
-    fp.max_col_tiles = h->max_col_tiles;
+    fp.sky_split = (!h->cur_pipelined && !h->profiling && plan.ppl && plan.narrow && fp.sky_min > 0 && W <= SKY_MAX_W &&
+                    (long)Btot * H * W <= 28000000L) ? 1 : 0;
+    fp.max_col_tiles = MAX_COL_TILES;
     fp.mul_dist = 1u << (32 - DSH);
     fp.four = 4u;
     fp.one = 1u;
@@ -623,20 +617,16 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, cudaStream_t s_front, co
         int grid = (int)(want < 1 ? 1 : want);
         if (!h->in_u16) {
             const float* in_s = (const float*)in + npx0;
-            if ((W & 15) == 0) k1_mask_rows_v16<float, true><<<grid, k1_threads, 0, s_front>>>(in_s, fp, ws, om, nullptr);
-            else if ((W & 3) == 0) k1_mask_rows_v16<float, false><<<grid, k1_threads, 0, s_front>>>(in_s, fp, ws, om, nullptr);
-            else k1_mask_rows<float><<<grid, k1_threads, 0, s_front>>>(in_s, fp, ws, om, nullptr);
+            if ((W & 15) == 0) k1_mask_rows_v16<float, true><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
+            else if ((W & 3) == 0) k1_mask_rows_v16<float, false><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
+            else k1_mask_rows<float><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
         } else {
             const uint16_t* in_s = (const uint16_t*)in + (size_t)b0 * h->in_H * W;
-            if ((W & 15) == 0) k1_mask_rows_v16<uint16_t, true><<<grid, k1_threads, 0, s_front>>>(in_s, fp, ws, om, olid);
-            else if ((W & 7) == 0) k1_mask_rows_v16<uint16_t, false><<<grid, k1_threads, 0, s_front>>>(in_s, fp, ws, om, olid);
-            else k1_mask_rows<uint16_t><<<grid, k1_threads, 0, s_front>>>(in_s, fp, ws, om, olid);
+            if ((W & 15) == 0) k1_mask_rows_v16<uint16_t, true><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
+            else if ((W & 7) == 0) k1_mask_rows_v16<uint16_t, false><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
+            else k1_mask_rows<uint16_t><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
         }
         ++*launches;
-        if (s_front != s) {                 // the later stages run on the lane's high-priority stream
-            CU(cudaEventRecord(L->front_done, s_front));
-            CU(cudaStreamWaitEvent(s, L->front_done, 0));
-        }
     }
     if (h->profiling) CU(cudaEventRecord(h->ev[1], s));
     if (!(h->debug_skip & 2)) {
@@ -655,10 +645,11 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, cudaStream_t s_front, co
     const bool want_lbl = ol != nullptr;
     // half-width and full-width tiles are different kernel instances and run next to each other on two streams.  The
     // instance that a frame of this shape normally uses stays on the call's own stream, so that the chain
-    // K1 -> K1b -> scan -> k3_sky does not cross streams twice (narrow_main; the other instance finds no task as a rule)
+    // K1 -> K1b -> scan -> k3_sky does not cross streams twice (narrow_main; the other instance finds no task as a rule;
+    // measured with the instances the other way round: strict step of 256 KITTI frames 0.536 ms against 0.519)
     const bool run_k2 = !(h->debug_skip & 4);
     const bool two = fp.narrow_ppl && run_k2;
-    const bool narrow_main = two && h->narrow_main && !h->profiling;
+    const bool narrow_main = two && !h->profiling;
     cudaStream_t s_side = s;
     if (two) {
         s_side = L->side[sub_index];
@@ -757,24 +748,13 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
         }
     }
 
-    cudaStream_t s = h->stream, s_front = h->stream;
+    cudaStream_t s = h->stream;
     if (pipelined) {
         // this call runs on the lane's own stream, behind whatever the caller queued so far and behind the lane's
         // previous call (stream order); the handle's stream only joins at dtfill_flush / dtfill_status.
-        // DTFILL_PRIO_SPLIT=1 (experiment, off): the first stage (HBM bound, thousands of small blocks) on a low-priority
-        // stream and the later stages on a high-priority one.  The calls then form a clean staggered pipeline instead of
-        // running in rounds (all K1, all K1b, all K2 ... of the calls in flight), but the low-priority stage starves and
-        // the step is 2 % slower (profiles/r02_timeline_*.txt).
         CU(cudaEventRecord(h->pipe_fork, h->stream));
         s = L->pipe;
-        if (h->prio_split) {
-            s_front = L->pipe_front;
-            CU(cudaStreamWaitEvent(s_front, h->pipe_fork, 0));
-            if (L->pending) CU(cudaStreamWaitEvent(s_front, L->done, 0));      // workspace of the call `depth` back
-        } else {
-            s_front = s;
-            CU(cudaStreamWaitEvent(s, h->pipe_fork, 0));
-        }
+        CU(cudaStreamWaitEvent(s, h->pipe_fork, 0));
     } else {
         // strict mode: everything still in flight on the lanes joins the handle's stream first
         for (Lane& o : h->lanes)
@@ -792,7 +772,7 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
     h->cur_slot = slot;
     h->cur_status = h->status_dev + (size_t)slot * dtfill_ctx::STATUS_STRIDE;
     if (h->slot_rearm[slot] || (h->debug_skip & 2)) {      // (a run without k1b_scan_compact reports nothing)
-        CU(cudaMemcpyAsync(h->cur_status, h->status_init, 8, cudaMemcpyHostToDevice, s_front));
+        CU(cudaMemcpyAsync(h->cur_status, h->status_init, 8, cudaMemcpyHostToDevice, s));
         h->slot_rearm[slot] = false;
     }
     h->cur_status_copied = false;
@@ -864,7 +844,7 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
     };
     if (nsub == 1 && !(hio && hio->any_out_pin())) {
         if ((rc = copy_in(s, 0, B))) return rc;
-        if ((rc = enqueue_range(h, L, s, s_front, plan, 0, B, B, in, H, W, src_thr, val_thr, out_depth, out_dt, out_lbl, out_mask,
+        if ((rc = enqueue_range(h, L, s, plan, 0, B, B, in, H, W, src_thr, val_thr, out_depth, out_dt, out_lbl, out_mask,
                                 out_counts, scratch_units_per_frame, 0, &launches))) return rc;
         if ((rc = copy_out(s, 0, B))) return rc;
     } else {
@@ -900,7 +880,7 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
                 CU(cudaStreamWaitEvent(L->sub[i], L->fork_ev, 0));
                 int r;
                 if ((r = copy_in(L->sub[i], b0, b1 - b0))) return r;
-                if ((r = enqueue_range(h, L, L->sub[i], L->sub[i], plan, b0, b1 - b0, B, in, H, W, src_thr, val_thr, out_depth, out_dt,
+                if ((r = enqueue_range(h, L, L->sub[i], plan, b0, b1 - b0, B, in, H, W, src_thr, val_thr, out_depth, out_dt,
                                        out_lbl, out_mask, out_counts, scratch_units_per_frame, i, &launches))) return r;
                 if ((r = copy_out(L->sub[i], b0, b1 - b0))) return r;
                 CU(cudaEventRecord(L->join_ev[i], L->sub[i]));
@@ -1003,12 +983,10 @@ int dtfill_create(int device, dtfill_t** out_handle) {
         CU(cudaStreamCreateWithFlags(&h->status_stream, cudaStreamNonBlocking));
         CU(cudaEventCreateWithFlags(&h->status_fork, cudaEventDisableTiming));
     }
-    int prio_lo = 0, prio_hi = 0;
-    CU(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));      // numerically lower = higher priority
+    int prio_hi = 0;
+    CU(cudaDeviceGetStreamPriorityRange(nullptr, &prio_hi));      // numerically lower = higher priority
     for (Lane& L : h->lanes) {
         CU(cudaStreamCreateWithPriority(&L.pipe, cudaStreamNonBlocking, prio_hi));
-        CU(cudaStreamCreateWithPriority(&L.pipe_front, cudaStreamNonBlocking, prio_lo));
-        CU(cudaEventCreateWithFlags(&L.front_done, cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&L.done, cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&L.fork_ev, cudaEventDisableTiming));
         for (int i = 0; i < Lane::MAX_SUB; ++i) {
@@ -1019,14 +997,9 @@ int dtfill_create(int device, dtfill_t** out_handle) {
             CU(cudaEventCreateWithFlags(&L.side_join[i], cudaEventDisableTiming));
         }
     }
-    if (const char* e = getenv("DTFILL_PRIO_SPLIT")) h->prio_split = atoi(e) != 0;
-    if (const char* e = getenv("DTFILL_TILES2D")) h->tiles2d = atoi(e) != 0;
     if (const char* e = getenv("DTFILL_SUBBATCHES")) h->nsub = atoi(e);
-    if (const char* e = getenv("DTFILL_MAX_COL_TILES")) h->max_col_tiles = atoi(e);
     if (const char* e = getenv("DTFILL_SKY_MIN")) h->sky_min = atoi(e) < -1 ? -1 : atoi(e);
     if (const char* e = getenv("DTFILL_BAND_CAP")) h->band_cap = atoi(e);
-    if (const char* e = getenv("DTFILL_NARROW_MAIN")) h->narrow_main = atoi(e) != 0;
-    if (const char* e = getenv("DTFILL_SKY_SPLIT")) h->sky_split = atoi(e) != 0;
     if (const char* e = getenv("DTFILL_STAGE_THREADS")) h->stage_threads = atoi(e);
     if (const char* e = getenv("DTFILL_SPARSE_UPLOAD")) h->sparse_upload = atoi(e) != 0;
     if (const char* e = getenv("DTFILL_METRICS_EXACT")) h->metrics_exact = atoi(e) != 0;
@@ -1050,8 +1023,6 @@ void dtfill_destroy(dtfill_t* h) {
         if (L.fork_ev) cudaEventDestroy(L.fork_ev);
         if (L.done) cudaEventDestroy(L.done);
         if (L.pipe) cudaStreamDestroy(L.pipe);
-        if (L.pipe_front) cudaStreamDestroy(L.pipe_front);
-        if (L.front_done) cudaEventDestroy(L.front_done);
         for (int i = 0; i < Lane::MAX_SUB; ++i) {
             if (L.join_ev[i]) cudaEventDestroy(L.join_ev[i]);
             if (L.sub[i]) cudaStreamDestroy(L.sub[i]);

@@ -174,34 +174,6 @@ struct TraceScope {
 #define DTFILL_TRACE_SCOPE(fp, k)
 #endif
 
-// depth_list is the one buffer of the path that is read at random (the gather depth_list[lbl - 1], tools.py:26) and
-// read more than once: 21 MB per batch of 256 KITTI frames.  Its stores and loads carry an L2 evict-last policy so that
-// the streaming traffic of the step (2 GB) does not push it out of the 126 MB L2 before the gather comes.
-#ifndef DTFILL_DLIST_KEEP
-#define DTFILL_DLIST_KEEP 0
-#endif
-__device__ __forceinline__ uint64_t l2_policy_keep() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ float ld_keep_f32(const void* p, uint64_t pol) {
-    float v;
-#if DTFILL_DLIST_KEEP
-    asm volatile("ld.global.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol));
-#else
-    v = *reinterpret_cast<const float*>(p);
-#endif
-    return v;
-}
-__device__ __forceinline__ void st_keep_f32(float* p, float v, uint64_t pol) {
-#if DTFILL_DLIST_KEEP
-    asm volatile("st.global.L2::cache_hint.f32 [%0], %1, %2;" ::"l"(p), "f"(v), "l"(pol) : "memory");
-#else
-    *p = v;
-#endif
-}
-
 __device__ __forceinline__ uint32_t lanemask_lt() {
     uint32_t m;
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));

@@ -102,7 +102,6 @@ __global__ void __launch_bounds__(K1B_THREADS) k1b_scan_compact(FrameParams fp, 
         // ---- warps 0..7: depth_list = in[valid] in raster order (tools.py:24).  K1 left every row's valid depths
         // compacted at the start of the row's slot in ws.scratch; concatenate the non-empty rows.
         float* dl = ws.dlist + (long)b * H * W;
-        const uint64_t pol_dlist = l2_policy_keep();
         const float* rowvals = reinterpret_cast<const float*>(ws.scratch) + (long)b * H * W;
         for (int yb = wid * 32; yb < H; yb += 8 * 32) {
             // one coalesced read of 33 row bases per 32 rows instead of two dependent loads per row
@@ -126,7 +125,7 @@ __global__ void __launch_bounds__(K1B_THREADS) k1b_scan_compact(FrameParams fp, 
                     for (int k = 0; k < 12; ++k) v[k] = 32 * k < rem ? sp[32 * k] : 0.f;
 #pragma unroll
                     for (int k = 0; k < 12; ++k)
-                        if (32 * k < rem) st_keep_f32(dp + 32 * k, v[k], pol_dlist);
+                        if (32 * k < rem) dp[32 * k] = v[k];
                 }
             }
         }

@@ -73,37 +73,12 @@ __device__ __forceinline__ uint32_t lane_carry(uint32_t e, int lane, uint32_t cl
 __device__ __forceinline__ void cp_async8(uint32_t smem_addr, const void* gptr) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_addr), "l"(gptr) : "memory");
 }
-__device__ __forceinline__ void cp_async16_l2only(uint32_t smem_addr, const void* gptr) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(gptr) : "memory");
-}
 // forward-state scratch is written once and read once, a whole pass later: keep it out of L1 (L2 only)
 __device__ __forceinline__ void st_scratch_v4(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
     asm volatile("st.global.cg.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 __device__ __forceinline__ void st_scratch_v2(void* p, uint32_t a, uint32_t b) {
     asm volatile("st.global.cg.v2.u32 [%0], {%1, %2};" ::"l"(p), "r"(a), "r"(b) : "memory");
-}
-// L2 residency of the forward state (DTFILL_L2POLICY): the scratch is written once and read back once in LIFO order, so
-// its most recent rows can live and die in the 126 MB L2 without ever reaching HBM: stores carry an evict-last policy,
-// the read-back an evict-first one, and a consumed row is discarded (dropped from L2 without write-back).
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void st_scratch_v4_hint(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d, uint64_t pol) {
-    asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(p), "r"(a), "r"(b), "r"(c), "r"(d), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void cp_async16_hint(uint32_t smem_addr, const void* gptr, uint64_t pol) {
-    asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"(smem_addr), "l"(gptr), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void l2_discard_128(const void* p) {
-    asm volatile("discard.global.L2 [%0], 128;" ::"l"(p) : "memory");
 }
 // One row of the forward state (128 * PPL contiguous bytes of scratch) -> shared memory as a single bulk-copy (TMA)
 // transaction; completion is signalled on an mbarrier that the whole warp waits on, phase by phase.
@@ -182,60 +157,11 @@ __device__ __forceinline__ void decode_row_bits(const RowBits& r, int x0, typena
 // fields, so their minimum is OpenCV's "first strictly smaller candidate wins" however it is grouped.  The ALU pipe
 // (VIADDMNMX, VIMNMX3, LOP3: one warp instruction per 2 cycles and SM sub-partition) is what the scan saturates;
 // the FMA pipe (IMAD) runs beside it at the same rate (profiles/ubench/pipes.cu: 3.8 warp instructions per clock
-// and SM for a 1:1 mix against 1.9 for either alone).  DTFILL_STENCIL chooses how many of the additions are plain
-// IMADs whose results meet in a 3-input minimum:
-//   0: 1 IMAD + 6 VIADDMNMX                    (forward; backward 7 VIADDMNMX)
-//   1: 3 IMAD + 4 VIADDMNMX + 1 VIMNMX3        (backward 2 IMAD + 5 VIADDMNMX + 1 VIMNMX3)
-//   2: 5 IMAD + 2 VIADDMNMX + 2 VIMNMX3        (backward 4 IMAD + 3 VIADDMNMX + 2 VIMNMX3)
-//   3: 7 IMAD + 3 VIMNMX3                      (backward 6 IMAD + 1 VIADDMNMX + 3 VIMNMX3)
+// and SM for a 1:1 mix against 1.9 for either alone).  Three of the forward additions (two backward) are plain IMADs
+// whose results meet in a 3-input minimum; DESIGN.md §5 records the other splits that were measured.
 // ------------------------------------------------------------------------------------------------------
-#ifndef DTFILL_STENCIL
-#define DTFILL_STENCIL 1
-#endif
-#ifndef DTFILL_SPLITSCAN
-#define DTFILL_SPLITSCAN 1
-#endif
-#ifndef DTFILL_FAKE_SCRATCH_DIV
-#define DTFILL_FAKE_SCRATCH_DIV 1   // > 1: timing experiment only (part of the forward state is dropped: wrong results)
-#endif
-#ifndef DTFILL_L2POLICY
-#define DTFILL_L2POLICY 0       // 1: evict-last stores + evict-first read-back of the scratch; 2: and discard of consumed rows
-#endif
-#ifndef DTFILL_K2_TMA
-#define DTFILL_K2_TMA 1         // forward rows scratch -> shared memory: 1 = one cp.async.bulk (TMA) per row issued by an
-#endif                          // elected lane and signalled on an mbarrier; 0 = 16-byte cp.async per lane (LDGSTS)
-#ifndef DTFILL_FLUSH_LATE
-#define DTFILL_FLUSH_LATE 0     // where a step stores the depths gathered by the previous one: 0 at its start, 1 after the
-#endif                          // stencil, 2 after the scan (the gather's latency is then covered by the whole step)
-#ifndef DTFILL_K2_SMEMROW
-#define DTFILL_K2_SMEMROW 0     // 1 (PPL = 20 only): the row two steps back (y-2 / y+2) lives in shared memory in column
-#endif                          // order (a ring of two rows that doubles as the output transposition buffer) instead of
-                                // 24 registers; the neighbours' columns are then plain loads
-#ifndef DTFILL_K2_WARPS
-#define DTFILL_K2_WARPS (DTFILL_K2_SMEMROW ? 28 : 20)      // resident warps per SM the PPL = 20 instance is compiled for (register budget)
-#endif
-
-// row of a tile in shared memory, column order: lane l owns columns [l*PPL, (l+1)*PPL); v[] by 128-bit accesses
-// (80-byte lane stride: conflict-free per quarter warp), the two neighbouring columns by 32-bit loads
-template <int PPL>
-__device__ __forceinline__ void load_row_smem(Row<PPL>& r, const uint32_t* row, int lane, uint32_t init_key) {
-    const uint4* p = reinterpret_cast<const uint4*>(row + lane * PPL);
-#pragma unroll
-    for (int j = 0; j < PPL / 4; ++j) {
-        const uint4 q = p[j];
-        r.v[4 * j] = q.x; r.v[4 * j + 1] = q.y; r.v[4 * j + 2] = q.z; r.v[4 * j + 3] = q.w;
-    }
-    const uint32_t a = row[lane == 0 ? 0 : lane * PPL - 1], c = row[lane == 31 ? 0 : lane * PPL + PPL];
-    r.l1 = lane == 0 ? init_key : a;
-    r.r0 = lane == 31 ? init_key : c;
-    r.l2 = r.r1 = init_key;       // never read for the row two steps back
-}
-template <int PPL>
-__device__ __forceinline__ void store_row_smem(uint32_t* row, const Row<PPL>& r, int lane) {
-    uint4* p = reinterpret_cast<uint4*>(row + lane * PPL);
-#pragma unroll
-    for (int j = 0; j < PPL / 4; ++j) p[j] = make_uint4(r.v[4 * j], r.v[4 * j + 1], r.v[4 * j + 2], r.v[4 * j + 3]);
-}
+// Resident warps per SM the PPL = 20 instance is compiled for: its register budget (more warps spill).
+constexpr int K2_WARPS_PPL20 = 20;
 
 template <int PPL>
 __device__ __forceinline__ uint32_t stencil_fwd(const Row<PPL>& A /*row y-1*/, const Row<PPL>& Bq /*row y-2*/, int i, uint32_t one)
@@ -243,31 +169,11 @@ __device__ __forceinline__ uint32_t stencil_fwd(const Row<PPL>& A /*row y-1*/, c
     const uint32_t b0 = at(Bq, i - 1), b1 = at(Bq, i + 1);
     const uint32_t a0 = at(A, i - 2), a1 = at(A, i - 1), a2 = at(A, i), a3 = at(A, i + 1), a4 = at(A, i + 2);
     // OpenCV's order: (-2,-1) (-2,+1) (-1,-2) (-1,-1) (-1,0) (-1,+1) (-1,+2); orders 0,2,..,12 (even: see header)
-#if DTFILL_STENCIL == 0
-    uint32_t m = b0 * one + KC(3, 0);
-    m = __viaddmin_u32(b1, KC(3, 2), m);
-    m = __viaddmin_u32(a0, KC(3, 4), m);
-    m = __viaddmin_u32(a1, KC(2, 6), m);
-    m = __viaddmin_u32(a2, KC(1, 8), m);
-    m = __viaddmin_u32(a3, KC(2, 10), m);
-    m = __viaddmin_u32(a4, KC(3, 12), m);
-    return m;
-#elif DTFILL_STENCIL == 1
     const uint32_t m0 = __viaddmin_u32(b1, KC(3, 2), b0 * one + KC(3, 0));
     const uint32_t m1 = __viaddmin_u32(a1, KC(2, 6), a0 * one + KC(3, 4));
     uint32_t m2 = __viaddmin_u32(a3, KC(2, 10), a2 * one + KC(1, 8));
     m2 = __viaddmin_u32(a4, KC(3, 12), m2);
     return __vimin3_u32(m0, m1, m2);
-#elif DTFILL_STENCIL == 2
-    const uint32_t p = __vimin3_u32(b0 * one + KC(3, 0), b1 * one + KC(3, 2), a0 * one + KC(3, 4));
-    const uint32_t q = __viaddmin_u32(a1, KC(2, 6), a2 * one + KC(1, 8));
-    const uint32_t r = __viaddmin_u32(a3, KC(2, 10), a4 * one + KC(3, 12));
-    return __vimin3_u32(p, q, r);
-#else
-    const uint32_t p = __vimin3_u32(b0 * one + KC(3, 0), b1 * one + KC(3, 2), a0 * one + KC(3, 4));
-    const uint32_t q = __vimin3_u32(a1 * one + KC(2, 6), a2 * one + KC(1, 8), a3 * one + KC(2, 10));
-    return __vimin3_u32(p, q, a4 * one + KC(3, 12));
-#endif
 }
 
 template <int PPL>
@@ -277,50 +183,24 @@ __device__ __forceinline__ uint32_t stencil_bwd(uint32_t own /*forward key, orde
     const uint32_t b0 = at(Bq, i + 1), b1 = at(Bq, i - 1);
     const uint32_t a0 = at(A, i + 2), a1 = at(A, i + 1), a2 = at(A, i), a3 = at(A, i - 1), a4 = at(A, i - 2);
     // own value first, then (+2,+1) (+2,-1) (+1,+2) (+1,+1) (+1,0) (+1,-1) (+1,-2); orders 2,4,..,14
-#if DTFILL_STENCIL == 0
-    uint32_t m = own;
-    m = __viaddmin_u32(b0, KC(3, 2), m);
-    m = __viaddmin_u32(b1, KC(3, 4), m);
-    m = __viaddmin_u32(a0, KC(3, 6), m);
-    m = __viaddmin_u32(a1, KC(2, 8), m);
-    m = __viaddmin_u32(a2, KC(1, 10), m);
-    m = __viaddmin_u32(a3, KC(2, 12), m);
-    m = __viaddmin_u32(a4, KC(3, 14), m);
-    return m;
-#elif DTFILL_STENCIL == 1
     uint32_t m0 = __viaddmin_u32(b0, KC(3, 2), own);
     m0 = __viaddmin_u32(b1, KC(3, 4), m0);
     const uint32_t m1 = __viaddmin_u32(a1, KC(2, 8), a0 * one + KC(3, 6));
     uint32_t m2 = __viaddmin_u32(a3, KC(2, 12), a2 * one + KC(1, 10));
     m2 = __viaddmin_u32(a4, KC(3, 14), m2);
     return __vimin3_u32(m0, m1, m2);
-#elif DTFILL_STENCIL == 2
-    const uint32_t p = __vimin3_u32(own, b0 * one + KC(3, 2), b1 * one + KC(3, 4));
-    const uint32_t q = __viaddmin_u32(a1, KC(2, 8), a0 * one + KC(3, 6));
-    uint32_t r = __viaddmin_u32(a3, KC(2, 12), a2 * one + KC(1, 10));
-    r = __viaddmin_u32(a4, KC(3, 14), r);
-    return __vimin3_u32(p, q, r);
-#else
-    const uint32_t p = __vimin3_u32(own, b0 * one + KC(3, 2), b1 * one + KC(3, 4));
-    const uint32_t q = __vimin3_u32(a0 * one + KC(3, 6), a1 * one + KC(2, 8), a2 * one + KC(1, 10));
-    const uint32_t r = __viaddmin_u32(a4, KC(3, 14), a3 * one + KC(2, 12));
-    return __vimin3_u32(p, q, r);
-#endif
 }
 
 template <int PPL, bool PAD, bool WANT_LBL, bool VEC>
-__global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_WARPS : 32))) k2_chamfer(FrameParams fp, Workspace ws, float* __restrict__ out_depth,
+__global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? K2_WARPS_PPL20 : 32))) k2_chamfer(FrameParams fp, Workspace ws, float* __restrict__ out_depth,
                                                   float* __restrict__ out_dt, int32_t* __restrict__ out_lbl, int my_kind)
 {
     // Transposition buffer for the keys of an output row.  Keeping shared memory small matters: what is left of the
     // 228 KB is the L1 that serves the depth_list gather.
-    constexpr bool SB = DTFILL_K2_SMEMROW && PPL == 20;
-    __shared__ __align__(16) uint32_t stage_ring[(SB ? 2 : 1) * 32 * PPL];   // SB: rows y and y -/+ 1 of the tile, slot = y & 1
-    uint32_t* stage = stage_ring;
+    __shared__ __align__(16) uint32_t stage_smem[32 * PPL];
+    uint32_t* stage = stage_smem;
     __shared__ __align__(16) uint2 fwdbuf[16 * PPL];      // forward keys of the next row to scan, [j][lane]
-#if DTFILL_K2_TMA
     __shared__ __align__(8) uint64_t fwdbar;              // completion of the bulk copy into fwdbuf
-#endif
 
     const Task task = ws.tasks[blockIdx.x];      // slot-major: blockIdx = slot * B + frame, longest tasks first
     if (task.kind != my_kind && !(task.kind == TASK_NOSRC && my_kind == TASK_CHAMFER)) return;
@@ -352,9 +232,6 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
     constexpr int VW = (PPL % 4 == 0) ? 4 : 2;   // keys per scratch vector
     uint2* scr = reinterpret_cast<uint2*>(ws.scratch) + (long)task.scratch_off * 16;   // 32*PPL keys per row
 
-#if DTFILL_L2POLICY
-    const uint64_t pol_keep = l2_policy_evict_last(), pol_drop = l2_policy_evict_first();
-#endif
     Row<PPL> ra, rb;
     fill_row(ra, init_key);
     fill_row(rb, init_key);
@@ -380,9 +257,8 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
                 rank += s ? 1u : 0u;
             }
         }
-        // in-lane scan: T[x] = min(c[x], T[x-1] + 1); the left neighbour is OpenCV's last candidate (order 14)
-#if DTFILL_SPLITSCAN
-        // two independent half-lane chains (twice the instruction-level parallelism of one chain of PPL dependent
+        // in-lane scan: T[x] = min(c[x], T[x-1] + 1); the left neighbour is OpenCV's last candidate (order 14).
+        // Two independent half-lane chains (twice the instruction-level parallelism of one chain of PPL dependent
         // steps), joined afterwards: a value entering the second half from the first is one more "left" candidate
         // (order 1, loses ties against anything the second half holds itself)
         constexpr int HF = PPL / 2;
@@ -403,34 +279,14 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
             if (PAD && x0 + i >= W) t = init_key;
             Bq.v[i] = t;
         }
-#else
-        uint32_t u = c[0] & ORDCLR;
-        c[0] = u;
-#pragma unroll
-        for (int i = 1; i < PPL; ++i) {
-            u = __viaddmin_u32(u, KC(1, 14), c[i]) & ORDCLR;
-            c[i] = u;
-        }
-        const uint32_t cin = lane_carry<PPL, +1>(u, lane, clamp_dist);
-#pragma unroll
-        for (int i = 0; i < PPL; ++i) {
-            uint32_t t = __viaddmin_u32(cin, uint32_t(i + 1) << DSH, c[i]);   // order bit 0/1 stays (see header)
-            if (PAD && x0 + i >= W) t = init_key;
-            Bq.v[i] = t;
-        }
-#endif
         refresh_halo(Bq, lane, init_key);
         // forward state -> scratch, [vector j][lane] so that every store instruction is fully coalesced; the rows of
         // the upper halo are never read back (the backward pass ends at r0)
         if (y >= task.r0) {
             char* dst = reinterpret_cast<char*>(scr) + (long)(y - task.lo) * (128 * PPL) + lane * (4 * VW);
 #pragma unroll
-            for (int j = 0; j < PPL / VW / DTFILL_FAKE_SCRATCH_DIV; ++j) {
-#if DTFILL_L2POLICY
-                if (VW == 4) st_scratch_v4_hint(dst + j * 512, Bq.v[4 * j], Bq.v[4 * j + 1], Bq.v[4 * j + 2], Bq.v[4 * j + 3], pol_keep);
-#else
+            for (int j = 0; j < PPL / VW; ++j) {
                 if (VW == 4) st_scratch_v4(dst + j * 512, Bq.v[4 * j], Bq.v[4 * j + 1], Bq.v[4 * j + 2], Bq.v[4 * j + 3]);
-#endif
                 else st_scratch_v2(dst + j * 256, Bq.v[2 * j], Bq.v[2 * j + 1]);
             }
         }
@@ -438,41 +294,22 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
 
     // one copy of the step in the instruction stream (the unrolled step is ~13 KB of code); the two live rows
     // are rotated with register moves, which go to the otherwise idle FMA pipe
-    if (SB) {
-        store_row_smem<PPL>(stage_ring, ra, lane);
-        store_row_smem<PPL>(stage_ring + 32 * PPL, ra, lane);
-        __syncwarp();
-#pragma unroll 1
-        for (int y = task.fstart; y < task.hi; ++y) {
-            uint32_t* slot = stage_ring + (y & 1) * (32 * PPL);      // holds row y-2, receives row y
-            load_row_smem<PPL>(rb, slot, lane, init_key);
-            fwd_step(ra, rb, y);
-            __syncwarp();                                            // every lane has read its neighbours' columns of row y-2
-            store_row_smem<PPL>(slot, rb, lane);
-            ra = rb;
-        }
-        __syncwarp();
-    } else {
 #pragma unroll 1
     for (int y = task.fstart; y < task.hi; ++y) {
         fwd_step(ra, rb, y);
         const Row<PPL> t = ra; ra = rb; rb = t;
     }
-    }
 
     // ---------------- backward pass: rows hi-1 .. r0 ----------------
-    // The forward keys of row y-1 are copied scratch -> fwdbuf with cp.async (16 B, L2 only) while row y is being
-    // scanned: no registers, no exposed latency, no L1 pollution.  (The depth gather is NOT done with cp.async: 4-byte
-    // LDGSTS cost 8 LSU cycles each and 20-38 of them per row step saturate the LSU -- measured.)
+    // The forward keys of row y-1 are copied scratch -> fwdbuf while row y is being scanned: no registers, no exposed
+    // latency.  With 4-key vectors (PPL % 4 == 0) the row is one bulk copy (TMA) issued by lane 0 and signalled on an
+    // mbarrier; otherwise every lane copies its own keys with 8-byte cp.async.  (The depth gather is NOT done with
+    // cp.async: 4-byte LDGSTS cost 8 LSU cycles each and 20-38 of them per row step saturate the LSU -- measured.)
     fill_row(ra, init_key);
     fill_row(rb, init_key);
-    if (SB) {
-        store_row_smem<PPL>(stage_ring, ra, lane);
-        store_row_smem<PPL>(stage_ring + 32 * PPL, ra, lane);
-        __syncwarp();
-    }
     const float* dl = ws.dlist + fpx;
-    const uint64_t pol_dlist = l2_policy_keep();
+    // depth_list is the one buffer of the path that is read at random and more than once (21 MB per batch of 256 KITTI
+    // frames); K1b writes it and the gather below reads it with plain stores and loads
     const char* dlm1_bytes = reinterpret_cast<const char*>(dl - 1);       // depth_list[lbl - 1]
     // output addressing that does not depend on the row: which 4-pixel groups of the transposed row this lane
     // writes (inside [c0,c1)), and where
@@ -484,16 +321,11 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
         if (lc < 32 * PPL && col >= task.c0 && col < task.c1) okmask |= 1u << j;
     }
     const long colbase = fpx + task.clo + lane * 4;
-    const uint4* sread0 = reinterpret_cast<const uint4*>(&stage[lane * 4]);
-    uint2* swrite0 = reinterpret_cast<uint2*>(&stage[xl]);
+    const uint4* sread = reinterpret_cast<const uint4*>(&stage[lane * 4]);
+    uint2* swrite = reinterpret_cast<uint2*>(&stage[xl]);
     const uint32_t fwdbuf_lane = (uint32_t)__cvta_generic_to_shared(fwdbuf) + lane * (4 * VW);
 
-#if DTFILL_K2_TMA
-    constexpr bool TMA_ROWS = (VW == 4) && DTFILL_FAKE_SCRATCH_DIV == 1;
-#else
-    constexpr bool TMA_ROWS = false;
-#endif
-#if DTFILL_K2_TMA
+    constexpr bool TMA_ROWS = VW == 4;
     const uint32_t fwdbar_a = (uint32_t)__cvta_generic_to_shared(&fwdbar);
     const uint32_t fwdbuf_a = (uint32_t)__cvta_generic_to_shared(fwdbuf);
     if (TMA_ROWS) {
@@ -508,39 +340,27 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
     }
     uint32_t fwd_phase = 0;           // parity of the transaction being waited for
     bool fwd_inflight = false;        // the last issue_fwd_row started a transaction (warp-uniform)
-#endif
     auto issue_fwd_row = [&](int y) {            // group A(y)
         const bool have = y >= task.fstart && y >= task.lo;
-#if DTFILL_K2_TMA
-        if (TMA_ROWS) {
+        if constexpr (TMA_ROWS) {
             fwd_inflight = have;
             if (have && lane == 0)
                 bulk_row_to_smem(fwdbuf_a, reinterpret_cast<const char*>(scr) + (long)(y - task.lo) * (128 * PPL), 128 * PPL, fwdbar_a);
-            return;
-        }
-#endif
-        if (have) {
-            const char* src = reinterpret_cast<const char*>(scr) + (long)(y - task.lo) * (128 * PPL) + lane * (4 * VW);
+        } else {
+            if (have) {
+                const char* src = reinterpret_cast<const char*>(scr) + (long)(y - task.lo) * (128 * PPL) + lane * (4 * VW);
 #pragma unroll
-            for (int j = 0; j < PPL / VW / DTFILL_FAKE_SCRATCH_DIV; ++j) {
-#if DTFILL_L2POLICY
-                if (VW == 4) cp_async16_hint(fwdbuf_lane + j * 512, src + j * 512, pol_drop);
-#else
-                if (VW == 4) cp_async16_l2only(fwdbuf_lane + j * 512, src + j * 512);
-#endif
-                else cp_async8(fwdbuf_lane + j * 256, src + j * 256);
+                for (int j = 0; j < PPL / VW; ++j) cp_async8(fwdbuf_lane + j * 256, src + j * 256);
             }
+            cp_async_commit();
         }
-        cp_async_commit();
     };
     auto wait_fwd_row = [&]() {
-#if DTFILL_K2_TMA
-        if (TMA_ROWS) {
+        if constexpr (TMA_ROWS) {
             if (fwd_inflight) { mbar_wait(fwdbar_a, fwd_phase); fwd_phase ^= 1u; }
-            return;
+        } else {
+            cp_async_wait<0>();
         }
-#endif
-        cp_async_wait<0>();
     };
     // Depths gathered for an output row stay in registers across the loop back-edge and are stored at the start of
     // the next step: the gather's latency is covered by the row rotation, and nothing else is live meanwhile.
@@ -555,24 +375,16 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
     issue_fwd_row(task.hi - 1);
 
     auto bwd_step = [&](const Row<PPL>& A /*row y+1*/, Row<PPL>& Bq /*row y+2 in, row y out*/, int y) {
-        if (lane < PPL / DTFILL_FAKE_SCRATCH_DIV && y - 3 >= task.fstart)      // forward row three steps ahead -> L2 (one 128 B line per lane)
+        if (lane < PPL && y - 3 >= task.fstart)      // forward row three steps ahead -> L2 (one 128 B line per lane)
             asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(scr) +
                                                           (long)(y - 3 - task.lo) * (128 * PPL) + lane * 128));
-#if DTFILL_FLUSH_LATE == 0
         if (VEC && y + 1 >= task.r0 && y + 1 < task.r1) flush_depth_row(y + 1);     // gathered during the last step
-#endif
         wait_fwd_row();                              // A(y), the only transfer in flight, has landed
-#if DTFILL_L2POLICY >= 2
-        if (VW == 4 && lane < PPL && y >= task.fstart && y >= task.lo)     // row y of the scratch is dead: one 128 B line per lane
-            l2_discard_128(reinterpret_cast<const char*>(scr) + (long)(y - task.lo) * (128 * PPL) + lane * 128);
-#endif
         uint32_t c[PPL];
         if (y >= task.fstart) {
 #pragma unroll
             for (int j = 0; j < PPL / VW; ++j) {
-                if (DTFILL_FAKE_SCRATCH_DIV > 1 && j >= PPL / VW / DTFILL_FAKE_SCRATCH_DIV) {
-                    for (int e = 0; e < VW; ++e) c[VW * j + e] = init_key;
-                } else if (VW == 4) {
+                if (VW == 4) {
                     const uint4 f = reinterpret_cast<const uint4*>(fwdbuf)[j * 32 + lane];
                     c[4 * j] = f.x; c[4 * j + 1] = f.y; c[4 * j + 2] = f.z; c[4 * j + 3] = f.w;
                 } else {
@@ -586,14 +398,8 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
         }
 #pragma unroll
         for (int i = 0; i < PPL; ++i) c[i] = stencil_bwd<PPL>(c[i], A, Bq, i, fp.one) & ORDCLR;
-#if DTFILL_K2_TMA
         if (TMA_ROWS) __syncwarp();                  // every lane has read fwdbuf before the next bulk copy overwrites it
-#endif
         issue_fwd_row(y - 1);                        // A(y-1): fwdbuf has been consumed above
-#if DTFILL_FLUSH_LATE == 1
-        if (VEC && y + 1 >= task.r0 && y + 1 < task.r1) flush_depth_row(y + 1);     // gathered during the last step
-#endif
-#if DTFILL_SPLITSCAN
         constexpr int HF = PPL / 2;                  // chains over columns [HF, PPL) and [0, HF), both right to left
         uint32_t u = c[PPL - 1], u2 = c[HF - 1];
 #pragma unroll
@@ -611,43 +417,18 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
             if (PAD && x0 + i >= W) t = init_key;
             Bq.v[i] = t;
         }
-#else
-        uint32_t u = c[PPL - 1];
-#pragma unroll
-        for (int i = PPL - 2; i >= 0; --i) {
-            u = __viaddmin_u32(u, KC(1, 1), c[i]) & ORDCLR;              // right neighbour is compared last
-            c[i] = u;
-        }
-        const uint32_t cin = lane_carry<PPL, -1>(u, lane, clamp_dist);
-#pragma unroll
-        for (int i = 0; i < PPL; ++i) {
-            uint32_t t = __viaddmin_u32(cin, uint32_t(PPL - i) << DSH, c[i]);   // order bit 0/1 stays
-            if (PAD && x0 + i >= W) t = init_key;
-            Bq.v[i] = t;
-        }
-#endif
         refresh_halo(Bq, lane, init_key);
-#if DTFILL_FLUSH_LATE == 2
-        if (VEC && y + 1 >= task.r0 && y + 1 < task.r1) flush_depth_row(y + 1);     // gathered during the last step
-#endif
 
         // ---- output of row y: keys -> shared memory (transpose), then per lane 4 consecutive pixels per group:
         // dt / lbl stores and the gather depth_list[lbl-1] (tools.py:26).  In this layout neighbouring lanes ask
         // for neighbouring labels (consecutive ranks along a beam), so a gather instruction touches few lines.
-        const int slot_off = SB ? (y & 1) * (32 * PPL) : 0;     // SB: the row goes to its slot of the ring in any case
-        const uint4* sread = sread0 + slot_off / 4;
-        uint2* swrite = swrite0 + slot_off / 2;
-        stage = stage_ring + slot_off;
-        if (SB) {
-            store_row_smem<PPL>(stage, Bq, lane);
-            __syncwarp();
-        }
+        // `stage` is re-set every step although it never moves: with `stage_smem` used directly, ptxas orders a few
+        // instructions of every instance differently.  This form keeps the SASS that was tuned and measured.
+        stage = stage_smem;
         if (y >= task.r0 && y < task.r1) {
-            if (!SB) {
 #pragma unroll
-                for (int j = 0; j < PPL / 2; ++j) swrite[j] = make_uint2(Bq.v[2 * j], Bq.v[2 * j + 1]);
-                __syncwarp();
-            }
+            for (int j = 0; j < PPL / 2; ++j) swrite[j] = make_uint2(Bq.v[2 * j], Bq.v[2 * j + 1]);
+            __syncwarp();
             const long ro = (long)y * W;
             if (VEC) {
                 float* pdt = out_dt + colbase + ro;
@@ -666,9 +447,8 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
                         const uint32_t kk[4] = {k.x, k.y, k.z, k.w};
 #pragma unroll
                         for (int e = 0; e < 4; ++e) {
-                            uint32_t l = kk[e] & LMASK;                                      // >= 1 inside [c0,c1)
-                            if (DTFILL_FAKE_SCRATCH_DIV > 1) l = max(l, 1u);
-                            g[4 * j + e] = __float_as_uint(ld_keep_f32(dlm1_bytes + (uint64_t)l * fp.four, pol_dlist));
+                            const uint32_t l = kk[e] & LMASK;                                // >= 1 inside [c0,c1)
+                            g[4 * j + e] = __float_as_uint(*reinterpret_cast<const float*>(dlm1_bytes + (uint64_t)l * fp.four));
                         }
                     }
                 }
@@ -693,23 +473,14 @@ __global__ void __launch_bounds__(32, (PPL >= 38 ? 12 : (PPL >= 20 ? DTFILL_K2_W
                     }
                 }
             }
-            if (!SB) __syncwarp();                   // stage is free for the next row
+            __syncwarp();                            // stage is free for the next row
         }
     };
 
-    if (SB) {
-#pragma unroll 1
-        for (int y = task.hi - 1; y >= task.r0; --y) {
-            load_row_smem<PPL>(rb, stage_ring + (y & 1) * (32 * PPL), lane, init_key);      // row y+2
-            bwd_step(ra, rb, y);
-            ra = rb;
-        }
-    } else {
 #pragma unroll 1
     for (int y = task.hi - 1; y >= task.r0; --y) {
         bwd_step(ra, rb, y);
         const Row<PPL> t = ra; ra = rb; rb = t;
-    }
     }
     wait_fwd_row();
     if (VEC) flush_depth_row(task.r0);
