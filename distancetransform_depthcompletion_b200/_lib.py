@@ -18,7 +18,7 @@ LIB_PATH = os.environ.get("DTFILL_LIB") or os.path.join(_HERE, "libdtfill.so")
 E_ARG, E_CUDA, E_INDEX, E_NOMEM, E_DATA = -1, -2, -3, -4, -5
 METRICS_KITTI, METRICS_NYU = 0, 1
 METRIC_COLS = 9
-ABI_VERSION = 7          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
+ABI_VERSION = 8          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
 METRIC_NAMES = ("mse", "rmse", "mae", "irmse", "imae", "delta1", "delta2", "delta3", "count")
 
 _c_float_p = ctypes.POINTER(ctypes.c_float)
@@ -98,6 +98,7 @@ def load() -> ctypes.CDLL:
         L.dtfill_run_png_to_png.argtypes = [vp, vp, vp, ci, ci, ci, ci, ci, cf, cf, vp, i64, vp, ci, ctypes.POINTER(ci)]
         L.dtfill_debug_png_encode_host.argtypes = [vp, ci, ci, vp, ctypes.c_long]
         L.dtfill_debug_png_encode_host.restype = ctypes.c_long
+        L.dtfill_eval_png.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, cf, cf, vp, vp, ctypes.POINTER(ci)]
         L.dtfill_debug_depth_samples_host.argtypes = [vp, ctypes.c_long, vp]
         L.dtfill_debug_depth_samples_host.restype = ci
         L.dtfill_host_alloc.argtypes = [ctypes.POINTER(vp), ctypes.c_size_t]
@@ -111,7 +112,7 @@ def load() -> ctypes.CDLL:
                      "dtfill_run_eval_async", "dtfill_eval_totals", "dtfill_edt", "dtfill_set_sparse_upload",
                      "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo", "dtfill_png_decode",
                      "dtfill_run_png", "dtfill_debug_png_decode_host", "dtfill_png_encode", "dtfill_png_encode_depth",
-                     "dtfill_run_png_to_png"):
+                     "dtfill_run_png_to_png", "dtfill_eval_png"):
             getattr(L, name).restype = ci
         _lib = L
         return L
@@ -323,6 +324,25 @@ class Handle:
             _check(rc, "dtfill_run_png_to_png")
         res["files"] = _split_files(out, out_off)
         return res
+
+    def eval_png(self, lidar_data: np.ndarray, lidar_off: np.ndarray, gt_data: np.ndarray, gt_off: np.ndarray, H: int,
+                 W: int, src_thr: float, val_thr: float):
+        """B LiDAR and B ground-truth PNG files (each set packed as for png_decode) decoded, the LiDAR frames filled and
+        KITTI-mode metrics taken against the ground truth, all on the device -> (per_frame [B,9], sums [10]) float64,
+        bit-exact with Result.evaluate.  A decode failure raises ValueError naming the list and the frame; a frame
+        Distance_Transform rejects raises IndexError."""
+        lidar_data, lidar_off = _png_args(lidar_data, lidar_off)
+        gt_data, gt_off = _png_args(gt_data, gt_off)
+        B = lidar_off.size - 1
+        if gt_off.size - 1 != B:
+            raise ValueError(f"dtfill_eval_png: {B} LiDAR files but {gt_off.size - 1} ground-truth files")
+        per_frame = np.empty((B, METRIC_COLS), np.float64)
+        sums = np.empty(METRIC_COLS + 1, np.float64)
+        bad = ctypes.c_int(-1)
+        _check(self._L.dtfill_eval_png(self._h, _ptr(lidar_data), _ptr(lidar_off), _ptr(gt_data), _ptr(gt_off), B,
+                                       int(H), int(W), float(src_thr), float(val_thr), _ptr(per_frame), _ptr(sums),
+                                       ctypes.byref(bad)), "dtfill_eval_png")
+        return per_frame, sums
 
     def png_encode_device_async(self, in_ptr: int, is_float: bool, B: int, H: int, W: int, out_ptr: int,
                                 capacity: int, offsets_ptr: int):

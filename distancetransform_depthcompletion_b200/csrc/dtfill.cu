@@ -940,6 +940,32 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
     return 0;
 }
 
+// Per-frame metrics in numpy's own summation order (k4x_*): per-pixel terms of the valid pixels compacted in raster order,
+// then the pairwise tree of np.add.reduce; groups of frames share a scratch of at most ~4 GiB (a batch of 256 KITTI frames
+// with a float64 ground truth needs 3.5 GB: one group, every frame's tree in flight at once).  GT: the arithmetic type,
+// GS: the ground truth as stored.  Device pointers; enqueued on s.
+template <typename GT, int MODE, typename GS>
+int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, double* per_frame, cudaStream_t s) {
+    const size_t gsz = sizeof(GT);
+    const long maxl = npx / 64 + 2;
+    long G = (long)((1ull << 32) / ((size_t)4 * npx * gsz));
+    G = G < 1 ? 1 : (G > B ? B : G);
+    int rc;
+    if ((rc = ensure(h, h->mx_terms, (size_t)G * 4 * npx * gsz))) return rc;
+    if ((rc = ensure(h, h->mx_counts, (size_t)G * 4 * 4))) return rc;
+    if ((rc = ensure(h, h->mx_leaf_start, (size_t)G * maxl * 4))) return rc;
+    if ((rc = ensure(h, h->mx_leaf_sum, (size_t)G * 4 * maxl * gsz))) return rc;
+    for (long g0 = 0; g0 < B; g0 += G) {
+        const int ng = (int)(B - g0 < G ? B - g0 : G);
+        GT* tm = (GT*)h->mx_terms.p;
+        int* cn = (int*)h->mx_counts.p;
+        k4x_compact<GT, MODE, GS><<<ng, K4X_THREADS, 0, s>>>(pred + g0 * npx, gt + g0 * npx, npx, tm, cn);
+        k4x_reduce<GT><<<ng, K4X_RTHREADS, 0, s>>>(tm, cn, npx, MODE, (int*)h->mx_leaf_start.p, (GT*)h->mx_leaf_sum.p,
+                                                   per_frame + g0 * 9);
+    }
+    return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1315,32 +1341,57 @@ int png_verdict(const int32_t* st, int B, int* first_bad_frame) {
     return 0;
 }
 
+// One set of host files: file b = data[offsets[b], offsets[b+1]), b < B.
+struct PngFiles { const uint8_t* data; const int64_t* offsets; int B; };
+
+// Stage sets of host files into the pinned buffer, back to back in the order given (bytes, then the offsets of all of
+// them rebased to 0), and enqueue one copy of it to the device.  The caller waits for the call before the buffer is used
+// again.
+int png_stage(dtfill_t* h, const PngFiles* sets, int nsets, const uint8_t** d_data, const int64_t** d_off) {
+    int rc;
+    size_t nbytes = 0;
+    int nfiles = 0;
+    for (int k = 0; k < nsets; ++k) {
+        const PngFiles& f = sets[k];
+        if (f.offsets[0] < 0) return fail(DTFILL_E_ARG, "dtfill_png_decode: offsets[0] < 0");
+        for (int b = 0; b < f.B; ++b)
+            if (f.offsets[b + 1] < f.offsets[b]) return fail(DTFILL_E_ARG, "dtfill_png_decode: offsets decrease at file " + std::to_string(b));
+        nbytes += (size_t)(f.offsets[f.B] - f.offsets[0]);
+        nfiles += f.B;
+    }
+    const size_t off_at = (nbytes + 15) & ~(size_t)15;
+    const size_t total = off_at + (size_t)(nfiles + 1) * 8;
+    if ((rc = ensure_pinned(h->pin_png, total))) return rc;
+    if ((rc = ensure(h, h->png_data, total))) return rc;
+    uint8_t* pin = (uint8_t*)h->pin_png.p;
+    int64_t* po = (int64_t*)(pin + off_at);
+    int64_t pos = 0;
+    int i = 0;
+    for (int k = 0; k < nsets; ++k) {
+        const PngFiles& f = sets[k];
+        const int64_t o0 = f.offsets[0];
+        memcpy(pin + pos, f.data + o0, (size_t)(f.offsets[f.B] - o0));
+        for (int b = 0; b < f.B; ++b) po[i++] = pos + f.offsets[b] - o0;
+        pos += f.offsets[f.B] - o0;
+    }
+    po[i] = pos;
+    CU(cudaMemcpyAsync(h->png_data.p, pin, total, cudaMemcpyHostToDevice, h->stream));
+    h->last_h2d_bytes = total;
+    *d_data = (const uint8_t*)h->png_data.p;
+    *d_off = (const int64_t*)((uint8_t*)h->png_data.p + off_at);
+    return 0;
+}
+
 // Enqueue the decode of B files on the handle's stream: samples into out_dev [B,H,W], status into status_dev [B].  Host
-// files go up in one copy through a pinned staging buffer (bytes, then the offsets rebased to 0); the caller waits for
-// the call before the buffer is used again.
+// files go up in one copy through the pinned staging buffer (png_stage).
 int png_enqueue(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H, int W,
                 uint16_t* out_dev, int32_t* status_dev) {
     int rc;
     const uint8_t* d_data = data;
     const int64_t* d_off = offsets;
     if (!in_is_device) {
-        const int64_t o0 = offsets[0];
-        if (o0 < 0) return fail(DTFILL_E_ARG, "dtfill_png_decode: offsets[0] < 0");
-        for (int b = 0; b < B; ++b)
-            if (offsets[b + 1] < offsets[b]) return fail(DTFILL_E_ARG, "dtfill_png_decode: offsets decrease at file " + std::to_string(b));
-        const size_t nbytes = (size_t)(offsets[B] - o0);
-        const size_t off_at = (nbytes + 15) & ~(size_t)15;
-        const size_t total = off_at + (size_t)(B + 1) * 8;
-        if ((rc = ensure_pinned(h->pin_png, total))) return rc;
-        if ((rc = ensure(h, h->png_data, total))) return rc;
-        uint8_t* pin = (uint8_t*)h->pin_png.p;
-        memcpy(pin, data + o0, nbytes);
-        int64_t* po = (int64_t*)(pin + off_at);
-        for (int b = 0; b <= B; ++b) po[b] = offsets[b] - o0;
-        CU(cudaMemcpyAsync(h->png_data.p, pin, total, cudaMemcpyHostToDevice, h->stream));
-        h->last_h2d_bytes = total;
-        d_data = (const uint8_t*)h->png_data.p;
-        d_off = (const int64_t*)((uint8_t*)h->png_data.p + off_at);
+        const PngFiles set{data, offsets, B};
+        if ((rc = png_stage(h, &set, 1, &d_data, &d_off))) return rc;
     }
     const size_t fbytes = (size_t)H * (1 + 2 * (size_t)W);
     if ((rc = ensure(h, h->png_scratch, (size_t)B * fbytes))) return rc;
@@ -1789,36 +1840,13 @@ int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_
     double* pf_d = (out_is_device && per_frame) ? per_frame : (double*)h->per_frame.p;
     double* sm_d = (out_is_device && sums) ? sums : (double*)h->sums.p;
     if (h->metrics_exact && npx < (1l << 31)) {
-        // numpy's own summation order (k4x_*): per-pixel terms of the valid pixels compacted in raster order, then the
-        // pairwise tree of np.add.reduce; groups of frames share a scratch of at most ~4 GiB (a batch of 256 KITTI frames
-        // with a float64 ground truth needs 3.5 GB: one group, every frame's tree in flight at once)
-        const long maxl = npx / 64 + 2;
-        long G = (long)((1ull << 32) / ((size_t)4 * npx * gsz));
-        G = G < 1 ? 1 : (G > B ? B : G);
-        if ((rc = ensure(h, h->mx_terms, (size_t)G * 4 * npx * gsz))) return rc;
-        if ((rc = ensure(h, h->mx_counts, (size_t)G * 4 * 4))) return rc;
-        if ((rc = ensure(h, h->mx_leaf_start, (size_t)G * maxl * 4))) return rc;
-        if ((rc = ensure(h, h->mx_leaf_sum, (size_t)G * 4 * maxl * gsz))) return rc;
-        for (long g0 = 0; g0 < B; g0 += G) {
-            const int ng = (int)(B - g0 < G ? B - g0 : G);
-            const float* pg = p_d + g0 * npx;
-            int* cn = (int*)h->mx_counts.p;
-            int* lst = (int*)h->mx_leaf_start.p;
-            double* pfg = pf_d + g0 * 9;
-            if (gt_is_f64) {
-                const double* gg = (const double*)g_d + g0 * npx;
-                double* tm = (double*)h->mx_terms.p;
-                if (mode == 0) k4x_compact<double, 0><<<ng, K4X_THREADS, 0, s>>>(pg, gg, npx, tm, cn);
-                else k4x_compact<double, 1><<<ng, K4X_THREADS, 0, s>>>(pg, gg, npx, tm, cn);
-                k4x_reduce<double><<<ng, K4X_RTHREADS, 0, s>>>(tm, cn, npx, mode, lst, (double*)h->mx_leaf_sum.p, pfg);
-            } else {
-                const float* gg = (const float*)g_d + g0 * npx;
-                float* tm = (float*)h->mx_terms.p;
-                if (mode == 0) k4x_compact<float, 0><<<ng, K4X_THREADS, 0, s>>>(pg, gg, npx, tm, cn);
-                else k4x_compact<float, 1><<<ng, K4X_THREADS, 0, s>>>(pg, gg, npx, tm, cn);
-                k4x_reduce<float><<<ng, K4X_RTHREADS, 0, s>>>(tm, cn, npx, mode, lst, (float*)h->mx_leaf_sum.p, pfg);
-            }
-        }
+        const double* g64 = (const double*)g_d;
+        const float* g32 = (const float*)g_d;
+        if (gt_is_f64)
+            rc = mode == 0 ? k4x_enqueue<double, 0>(h, p_d, g64, B, npx, pf_d, s) : k4x_enqueue<double, 1>(h, p_d, g64, B, npx, pf_d, s);
+        else
+            rc = mode == 0 ? k4x_enqueue<float, 0>(h, p_d, g32, B, npx, pf_d, s) : k4x_enqueue<float, 1>(h, p_d, g32, B, npx, pf_d, s);
+        if (rc) return rc;
         k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, accumulate);
     } else {
     int chunks = (int)((npx + 16383) / 16384);     // chunk boundaries stay multiples of 4 pixels when npx is
@@ -1842,6 +1870,91 @@ int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_
         if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
         if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
         CU(cudaStreamSynchronize(s));
+    }
+    return 0;
+}
+
+int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets, const uint8_t* gt,
+                    const int64_t* gt_offsets, int B, int H, int W, float src_thr, float val_thr, double* per_frame,
+                    double* sums, int* first_bad_frame) {
+    if (first_bad_frame) *first_bad_frame = -1;
+    if (!h || !lidar || !lidar_offsets || !gt || !gt_offsets)
+        return fail(DTFILL_E_ARG, "dtfill_eval_png: NULL handle, files or offsets");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_eval_png: B, H, W must be positive");
+    if ((int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28))
+        return fail(DTFILL_E_ARG, "dtfill_eval_png: frame too large (H * (1 + 2 W) < 2^28 bytes)");
+    CU(cudaSetDevice(h->device));
+    const long npx = (long)H * W;
+    cudaStream_t s = h->stream;
+    int rc;
+    // 1. one decode of the 2B files (one warp per file, so the call costs about the slowest file, not two files in a row):
+    //    LiDAR file b -> samples / status b, ground-truth file b -> samples / status B + b
+    if ((rc = ensure(h, h->png_samples, (size_t)2 * B * npx * 2))) return rc;
+    if ((rc = ensure(h, h->png_status, (size_t)2 * B * 4))) return rc;
+    int32_t* st_host = nullptr;                   // [2B] decode status, then the fill's counts [B][2]
+    if ((rc = png_status_host(h, 4 * B, &st_host))) return rc;
+    uint16_t* samples = (uint16_t*)h->png_samples.p;
+    int32_t* status = (int32_t*)h->png_status.p;
+    const PngFiles sets[2] = {{lidar, lidar_offsets, B}, {gt, gt_offsets, B}};
+    const uint8_t* d_data;
+    const int64_t* d_off;
+    if ((rc = png_stage(h, sets, 2, &d_data, &d_off))) return rc;
+    const size_t h2d = h->last_h2d_bytes;
+    if ((rc = png_enqueue(h, d_data, d_off, 1, 2 * B, H, W, samples, status))) return rc;
+    // 2. the fill of dtfill_run_u16 (no crop) on the LiDAR samples, strict order on the handle's stream; only the counts
+    //    leave the device
+    if ((rc = ensure(h, h->depth_dev, (size_t)B * npx * 4))) return rc;
+    if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc;
+    float* depth = (float*)h->depth_dev.p;
+    int32_t* counts = (int32_t*)h->counts_out_dev.p;
+    {
+        InputScope scope(h, true, H, 0, nullptr);
+        if ((rc = enqueue(h, samples, B, H, W, src_thr, val_thr, depth, nullptr, nullptr, nullptr, counts, nullptr, true)))
+            return rc;
+    }
+    // 3. Result.evaluate of the filled depth against the ground-truth samples, in numpy's summation order whatever
+    //    dtfill_set_metrics_exact says
+    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
+    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
+    double* pf_d = (double*)h->per_frame.p;
+    double* sm_d = (double*)h->sums.p;
+    if ((rc = k4x_enqueue<double, 0>(h, depth, samples + (size_t)B * npx, B, npx, pf_d, s))) return rc;
+    k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(st_host, status, (size_t)2 * B * 4, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(st_host + 2 * B, counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
+    if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
+    if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
+    int fill_bad = -1;
+    rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
+    h->last_h2d_bytes = h2d;
+    h->last_d2h_bytes = (size_t)B * (2 * 4 + 8 + (per_frame ? 9 * 8 : 0)) + (sums ? 10 * 8 : 0);
+    if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
+    // 4. the verdict, frame by frame as the notebook's loop meets it: a decode failure (LiDAR before ground truth) wins
+    //    over an IndexError of Distance_Transform
+    for (int b = 0; b < B; ++b) {
+        const bool lid_bad = st_host[b] != png::ST_OK;
+        if (lid_bad || st_host[B + b] != png::ST_OK) {
+            const int st = lid_bad ? st_host[b] : st_host[B + b];
+            if (first_bad_frame) *first_bad_frame = b;
+            return fail(DTFILL_E_DATA, std::string(lid_bad ? "LiDAR" : "ground-truth") + " file " + std::to_string(b) + ": " +
+                                           png_reason(st) + " (status " + std::to_string(st) + ")");
+        }
+    }
+    const int32_t* cnt = st_host + 2 * B;
+    const int lim = rc == DTFILL_E_INDEX ? fill_bad : B;
+    for (int b = 0; b < lim; ++b)
+        if (cnt[2 * b + 1] == 1) {
+            // eval_NYU.py:126 np.squeeze(lidar[with_value]) makes a single valid depth 0-dimensional; :128 then fails
+            if (first_bad_frame) *first_bad_frame = b;
+            return fail(DTFILL_E_INDEX, "LiDAR file " + std::to_string(b) +
+                                            ": one valid depth (numpy IndexError: too many indices for array: array is "
+                                            "0-dimensional, but 1 were indexed)");
+        }
+    if (rc == DTFILL_E_INDEX) {
+        if (first_bad_frame) *first_bad_frame = fill_bad;
+        return fail(DTFILL_E_INDEX, "LiDAR file " + std::to_string(fill_bad) +
+                                        ": labels index outside the list of valid depths (numpy IndexError)");
     }
     return 0;
 }

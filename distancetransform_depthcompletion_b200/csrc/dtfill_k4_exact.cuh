@@ -1,5 +1,7 @@
 // dtfill_k4_exact.cuh -- K4x: evaluation.py:82-123, 196-239 with numpy's own summation order
 #pragma once
+#include <type_traits>
+
 #include "dtfill_k4_metrics.cuh"
 
 namespace dtfill {
@@ -16,7 +18,8 @@ namespace dtfill {
 // (numpy/_core/src/umath/loops_utils.h.src; pinned by tests/test_host_logic.py against np.add.reduce).  The kernels below
 // reproduce exactly that tree, so the metrics are the reference's bit for bit -- the fixed-order float64 sums of
 // k4_metrics_partial agree with numpy's float32 pairwise sums only to ~1e-5.
-//   k4x_compact  one block per frame: the terms of the valid pixels, compacted in raster order (ballots + warp ranks)
+//   k4x_compact  one block per frame: the terms of the valid pixels, compacted in raster order (ballots + warp ranks);
+//                the ground truth is stored as the arithmetic type or, in KITTI mode, as 16-bit PNG samples
 //   k4x_reduce   one block per frame: the leaves (<= 128 elements) of the tree in parallel, then the tree itself
 // Terms: 0 |d|^2, 1 |d| (KITTI) or |d| / t (NYU), 2 |dinv|^2, 3 |dinv|; counts: valid, delta1..3.
 // ------------------------------------------------------------------------------------------------------
@@ -59,8 +62,21 @@ __device__ __forceinline__ bool metric_terms(float o, GT t, GT* term, int* hit)
     return true;
 }
 
-template <typename GT, int MODE>
-__global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restrict__ pred, const GT* __restrict__ gt, long npx,
+// The ground truth as stored (GS) -> its value in the arithmetic type (GT): the identity, or, for the samples of a KITTI
+// 16-bit depth PNG, data_read.py:223 `png / 256.` in float64 -- exact, so a ground truth read from its files costs 2 B/px
+// and no float64 copy of it exists
+template <typename GT, typename GS>
+__device__ __forceinline__ GT gt_value(GS s)
+{
+    if constexpr (std::is_same<GT, GS>::value) return s;
+    else {
+        static_assert(std::is_same<GT, double>::value && std::is_same<GS, uint16_t>::value, "u16 samples are read as float64");
+        return (double)s * (1.0 / 256);
+    }
+}
+
+template <typename GT, int MODE, typename GS = GT>
+__global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restrict__ pred, const GS* __restrict__ gt, long npx,
                                                             GT* __restrict__ terms /*[frames][4][npx]*/,
                                                             int* __restrict__ counts /*[frames][4]*/)
 {
@@ -68,7 +84,7 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
     __shared__ int hits[3];
     const int b = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const float* p = pred + (long)b * npx;
-    const GT* g = gt + (long)b * npx;
+    const GS* g = gt + (long)b * npx;
     GT* tb = terms + (long)b * 4 * npx;
     const long seg = ((npx + K4X_THREADS - 1) / K4X_THREADS) * 32;     // pixels per warp, a multiple of 32
     const long i0 = min(npx, wid * seg), i1 = min(npx, i0 + seg);
@@ -77,7 +93,7 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
     int cnt = 0;
     for (long c = i0; c < i1; c += 32) {
         const long i = c + lane;
-        const bool v = i < i1 && (p[i] > 0.01f) && (g[i] > (GT)0.01);
+        const bool v = i < i1 && (p[i] > 0.01f) && (gt_value<GT>(g[i]) > (GT)0.01);     // u16: s >= 3
         cnt += __popc(__ballot_sync(0xffffffffu, v));
     }
     if (lane == 0) wtot[wid] = cnt;
@@ -98,7 +114,7 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
         const long i = c + lane;
         GT term[4] = {0, 0, 0, 0};
         int hit[3] = {0, 0, 0};
-        const bool v = i < i1 && metric_terms<GT, MODE>(p[i], g[i], term, hit);
+        const bool v = i < i1 && metric_terms<GT, MODE>(p[i], gt_value<GT>(g[i]), term, hit);
         const uint32_t m = __ballot_sync(0xffffffffu, v);
         if (v) {
             const long k = run + __popc(m & lanemask_lt());

@@ -5,6 +5,8 @@
 
 ``evaluate`` sets the same attributes as the reference and returns None.  ``evaluate_batch`` is the batched form
 the eval loops (eval.py:212-232, eval_NYU.py:207-229) reduce to: per-frame metrics and their running sums.
+``evaluate_fill_png_files`` runs the KITTI ablation notebook's loop (PNG files -> Distance_Transform -> Result.evaluate)
+from the files, decoding, filling and evaluating on the GPU.
 """
 from __future__ import annotations
 
@@ -31,6 +33,42 @@ def evaluate_batch(output, target, mode: int, device: int | None = None):
     B = output.shape[0]
     n = int(np.prod(output.shape[1:]))
     return _lib.get_handle(device).metrics(output, target, B, 1, n, mode, target.dtype == np.float64)
+
+
+def evaluate_fill_png_files(lidar_files, gt_files, src_thr: float = 0.1, device: int | None = None):
+    """The evaluation loop of the KITTI ablation notebook (SURVEY.md section 3 C), from the PNG files, in one call:
+
+        for i in range(B):
+            lidar = np.array(Image.open(lidar_files[i])).astype(np.float32) / 256    data_read.py:215
+            gt = np.array(Image.open(gt_files[i])) / 256.                            data_read.py:223 (float64)
+            pred = Distance_Transform(lidar, src_thr)                                 eval_NYU.py:120-133
+            result.evaluate(pred, gt)                                                 evaluation.py:82-123
+
+    lidar_files, gt_files: paths or the files' bytes, 16-bit grayscale PNGs all of the size of the first LiDAR file,
+    evaluated at that size (no crop).  Returns (per_frame float64 [B,9], sums float64 [10]) in the layout of
+    evaluate_batch: row b is [mse, rmse, mae, irmse, imae, 0, 0, 0, n_valid] of frame b, equal to Result.evaluate's bit for
+    bit (a frame whose ground truth has no valid pixel gives numpy's mean of an empty array), and sums holds the column
+    sums followed by B, ready for sharding.finalize_means.  The files are decoded, filled and evaluated on the GPU; only the
+    files go up and only the metrics come back.
+
+    Raises ValueError for lists of different lengths or empty lists, and for the first frame with a file that is not an
+    intact 16-bit grayscale PNG of that size (naming the LiDAR or the ground-truth list and the frame; the LiDAR file wins
+    at the same frame).  Otherwise raises IndexError for the first frame Distance_Transform rejects (no valid depth,
+    exactly one valid depth, labels outside the list of valid depths)."""
+    from .data_read import pack_png_files
+    from .tools import VALID_THR
+    lidar_files, gt_files = list(lidar_files), list(gt_files)
+    if not lidar_files or not gt_files:
+        raise ValueError("evaluate_fill_png_files: no files")
+    if len(lidar_files) != len(gt_files):
+        raise ValueError(f"evaluate_fill_png_files: {len(lidar_files)} LiDAR files but {len(gt_files)} ground-truth files")
+    B = len(lidar_files)
+    # one buffer for both lists; the size comes from the first LiDAR file's IHDR
+    try:
+        data, offsets, H, W = pack_png_files(lidar_files + gt_files)
+    except ValueError:
+        raise ValueError("evaluate_fill_png_files: LiDAR file 0 is not a PNG file") from None
+    return _lib.get_handle(device).eval_png(data, offsets[:B + 1], data, offsets[B:], H, W, src_thr, VALID_THR)
 
 
 class _ResultBase(object):

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DTFILL_ABI_VERSION 7      /* 7: PNG encode (dtfill_png_encode, dtfill_png_encode_depth, dtfill_run_png_to_png); 6: PNG decode (dtfill_png_decode, dtfill_run_png, DTFILL_E_DATA); 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
+#define DTFILL_ABI_VERSION 8      /* 8: dtfill_eval_png; 7: PNG encode (dtfill_png_encode, dtfill_png_encode_depth, dtfill_run_png_to_png); 6: PNG decode (dtfill_png_decode, dtfill_run_png, DTFILL_E_DATA); 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
 
 enum {
     DTFILL_OK = 0,
@@ -212,6 +212,25 @@ int dtfill_set_metrics_exact(dtfill_t* h, int enabled);
 int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_f64, int in_is_device,
                       int B, int H, int W, int mode, double* per_frame, double* sums, int out_is_device,
                       int accumulate);
+
+/*
+ * The evaluation loop of the reference's KITTI ablation notebook, from the files (SURVEY.md section 3 C):
+ *     lidar = png.astype(float32) / 256        data_read.py:215
+ *     gt    = png / 256.  (float64)            data_read.py:223
+ *     Result().evaluate(Distance_Transform(lidar, src_thr), gt)
+ * for B pairs of 16-bit grayscale PNG files of H x W (no crop), host files laid out as for dtfill_png_decode.  The 2B
+ * files are decoded in one launch, the LiDAR frames filled as by dtfill_run_u16, and the metrics computed against the
+ * ground-truth samples in KITTI mode and numpy's summation order (whatever dtfill_set_metrics_exact says), so that
+ * per_frame [B][DTFILL_METRIC_COLS] and sums [DTFILL_METRIC_COLS + 1] (host, nullable; layout of dtfill_metrics) equal
+ * the reference's bit for bit.  No per-pixel data crosses the link.  Synchronous.
+ * Errors, frame by frame as the loop meets them: DTFILL_E_DATA for the first frame with a file that fails to decode
+ * (LiDAR before ground truth at the same frame), which wins over DTFILL_E_INDEX for the first LiDAR frame
+ * Distance_Transform rejects (no valid depth, exactly one valid depth, labels outside the list of valid depths);
+ * *first_bad_frame receives the frame.  On an error the contents of per_frame and sums are unspecified.
+ */
+int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets, const uint8_t* gt,
+                    const int64_t* gt_offsets, int B, int H, int W, float src_thr, float val_thr, double* per_frame,
+                    double* sums, int* first_bad_frame);
 
 /*
  * One step of an evaluation sweep, fused (BASELINE.json configs[4]; the loop body of eval.py:212-232: DT_complete_batch,
