@@ -7,7 +7,8 @@ namespace dtfill {
 // ------------------------------------------------------------------------------------------------------
 // K6: KITTI outlier filter, data_read.py:103-128 (SURVEY.md 8 f-2): sum and count over the 7 x 7 diamond
 // (cv2.filter2D, default border BORDER_REFLECT_101), average = sum / (count + 1e-5) in float64 (the reference's
-// valid_pixels array is float64), a point more than 1.0 m FARTHER than the local average is dropped.
+// valid_pixels array is float64), a point more than 1.0 m FARTHER than the local average is dropped.  A dropped depth
+// becomes a zero of its own sign: x * (1 - 1) in float64 (:128) gives -0.0 for a negative x.
 // ------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int reflect101(int i, int n) {
     if (n == 1) return 0;
@@ -41,6 +42,7 @@ __device__ __forceinline__ bool k6_verdict(const float* __restrict__ frame, int 
 __device__ __noinline__ bool k6_verdict_border(const float* __restrict__ frame, int H, int W, int y, int x_, float x) {
     return k6_verdict<true>(frame, H, W, y, x_, x);
 }
+__device__ __forceinline__ float k6_dropped(float x) { return __uint_as_float(__float_as_uint(x) & 0x80000000u); }
 __device__ __forceinline__ bool k6_is_outlier(const float* __restrict__ frame, int H, int W, int y, int x_, float x) {
     if (y >= 3 && y < H - 3 && x_ >= 3 && x_ < W - 3) return k6_verdict<false>(frame, H, W, y, x_, x);
     return k6_verdict_border(frame, H, W, y, x_, x);
@@ -99,10 +101,10 @@ __global__ void __launch_bounds__(256) k6_outlier_removal(const float* __restric
             d3 |= __reduce_or_sync(0xffffffffu, e == 3 ? bit : 0u);
         }
         if (!live) return;
-        if ((d0 >> lane) & 1u) v.x = 0.0f;
-        if ((d1 >> lane) & 1u) v.y = 0.0f;
-        if ((d2 >> lane) & 1u) v.z = 0.0f;
-        if ((d3 >> lane) & 1u) v.w = 0.0f;
+        if ((d0 >> lane) & 1u) v.x = k6_dropped(v.x);
+        if ((d1 >> lane) & 1u) v.y = k6_dropped(v.y);
+        if ((d2 >> lane) & 1u) v.z = k6_dropped(v.z);
+        if ((d3 >> lane) & 1u) v.w = k6_dropped(v.w);
         st_stream_v4(out + g * 4, __float_as_uint(v.x), __float_as_uint(v.y), __float_as_uint(v.z), __float_as_uint(v.w));
     } else {
         if (g >= ngroups) return;
@@ -111,7 +113,7 @@ __global__ void __launch_bounds__(256) k6_outlier_removal(const float* __restric
         const long frame = row / H;
         const int y = (int)(row - frame * H);
         const float x = in[g];
-        out[g] = ((__float_as_uint(x) << 1) != 0u && k6_is_outlier(in + frame * H * W, H, W, y, x0, x)) ? 0.0f : x;
+        out[g] = ((__float_as_uint(x) << 1) != 0u && k6_is_outlier(in + frame * H * W, H, W, y, x0, x)) ? k6_dropped(x) : x;
     }
 }
 

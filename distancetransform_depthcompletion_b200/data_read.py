@@ -18,7 +18,8 @@ from . import _lib
 
 def outlier_removal(lidar, device: int | None = None):
     """data_read.py:103-128: zero every depth that is more than 1.0 m farther than the average of the valid depths
-    inside its 7 x 7 diamond.  Any shape that squeezes to [H,W]; returns float32 [H,W]."""
+    inside its 7 x 7 diamond.  A dropped depth becomes a zero of its own sign, as the reference's float64
+    ``x * (1 - 1)`` gives (-0.0 for a negative depth).  Any shape that squeezes to [H,W]; returns float32 [H,W]."""
     sparse_lidar = np.squeeze(np.asarray(lidar))                              # :114
     if sparse_lidar.ndim != 2:
         raise ValueError(f"outlier_removal: input must squeeze to 2-D, got {np.shape(lidar)}")

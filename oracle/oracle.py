@@ -294,19 +294,51 @@ def demo_generate_multi_channel(lidar_data: np.ndarray, table_size: int = 11, sc
 # ---------------------------------------------------------------------------------------------------------
 # KITTI outlier filter (SURVEY.md section 8 f-2): data_read.py:103-128 with the real cv2.filter2D.
 # ---------------------------------------------------------------------------------------------------------
-def cv2_port_outlier_removal(lidar):
-    """data_read.py:103-128 line by line (np.float, removed from numpy, is spelled float64 = what it aliased)."""
+DIAMOND_KERNEL_7 = np.asarray([[0, 0, 0, 1, 0, 0, 0], [0, 0, 1, 1, 1, 0, 0], [0, 1, 1, 1, 1, 1, 0],
+                               [1, 1, 1, 1, 1, 1, 1], [0, 1, 1, 1, 1, 1, 0], [0, 0, 1, 1, 1, 0, 0],
+                               [0, 0, 0, 1, 0, 0, 0]], dtype=np.uint8)                          # data_read.py:104-113
+
+
+def cv2_port_outlier_removal(lidar, squeeze: bool = True):
+    """data_read.py:103-128 line by line (np.float, removed from numpy, is spelled float64 = what it aliased).
+    ``squeeze=False`` takes a 2-D frame as given: the reference squeezes a 1 x W or H x 1 frame to 1-D, which cv2
+    reads as a column and the lines after it then broadcast to W x W."""
     import cv2
-    DIAMOND_KERNEL_7 = np.asarray([[0, 0, 0, 1, 0, 0, 0], [0, 0, 1, 1, 1, 0, 0], [0, 1, 1, 1, 1, 1, 0],
-                                   [1, 1, 1, 1, 1, 1, 1], [0, 1, 1, 1, 1, 1, 0], [0, 0, 1, 1, 1, 0, 0],
-                                   [0, 0, 0, 1, 0, 0, 0]], dtype=np.uint8)                      # :104-113
-    sparse_lidar = np.squeeze(lidar)                                                            # :115
+    sparse_lidar = np.squeeze(lidar) if squeeze else np.asarray(lidar)                         # :115
     valid_pixels = (sparse_lidar > 0.1).astype(np.float64)                                      # :116
     lidar_sum = cv2.filter2D(sparse_lidar, -1, DIAMOND_KERNEL_7)                                # :119
     lidar_count = cv2.filter2D(valid_pixels, -1, DIAMOND_KERNEL_7)                              # :121
     lidar_aveg = lidar_sum / (lidar_count + 0.00001)                                            # :123
     potential_outliers = ((sparse_lidar - lidar_aveg) > 1.0).astype(np.float64)                 # :125
     return (sparse_lidar * (1 - potential_outliers)).astype(np.float32)                         # :128
+
+
+def outlier_removal_numpy(lidar: np.ndarray) -> np.ndarray:
+    """data_read.py:103-128 without cv2, bit for bit, for float32 [H,W] or [B,H,W] (frame by frame).  cv2.filter2D of a
+    float32 frame with the 0/1 diamond is, for any float32 values, the 25 taps added in float32 starting from 0, row by
+    row (dy = -3..3) and left to right within a row, over the frame padded BORDER_REFLECT_101 (np.pad's "reflect"); the
+    count of valid pixels is exact.  Then the float64 average sum / (count + 1e-5), the strict ``> 1.0`` and
+    ``x * (1 - outlier)`` in float64, which keeps the sign of a dropped depth (-0.0 for a negative one).  Pinned to
+    cv2_port_outlier_removal by tests/test_outlier_edges.py."""
+    x = np.asarray(lidar)
+    assert x.dtype == np.float32 and x.ndim in (2, 3), (x.dtype, x.shape)
+    xb = x[None] if x.ndim == 2 else x
+    B, H, W = xb.shape
+    R = 3
+    p = np.pad(xb, ((0, 0), (R, R), (R, R)), mode="reflect")
+    total = np.zeros((B, H, W), np.float32)
+    count = np.zeros((B, H, W), np.int64)
+    with np.errstate(all="ignore"):
+        for dy in range(-R, R + 1):
+            for dx in range(-R, R + 1):
+                if DIAMOND_KERNEL_7[R + dy, R + dx]:
+                    v = p[:, R + dy:R + dy + H, R + dx:R + dx + W]
+                    total += v                                                                 # :119, float32
+                    count += v > np.float32(0.1)                                               # :116, :121
+        aveg = total.astype(np.float64) / (count + 0.00001)                                    # :123
+        outlier = ((xb.astype(np.float64) - aveg) > 1.0).astype(np.float64)                    # :125
+        out = (xb.astype(np.float64) * (1 - outlier)).astype(np.float32)                       # :128
+    return out[0] if x.ndim == 2 else out
 
 
 # ------------------------------------------------------------------------------------------------------------
