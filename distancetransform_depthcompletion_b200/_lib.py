@@ -18,7 +18,7 @@ LIB_PATH = os.environ.get("DTFILL_LIB") or os.path.join(_HERE, "libdtfill.so")
 E_ARG, E_CUDA, E_INDEX, E_NOMEM, E_DATA = -1, -2, -3, -4, -5
 METRICS_KITTI, METRICS_NYU = 0, 1
 METRIC_COLS = 9
-ABI_VERSION = 8          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
+ABI_VERSION = 9          # DTFILL_ABI_VERSION of include/dtfill.h this module was written against
 METRIC_NAMES = ("mse", "rmse", "mae", "irmse", "imae", "delta1", "delta2", "delta3", "count")
 
 _c_float_p = ctypes.POINTER(ctypes.c_float)
@@ -99,6 +99,8 @@ def load() -> ctypes.CDLL:
         L.dtfill_debug_png_encode_host.argtypes = [vp, ci, ci, vp, ctypes.c_long]
         L.dtfill_debug_png_encode_host.restype = ctypes.c_long
         L.dtfill_eval_png.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, cf, cf, vp, vp, ctypes.POINTER(ci)]
+        L.dtfill_eval_sampled.argtypes = [vp, vp, ci, ci, ci, ci, vp, vp, vp, ci, ci, ci, ci, ci, cf, cf, vp, vp, vp,
+                                          ctypes.POINTER(ci)]
         L.dtfill_debug_depth_samples_host.argtypes = [vp, ctypes.c_long, vp]
         L.dtfill_debug_depth_samples_host.restype = ci
         L.dtfill_host_alloc.argtypes = [ctypes.POINTER(vp), ctypes.c_size_t]
@@ -112,7 +114,7 @@ def load() -> ctypes.CDLL:
                      "dtfill_run_eval_async", "dtfill_eval_totals", "dtfill_edt", "dtfill_set_sparse_upload",
                      "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo", "dtfill_png_decode",
                      "dtfill_run_png", "dtfill_debug_png_decode_host", "dtfill_png_encode", "dtfill_png_encode_depth",
-                     "dtfill_run_png_to_png", "dtfill_eval_png"):
+                     "dtfill_run_png_to_png", "dtfill_eval_png", "dtfill_eval_sampled"):
             getattr(L, name).restype = ci
         _lib = L
         return L
@@ -343,6 +345,29 @@ class Handle:
                                        int(H), int(W), float(src_thr), float(val_thr), _ptr(per_frame), _ptr(sums),
                                        ctypes.byref(bad)), "dtfill_eval_png")
         return per_frame, sums
+
+    def eval_sampled(self, gt, B: int, H: int, W: int, rows, cols, offsets, crop, src_thr: float, val_thr: float,
+                     gt_is_device: bool = False, coords_are_device: bool = False, want_lidar: bool = False):
+        """The NYU evaluation loop on B frames of dense float32 ground truth gt [B,H,W] (a numpy array, or a device pointer
+        with gt_is_device): frame b keeps the pixels rows[k], cols[k] for k in [offsets[b], offsets[b+1]) (int32 / int64
+        numpy arrays, or device pointers with coords_are_device), is filled, and the crop window (r0, r1, c0, c1) is scored
+        in NYU mode, all on the device -> (per_frame [B,9], sums [10]) float64, plus the sparse frames gt * Mask float32
+        [B,H,W] with want_lidar.  Coordinates outside the frame and decreasing offsets raise ValueError, a frame
+        Distance_Transform rejects raises IndexError."""
+        r0, r1, c0, c1 = (int(v) for v in crop)
+        if not gt_is_device:
+            assert gt.dtype == np.float32 and gt.shape == (B, H, W) and gt.flags.c_contiguous
+        if not coords_are_device:
+            assert rows.dtype == np.int32 and cols.dtype == np.int32 and offsets.dtype == np.int64 and offsets.size == B + 1
+        per_frame = np.empty((B, METRIC_COLS), np.float64)
+        sums = np.empty(METRIC_COLS + 1, np.float64)
+        lidar = np.empty((B, H, W), np.float32) if want_lidar else None
+        bad = ctypes.c_int(-1)
+        _check(self._L.dtfill_eval_sampled(self._h, _ptr(gt), int(bool(gt_is_device)), int(B), int(H), int(W), _ptr(rows),
+                                           _ptr(cols), _ptr(offsets), int(bool(coords_are_device)), r0, r1, c0, c1,
+                                           float(src_thr), float(val_thr), _ptr(lidar), _ptr(per_frame), _ptr(sums),
+                                           ctypes.byref(bad)), "dtfill_eval_sampled")
+        return (per_frame, sums, lidar) if want_lidar else (per_frame, sums)
 
     def png_encode_device_async(self, in_ptr: int, is_float: bool, B: int, H: int, W: int, out_ptr: int,
                                 capacity: int, offsets_ptr: int):

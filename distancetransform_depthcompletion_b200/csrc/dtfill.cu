@@ -359,6 +359,9 @@ struct dtfill_ctx {
     bool in_u16 = false;
     int in_H = 0, in_crop = 0;
     float* lidar_dev = nullptr;
+    // ... or dense float32 ground truth [B,H,W] of which K1 keeps the pixels of the sample bitmap that k10_sample_bits left
+    // in lane 0's srcbits (dtfill_eval_sampled)
+    bool in_sampled = false;
     // evaluation fused behind the call being enqueued (dtfill_run_eval_async): ground truth, mode
     const void* ev_gt = nullptr;
     int ev_gt_f64 = 0, ev_mode = 0;
@@ -377,6 +380,10 @@ struct dtfill_ctx {
     // their offsets (host outputs), filled depth of dtfill_run_png_to_png
     Buf enc_in, enc_filt, enc_adler, enc_slots, enc_seg, enc_out, enc_off, enc_depth;
     PinBuf pin_enc_off;
+    // dtfill_eval_sampled: uploaded host coordinates, the flag word of k10_sample_bits; pinned staging of host coordinates,
+    // and of the counts and the flag word on their way back
+    Buf smp_coords, smp_bad;
+    PinBuf pin_smp, pin_smp_out;
     bool metrics_exact = true;        // dtfill_metrics / _ex reproduce np.mean's pairwise sums bit for bit
     bool sparse_upload = true;        // pageable float32 inputs are compacted on the host instead of mirrored (see CopyPool)
     size_t last_h2d_bytes = 0, last_d2h_bytes = 0;   // bytes the last synchronous host call moved over the link
@@ -615,7 +622,12 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
         const int wpb = k1_threads / 32;
         long want = ((long)rows + wpb - 1) / wpb;
         int grid = (int)(want < 1 ? 1 : want);
-        if (!h->in_u16) {
+        if (h->in_sampled) {
+            const SampledGt* in_s = (const SampledGt*)in + npx0;
+            if ((W & 15) == 0) k1_mask_rows_v16<SampledGt, true><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
+            else if ((W & 3) == 0) k1_mask_rows_v16<SampledGt, false><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
+            else k1_mask_rows<SampledGt><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
+        } else if (!h->in_u16) {
             const float* in_s = (const float*)in + npx0;
             if ((W & 15) == 0) k1_mask_rows_v16<float, true><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
             else if ((W & 3) == 0) k1_mask_rows_v16<float, false><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
@@ -943,9 +955,12 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
 // Per-frame metrics in numpy's own summation order (k4x_*): per-pixel terms of the valid pixels compacted in raster order,
 // then the pairwise tree of np.add.reduce; groups of frames share a scratch of at most ~4 GiB (a batch of 256 KITTI frames
 // with a float64 ground truth needs 3.5 GB: one group, every frame's tree in flight at once).  GT: the arithmetic type,
-// GS: the ground truth as stored.  Device pointers; enqueued on s.
-template <typename GT, int MODE, typename GS>
-int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, double* per_frame, cudaStream_t s) {
+// GS: the ground truth as stored.  WIN: npx is the area of the crop window `win` of frames of win.frame_px pixels.  Device
+// pointers; enqueued on s.
+template <typename GT, int MODE, typename GS, bool WIN = false>
+int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, double* per_frame, cudaStream_t s,
+                const K4xWindow& win = K4xWindow{}) {
+    const long fstride = WIN ? win.frame_px : npx;
     const size_t gsz = sizeof(GT);
     const long maxl = npx / 64 + 2;
     long G = (long)((1ull << 32) / ((size_t)4 * npx * gsz));
@@ -959,7 +974,7 @@ int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, d
         const int ng = (int)(B - g0 < G ? B - g0 : G);
         GT* tm = (GT*)h->mx_terms.p;
         int* cn = (int*)h->mx_counts.p;
-        k4x_compact<GT, MODE, GS><<<ng, K4X_THREADS, 0, s>>>(pred + g0 * npx, gt + g0 * npx, npx, tm, cn);
+        k4x_compact<GT, MODE, GS, WIN><<<ng, K4X_THREADS, 0, s>>>(pred + g0 * fstride, gt + g0 * fstride, npx, tm, cn, win);
         k4x_reduce<GT><<<ng, K4X_RTHREADS, 0, s>>>(tm, cn, npx, MODE, (int*)h->mx_leaf_start.p, (GT*)h->mx_leaf_sum.p,
                                                    per_frame + g0 * 9);
     }
@@ -1061,7 +1076,7 @@ void dtfill_destroy(dtfill_t* h) {
                    &h->gt_dev, &h->partial, &h->per_frame, &h->sums, &h->edt_rows, &h->edt_stack, &h->sparse_dev,
                    &h->mx_terms, &h->mx_counts, &h->mx_leaf_start, &h->mx_leaf_sum, &h->png_data, &h->png_scratch,
                    &h->png_samples, &h->png_status, &h->enc_in, &h->enc_filt, &h->enc_adler, &h->enc_slots, &h->enc_seg,
-                   &h->enc_out, &h->enc_off, &h->enc_depth};
+                   &h->enc_out, &h->enc_off, &h->enc_depth, &h->smp_coords, &h->smp_bad};
     for (Buf* b : bufs)
         if (b->p) cudaFree(b->p);
     for (void* q : h->retired) cudaFree(q);
@@ -1069,7 +1084,7 @@ void dtfill_destroy(dtfill_t* h) {
     delete h->pool_in;
     delete h->pool_out;
     for (PinBuf* b : {&h->pin_in, &h->pin_depth, &h->pin_dt, &h->pin_lbl, &h->pin_mask, &h->pin_lidar, &h->pin_sparse, &h->pin_png,
-                      &h->pin_png_status, &h->pin_enc_off})
+                      &h->pin_png_status, &h->pin_enc_off, &h->pin_smp, &h->pin_smp_out})
         if (b->p) cudaFreeHost(b->p);
     if (h->status_ring) cudaFreeHost(h->status_ring);
     if (h->status_dev) cudaFree(h->status_dev);
@@ -1779,6 +1794,26 @@ struct EvalScope {
     EvalScope(dtfill_t* h_, const void* gt, int f64, int mode) : h(h_) { h->ev_gt = gt; h->ev_gt_f64 = f64; h->ev_mode = mode; }
     ~EvalScope() { h->ev_gt = nullptr; }
 };
+
+// Distance_Transform's verdict on the frames of a synchronous fill, frame by frame as the evaluation loop meets them: rc and
+// fill_bad are what dtfill_status reported, cnt the fill's counts [B][2].  `what` names a frame in the message.
+int fill_verdict(int rc, int fill_bad, const int32_t* cnt, int B, const char* what, int* first_bad_frame) {
+    const int lim = rc == DTFILL_E_INDEX ? fill_bad : B;
+    for (int b = 0; b < lim; ++b)
+        if (cnt[2 * b + 1] == 1) {
+            // eval_NYU.py:126 np.squeeze(lidar[with_value]) makes a single valid depth 0-dimensional; :128 then fails
+            if (first_bad_frame) *first_bad_frame = b;
+            return fail(DTFILL_E_INDEX, what + std::to_string(b) +
+                                            ": one valid depth (numpy IndexError: too many indices for array: array is "
+                                            "0-dimensional, but 1 were indexed)");
+        }
+    if (rc == DTFILL_E_INDEX) {
+        if (first_bad_frame) *first_bad_frame = fill_bad;
+        return fail(DTFILL_E_INDEX, what + std::to_string(fill_bad) +
+                                        ": labels index outside the list of valid depths (numpy IndexError)");
+    }
+    return 0;
+}
 }  // namespace
 
 int dtfill_run_eval_async(dtfill_t* h, const float* in_dev, const void* gt_dev, int gt_is_f64, int B, int H, int W,
@@ -1941,22 +1976,137 @@ int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offs
                                            png_reason(st) + " (status " + std::to_string(st) + ")");
         }
     }
-    const int32_t* cnt = st_host + 2 * B;
-    const int lim = rc == DTFILL_E_INDEX ? fill_bad : B;
-    for (int b = 0; b < lim; ++b)
-        if (cnt[2 * b + 1] == 1) {
-            // eval_NYU.py:126 np.squeeze(lidar[with_value]) makes a single valid depth 0-dimensional; :128 then fails
-            if (first_bad_frame) *first_bad_frame = b;
-            return fail(DTFILL_E_INDEX, "LiDAR file " + std::to_string(b) +
-                                            ": one valid depth (numpy IndexError: too many indices for array: array is "
-                                            "0-dimensional, but 1 were indexed)");
+    return fill_verdict(rc, fill_bad, st_host + 2 * B, B, "LiDAR file ", first_bad_frame);
+}
+
+int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, const int32_t* rows,
+                        const int32_t* cols, const int64_t* sample_offsets, int coords_are_device, int r0, int r1, int c0,
+                        int c1, float src_thr, float val_thr, float* out_lidar, double* per_frame, double* sums,
+                        int* first_bad_frame) {
+    const char* who = "dtfill_eval_sampled";
+    if (first_bad_frame) *first_bad_frame = -1;
+    if (!h || !gt || !rows || !cols || !sample_offsets)
+        return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, ground truth, coordinates or offsets");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H, W must be positive");
+    if ((long)H + W >= 60000 || (long)H * W >= (1l << 31) || W > 28000)
+        return fail(DTFILL_E_ARG, std::string(who) + ": frame size not supported (H + W < 60000, W <= 28000)");
+    if (r0 < 0 || r1 > H || r0 >= r1 || c0 < 0 || c1 > W || c0 >= c1)
+        return fail(DTFILL_E_ARG, std::string(who) + ": window [" + std::to_string(r0) + ":" + std::to_string(r1) + ", " +
+                                      std::to_string(c0) + ":" + std::to_string(c1) + "] is not a non-empty window of the " +
+                                      std::to_string(H) + " x " + std::to_string(W) + " frame");
+    if (gt_is_device && (W & 3) == 0 && ((uintptr_t)gt & 15))
+        return fail(DTFILL_E_ARG, std::string(who) + ": device ground truth must be 16-byte aligned");
+    CU(cudaSetDevice(h->device));
+    int rc = dtfill_flush(h);        // fills in flight (pipelined mode) may still use lane 0's workspace
+    if (rc) return rc;
+    const long npx = (long)H * W;
+    const int WW = (W + 31) / 32;
+    cudaStream_t s = h->stream;
+    size_t h2d = 0;
+    // 1. coordinates: host ones are checked here and go up in one copy through the pinned staging buffer (rows, cols, then
+    //    the offsets rebased to 0); device ones are checked by k10_sample_bits
+    const int32_t* d_rows = rows;
+    const int32_t* d_cols = cols;
+    const int64_t* d_off = sample_offsets;
+    if (!coords_are_device) {
+        const int64_t* o = sample_offsets;
+        if (o[0] < 0) return fail(DTFILL_E_ARG, std::string(who) + ": sample_offsets[0] < 0");
+        for (int b = 0; b < B; ++b) {
+            if (o[b + 1] < o[b]) {
+                if (first_bad_frame) *first_bad_frame = b;
+                return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(b) + " has a negative sample count");
+            }
+            for (int64_t i = o[b]; i < o[b + 1]; ++i)
+                if ((unsigned)rows[i] >= (unsigned)H || (unsigned)cols[i] >= (unsigned)W) {
+                    if (first_bad_frame) *first_bad_frame = b;
+                    return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(b) + ": sample (" +
+                                                  std::to_string(rows[i]) + ", " + std::to_string(cols[i]) +
+                                                  ") outside the frame");
+                }
         }
-    if (rc == DTFILL_E_INDEX) {
-        if (first_bad_frame) *first_bad_frame = fill_bad;
-        return fail(DTFILL_E_INDEX, "LiDAR file " + std::to_string(fill_bad) +
-                                        ": labels index outside the list of valid depths (numpy IndexError)");
+        const size_t n = (size_t)(o[B] - o[0]);
+        const size_t off_at = (2 * n * 4 + 15) & ~(size_t)15;
+        const size_t total = off_at + (size_t)(B + 1) * 8;
+        if ((rc = ensure_pinned(h->pin_smp, total))) return rc;
+        if ((rc = ensure(h, h->smp_coords, total))) return rc;
+        uint8_t* pin = (uint8_t*)h->pin_smp.p;
+        if (n) {
+            memcpy(pin, rows + o[0], n * 4);
+            memcpy(pin + n * 4, cols + o[0], n * 4);
+        }
+        int64_t* po = (int64_t*)(pin + off_at);
+        for (int b = 0; b <= B; ++b) po[b] = o[b] - o[0];
+        CU(cudaMemcpyAsync(h->smp_coords.p, pin, total, cudaMemcpyHostToDevice, s));
+        h2d += total;
+        d_rows = (const int32_t*)h->smp_coords.p;
+        d_cols = d_rows + n;
+        d_off = (const int64_t*)((uint8_t*)h->smp_coords.p + off_at);
     }
-    return 0;
+    // 2. the ground truth, unless it is resident
+    const float* g_d = gt;
+    if (!gt_is_device) {
+        if ((rc = ensure(h, h->gt_dev, (size_t)B * npx * 4))) return rc;
+        CU(cudaMemcpyAsync(h->gt_dev.p, gt, (size_t)B * npx * 4, cudaMemcpyHostToDevice, s));
+        h2d += (size_t)B * npx * 4;
+        g_d = (const float*)h->gt_dev.p;
+    }
+    // 3. the sample bitmap in lane 0's srcbits (the lane of a strict-order fill), sized as the fill sizes it so that the
+    //    fill does not reallocate it
+    Lane* L = &h->lanes[0];
+    if ((rc = ensure(h, L->srcbits, (size_t)B * H * WW * 4))) return rc;
+    if ((rc = ensure(h, h->smp_bad, 4))) return rc;
+    CU(cudaMemsetAsync(L->srcbits.p, 0, (size_t)B * H * WW * 4, s));
+    CU(cudaMemsetAsync(h->smp_bad.p, 0x7F, 4, s));           // 0x7F7F7F7F: above every frame index
+    k10_sample_bits<<<B, K10_THREADS, 0, s>>>(d_rows, d_cols, d_off, H, W, WW, (uint32_t*)L->srcbits.p, (int*)h->smp_bad.p);
+    CU(cudaGetLastError());
+    // 4. the fill with K1's sampled input kind, strict order on the handle's stream; the filled depth stays on the device
+    if ((rc = ensure(h, h->depth_dev, (size_t)B * npx * 4))) return rc;
+    if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc;
+    float* lid_d = nullptr;
+    if (out_lidar) {
+        if ((rc = ensure(h, h->lidar_out_dev, (size_t)B * npx * 4))) return rc;
+        lid_d = (float*)h->lidar_out_dev.p;
+    }
+    float* depth = (float*)h->depth_dev.p;
+    int32_t* counts = (int32_t*)h->counts_out_dev.p;
+    {
+        InputScope scope(h, false, H, 0, lid_d);
+        h->in_sampled = true;
+        rc = enqueue(h, g_d, B, H, W, src_thr, val_thr, depth, nullptr, nullptr, nullptr, counts, nullptr, true);
+        h->in_sampled = false;
+        if (rc) return rc;
+    }
+    // 5. Result_NYU.evaluate of the window of the filled depth against the same window of the ground truth, in numpy's
+    //    summation order whatever dtfill_set_metrics_exact says
+    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
+    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
+    double* pf_d = (double*)h->per_frame.p;
+    double* sm_d = (double*)h->sums.p;
+    const K4xWindow win{npx, W, r0, c0, c1 - c0};
+    if ((rc = k4x_enqueue<float, 1, float, true>(h, depth, g_d, B, (long)(r1 - r0) * (c1 - c0), pf_d, s, win))) return rc;
+    k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
+    CU(cudaGetLastError());
+    if ((rc = ensure_pinned(h->pin_smp_out, (size_t)B * 8 + 4))) return rc;
+    int32_t* out_h = (int32_t*)h->pin_smp_out.p;            // the fill's counts [B][2], then the flag word
+    CU(cudaMemcpyAsync(out_h, counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(out_h + 2 * B, h->smp_bad.p, 4, cudaMemcpyDeviceToHost, s));
+    if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
+    if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
+    if (out_lidar) CU(cudaMemcpyAsync(out_lidar, lid_d, (size_t)B * npx * 4, cudaMemcpyDeviceToHost, s));
+    int fill_bad = -1;
+    rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
+    h->last_h2d_bytes = h2d;
+    h->last_d2h_bytes = (size_t)B * 8 + 4 + (per_frame ? (size_t)B * 9 * 8 : 0) + (sums ? 10 * 8 : 0) +
+                        (out_lidar ? (size_t)B * npx * 4 : 0);
+    if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
+    // 6. the verdict: device coordinates outside the frame, then Distance_Transform's frame by frame
+    const int bad = out_h[2 * B];
+    if (bad < B) {
+        if (first_bad_frame) *first_bad_frame = bad;
+        return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(bad) +
+                                      ": a sample outside the frame, or a negative sample count");
+    }
+    return fill_verdict(rc, fill_bad, out_h, B, "frame ", first_bad_frame);
 }
 
 int dtfill_set_band_cap(dtfill_t* h, int cap) {

@@ -153,6 +153,14 @@ template <> struct In16<uint16_t> {
         return make_float4(u16_depth(a & 0xFFFFu), u16_depth(a >> 16), u16_depth(b & 0xFFFFu), u16_depth(b >> 16));
     }
 };
+// Input kind of K1 for the NYU loop (dtfill_eval_sampled): dense float32 ground truth, of which only the pixels set in the
+// sample bitmap (k10_sample_bits) are kept; the sparse frame `gt * Mask` is formed in registers (dtfill_k1_mask.cuh)
+struct SampledGt { float v; };
+template <> struct In16<SampledGt> : In16<float> {
+    __device__ __forceinline__ void load(const SampledGt* p, int col, int W) { In16<float>::load(&p->v, col, W); }
+    __device__ __forceinline__ void load_all(const SampledGt* p, bool inside) { In16<float>::load_all(&p->v, inside); }
+};
+__device__ __forceinline__ float load_px_stream(const SampledGt* p) { return ld_stream(&p->v); }
 
 // Tuning build (-DDTFILL_TRACE): every block that does work records its start and end (globaltimer, ns) into the
 // launch's trace slot, so that the overlap of the kernels of consecutive calls can be reconstructed without a profiler.

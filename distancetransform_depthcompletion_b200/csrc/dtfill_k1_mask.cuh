@@ -1,5 +1,7 @@
 // dtfill_k1_mask.cuh -- K1: predicates, bit rows, validity mask, row-local compaction (tools.py:8, :22; net.py:131-132; data_read.py:215)
 #pragma once
+#include <type_traits>
+
 #include "dtfill_common.cuh"
 
 namespace dtfill {
@@ -30,6 +32,18 @@ __device__ __forceinline__ uint32_t sign_nibble_bytes(float t0, float t1, float 
     return (w * 0x00204081u) >> 28;
 }
 
+// Sampled input (T = SampledGt, dtfill_eval_sampled): the sample bitmap of k10_sample_bits lies in ws.srcbits, in the layout
+// K1 writes its source bits in.  A word is read by the two lanes (or, in the scalar kernel, the warp) that later overwrite
+// it, and every read value is consumed before the warp's shuffles / ballots that precede the write.  A pixel keeps its
+// ground-truth value when its bit is set and becomes g * 0 otherwise, as `gt * Mask` does (data_read.py:364): -0 for a
+// negative g, NaN for a NaN or infinite g (a source, tools.py:8).
+__device__ __forceinline__ float sampled_px(float g, uint32_t bit) { return bit ? g : __fmul_rn(g, 0.0f); }
+// the 16 bits of the lane's pixels [col, col + 16) of row `row` (col a multiple of 16)
+__device__ __forceinline__ uint32_t sample_half(const Workspace& ws, long row, int WW, int col, int W)
+{
+    return col < W ? (ws.srcbits[row * WW + (col >> 5)] >> (col & 16)) & 0xFFFFu : 0u;
+}
+
 // W16: W % 16 == 0 (KITTI 1216, NYU 640): a lane's 16 pixels are inside the row or outside it as a whole.
 template <typename T, bool W16>
 __global__ void __launch_bounds__(256) k1_mask_rows_v16(const T* __restrict__ in, FrameParams fp, Workspace ws,
@@ -57,16 +71,28 @@ __global__ void __launch_bounds__(256) k1_mask_rows_v16(const T* __restrict__ in
         In16<T> nq;
         if (W16) nq.load_all(rp + lane * 16, lane * 16 < W);
         else nq.load(rp + lane * 16, lane * 16, W);
+        uint32_t nbits = 0;
+        if constexpr (std::is_same<T, SampledGt>::value) nbits = sample_half(ws, row, WW, lane * 16, W);
         for (int ch = 0; ch < nchunks; ++ch) {
             const int col = (ch << 9) + lane * 16;
             float4 q[4];
 #pragma unroll
             for (int g = 0; g < 4; ++g) q[g] = nq.get(g);
+            const uint32_t bits = nbits;
             if (ch + 1 < nchunks) {
                 if (W16) nq.load_all(rp + col + 512, col + 512 < W);
                 else nq.load(rp + col + 512, col + 512, W);
+                if constexpr (std::is_same<T, SampledGt>::value) nbits = sample_half(ws, row, WW, col + 512, W);
             }
-            if (out_lidar && col < W) {                  // decoded frame (uint16 input): what the CNN reads as lidar
+            if constexpr (std::is_same<T, SampledGt>::value) {
+#pragma unroll
+                for (int g = 0; g < 4; ++g) {
+                    const uint32_t b4 = bits >> (4 * g);
+                    q[g] = make_float4(sampled_px(q[g].x, b4 & 1u), sampled_px(q[g].y, b4 & 2u), sampled_px(q[g].z, b4 & 4u),
+                                       sampled_px(q[g].w, b4 & 8u));
+                }
+            }
+            if (out_lidar && col < W) {                  // decoded (uint16) or sampled frame: what the CNN reads as lidar
 #pragma unroll
                 for (int g = 0; g < 4; ++g)
                     if (W16 || col + 4 * g < W)
@@ -190,6 +216,8 @@ __global__ void __launch_bounds__(256) k1_mask_rows(const T* __restrict__ in, Fr
             for (int k = 0; k < 16; ++k) {
                 const int col = (c0 + k) * 32 + lane;
                 x[k] = col < W ? load_px_stream(rp + col) : 0.0f;
+                if constexpr (std::is_same<T, SampledGt>::value)
+                    if (col < W) x[k] = sampled_px(x[k], (ws.srcbits[row * WW + c0 + k] >> lane) & 1u);
                 if (out_lidar && col < W) out_lidar[row * W + col] = x[k];
             }
             uint32_t mys = 0, mypre = 0;

@@ -19,7 +19,8 @@ namespace dtfill {
 // reproduce exactly that tree, so the metrics are the reference's bit for bit -- the fixed-order float64 sums of
 // k4_metrics_partial agree with numpy's float32 pairwise sums only to ~1e-5.
 //   k4x_compact  one block per frame: the terms of the valid pixels, compacted in raster order (ballots + warp ranks);
-//                the ground truth is stored as the arithmetic type or, in KITTI mode, as 16-bit PNG samples
+//                the ground truth is stored as the arithmetic type or, in KITTI mode, as 16-bit PNG samples; the WIN
+//                instance (NYU mode, float32) scores a crop window of the frames
 //   k4x_reduce   one block per frame: the leaves (<= 128 elements) of the tree in parallel, then the tree itself
 // Terms: 0 |d|^2, 1 |d| (KITTI) or |d| / t (NYU), 2 |dinv|^2, 3 |dinv|; counts: valid, delta1..3.
 // ------------------------------------------------------------------------------------------------------
@@ -75,16 +76,31 @@ __device__ __forceinline__ GT gt_value(GS s)
     }
 }
 
-template <typename GT, int MODE, typename GS = GT>
+// A crop window of the frames (WIN instances, dtfill_eval_sampled: eval_NYU.py:202-207 scores pred[6:234, 8:312]): pixel i
+// of the window in its raster order is pixel (r0 + i / cw) * W + c0 + i % cw of a frame of frame_px pixels.  The terms of
+// the window's valid pixels are then compacted in the order numpy's boolean index of the cropped view gives them.
+struct K4xWindow {
+    long frame_px;
+    int W, r0, c0, cw;
+    __device__ __forceinline__ long at(long i) const
+    {
+        const int y = (int)i / cw;
+        return (long)(r0 + y) * W + c0 + ((int)i - y * cw);
+    }
+};
+
+// npx: pixels per frame, or per window (WIN); the term arrays hold npx entries per frame either way
+template <typename GT, int MODE, typename GS = GT, bool WIN = false>
 __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restrict__ pred, const GS* __restrict__ gt, long npx,
                                                             GT* __restrict__ terms /*[frames][4][npx]*/,
-                                                            int* __restrict__ counts /*[frames][4]*/)
+                                                            int* __restrict__ counts /*[frames][4]*/, const K4xWindow win)
 {
     __shared__ int wtot[K4X_THREADS / 32], wbase[K4X_THREADS / 32];
     __shared__ int hits[3];
     const int b = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const float* p = pred + (long)b * npx;
-    const GS* g = gt + (long)b * npx;
+    auto px = [&](long i) -> long { if constexpr (WIN) return win.at(i); else return i; };
+    const float* p = pred + (long)b * (WIN ? win.frame_px : npx);
+    const GS* g = gt + (long)b * (WIN ? win.frame_px : npx);
     GT* tb = terms + (long)b * 4 * npx;
     const long seg = ((npx + K4X_THREADS - 1) / K4X_THREADS) * 32;     // pixels per warp, a multiple of 32
     const long i0 = min(npx, wid * seg), i1 = min(npx, i0 + seg);
@@ -93,7 +109,7 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
     int cnt = 0;
     for (long c = i0; c < i1; c += 32) {
         const long i = c + lane;
-        const bool v = i < i1 && (p[i] > 0.01f) && (gt_value<GT>(g[i]) > (GT)0.01);     // u16: s >= 3
+        const bool v = i < i1 && (p[px(i)] > 0.01f) && (gt_value<GT>(g[px(i)]) > (GT)0.01);     // u16: s >= 3
         cnt += __popc(__ballot_sync(0xffffffffu, v));
     }
     if (lane == 0) wtot[wid] = cnt;
@@ -114,7 +130,7 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
         const long i = c + lane;
         GT term[4] = {0, 0, 0, 0};
         int hit[3] = {0, 0, 0};
-        const bool v = i < i1 && metric_terms<GT, MODE>(p[i], gt_value<GT>(g[i]), term, hit);
+        const bool v = i < i1 && metric_terms<GT, MODE>(p[px(i)], gt_value<GT>(g[px(i)]), term, hit);
         const uint32_t m = __ballot_sync(0xffffffffu, v);
         if (v) {
             const long k = run + __popc(m & lanemask_lt());

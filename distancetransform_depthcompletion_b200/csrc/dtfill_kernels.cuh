@@ -21,6 +21,8 @@
 //                         of the uint16 entry (data_read.py:215 reads the files with PIL)
 //   K9  k9_png_*          uint16 samples or float32 depth -> 16-bit grayscale PNG files (row filter, deflate per segment,
 //                         offsets, pack), so that filled maps leave the device compressed
+//   K10 k10_sample_bits   NYU sample coordinates -> a bitmap of 1 bit per pixel, read by K1's sampled input kind, which
+//                         forms `gt * Mask` from the dense ground truth in registers (dtfill_eval_sampled)
 // One header per kernel (dtfill_k*.cuh); dtfill_common.cuh holds the key format, the structs and the helpers.
 //
 // Key format of the fast path (SURVEY.md section 7 H1): dist:11 | order:4 | label:17.  "order" is the position
@@ -43,3 +45,4 @@
 #include "dtfill_k7_edt.cuh"
 #include "dtfill_k8_png.cuh"
 #include "dtfill_k9_png_encode.cuh"
+#include "dtfill_k10_sample.cuh"

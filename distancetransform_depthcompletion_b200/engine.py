@@ -166,6 +166,45 @@ class DTFillEngine:
         self._hold(t, data, offsets)
         return data, offsets
 
+    def eval_sampled(self, gt, rows, cols, offsets=None, crop=None, src_thr: float | None = None, want_lidar: bool = False):
+        """The NYU evaluation loop (eval_nyu.evaluate_fill_sampled) against the float32 CUDA tensor gt [B,H,W], used in
+        place, on torch's current stream, so that repeated draws against the same resident ground truth move only their
+        coordinates.  rows / cols: the host forms evaluate_fill_sampled takes, or int32 CUDA tensors of the concatenated
+        coordinates with ``offsets`` an int64 CUDA tensor [B+1] (frame b: entries offsets[b]:offsets[b+1]; checked on the
+        device, a coordinate outside the frame raises ValueError).  Synchronous: returns (per_frame [B,9], sums [10]) float64
+        numpy arrays (and the sparse frames gt * Mask with want_lidar).  Fills still in flight are joined first."""
+        from . import eval_nyu
+        torch = self.torch
+        assert gt.is_cuda and gt.dtype == torch.float32 and gt.dim() == 3
+        gt = eval_nyu._aligned(gt)
+        B, H, W = (int(v) for v in gt.shape)
+        crop = eval_nyu._check_crop(eval_nyu.NYU_EVAL_CROP if crop is None else crop, H, W)
+        src_thr = eval_nyu.NYU_SRC_THR if src_thr is None else src_thr
+        on_device = isinstance(rows, torch.Tensor) and rows.is_cuda
+        if on_device:
+            assert cols.is_cuda and rows.dtype == cols.dtype == torch.int32 and rows.is_contiguous() and cols.is_contiguous()
+            assert offsets is not None and offsets.is_cuda and offsets.dtype == torch.int64 and offsets.numel() == B + 1
+            assert offsets.is_contiguous()
+            if rows.numel() != cols.numel():
+                raise ValueError(f"eval_sampled: {rows.numel()} rows but {cols.numel()} cols")
+            # the kernel reads rows / cols between offsets[0] and offsets[B], so non-decreasing offsets whose ends lie within
+            # the arrays keep every read inside them (a synchronous call: these checks cost two small copies)
+            lo, hi = (int(v) for v in offsets[[0, B]].tolist())
+            if lo < 0 or hi > rows.numel():
+                raise ValueError(f"eval_sampled: offsets span [{lo}, {hi}) but there are {rows.numel()} coordinates")
+            dec = torch.nonzero(offsets[1:] < offsets[:-1])
+            if dec.numel():
+                raise ValueError(f"eval_sampled: frame {int(dec[0, 0])} has a negative sample count")
+            r, c, off = rows.data_ptr(), cols.data_ptr(), offsets.data_ptr()
+        else:
+            r, c, off = eval_nyu._sample_arrays(rows, cols, B, H, W)
+        from .tools import VALID_THR
+        self._bind_stream()
+        res = self.handle.eval_sampled(gt.data_ptr(), B, H, W, r, c, off, crop, src_thr, VALID_THR, gt_is_device=True,
+                                       coords_are_device=on_device, want_lidar=want_lidar)
+        self._inflight = {}       # the call synchronised: every earlier call has finished
+        return res
+
     def flush(self):
         """Pipelined mode: torch's current stream waits for every fill still in flight."""
         self._bind_stream()

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DTFILL_ABI_VERSION 8      /* 8: dtfill_eval_png; 7: PNG encode (dtfill_png_encode, dtfill_png_encode_depth, dtfill_run_png_to_png); 6: PNG decode (dtfill_png_decode, dtfill_run_png, DTFILL_E_DATA); 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
+#define DTFILL_ABI_VERSION 9      /* 9: dtfill_eval_sampled; 8: dtfill_eval_png; 7: PNG encode (dtfill_png_encode, dtfill_png_encode_depth, dtfill_run_png_to_png); 6: PNG decode (dtfill_png_decode, dtfill_run_png, DTFILL_E_DATA); 5: sparse upload (dtfill_set_sparse_upload, dtfill_transfer_bytes); 4: dtfill_run_eval_async + dtfill_eval_totals, dtfill_edt; 3: metrics_ex, allreduce, status ring */
 
 enum {
     DTFILL_OK = 0,
@@ -231,6 +231,32 @@ int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_
 int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets, const uint8_t* gt,
                     const int64_t* gt_offsets, int B, int H, int W, float src_thr, float val_thr, double* per_frame,
                     double* sums, int* first_bad_frame);
+
+/*
+ * The evaluation loop of the reference's NYU script (eval_NYU.py:138-254, data_read.py:337-371) from dense ground truth:
+ *     Mask = zeros(H, W);  Mask[rows_b, cols_b] = 1                 data_read.py:360-364 (duplicates collapse)
+ *     pred = Distance_Transform(gt_b * Mask, src_thr)               eval_NYU.py:120-133
+ *     Result_NYU().evaluate(pred[r0:r1, c0:c1], gt_b[r0:r1, c0:c1]) eval_NYU.py:202-207
+ * for the B frames of gt (float32 [B,H,W]; a device pointer when gt_is_device, used in place and never copied, else host).
+ * Frame b's sample coordinates are rows[k], cols[k] for k in [sample_offsets[b], sample_offsets[b+1]) (int32, int64
+ * offsets [B+1]; device pointers when coords_are_device, in which case every index from the smallest to the largest
+ * offset must lie within rows and cols: the device can check the coordinates' values, not the arrays' length).  The
+ * coordinates become a bitmap of 1 bit per pixel
+ * (k10_sample_bits), K1 forms `gt * Mask` from the ground truth and the bitmap in registers (out_lidar, host, nullable:
+ * that sparse frame [B,H,W]), the fill keeps the filled depth on the device, and the NYU-mode metrics of the window are
+ * computed against the same ground-truth buffer in numpy's summation order (whatever dtfill_set_metrics_exact says), so
+ * that per_frame [B][DTFILL_METRIC_COLS] and sums [DTFILL_METRIC_COLS + 1] (host, nullable; layout of dtfill_metrics) equal
+ * the reference's bit for bit.  With a resident ground truth only the coordinates and offsets go up and only the counts and
+ * the metrics come back (dtfill_transfer_bytes).  Synchronous; strict order on the handle's stream.
+ * Errors: DTFILL_E_ARG for a window that is empty or leaves the frame, decreasing offsets (a negative count) and
+ * coordinates outside [0,H) x [0,W) (host coordinates are checked on the host, device ones on the device; *first_bad_frame
+ * receives the frame); then DTFILL_E_INDEX for the first frame Distance_Transform rejects (no valid depth, exactly one
+ * valid depth, labels outside the list of valid depths).  On an error the contents of the outputs are unspecified.
+ */
+int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, const int32_t* rows,
+                        const int32_t* cols, const int64_t* sample_offsets, int coords_are_device, int r0, int r1, int c0,
+                        int c1, float src_thr, float val_thr, float* out_lidar, double* per_frame, double* sums,
+                        int* first_bad_frame);
 
 /*
  * One step of an evaluation sweep, fused (BASELINE.json configs[4]; the loop body of eval.py:212-232: DT_complete_batch,
