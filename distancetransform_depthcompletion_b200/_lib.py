@@ -101,6 +101,11 @@ def load() -> ctypes.CDLL:
         L.dtfill_eval_png.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, cf, cf, vp, vp, ctypes.POINTER(ci)]
         L.dtfill_eval_sampled.argtypes = [vp, vp, ci, ci, ci, ci, vp, vp, vp, ci, ci, ci, ci, ci, cf, cf, vp, vp, vp,
                                           ctypes.POINTER(ci)]
+        try:
+            L.dtfill_eval_png_kitti.argtypes = [vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, cf, cf, vp, vp, ctypes.POINTER(ci)]
+        except AttributeError:      # an older build of the same ABI version
+            raise DTFillError(f"{LIB_PATH} lacks dtfill_eval_png_kitti: rebuild it with "
+                              "`python -m distancetransform_depthcompletion_b200.build`") from None
         L.dtfill_debug_depth_samples_host.argtypes = [vp, ctypes.c_long, vp]
         L.dtfill_debug_depth_samples_host.restype = ci
         L.dtfill_host_alloc.argtypes = [ctypes.POINTER(vp), ctypes.c_size_t]
@@ -114,7 +119,7 @@ def load() -> ctypes.CDLL:
                      "dtfill_run_eval_async", "dtfill_eval_totals", "dtfill_edt", "dtfill_set_sparse_upload",
                      "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo", "dtfill_png_decode",
                      "dtfill_run_png", "dtfill_debug_png_decode_host", "dtfill_png_encode", "dtfill_png_encode_depth",
-                     "dtfill_run_png_to_png", "dtfill_eval_png", "dtfill_eval_sampled"):
+                     "dtfill_run_png_to_png", "dtfill_eval_png", "dtfill_eval_sampled", "dtfill_eval_png_kitti"):
             getattr(L, name).restype = ci
         _lib = L
         return L
@@ -344,6 +349,29 @@ class Handle:
         _check(self._L.dtfill_eval_png(self._h, _ptr(lidar_data), _ptr(lidar_off), _ptr(gt_data), _ptr(gt_off), B,
                                        int(H), int(W), float(src_thr), float(val_thr), _ptr(per_frame), _ptr(sums),
                                        ctypes.byref(bad)), "dtfill_eval_png")
+        return per_frame, sums
+
+    def eval_png_kitti(self, lidar_data: np.ndarray, lidar_off: np.ndarray, gt_data, gt_off, gt_ptr, H_in: int, W: int,
+                       crop_top: int, src_thr: float, val_thr: float):
+        """The KITTI branch of eval_NYU.py's loop: B LiDAR PNG files (packed as for png_decode) decoded, rows crop_top:
+        filled, floored at 0.9 and scored in KITTI mode against the same rows of the ground truth, all on the device ->
+        (per_frame [B,9], sums [10]) float64, bit-exact with the loop.  The ground truth is B PNG files (gt_data, gt_off;
+        gt_ptr None) or a device pointer to uint16 samples [B,H_in,W] on this handle's device (gt_data and gt_off None),
+        read in place.  A decode failure raises ValueError naming the list and the frame; a frame Distance_Transform
+        rejects raises IndexError."""
+        lidar_data, lidar_off = _png_args(lidar_data, lidar_off)
+        B = lidar_off.size - 1
+        if gt_ptr is None:
+            gt_data, gt_off = _png_args(gt_data, gt_off)
+            if gt_off.size - 1 != B:
+                raise ValueError(f"dtfill_eval_png_kitti: {B} LiDAR files but {gt_off.size - 1} ground-truth files")
+        per_frame = np.empty((B, METRIC_COLS), np.float64)
+        sums = np.empty(METRIC_COLS + 1, np.float64)
+        bad = ctypes.c_int(-1)
+        _check(self._L.dtfill_eval_png_kitti(self._h, _ptr(lidar_data), _ptr(lidar_off), _ptr(gt_data), _ptr(gt_off),
+                                             _ptr(gt_ptr), B, int(H_in), int(W), int(crop_top), float(src_thr),
+                                             float(val_thr), _ptr(per_frame), _ptr(sums), ctypes.byref(bad)),
+               "dtfill_eval_png_kitti")
         return per_frame, sums
 
     def eval_sampled(self, gt, B: int, H: int, W: int, rows, cols, offsets, crop, src_thr: float, val_thr: float,

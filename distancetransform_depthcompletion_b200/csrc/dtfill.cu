@@ -955,12 +955,13 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
 // Per-frame metrics in numpy's own summation order (k4x_*): per-pixel terms of the valid pixels compacted in raster order,
 // then the pairwise tree of np.add.reduce; groups of frames share a scratch of at most ~4 GiB (a batch of 256 KITTI frames
 // with a float64 ground truth needs 3.5 GB: one group, every frame's tree in flight at once).  GT: the arithmetic type,
-// GS: the ground truth as stored.  WIN: npx is the area of the crop window `win` of frames of win.frame_px pixels.  Device
-// pointers; enqueued on s.
-template <typename GT, int MODE, typename GS, bool WIN = false>
+// GS: the ground truth as stored.  WIN: npx is the area of the crop window `win` of frames of win.frame_px pixels.
+// CROP_FLOOR: npx pixels per prediction frame against rows win.r0: of ground-truth frames of win.frame_px samples, the
+// prediction floored at 0.9 (k4x_compact).  Device pointers; enqueued on s.
+template <typename GT, int MODE, typename GS, bool WIN = false, bool CROP_FLOOR = false>
 int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, double* per_frame, cudaStream_t s,
                 const K4xWindow& win = K4xWindow{}) {
-    const long fstride = WIN ? win.frame_px : npx;
+    const long pstride = WIN ? win.frame_px : npx, gstride = WIN || CROP_FLOOR ? win.frame_px : npx;
     const size_t gsz = sizeof(GT);
     const long maxl = npx / 64 + 2;
     long G = (long)((1ull << 32) / ((size_t)4 * npx * gsz));
@@ -974,7 +975,8 @@ int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, d
         const int ng = (int)(B - g0 < G ? B - g0 : G);
         GT* tm = (GT*)h->mx_terms.p;
         int* cn = (int*)h->mx_counts.p;
-        k4x_compact<GT, MODE, GS, WIN><<<ng, K4X_THREADS, 0, s>>>(pred + g0 * fstride, gt + g0 * fstride, npx, tm, cn, win);
+        k4x_compact<GT, MODE, GS, WIN, CROP_FLOOR><<<ng, K4X_THREADS, 0, s>>>(pred + g0 * pstride, gt + g0 * gstride, npx, tm,
+                                                                                cn, win);
         k4x_reduce<GT><<<ng, K4X_RTHREADS, 0, s>>>(tm, cn, npx, MODE, (int*)h->mx_leaf_start.p, (GT*)h->mx_leaf_sum.p,
                                                    per_frame + g0 * 9);
     }
@@ -1909,6 +1911,86 @@ int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_
     return 0;
 }
 
+namespace {
+
+// The body of dtfill_eval_png (no crop, no floor) and dtfill_eval_png_kitti (rows crop_top: of both, the prediction
+// floored at 0.9): B LiDAR files and the ground truth as B files (gt, gt_offsets) or as resident samples gt_dev
+// [B,H_in,W], which are read in place.
+int eval_png_run(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets, const uint8_t* gt,
+                 const int64_t* gt_offsets, const uint16_t* gt_dev, int B, int H_in, int W, int crop_top, bool floor,
+                 float src_thr, float val_thr, double* per_frame, double* sums, int* first_bad_frame) {
+    CU(cudaSetDevice(h->device));
+    const long npx_in = (long)H_in * W, npx = (long)(H_in - crop_top) * W;
+    const int nfiles = gt_dev ? B : 2 * B;
+    cudaStream_t s = h->stream;
+    int rc;
+    // 1. one decode of the files (one warp per file, so the call costs about the slowest file, not two files in a row):
+    //    LiDAR file b -> samples / status b, ground-truth file b -> samples / status B + b
+    if ((rc = ensure(h, h->png_samples, (size_t)nfiles * npx_in * 2))) return rc;
+    if ((rc = ensure(h, h->png_status, (size_t)nfiles * 4))) return rc;
+    int32_t* st_host = nullptr;                   // [nfiles] decode status, then the fill's counts [B][2]
+    if ((rc = png_status_host(h, nfiles + 2 * B, &st_host))) return rc;
+    uint16_t* samples = (uint16_t*)h->png_samples.p;
+    int32_t* status = (int32_t*)h->png_status.p;
+    const PngFiles sets[2] = {{lidar, lidar_offsets, B}, {gt, gt_offsets, B}};
+    const uint8_t* d_data;
+    const int64_t* d_off;
+    if ((rc = png_stage(h, sets, gt_dev ? 1 : 2, &d_data, &d_off))) return rc;
+    const size_t h2d = h->last_h2d_bytes;
+    if ((rc = png_enqueue(h, d_data, d_off, 1, nfiles, H_in, W, samples, status))) return rc;
+    // 2. the fill of dtfill_run_u16 on rows crop_top: of the LiDAR samples, strict order on the handle's stream; only the
+    //    counts leave the device
+    if ((rc = ensure(h, h->depth_dev, (size_t)B * npx * 4))) return rc;
+    if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc;
+    float* depth = (float*)h->depth_dev.p;
+    int32_t* counts = (int32_t*)h->counts_out_dev.p;
+    {
+        InputScope scope(h, true, H_in, crop_top, nullptr);
+        if ((rc = enqueue(h, samples, B, H_in - crop_top, W, src_thr, val_thr, depth, nullptr, nullptr, nullptr, counts,
+                          nullptr, true)))
+            return rc;
+    }
+    // 3. Result.evaluate of the filled depth against the same rows of the ground-truth samples, in numpy's summation
+    //    order whatever dtfill_set_metrics_exact says
+    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
+    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
+    double* pf_d = (double*)h->per_frame.p;
+    double* sm_d = (double*)h->sums.p;
+    const uint16_t* g_d = gt_dev ? gt_dev : samples + (size_t)B * npx_in;
+    if (floor) {
+        const K4xWindow rows{npx_in, W, crop_top, 0, W};
+        rc = k4x_enqueue<double, 0, uint16_t, false, true>(h, depth, g_d, B, npx, pf_d, s, rows);
+    } else {
+        rc = k4x_enqueue<double, 0>(h, depth, g_d, B, npx, pf_d, s);
+    }
+    if (rc) return rc;
+    k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(st_host, status, (size_t)nfiles * 4, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(st_host + nfiles, counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
+    if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
+    if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
+    int fill_bad = -1;
+    rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
+    h->last_h2d_bytes = h2d;
+    h->last_d2h_bytes = (size_t)nfiles * 4 + (size_t)B * (8 + (per_frame ? 9 * 8 : 0)) + (sums ? 10 * 8 : 0);
+    if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
+    // 4. the verdict, frame by frame as the loop meets it: a decode failure (LiDAR before ground truth) wins over an
+    //    IndexError of Distance_Transform
+    for (int b = 0; b < B; ++b) {
+        const bool lid_bad = st_host[b] != png::ST_OK;
+        if (lid_bad || (!gt_dev && st_host[B + b] != png::ST_OK)) {
+            const int st = lid_bad ? st_host[b] : st_host[B + b];
+            if (first_bad_frame) *first_bad_frame = b;
+            return fail(DTFILL_E_DATA, std::string(lid_bad ? "LiDAR" : "ground-truth") + " file " + std::to_string(b) + ": " +
+                                           png_reason(st) + " (status " + std::to_string(st) + ")");
+        }
+    }
+    return fill_verdict(rc, fill_bad, st_host + nfiles, B, "LiDAR file ", first_bad_frame);
+}
+
+}  // namespace
+
 int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets, const uint8_t* gt,
                     const int64_t* gt_offsets, int B, int H, int W, float src_thr, float val_thr, double* per_frame,
                     double* sums, int* first_bad_frame) {
@@ -1918,65 +2000,25 @@ int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offs
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_eval_png: B, H, W must be positive");
     if ((int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28))
         return fail(DTFILL_E_ARG, "dtfill_eval_png: frame too large (H * (1 + 2 W) < 2^28 bytes)");
-    CU(cudaSetDevice(h->device));
-    const long npx = (long)H * W;
-    cudaStream_t s = h->stream;
-    int rc;
-    // 1. one decode of the 2B files (one warp per file, so the call costs about the slowest file, not two files in a row):
-    //    LiDAR file b -> samples / status b, ground-truth file b -> samples / status B + b
-    if ((rc = ensure(h, h->png_samples, (size_t)2 * B * npx * 2))) return rc;
-    if ((rc = ensure(h, h->png_status, (size_t)2 * B * 4))) return rc;
-    int32_t* st_host = nullptr;                   // [2B] decode status, then the fill's counts [B][2]
-    if ((rc = png_status_host(h, 4 * B, &st_host))) return rc;
-    uint16_t* samples = (uint16_t*)h->png_samples.p;
-    int32_t* status = (int32_t*)h->png_status.p;
-    const PngFiles sets[2] = {{lidar, lidar_offsets, B}, {gt, gt_offsets, B}};
-    const uint8_t* d_data;
-    const int64_t* d_off;
-    if ((rc = png_stage(h, sets, 2, &d_data, &d_off))) return rc;
-    const size_t h2d = h->last_h2d_bytes;
-    if ((rc = png_enqueue(h, d_data, d_off, 1, 2 * B, H, W, samples, status))) return rc;
-    // 2. the fill of dtfill_run_u16 (no crop) on the LiDAR samples, strict order on the handle's stream; only the counts
-    //    leave the device
-    if ((rc = ensure(h, h->depth_dev, (size_t)B * npx * 4))) return rc;
-    if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc;
-    float* depth = (float*)h->depth_dev.p;
-    int32_t* counts = (int32_t*)h->counts_out_dev.p;
-    {
-        InputScope scope(h, true, H, 0, nullptr);
-        if ((rc = enqueue(h, samples, B, H, W, src_thr, val_thr, depth, nullptr, nullptr, nullptr, counts, nullptr, true)))
-            return rc;
-    }
-    // 3. Result.evaluate of the filled depth against the ground-truth samples, in numpy's summation order whatever
-    //    dtfill_set_metrics_exact says
-    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
-    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
-    double* pf_d = (double*)h->per_frame.p;
-    double* sm_d = (double*)h->sums.p;
-    if ((rc = k4x_enqueue<double, 0>(h, depth, samples + (size_t)B * npx, B, npx, pf_d, s))) return rc;
-    k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(st_host, status, (size_t)2 * B * 4, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(st_host + 2 * B, counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
-    if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
-    int fill_bad = -1;
-    rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
-    h->last_h2d_bytes = h2d;
-    h->last_d2h_bytes = (size_t)B * (2 * 4 + 8 + (per_frame ? 9 * 8 : 0)) + (sums ? 10 * 8 : 0);
-    if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
-    // 4. the verdict, frame by frame as the notebook's loop meets it: a decode failure (LiDAR before ground truth) wins
-    //    over an IndexError of Distance_Transform
-    for (int b = 0; b < B; ++b) {
-        const bool lid_bad = st_host[b] != png::ST_OK;
-        if (lid_bad || st_host[B + b] != png::ST_OK) {
-            const int st = lid_bad ? st_host[b] : st_host[B + b];
-            if (first_bad_frame) *first_bad_frame = b;
-            return fail(DTFILL_E_DATA, std::string(lid_bad ? "LiDAR" : "ground-truth") + " file " + std::to_string(b) + ": " +
-                                           png_reason(st) + " (status " + std::to_string(st) + ")");
-        }
-    }
-    return fill_verdict(rc, fill_bad, st_host + 2 * B, B, "LiDAR file ", first_bad_frame);
+    return eval_png_run(h, lidar, lidar_offsets, gt, gt_offsets, nullptr, B, H, W, 0, false, src_thr,
+                        val_thr, per_frame, sums, first_bad_frame);
+}
+
+int dtfill_eval_png_kitti(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets, const uint8_t* gt,
+                          const int64_t* gt_offsets, const uint16_t* gt_samples_dev, int B, int H_in, int W, int crop_top,
+                          float src_thr, float val_thr, double* per_frame, double* sums, int* first_bad_frame) {
+    const char* who = "dtfill_eval_png_kitti";
+    if (first_bad_frame) *first_bad_frame = -1;
+    if (!h || !lidar || !lidar_offsets) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, LiDAR files or offsets");
+    const bool files = gt || gt_offsets;
+    if (files == (gt_samples_dev != nullptr) || (files && !(gt && gt_offsets)))
+        return fail(DTFILL_E_ARG, std::string(who) + ": give the ground truth either as files and offsets or as device samples");
+    if (B <= 0 || H_in <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H_in, W must be positive");
+    if (crop_top < 0 || crop_top >= H_in) return fail(DTFILL_E_ARG, std::string(who) + ": crop_top must lie in [0, H_in)");
+    if ((int64_t)H_in * (1 + 2 * (int64_t)W) >= (1ll << 28))
+        return fail(DTFILL_E_ARG, std::string(who) + ": frame too large (H_in * (1 + 2 W) < 2^28 bytes)");
+    return eval_png_run(h, lidar, lidar_offsets, gt, gt_offsets, gt_samples_dev, B, H_in, W, crop_top, true, src_thr,
+                        val_thr, per_frame, sums, first_bad_frame);
 }
 
 int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, const int32_t* rows,

@@ -20,7 +20,8 @@ namespace dtfill {
 // k4_metrics_partial agree with numpy's float32 pairwise sums only to ~1e-5.
 //   k4x_compact  one block per frame: the terms of the valid pixels, compacted in raster order (ballots + warp ranks);
 //                the ground truth is stored as the arithmetic type or, in KITTI mode, as 16-bit PNG samples; the WIN
-//                instance (NYU mode, float32) scores a crop window of the frames
+//                instance (NYU mode, float32) scores a crop window of the frames, the CROP_FLOOR instance (KITTI mode,
+//                u16 samples) the rows crop_top: of the ground truth against a floored prediction of those rows
 //   k4x_reduce   one block per frame: the leaves (<= 128 elements) of the tree in parallel, then the tree itself
 // Terms: 0 |d|^2, 1 |d| (KITTI) or |d| / t (NYU), 2 |dinv|^2, 3 |dinv|; counts: valid, delta1..3.
 // ------------------------------------------------------------------------------------------------------
@@ -89,18 +90,26 @@ struct K4xWindow {
     }
 };
 
+// The KITTI branch of eval_NYU.py (CROP_FLOOR instances, dtfill_eval_png_kitti): the prediction holds only rows
+// win.r0: of the ground truth's frames of win.frame_px = H_in * W samples, so prediction frame b is the npx pixels from
+// b * npx and ground-truth frame b the npx samples from b * win.frame_px + win.r0 * win.W (the rows are a contiguous
+// suffix of the frame).  The prediction is floored in registers, before the validity test and the terms:
+// relu(pred - 0.9) + 0.9 (eval_NYU.py:202-206, float32) equals fmaxf(pred, 0.9f) on every value the fill gives from PNG
+// samples (s / 256, s in 0..65535; pinned by tests/test_eval_kitti_png.py).
 // npx: pixels per frame, or per window (WIN); the term arrays hold npx entries per frame either way
-template <typename GT, int MODE, typename GS = GT, bool WIN = false>
+template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool CROP_FLOOR = false>
 __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restrict__ pred, const GS* __restrict__ gt, long npx,
                                                             GT* __restrict__ terms /*[frames][4][npx]*/,
                                                             int* __restrict__ counts /*[frames][4]*/, const K4xWindow win)
 {
+    static_assert(!(WIN && CROP_FLOOR), "a window or the KITTI branch's crop, not both");
     __shared__ int wtot[K4X_THREADS / 32], wbase[K4X_THREADS / 32];
     __shared__ int hits[3];
     const int b = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     auto px = [&](long i) -> long { if constexpr (WIN) return win.at(i); else return i; };
     const float* p = pred + (long)b * (WIN ? win.frame_px : npx);
-    const GS* g = gt + (long)b * (WIN ? win.frame_px : npx);
+    const GS* g = gt + (CROP_FLOOR ? (long)b * win.frame_px + (long)win.r0 * win.W : (long)b * (WIN ? win.frame_px : npx));
+    auto out = [&](long i) -> float { if constexpr (CROP_FLOOR) return fmaxf(p[i], 0.9f); else return p[px(i)]; };
     GT* tb = terms + (long)b * 4 * npx;
     const long seg = ((npx + K4X_THREADS - 1) / K4X_THREADS) * 32;     // pixels per warp, a multiple of 32
     const long i0 = min(npx, wid * seg), i1 = min(npx, i0 + seg);
@@ -109,7 +118,7 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
     int cnt = 0;
     for (long c = i0; c < i1; c += 32) {
         const long i = c + lane;
-        const bool v = i < i1 && (p[px(i)] > 0.01f) && (gt_value<GT>(g[px(i)]) > (GT)0.01);     // u16: s >= 3
+        const bool v = i < i1 && (out(i) > 0.01f) && (gt_value<GT>(g[px(i)]) > (GT)0.01);     // u16: s >= 3
         cnt += __popc(__ballot_sync(0xffffffffu, v));
     }
     if (lane == 0) wtot[wid] = cnt;
@@ -130,7 +139,7 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
         const long i = c + lane;
         GT term[4] = {0, 0, 0, 0};
         int hit[3] = {0, 0, 0};
-        const bool v = i < i1 && metric_terms<GT, MODE>(p[px(i)], gt_value<GT>(g[px(i)]), term, hit);
+        const bool v = i < i1 && metric_terms<GT, MODE>(out(i), gt_value<GT>(g[px(i)]), term, hit);
         const uint32_t m = __ballot_sync(0xffffffffu, v);
         if (v) {
             const long k = run + __popc(m & lanemask_lt());

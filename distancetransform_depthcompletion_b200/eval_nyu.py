@@ -5,6 +5,7 @@ script's evaluation loop on the GPU.
     Distance_Transform(lidar)      -> depth_map [H,W]    eval_NYU.py:120-133  (any size, dtype of the input)
     nyu_sample_coords(n)           -> (rows, cols)       data_read.py:360-364 (the random sample of one frame)
     evaluate_fill_sampled(gt, rows, cols) -> (per_frame [B,9], sums [10])   eval_NYU.py:138-254 from dense ground truth
+    evaluate_fill_kitti_png_files(lidar_files, gt) -> (per_frame [B,9], sums [10])   the script's KITTI branch, from files
 """
 from __future__ import annotations
 
@@ -16,6 +17,7 @@ from .tools import nearest_point as _nearest_point
 
 NYU_SRC_THR = 0.001     # eval_NYU.py:115
 NYU_EVAL_CROP = (6, 234, 8, 312)      # eval_NYU.py:202-207: rows 6:234, columns 8:312 of the 240 x 320 frames are scored
+KITTI_CROP_TOP = 96     # eval_NYU.py:151-165: the KITTI branch drops the first 96 rows of LiDAR and ground truth
 
 
 def nearest_point(refined_lidar, device: int | None = None):
@@ -175,3 +177,68 @@ def _aligned(t):
     as a rule, else a copy."""
     t = t.contiguous()
     return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+def evaluate_fill_kitti_png_files(lidar_files, gt, crop_top: int = KITTI_CROP_TOP, src_thr: float = NYU_SRC_THR,
+                                  device: int | None = None):
+    """The KITTI branch of eval_NYU.py's evaluation loop, from the PNG files, in one call on the GPU.  The script is not
+    part of this checkout; this follows SURVEY.md's record of it (section 3 B):
+
+        for i in range(B):
+            lidar = np.array(Image.open(lidar_files[i])).astype(np.float32) / 256    data_read.py:215
+            gt = np.array(Image.open(gt_files[i])) / 256.                            data_read.py:223 (float64)
+            lidar, gt = lidar[crop_top:], gt[crop_top:]                              eval_NYU.py:151-165
+            pred = Distance_Transform(lidar, src_thr)                                eval_NYU.py:120-133 (0.001, :115)
+            pred = relu(pred - 0.9) + 0.9                                            eval_NYU.py:202-206 (float32)
+            result.evaluate(pred, gt)                                                evaluation.py:82-123
+
+    lidar_files: paths or the files' bytes, 16-bit grayscale PNGs all of the size H_in x W of the first file.  gt: the
+    ground truth as B such files, or as a uint16 CUDA tensor [B,H_in,W] of their samples (DTFillEngine.decode_png gives
+    one), used in place on its own device: then only the LiDAR files go up, so a sweep over LiDAR densities against the
+    same ground truth decodes it once.  Returns (per_frame float64 [B,9], sums float64 [10]) in the layout of
+    evaluation.evaluate_batch: row b is [mse, rmse, mae, irmse, imae, 0, 0, 0, n_valid] of frame b, equal to
+    Result.evaluate's bit for bit (a frame whose ground truth has no valid pixel gives numpy's mean of an empty array),
+    and sums holds the column sums followed by B.  The division by the frame count (1000 in the reference) stays with
+    the caller: sharding.finalize_means(sums).  device: the GPU that runs the call for ground-truth files; a tensor runs
+    on its own device (a different device raises ValueError).
+
+    Raises, before the device is touched: ValueError for empty or unequal lists, a first LiDAR file that is not a PNG,
+    crop_top outside [0, H_in) and a tensor whose shape is not [B,H_in,W]; TypeError for a tensor that is not uint16 or
+    not on a CUDA device.  Then ValueError for the first frame with a file that is not an intact 16-bit grayscale PNG of
+    that size (naming the LiDAR or the ground-truth list and the frame; the LiDAR file wins at the same frame), and
+    otherwise IndexError for the first frame Distance_Transform rejects in the cropped rows (no valid depth, exactly one
+    valid depth, labels outside the list of valid depths)."""
+    from .data_read import pack_png_files
+    from .tools import VALID_THR
+    who = "evaluate_fill_kitti_png_files"
+    lidar_files = list(lidar_files)
+    is_tensor = type(gt).__module__.startswith("torch")
+    gt_files = None if is_tensor else list(gt)
+    if not lidar_files or (gt_files is not None and not gt_files):
+        raise ValueError(f"{who}: no files")
+    B = len(lidar_files)
+    if gt_files is not None and len(gt_files) != B:
+        raise ValueError(f"{who}: {B} LiDAR files but {len(gt_files)} ground-truth files")
+    try:       # the size comes from the first LiDAR file's IHDR
+        data, offsets, H_in, W = pack_png_files(lidar_files + (gt_files or []))
+    except ValueError:
+        raise ValueError(f"{who}: LiDAR file 0 is not a PNG file") from None
+    crop_top = int(crop_top)
+    if not 0 <= crop_top < H_in:
+        raise ValueError(f"{who}: crop_top {crop_top} outside [0, {H_in}) for frames of {H_in} rows")
+    if gt_files is not None:
+        return _lib.get_handle(device).eval_png_kitti(data, offsets[:B + 1], data, offsets[B:], None, H_in, W, crop_top,
+                                                      src_thr, VALID_THR)
+    import torch
+    if gt.dtype != torch.uint16:
+        raise TypeError(f"{who}: ground-truth tensor dtype {gt.dtype} not supported (uint16 PNG samples only)")
+    if tuple(gt.shape) != (B, H_in, W):
+        raise ValueError(f"{who}: ground-truth tensor of shape {tuple(gt.shape)}, the LiDAR files need {(B, H_in, W)}")
+    if not gt.is_cuda:
+        raise TypeError(f"{who}: the ground-truth tensor must be on a CUDA device, got {gt.device}")
+    if device is not None and int(device) != gt.device.index:
+        raise ValueError(f"{who}: device={device} but the ground truth is on {gt.device}")
+    gt = gt.contiguous()
+    torch.cuda.current_stream(gt.device).synchronize()      # the handle's stream reads gt
+    return _lib.get_handle(gt.device.index).eval_png_kitti(data, offsets, None, None, gt.data_ptr(), H_in, W, crop_top,
+                                                           src_thr, VALID_THR)

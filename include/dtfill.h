@@ -233,6 +233,32 @@ int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offs
                     double* sums, int* first_bad_frame);
 
 /*
+ * The KITTI branch of the reference's eval_NYU.py evaluation loop, from the files (SURVEY.md section 3 B; the script is
+ * not part of this checkout, so this follows that record):
+ *     lidar = png.astype(float32) / 256;  gt = png / 256.  (float64)     data_read.py:215 / :223
+ *     lidar, gt = lidar[crop_top:], gt[crop_top:]                         eval_NYU.py:151-165 (crop_top 96)
+ *     pred = Distance_Transform(lidar, src_thr)                           eval_NYU.py:120-133 (src_thr 0.001, :115)
+ *     pred = relu(pred - 0.9) + 0.9                                       eval_NYU.py:202-206 (float32)
+ *     Result().evaluate(pred, gt)                                         evaluation.py:82-123
+ * for B LiDAR files of H_in x W (host, laid out as for dtfill_png_decode) against B ground-truth frames given either as
+ * host files (gt, gt_offsets; gt_samples_dev NULL) or as resident uint16 samples gt_samples_dev [B,H_in,W] on the handle's
+ * device (gt and gt_offsets NULL), which are read in place and never copied: exactly one form.  Files are decoded in one
+ * launch, rows crop_top: of the LiDAR samples filled as by dtfill_run_u16, and the metrics of the filled rows, floored at
+ * 0.9 in registers, computed against the same rows of the ground truth in KITTI mode and numpy's summation order, so
+ * that per_frame [B][DTFILL_METRIC_COLS] and sums [DTFILL_METRIC_COLS + 1] (host, nullable; layout of dtfill_metrics)
+ * equal the reference's bit for bit.  No per-pixel data crosses the link; with resident ground truth only the LiDAR files
+ * and their offsets go up.  Synchronous.
+ * Errors: DTFILL_E_ARG for crop_top outside [0, H_in) or not exactly one ground-truth form; then, frame by frame as the
+ * loop meets them, DTFILL_E_DATA for the first frame with a file that fails to decode (LiDAR before ground truth), which
+ * wins over DTFILL_E_INDEX for the first frame Distance_Transform rejects in the cropped rows (no valid depth, exactly one
+ * valid depth, labels outside the list of valid depths); *first_bad_frame receives the frame.  On an error the contents
+ * of per_frame and sums are unspecified.
+ */
+int dtfill_eval_png_kitti(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets, const uint8_t* gt,
+                          const int64_t* gt_offsets, const uint16_t* gt_samples_dev, int B, int H_in, int W, int crop_top,
+                          float src_thr, float val_thr, double* per_frame, double* sums, int* first_bad_frame);
+
+/*
  * The evaluation loop of the reference's NYU script (eval_NYU.py:138-254, data_read.py:337-371) from dense ground truth:
  *     Mask = zeros(H, W);  Mask[rows_b, cols_b] = 1                 data_read.py:360-364 (duplicates collapse)
  *     pred = Distance_Transform(gt_b * Mask, src_thr)               eval_NYU.py:120-133
