@@ -14,6 +14,7 @@
 #include <mutex>
 #include <thread>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "dtfill_kernels.cuh"
@@ -36,9 +37,14 @@ int fail(int code, const std::string& msg) {
             return fail(DTFILL_E_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));           \
     } while (0)
 
+// A device buffer of the handle, grown by ensure(); freed with the handle (dtfill_destroy synchronises first).
 struct Buf {
     void* p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(const Buf&) = delete;
+    Buf& operator=(const Buf&) = delete;
+    ~Buf() { if (p) cudaFree(p); }
 };
 
 }  // namespace
@@ -293,9 +299,14 @@ private:
     size_t nparts_ = 0, next_ = 0, done_ = 0;
 };
 
+// A pinned host buffer of the handle, grown by ensure_pinned(); freed with the handle.
 struct PinBuf {
     void* p = nullptr;
     size_t cap = 0;
+    PinBuf() = default;
+    PinBuf(const PinBuf&) = delete;
+    PinBuf& operator=(const PinBuf&) = delete;
+    ~PinBuf() { if (p) cudaFreeHost(p); }
 };
 
 // One "lane" = everything a call needs while it is in flight: workspace, streams, events.  A handle has two, so
@@ -346,25 +357,9 @@ struct dtfill_ctx {
     bool slot_rearm[STATUS_RING] = {}; // the slot's device words left their initial state: re-arm before the next use
     cudaStream_t status_stream = nullptr;
     cudaEvent_t status_fork = nullptr;
-    int* cur_status = nullptr;        // device status words of the call being enqueued
-    int cur_slot = 0;
-    bool cur_status_early = false;    // this call copies its status words to the host right behind k1b_scan_compact
-    bool cur_status_copied = false;
     int last_slot = 0;
     std::vector<void*> retired;       // device buffers replaced by larger ones; freed at the next synchronisation point
     size_t wide_smem_configured = 0;  // dynamic shared memory limit of k2_chamfer_wide raised so far on this device
-    bool cur_pipelined = false;       // the call being enqueued runs on a lane's own stream
-    // input of the call being enqueued: float32 frames [B,H,W], or uint16 PNG samples [B,in_H,W] of which rows
-    // [in_crop, in_crop + H) are the frame (dtfill_run_u16); lidar_dev: decoded float32 frames, optional
-    bool in_u16 = false;
-    int in_H = 0, in_crop = 0;
-    float* lidar_dev = nullptr;
-    // ... or dense float32 ground truth [B,H,W] of which K1 keeps the pixels of the sample bitmap that k10_sample_bits left
-    // in lane 0's srcbits (dtfill_eval_sampled)
-    bool in_sampled = false;
-    // evaluation fused behind the call being enqueued (dtfill_run_eval_async): ground truth, mode
-    const void* ev_gt = nullptr;
-    int ev_gt_f64 = 0, ev_mode = 0;
     int pipeline_depth = 1;           // 1: strict stream order (default); 2: consecutive calls may overlap
     cudaEvent_t pipe_fork = nullptr;
     Buf in_dev, depth_dev, dt_dev, lbl_dev, mask_dev, counts_out_dev, lidar_out_dev;   // staging for host-pointer calls
@@ -541,20 +536,65 @@ static float source_cut(float thr) {
 
 constexpr int MAX_COL_TILES = 4;      // planner: at most this many half-width tiles side by side in a band
 
-// Enqueue the path for frames [b0, b0+nb) of the batch on stream s; all pointers are device pointers to the whole
-// batch, the workspace is sliced per frame so sub-batches never share anything but the status words.
-int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0, int nb, int Btot, const void* in, int H, int W,
-                  float src_thr, float val_thr, float* out_depth, float* out_dt, int32_t* out_lbl, uint8_t* out_mask,
-                  int32_t* out_counts, int scratch_units_per_frame, int sub_index, int* launches) {
+// What one fill reads and writes, built by each entry point and passed down to enqueue.  Device pointers to the whole
+// batch.
+struct FillCall {
+    // F32: float32 frames [B,H,W].  U16: uint16 PNG samples [B,in_H,W] of which rows [crop, crop + H) are the frame
+    // (dtfill_run_u16).  SAMPLED: dense float32 ground truth [B,H,W] of which K1 keeps the pixels of the sample bitmap
+    // that k10_sample_bits left in lane 0's srcbits (dtfill_eval_sampled).
+    enum Kind { F32, U16, SAMPLED };
+    Kind kind = F32;
+    const void* in = nullptr;
+    int in_H = 0, crop = 0;           // U16 only
+    float* lidar = nullptr;           // optional: the decoded float32 frames (U16, SAMPLED)
+    int B = 0, H = 0, W = 0;
+    float src_thr = 0.f, val_thr = 0.f;
+    float* depth = nullptr;
+    float* dt = nullptr;
+    int32_t* lbl = nullptr;
+    uint8_t* mask = nullptr;
+    int32_t* counts = nullptr;
+    // optional evaluation fused behind the fill (dtfill_run_eval_async): ground truth [B,H,W], float64 or float32, mode
+    const void* eval_gt = nullptr;
+    int eval_gt_f64 = 0, eval_mode = 0;
+};
+
+// Bookkeeping of one enqueue, shared by its sub-batches.
+struct EnqueueState {
+    bool pipelined = false;           // the call runs on a lane's own stream
+    int* status = nullptr;            // the call's device status words, slot `slot` of the ring
+    int slot = 0;
+    bool status_early = false;        // copy the status words to the host right behind k1b_scan_compact ...
+    bool status_copied = false;       // ... which enqueue_range did
+    int launches = 0;
+};
+
+// K1 on input of type T, one warp per row: the 128-bit-load kernel where rows start 16-byte aligned (W % 4 for 4-byte
+// pixels, W % 8 for uint16 samples), in its whole-group form when W % 16 == 0; the scalar kernel otherwise.  Frame
+// fp.frame0 starts fp.in_H rows into the input (in_H = H but for uint16 samples with a crop).
+template <typename T>
+void launch_k1(const void* in, int grid, int threads, cudaStream_t s, const FrameParams& fp, const Workspace& ws, uint8_t* om,
+               float* olid) {
+    const T* in_s = (const T*)in + (size_t)fp.frame0 * fp.in_H * fp.W;
+    if ((fp.W & 15) == 0) k1_mask_rows_v16<T, true><<<grid, threads, 0, s>>>(in_s, fp, ws, om, olid);
+    else if (fp.W % (int)(16 / sizeof(T)) == 0) k1_mask_rows_v16<T, false><<<grid, threads, 0, s>>>(in_s, fp, ws, om, olid);
+    else k1_mask_rows<T><<<grid, threads, 0, s>>>(in_s, fp, ws, om, olid);
+}
+
+// Enqueue the path for frames [b0, b0+nb) of call c on stream s; the workspace is sliced per frame so sub-batches never
+// share anything but the status words.
+int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const FillCall& c, const Plan& plan, int b0, int nb,
+                  int scratch_units_per_frame, int sub_index, EnqueueState& state) {
+    const int H = c.H, W = c.W;
     const int WW = (W + 31) / 32;
     const size_t rows0 = (size_t)b0 * H, npx0 = rows0 * W;
     const size_t rows = (size_t)nb * H;
     FrameParams fp;
     fp.B = nb; fp.H = H; fp.W = W; fp.WW = WW;
-    fp.in_H = h->in_u16 ? h->in_H : H;
-    fp.in_crop = h->in_u16 ? h->in_crop : 0;
-    fp.src_thr = src_thr; fp.val_thr = val_thr;
-    fp.src_cut = source_cut(src_thr);
+    fp.in_H = c.kind == FillCall::U16 ? c.in_H : H;
+    fp.in_crop = c.kind == FillCall::U16 ? c.crop : 0;
+    fp.src_thr = c.src_thr; fp.val_thr = c.val_thr;
+    fp.src_cut = source_cut(c.src_thr);
     fp.init_dist = H + W + 8;
     fp.force_wide = plan.ppl == 0;
     fp.scratch_units_per_frame = scratch_units_per_frame;
@@ -565,8 +605,8 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
     // strict order with two scan instances: k3_sky follows the full-width instance on the side stream (see the planner)
     // -- while the scan leaves SMs idle: measured on KITTI frames, 4 / 16 / 32 / 64 frames per call -4 / -10 / -9 / -2 %,
     // 128 / 256 frames +4 / +2 % (the wide instance then takes registers from the narrow tiles)
-    fp.sky_split = (!h->cur_pipelined && !h->profiling && plan.ppl && plan.narrow && fp.sky_min > 0 && W <= SKY_MAX_W &&
-                    (long)Btot * H * W <= 28000000L) ? 1 : 0;
+    fp.sky_split = (!state.pipelined && !h->profiling && plan.ppl && plan.narrow && fp.sky_min > 0 && W <= SKY_MAX_W &&
+                    (long)c.B * H * W <= 28000000L) ? 1 : 0;
     fp.max_col_tiles = MAX_COL_TILES;
     fp.mul_dist = 1u << (32 - DSH);
     fp.four = 4u;
@@ -580,7 +620,7 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
             // tiles wanted per frame; with batches overlapping (pipelined mode) fewer, taller tiles do: they carry
             // less halo redundancy and the other batches in flight fill the SMs
             // (measured on 256 KITTI frames, 4 batches in flight: target 260 -> 0.417 ms per step, 202 -> 0.426, 330 -> 0.419)
-            const long beff = h->pipeline_depth > 1 ? (9L * Btot + 3) / 4 : Btot;
+            const long beff = h->pipeline_depth > 1 ? (9L * c.B + 3) / 4 : c.B;
             const long per_frame = ((long)h->sm_count * 28 + beff - 1) / beff;
             if (per_frame <= 1) cap = 0;                                              // batch alone fills the GPU
             else {
@@ -588,7 +628,7 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
                 cap = (int)(2 * band_rows + 42);
                 // (the floor: bands shorter than twice their halo are not cut anyway; measured on KITTI frames, 1 / 4 frames
                 // per call 0.129 -> 0.119 / 0.133 -> 0.126 ms with 80 instead of 96, 16 frames 0.144 -> 0.150)
-                const int floor_cap = Btot <= 8 ? 80 : 96;
+                const int floor_cap = c.B <= 8 ? 80 : 96;
                 if (cap < floor_cap) cap = floor_cap;
             }
         }
@@ -604,15 +644,15 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
     ws.dlist = (float*)L->dlist.p + npx0;
     ws.scratch = (uint32_t*)L->scratch.p + (size_t)b0 * scratch_units_per_frame * 32;
     ws.tasks = (Task*)L->tasks.p + (size_t)b0 * MAXT;
-    ws.status = h->cur_status;
+    ws.status = state.status;
     ws.sky = (int*)L->sky.p + b0;
     ws.skykeys = (uint32_t*)L->skykeys.p + (size_t)b0 * 2 * W;
-    float* olid = h->lidar_dev ? h->lidar_dev + npx0 : nullptr;
-    float* od = out_depth + npx0;
-    float* odt = out_dt ? out_dt + npx0 : nullptr;
-    int32_t* ol = out_lbl ? out_lbl + npx0 : nullptr;
-    uint8_t* om = out_mask ? out_mask + npx0 : nullptr;
-    int32_t* oc = out_counts ? out_counts + 2 * (size_t)b0 : nullptr;
+    float* olid = c.lidar ? c.lidar + npx0 : nullptr;
+    float* od = c.depth + npx0;
+    float* odt = c.dt ? c.dt + npx0 : nullptr;
+    int32_t* ol = c.lbl ? c.lbl + npx0 : nullptr;
+    uint8_t* om = c.mask ? c.mask + npx0 : nullptr;
+    int32_t* oc = c.counts ? c.counts + 2 * (size_t)b0 : nullptr;
 
     if (h->profiling) CU(cudaEventRecord(h->ev[0], s));
     if (!(h->debug_skip & 1)) {   // K1: one warp per row
@@ -622,34 +662,23 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
         const int wpb = k1_threads / 32;
         long want = ((long)rows + wpb - 1) / wpb;
         int grid = (int)(want < 1 ? 1 : want);
-        if (h->in_sampled) {
-            const SampledGt* in_s = (const SampledGt*)in + npx0;
-            if ((W & 15) == 0) k1_mask_rows_v16<SampledGt, true><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
-            else if ((W & 3) == 0) k1_mask_rows_v16<SampledGt, false><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
-            else k1_mask_rows<SampledGt><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
-        } else if (!h->in_u16) {
-            const float* in_s = (const float*)in + npx0;
-            if ((W & 15) == 0) k1_mask_rows_v16<float, true><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
-            else if ((W & 3) == 0) k1_mask_rows_v16<float, false><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
-            else k1_mask_rows<float><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, nullptr);
-        } else {
-            const uint16_t* in_s = (const uint16_t*)in + (size_t)b0 * h->in_H * W;
-            if ((W & 15) == 0) k1_mask_rows_v16<uint16_t, true><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
-            else if ((W & 7) == 0) k1_mask_rows_v16<uint16_t, false><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
-            else k1_mask_rows<uint16_t><<<grid, k1_threads, 0, s>>>(in_s, fp, ws, om, olid);
+        switch (c.kind) {
+            case FillCall::F32: launch_k1<float>(c.in, grid, k1_threads, s, fp, ws, om, olid); break;
+            case FillCall::U16: launch_k1<uint16_t>(c.in, grid, k1_threads, s, fp, ws, om, olid); break;
+            case FillCall::SAMPLED: launch_k1<SampledGt>(c.in, grid, k1_threads, s, fp, ws, om, olid); break;
         }
-        ++*launches;
+        ++state.launches;
     }
     if (h->profiling) CU(cudaEventRecord(h->ev[1], s));
     if (!(h->debug_skip & 2)) {
         k1b_scan_compact<<<nb, K1B_THREADS, 0, s>>>(fp, ws, oc);
-        ++*launches;
-        if (h->cur_status_early) {       // the status words are final: to the host on the status stream
+        ++state.launches;
+        if (state.status_early) {        // the status words are final: to the host on the status stream
             CU(cudaEventRecord(h->status_fork, s));
             CU(cudaStreamWaitEvent(h->status_stream, h->status_fork, 0));
-            CU(cudaMemcpyAsync(h->status_ring + 2 * h->cur_slot, h->cur_status, 8, cudaMemcpyDeviceToHost, h->status_stream));
-            CU(cudaEventRecord(h->slot_done[h->cur_slot], h->status_stream));
-            h->cur_status_copied = true;
+            CU(cudaMemcpyAsync(h->status_ring + 2 * state.slot, state.status, 8, cudaMemcpyDeviceToHost, h->status_stream));
+            CU(cudaEventRecord(h->slot_done[state.slot], h->status_stream));
+            state.status_copied = true;
         }
     }
     if (h->profiling) CU(cudaEventRecord(h->ev[2], s));
@@ -672,7 +701,7 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
     if (two) {
         if (fp.narrow_ppl == 20) launch_k2<20>(false, want_lbl, nb * MAXT, s_narrow, fp, ws, od, odt, ol, TASK_NARROW);
         else launch_k2<10>(false, want_lbl, nb * MAXT, s_narrow, fp, ws, od, odt, ol, TASK_NARROW);
-        ++*launches;
+        ++state.launches;
     }
     if (run_k2) switch (plan.ppl) {
         case 10: launch_k2<10>(plan.pad, want_lbl, nb * MAXT, s_full, fp, ws, od, odt, ol, TASK_CHAMFER); break;
@@ -680,20 +709,20 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
         case 38: launch_k2<38>(plan.pad, want_lbl, nb * MAXT, s_full, fp, ws, od, odt, ol, TASK_CHAMFER); break;
         default: launch_k2<10>(true, want_lbl, nb * MAXT, s_full, fp, ws, od, odt, ol, TASK_CHAMFER); break;  // NOSRC only
     }
-    if (run_k2) ++*launches;
+    if (run_k2) ++state.launches;
     // 64-bit-key fallback: returns immediately for every task the fast kernels handle.  It touches other frames
     // than they do, so it runs next to the narrow tiles; only per-kernel profiling serialises it behind the join.
     const size_t wide_smem = (size_t)3 * (W + 4) * sizeof(uint64_t);
     if (!h->profiling && run_k2) {
         k2_chamfer_wide<<<nb, 32, wide_smem, s_full>>>(fp, ws, od, odt, ol);
-        ++*launches;
+        ++state.launches;
     }
     const bool run_sky = fp.band_cap > 0 && fp.sky_min > 0 && W <= SKY_MAX_W && !(h->debug_skip & 8);
     bool sky_done = false;
     if (two && narrow_main && fp.sky_split && run_sky) {
         // the base rows of every frame come from the full-width instance just launched on the side stream
         k3_sky<<<dim3(nb, (H + SKY_ROWS - 1) / SKY_ROWS), 256, 0, s_side>>>(fp, ws, od, odt, ol);
-        ++*launches;
+        ++state.launches;
         sky_done = true;
     }
     if (two) {
@@ -703,24 +732,52 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const Plan& plan, int b0
     if (h->profiling) {
         CU(cudaEventRecord(h->ev[3], s));
         k2_chamfer_wide<<<nb, 32, wide_smem, s>>>(fp, ws, od, odt, ol);
-        ++*launches;
+        ++state.launches;
         CU(cudaEventRecord(h->ev[4], s));
     }
     // rows above the first source row, from the two base rows the scan left in ws.skykeys (blocks of frames without
     // such rows return at once)
     if (run_sky && !sky_done) {
         k3_sky<<<dim3(nb, (H + SKY_ROWS - 1) / SKY_ROWS), 256, 0, s>>>(fp, ws, od, odt, ol);
-        ++*launches;
+        ++state.launches;
     }
     if (h->profiling) CU(cudaEventRecord(h->ev[5], s));
     return 0;
 }
 
-// Enqueue the whole path on h->stream; all pointers are device pointers.
-int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, float val_thr, float* out_depth,
-            float* out_dt, int32_t* out_lbl, uint8_t* out_mask, int32_t* out_counts, const HostIO* hio = nullptr,
-            bool force_strict = false) {
-    if (!h || !in || !out_depth) return fail(DTFILL_E_ARG, "dtfill_run: NULL handle, input or out_depth");
+// fn(GT(), std::integral_constant<int, MODE>()) for a float64 (gt_f64) or float32 ground truth and metric mode 0 or 1
+template <typename Fn>
+int with_gt_mode(int gt_f64, int mode, Fn&& fn) {
+    using Kitti = std::integral_constant<int, DTFILL_METRICS_KITTI>;
+    using Nyu = std::integral_constant<int, DTFILL_METRICS_NYU>;
+    if (gt_f64) return mode == DTFILL_METRICS_KITTI ? fn(double(), Kitti()) : fn(double(), Nyu());
+    return mode == DTFILL_METRICS_KITTI ? fn(float(), Kitti()) : fn(float(), Nyu());
+}
+
+// One-pass metrics of B frames of npx pixels (k4_metrics_partial, k4_metrics_final): per_frame [B,9], sums [10] (added to
+// when accumulate); the chunk partials go to `partial`.  Device pointers; enqueued on s.
+int metrics_onepass(dtfill_t* h, Buf& partial, const float* pred, const void* gt, int gt_f64, int mode, int B, long npx,
+                    double* per_frame, double* sums, int accumulate, cudaStream_t s) {
+    int chunks = (int)((npx + 16383) / 16384);     // chunk boundaries stay multiples of 4 pixels when npx is
+    if (chunks < 1) chunks = 1;
+    if (chunks > 64) chunks = 64;
+    while (chunks > 1 && (((npx + chunks - 1) / chunks) & 3)) --chunks;
+    int rc;
+    if ((rc = ensure(h, partial, (size_t)B * chunks * ACC * 8))) return rc;
+    double* part = (double*)partial.p;
+    with_gt_mode(gt_f64, mode, [&](auto g, auto m) {
+        using GT = decltype(g);
+        k4_metrics_partial<GT, decltype(m)::value><<<dim3(chunks, B), 256, 0, s>>>(pred, (const GT*)gt, npx, chunks, part);
+        return 0;
+    });
+    k4_metrics_final<<<1, 256, 0, s>>>(part, B, chunks, mode, per_frame, sums, accumulate);
+    return 0;
+}
+
+// Enqueue the whole path of call c on h->stream.  hio: host buffers of a synchronous call, which c's device buffers stage.
+int enqueue(dtfill_t* h, const FillCall& c, const HostIO* hio = nullptr, bool force_strict = false) {
+    const int B = c.B, H = c.H, W = c.W;
+    if (!h || !c.in || !c.depth) return fail(DTFILL_E_ARG, "dtfill_run: NULL handle, input or out_depth");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_run: B, H, W must be positive");
     if ((long)H + W >= 60000 || (long)H * W >= (1l << 31) || W > 28000)
         return fail(DTFILL_E_ARG, "dtfill_run: frame size not supported (H + W < 60000, W <= 28000)");
@@ -728,9 +785,9 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
     // lane and stream of this call
     // synchronous entries (dtfill_run*) always run in strict order on the handle's stream: their device-to-host copies
     // and their status follow the kernels in stream order
-    const bool pipelined = h->pipeline_depth > 1 && !h->profiling && !hio && !force_strict;
-    Lane* L = &h->lanes[pipelined ? (h->ncalls % h->pipeline_depth) : 0];
-    h->cur_pipelined = pipelined;
+    EnqueueState state;
+    state.pipelined = h->pipeline_depth > 1 && !h->profiling && !hio && !force_strict;
+    Lane* L = &h->lanes[state.pipelined ? (h->ncalls % h->pipeline_depth) : 0];
     const Plan plan = make_plan(H, W);
     const int WW = (W + 31) / 32;
     const size_t rows = (size_t)B * H;
@@ -761,7 +818,7 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
     }
 
     cudaStream_t s = h->stream;
-    if (pipelined) {
+    if (state.pipelined) {
         // this call runs on the lane's own stream, behind whatever the caller queued so far and behind the lane's
         // previous call (stream order); the handle's stream only joins at dtfill_flush / dtfill_status.
         CU(cudaEventRecord(h->pipe_fork, h->stream));
@@ -772,7 +829,6 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
         for (Lane& o : h->lanes)
             if (o.pending) { CU(cudaStreamWaitEvent(h->stream, o.done, 0)); o.pending = false; }
     }
-    int launches = 0;
     // this call's slot of the status ring; a slot that dtfill_status has not examined yet keeps its verdict
     const int slot = h->ncalls % dtfill_ctx::STATUS_RING;
     if (h->slot_dirty[slot]) {
@@ -781,13 +837,12 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
         if (h->status_ring[2 * slot] != INT_MAX || h->status_ring[2 * slot + 1] != 0) h->slot_rearm[slot] = true;
         h->slot_dirty[slot] = false;
     }
-    h->cur_slot = slot;
-    h->cur_status = h->status_dev + (size_t)slot * dtfill_ctx::STATUS_STRIDE;
+    state.slot = slot;
+    state.status = h->status_dev + (size_t)slot * dtfill_ctx::STATUS_STRIDE;
     if (h->slot_rearm[slot] || (h->debug_skip & 2)) {      // (a run without k1b_scan_compact reports nothing)
-        CU(cudaMemcpyAsync(h->cur_status, h->status_init, 8, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(state.status, h->status_init, 8, cudaMemcpyHostToDevice, s));
         h->slot_rearm[slot] = false;
     }
-    h->cur_status_copied = false;
 
     // sub-batches on forked streams (skipped while per-kernel profiling is on: the event pairs need one stream)
     int nsub = h->nsub;
@@ -797,11 +852,11 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
     if (nsub > Lane::MAX_SUB) nsub = Lane::MAX_SUB;
     if (nsub > B) nsub = B;
     if (h->profiling || nsub < 1) nsub = 1;
-    h->cur_status_early = nsub == 1 && !(h->debug_skip & 2);     // slices share the words: their copy follows the last slice
+    state.status_early = nsub == 1 && !(h->debug_skip & 2);     // slices share the words: their copy follows the last slice
     void* dense_pin = hio ? hio->in_pin : nullptr;      // pinned mirror of a pageable input (allocated late on the sparse path)
     auto copy_in = [&](cudaStream_t st, int b0, int nb) -> int {
         if (!hio || !hio->in) return 0;
-        const size_t frame_bytes = h->in_u16 ? (size_t)h->in_H * W * 2 : (size_t)H * W * 4;
+        const size_t frame_bytes = c.kind == FillCall::U16 ? (size_t)c.in_H * W * 2 : (size_t)H * W * 4;
         const char* src = (const char*)hio->in + b0 * frame_bytes;
         if (hio->sparse_pin) {     // pageable float32 input: compact the slice on the host, rebuild it on the device
             const size_t o = (size_t)b0 * H * W, n = (size_t)nb * H * W;
@@ -812,7 +867,7 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
             const size_t cnt = n < (1ull << 32) ? h->pool_in->compact(pi, pv, cap, (const float*)src, n, hio->sparse_scut, hio->sparse_vthr)
                                                 : SIZE_MAX;
             if (cnt != SIZE_MAX) {
-                float* dst = (float*)const_cast<void*>(in) + o;
+                float* dst = (float*)const_cast<void*>(c.in) + o;
                 CU(cudaMemsetAsync(dst, 0, n * 4, st));
                 if (cnt) {
                     uint32_t* di = (uint32_t*)h->sparse_dev.p + ro;
@@ -836,28 +891,27 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
             h->pool_in->copy(pin, src, nb * frame_bytes);
             src = pin;
         }
-        CU(cudaMemcpyAsync((char*)const_cast<void*>(in) + b0 * frame_bytes, src, nb * frame_bytes, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync((char*)const_cast<void*>(c.in) + b0 * frame_bytes, src, nb * frame_bytes, cudaMemcpyHostToDevice, st));
         h->last_h2d_bytes += nb * frame_bytes;
         return 0;
     };
     auto copy_out = [&](cudaStream_t st, int b0, int nb) -> int {
         if (!hio) return 0;
         const size_t o = (size_t)b0 * H * W, n = (size_t)nb * H * W;
-        CU(cudaMemcpyAsync((hio->depth_pin ? hio->depth_pin : hio->depth) + o, out_depth + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->lidar) CU(cudaMemcpyAsync((hio->lidar_pin ? hio->lidar_pin : hio->lidar) + o, h->lidar_dev + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->dt) CU(cudaMemcpyAsync((hio->dt_pin ? hio->dt_pin : hio->dt) + o, out_dt + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->lbl) CU(cudaMemcpyAsync((hio->lbl_pin ? hio->lbl_pin : hio->lbl) + o, out_lbl + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->mask) CU(cudaMemcpyAsync((hio->mask_pin ? hio->mask_pin : hio->mask) + o, out_mask + o, n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync((hio->depth_pin ? hio->depth_pin : hio->depth) + o, c.depth + o, n * 4, cudaMemcpyDeviceToHost, st));
+        if (hio->lidar) CU(cudaMemcpyAsync((hio->lidar_pin ? hio->lidar_pin : hio->lidar) + o, c.lidar + o, n * 4, cudaMemcpyDeviceToHost, st));
+        if (hio->dt) CU(cudaMemcpyAsync((hio->dt_pin ? hio->dt_pin : hio->dt) + o, c.dt + o, n * 4, cudaMemcpyDeviceToHost, st));
+        if (hio->lbl) CU(cudaMemcpyAsync((hio->lbl_pin ? hio->lbl_pin : hio->lbl) + o, c.lbl + o, n * 4, cudaMemcpyDeviceToHost, st));
+        if (hio->mask) CU(cudaMemcpyAsync((hio->mask_pin ? hio->mask_pin : hio->mask) + o, c.mask + o, n, cudaMemcpyDeviceToHost, st));
         if (hio->counts)
-            CU(cudaMemcpyAsync(hio->counts + 2 * (size_t)b0, out_counts + 2 * (size_t)b0, (size_t)nb * 8,
+            CU(cudaMemcpyAsync(hio->counts + 2 * (size_t)b0, c.counts + 2 * (size_t)b0, (size_t)nb * 8,
                                cudaMemcpyDeviceToHost, st));
         h->last_d2h_bytes += n * (4 + (hio->lidar ? 4 : 0) + (hio->dt ? 4 : 0) + (hio->lbl ? 4 : 0) + (hio->mask ? 1 : 0));
         return 0;
     };
     if (nsub == 1 && !(hio && hio->any_out_pin())) {
         if ((rc = copy_in(s, 0, B))) return rc;
-        if ((rc = enqueue_range(h, L, s, plan, 0, B, B, in, H, W, src_thr, val_thr, out_depth, out_dt, out_lbl, out_mask,
-                                out_counts, scratch_units_per_frame, 0, &launches))) return rc;
+        if ((rc = enqueue_range(h, L, s, c, plan, 0, B, scratch_units_per_frame, 0, state))) return rc;
         if ((rc = copy_out(s, 0, B))) return rc;
     } else {
         // pageable outputs: a drain thread waits for each slice's device-to-host copies and moves the slice from the
@@ -892,8 +946,7 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
                 CU(cudaStreamWaitEvent(L->sub[i], L->fork_ev, 0));
                 int r;
                 if ((r = copy_in(L->sub[i], b0, b1 - b0))) return r;
-                if ((r = enqueue_range(h, L, L->sub[i], plan, b0, b1 - b0, B, in, H, W, src_thr, val_thr, out_depth, out_dt,
-                                       out_lbl, out_mask, out_counts, scratch_units_per_frame, i, &launches))) return r;
+                if ((r = enqueue_range(h, L, L->sub[i], c, plan, b0, b1 - b0, scratch_units_per_frame, i, state))) return r;
                 if ((r = copy_out(L->sub[i], b0, b1 - b0))) return r;
                 CU(cudaEventRecord(L->join_ev[i], L->sub[i]));
                 CU(cudaStreamWaitEvent(s, L->join_ev[i], 0));
@@ -906,46 +959,32 @@ int enqueue(dtfill_t* h, const void* in, int B, int H, int W, float src_thr, flo
         if (drain.joinable()) drain.join();
         if (rc) return rc;
     }
-    if (h->ev_gt) {
+    if (c.eval_gt) {
         // evaluation.py:82-123 / :196-239 on the filled depth of this call, on the call's own stream: per-frame metrics,
         // their column sums added to the lane's running totals (eval.py:212-232 `+=`), no host synchronisation
-        const long fnpx = (long)H * W;
-        int chunks = (int)((fnpx + 16383) / 16384);
-        if (chunks < 1) chunks = 1;
-        if (chunks > 64) chunks = 64;
-        while (chunks > 1 && (((fnpx + chunks - 1) / chunks) & 3)) --chunks;
-        if ((rc = ensure(h, L->ev_partial, (size_t)B * chunks * ACC * 8))) return rc;
         if ((rc = ensure(h, L->ev_per_frame, (size_t)B * 9 * 8))) return rc;
         if (!L->ev_totals.p) {
             if ((rc = ensure(h, L->ev_totals, 10 * 8))) return rc;
             CU(cudaMemsetAsync(L->ev_totals.p, 0, 10 * 8, s));
         }
-        dim3 grid(chunks, B);
-        double* part = (double*)L->ev_partial.p;
-        if (h->ev_gt_f64) {
-            if (h->ev_mode == 0) k4_metrics_partial<double, 0><<<grid, 256, 0, s>>>(out_depth, (const double*)h->ev_gt, fnpx, chunks, part);
-            else k4_metrics_partial<double, 1><<<grid, 256, 0, s>>>(out_depth, (const double*)h->ev_gt, fnpx, chunks, part);
-        } else {
-            if (h->ev_mode == 0) k4_metrics_partial<float, 0><<<grid, 256, 0, s>>>(out_depth, (const float*)h->ev_gt, fnpx, chunks, part);
-            else k4_metrics_partial<float, 1><<<grid, 256, 0, s>>>(out_depth, (const float*)h->ev_gt, fnpx, chunks, part);
-        }
-        k4_metrics_final<<<1, 256, 0, s>>>(part, B, chunks, h->ev_mode, (double*)L->ev_per_frame.p, (double*)L->ev_totals.p, 1);
-        launches += 2;
+        if ((rc = metrics_onepass(h, L->ev_partial, c.depth, c.eval_gt, c.eval_gt_f64, c.eval_mode, B, (long)H * W,
+                                  (double*)L->ev_per_frame.p, (double*)L->ev_totals.p, 1, s)))
+            return rc;
+        state.launches += 2;
         L->ev_dirty = true;
     }
-    if (!h->cur_status_copied) {
-        CU(cudaMemcpyAsync(h->status_ring + 2 * slot, h->cur_status, 8, cudaMemcpyDeviceToHost, s));
+    if (!state.status_copied) {
+        CU(cudaMemcpyAsync(h->status_ring + 2 * slot, state.status, 8, cudaMemcpyDeviceToHost, s));
         CU(cudaEventRecord(h->slot_done[slot], s));
     }
-    h->cur_status_early = false;
     h->slot_dirty[slot] = true;
     h->last_slot = slot;
     CU(cudaGetLastError());
-    if (pipelined) {
+    if (state.pipelined) {
         CU(cudaEventRecord(L->done, s));
         L->pending = true;
     }
-    L->last_launches = launches;
+    L->last_launches = state.launches;
     L->last_B = B;
     h->last_lane = (int)(L - h->lanes);
     ++h->ncalls;
@@ -1059,10 +1098,6 @@ void dtfill_destroy(dtfill_t* h) {
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
     for (Lane& L : h->lanes) {
-        Buf* lb[] = {&L.srcbits, &L.wprefix, &L.rowcell, &L.rowsrc, &L.rowval, &L.counts, &L.dlist,
-                     &L.scratch, &L.tasks, &L.sky, &L.skykeys, &L.ev_partial, &L.ev_per_frame, &L.ev_totals};
-        for (Buf* b : lb)
-            if (b->p) cudaFree(b->p);
         if (L.fork_ev) cudaEventDestroy(L.fork_ev);
         if (L.done) cudaEventDestroy(L.done);
         if (L.pipe) cudaStreamDestroy(L.pipe);
@@ -1074,20 +1109,10 @@ void dtfill_destroy(dtfill_t* h) {
             if (L.side[i]) cudaStreamDestroy(L.side[i]);
         }
     }
-    Buf* bufs[] = {&h->in_dev, &h->depth_dev, &h->dt_dev, &h->lbl_dev, &h->mask_dev, &h->counts_out_dev, &h->lidar_out_dev,
-                   &h->gt_dev, &h->partial, &h->per_frame, &h->sums, &h->edt_rows, &h->edt_stack, &h->sparse_dev,
-                   &h->mx_terms, &h->mx_counts, &h->mx_leaf_start, &h->mx_leaf_sum, &h->png_data, &h->png_scratch,
-                   &h->png_samples, &h->png_status, &h->enc_in, &h->enc_filt, &h->enc_adler, &h->enc_slots, &h->enc_seg,
-                   &h->enc_out, &h->enc_off, &h->enc_depth, &h->smp_coords, &h->smp_bad};
-    for (Buf* b : bufs)
-        if (b->p) cudaFree(b->p);
     for (void* q : h->retired) cudaFree(q);
     if (h->counts_host) cudaFreeHost(h->counts_host);
     delete h->pool_in;
     delete h->pool_out;
-    for (PinBuf* b : {&h->pin_in, &h->pin_depth, &h->pin_dt, &h->pin_lbl, &h->pin_mask, &h->pin_lidar, &h->pin_sparse, &h->pin_png,
-                      &h->pin_png_status, &h->pin_enc_off, &h->pin_smp, &h->pin_smp_out})
-        if (b->p) cudaFreeHost(b->p);
     if (h->status_ring) cudaFreeHost(h->status_ring);
     if (h->status_dev) cudaFree(h->status_dev);
     if (h->status_stream) cudaStreamDestroy(h->status_stream);
@@ -1144,8 +1169,11 @@ int dtfill_synchronize(dtfill_t* h) {
 int dtfill_run_async(dtfill_t* h, const float* in_dev, int B, int H, int W, float src_thr, float val_thr,
                      float* out_depth_dev, float* out_dt_dev, int32_t* out_lbl_dev, uint8_t* out_mask_dev,
                      int32_t* out_counts_dev) {
-    return enqueue(h, in_dev, B, H, W, src_thr, val_thr, out_depth_dev, out_dt_dev, out_lbl_dev, out_mask_dev,
-                   out_counts_dev);
+    FillCall c;
+    c.in = in_dev;
+    c.B = B; c.H = H; c.W = W; c.src_thr = src_thr; c.val_thr = val_thr;
+    c.depth = out_depth_dev; c.dt = out_dt_dev; c.lbl = out_lbl_dev; c.mask = out_mask_dev; c.counts = out_counts_dev;
+    return enqueue(h, c);
 }
 
 int dtfill_status(dtfill_t* h, int* first_bad_frame, int* kernel_launches) {
@@ -1172,15 +1200,6 @@ int dtfill_status(dtfill_t* h, int* first_bad_frame, int* kernel_launches) {
 
 namespace {
 
-// Input description of one call, installed on the handle while the call is enqueued.
-struct InputScope {
-    dtfill_t* h;
-    InputScope(dtfill_t* h_, bool u16, int in_H, int in_crop, float* lidar_dev) : h(h_) {
-        h->in_u16 = u16; h->in_H = in_H; h->in_crop = in_crop; h->lidar_dev = lidar_dev;
-    }
-    ~InputScope() { h->in_u16 = false; h->in_H = 0; h->in_crop = 0; h->lidar_dev = nullptr; }
-};
-
 // dtfill_run / dtfill_run_u16: buffers on either side, synchronous.  u16: `in` holds uint16 samples [B,in_H,W].
 int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, int in_crop, int B, int H, int W,
              float src_thr, float val_thr, float* out_lidar, float* out_depth, float* out_dt, int32_t* out_lbl,
@@ -1189,27 +1208,27 @@ int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, 
     const size_t npx = (size_t)B * H * W;
     const size_t in_bytes = u16 ? (size_t)B * in_H * W * 2 : npx * 4;
     int rc;
-    const void* in_d = in;
+    FillCall c;
+    c.kind = u16 ? FillCall::U16 : FillCall::F32; c.in = in; c.in_H = in_H; c.crop = in_crop; c.lidar = out_lidar;
+    c.B = B; c.H = H; c.W = W; c.src_thr = src_thr; c.val_thr = val_thr;
+    c.depth = out_depth; c.dt = out_dt; c.lbl = out_lbl; c.mask = out_mask; c.counts = out_counts;
     // outputs on the host: copies are sliced.  in_resident: the input is a device buffer the library itself just produced
     // (dtfill_run_png), so only the outputs go through the slices
     const bool pipelined = !out_is_device && (!in_is_device || in_resident);
     if (!in_is_device) {
         if ((rc = ensure(h, h->in_dev, in_bytes))) return rc;
         if (!pipelined) CU(cudaMemcpyAsync(h->in_dev.p, in, in_bytes, cudaMemcpyHostToDevice, h->stream));
-        in_d = h->in_dev.p;
+        c.in = h->in_dev.p;
     }
-    float* olid = out_lidar; float* od = out_depth; float* odt = out_dt; int32_t* ol = out_lbl; uint8_t* om = out_mask;
-    int32_t* oc = out_counts;
     if (!out_is_device) {
         if ((rc = ensure(h, h->depth_dev, npx * 4))) return rc;
-        od = (float*)h->depth_dev.p;
-        if (out_lidar) { if ((rc = ensure(h, h->lidar_out_dev, npx * 4))) return rc; olid = (float*)h->lidar_out_dev.p; }
-        if (out_dt) { if ((rc = ensure(h, h->dt_dev, npx * 4))) return rc; odt = (float*)h->dt_dev.p; }
-        if (out_lbl) { if ((rc = ensure(h, h->lbl_dev, npx * 4))) return rc; ol = (int32_t*)h->lbl_dev.p; }
-        if (out_mask) { if ((rc = ensure(h, h->mask_dev, npx))) return rc; om = (uint8_t*)h->mask_dev.p; }
-        if (out_counts) { if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc; oc = (int32_t*)h->counts_out_dev.p; }
+        c.depth = (float*)h->depth_dev.p;
+        if (out_lidar) { if ((rc = ensure(h, h->lidar_out_dev, npx * 4))) return rc; c.lidar = (float*)h->lidar_out_dev.p; }
+        if (out_dt) { if ((rc = ensure(h, h->dt_dev, npx * 4))) return rc; c.dt = (float*)h->dt_dev.p; }
+        if (out_lbl) { if ((rc = ensure(h, h->lbl_dev, npx * 4))) return rc; c.lbl = (int32_t*)h->lbl_dev.p; }
+        if (out_mask) { if ((rc = ensure(h, h->mask_dev, npx))) return rc; c.mask = (uint8_t*)h->mask_dev.p; }
+        if (out_counts) { if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc; c.counts = (int32_t*)h->counts_out_dev.p; }
     }
-    InputScope scope(h, u16, in_H, in_crop, olid);
     h->last_h2d_bytes = h->last_d2h_bytes = 0;
     if (pipelined) {
         HostIO hio;
@@ -1262,19 +1281,19 @@ int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, 
             }
             hio.counts = h->counts_host;
         }
-        if ((rc = enqueue(h, in_d, B, H, W, src_thr, val_thr, od, odt, ol, om, oc, &hio, true))) return rc;
+        if ((rc = enqueue(h, c, &hio, true))) return rc;
         rc = dtfill_status(h, first_bad_frame, nullptr);
         if (out_counts && (rc == 0 || rc == DTFILL_E_INDEX)) memcpy(out_counts, h->counts_host, (size_t)B * 8);
         return rc;
     }
-    if ((rc = enqueue(h, in_d, B, H, W, src_thr, val_thr, od, odt, ol, om, oc, nullptr, true))) return rc;
+    if ((rc = enqueue(h, c, nullptr, true))) return rc;
     if (!out_is_device) {
-        CU(cudaMemcpyAsync(out_depth, od, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_lidar) CU(cudaMemcpyAsync(out_lidar, olid, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_dt) CU(cudaMemcpyAsync(out_dt, odt, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_lbl) CU(cudaMemcpyAsync(out_lbl, ol, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_mask) CU(cudaMemcpyAsync(out_mask, om, npx, cudaMemcpyDeviceToHost, h->stream));
-        if (out_counts) CU(cudaMemcpyAsync(out_counts, oc, (size_t)B * 8, cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaMemcpyAsync(out_depth, c.depth, npx * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (out_lidar) CU(cudaMemcpyAsync(out_lidar, c.lidar, npx * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (out_dt) CU(cudaMemcpyAsync(out_dt, c.dt, npx * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (out_lbl) CU(cudaMemcpyAsync(out_lbl, c.lbl, npx * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (out_mask) CU(cudaMemcpyAsync(out_mask, c.mask, npx, cudaMemcpyDeviceToHost, h->stream));
+        if (out_counts) CU(cudaMemcpyAsync(out_counts, c.counts, (size_t)B * 8, cudaMemcpyDeviceToHost, h->stream));
     }
     return dtfill_status(h, first_bad_frame, nullptr);
 }
@@ -1313,9 +1332,11 @@ int dtfill_run_u16_async(dtfill_t* h, const uint16_t* in_dev, int B, int H_in, i
                          uint8_t* out_mask_dev, int32_t* out_counts_dev) {
     int rc = check_u16_args("dtfill_run_u16_async", h, in_dev, out_depth_dev, B, H_in, W, crop_top);
     if (rc) return rc;
-    InputScope scope(h, true, H_in, crop_top, out_lidar_dev);
-    return enqueue(h, in_dev, B, H_in - crop_top, W, src_thr, val_thr, out_depth_dev, out_dt_dev, out_lbl_dev, out_mask_dev,
-                   out_counts_dev);
+    FillCall c;
+    c.kind = FillCall::U16; c.in = in_dev; c.in_H = H_in; c.crop = crop_top; c.lidar = out_lidar_dev;
+    c.B = B; c.H = H_in - crop_top; c.W = W; c.src_thr = src_thr; c.val_thr = val_thr;
+    c.depth = out_depth_dev; c.dt = out_dt_dev; c.lbl = out_lbl_dev; c.mask = out_mask_dev; c.counts = out_counts_dev;
+    return enqueue(h, c);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1338,11 +1359,14 @@ const char* png_reason(int st) {
     }
 }
 
+// The filtered bytes of an H x W frame, H * (1 + 2 W), stay below 2^28: the Adler-32 sums of k8_png_inflate are exact in
+// 64 bits below this size.
+bool png_frame_fits(int H, int W) { return (int64_t)H * (1 + 2 * (int64_t)W) < (1ll << 28); }
+
 int png_args(const char* who, dtfill_t* h, const void* data, const int64_t* offsets, const void* out, int B, int H, int W) {
     if (!h || !data || !offsets || !out) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, data, offsets or output");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H, W must be positive");
-    // the Adler-32 sums of k8_png_inflate are exact in 64 bits below this size
-    if ((int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28))
+    if (!png_frame_fits(H, W))
         return fail(DTFILL_E_ARG, std::string(who) + ": frame too large (H * (1 + 2 W) < 2^28 bytes)");
     return 0;
 }
@@ -1482,7 +1506,7 @@ int dtfill_run_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int
 
 int dtfill_debug_png_decode_host(const uint8_t* f, long nbytes, int H, int W, uint16_t* out) {
     using namespace png;
-    if (!f || !out || nbytes < 0 || H <= 0 || W <= 0 || (int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28)) return -1;
+    if (!f || !out || nbytes < 0 || H <= 0 || W <= 0 || !png_frame_fits(H, W)) return -1;
     const uint32_t total = (uint32_t)H * (uint32_t)(1 + 2 * W);
     std::vector<uint8_t> scr(total);
     std::vector<uint16_t> llut(1 << LBITS), dlut(1 << DBITS);
@@ -1546,7 +1570,7 @@ int png_encode_args(const char* who, dtfill_t* h, const void* in, const void* ou
                     int H, int W, int64_t out_capacity) {
     if (!h || !in || !out || !out_offsets) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, input, out or out_offsets");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H, W must be positive");
-    if ((int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28))
+    if (!png_frame_fits(H, W))
         return fail(DTFILL_E_ARG, std::string(who) + ": frame too large (H * (1 + 2 W) < 2^28 bytes)");
     const int64_t need = (int64_t)B * png::encode_bound(H, W);
     if (out_capacity < need)
@@ -1678,7 +1702,7 @@ int64_t png_deflate_segment_host(const uint8_t* f, int64_t s0, int64_t s1, int64
 }  // namespace
 
 int64_t dtfill_png_encode_bound(int H, int W) {
-    if (H <= 0 || W <= 0 || (int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28)) return DTFILL_E_ARG;
+    if (H <= 0 || W <= 0 || !png_frame_fits(H, W)) return DTFILL_E_ARG;
     return png::encode_bound(H, W);
 }
 
@@ -1729,7 +1753,7 @@ int dtfill_debug_depth_samples_host(const float* depth, long n, uint16_t* out) {
 
 long dtfill_debug_png_encode_host(const uint16_t* samples, int H, int W, uint8_t* out, long capacity) {
     using namespace png;
-    if (!samples || !out || H <= 0 || W <= 0 || (int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28)) return -1;
+    if (!samples || !out || H <= 0 || W <= 0 || !png_frame_fits(H, W)) return -1;
     if (capacity < encode_bound(H, W)) return -1;
     const int64_t stride = 1 + 2 * (int64_t)W;
     std::vector<uint8_t> filt((size_t)H * stride);
@@ -1791,11 +1815,6 @@ __global__ void k4_fold_totals(LaneTotals lanes, double* __restrict__ sums, int 
         if (lanes.p[l]) s += lanes.p[l][i];       // fixed order: lane 0, 1, 2, 3
     sums[i] = s;
 }
-struct EvalScope {
-    dtfill_t* h;
-    EvalScope(dtfill_t* h_, const void* gt, int f64, int mode) : h(h_) { h->ev_gt = gt; h->ev_gt_f64 = f64; h->ev_mode = mode; }
-    ~EvalScope() { h->ev_gt = nullptr; }
-};
 
 // Distance_Transform's verdict on the frames of a synchronous fill, frame by frame as the evaluation loop meets them: rc and
 // fill_bad are what dtfill_status reported, cnt the fill's counts [B][2].  `what` names a frame in the message.
@@ -1823,9 +1842,12 @@ int dtfill_run_eval_async(dtfill_t* h, const float* in_dev, const void* gt_dev, 
                           int32_t* out_lbl_dev, uint8_t* out_mask_dev, int32_t* out_counts_dev) {
     if (!h || !gt_dev) return fail(DTFILL_E_ARG, "dtfill_run_eval_async: NULL handle or ground truth");
     if (mode != DTFILL_METRICS_KITTI && mode != DTFILL_METRICS_NYU) return fail(DTFILL_E_ARG, "dtfill_run_eval_async: bad mode");
-    EvalScope scope(h, gt_dev, gt_is_f64, mode);
-    return enqueue(h, in_dev, B, H, W, src_thr, val_thr, out_depth_dev, out_dt_dev, out_lbl_dev, out_mask_dev,
-                   out_counts_dev);
+    FillCall c;
+    c.in = in_dev;
+    c.B = B; c.H = H; c.W = W; c.src_thr = src_thr; c.val_thr = val_thr;
+    c.depth = out_depth_dev; c.dt = out_dt_dev; c.lbl = out_lbl_dev; c.mask = out_mask_dev; c.counts = out_counts_dev;
+    c.eval_gt = gt_dev; c.eval_gt_f64 = gt_is_f64; c.eval_mode = mode;
+    return enqueue(h, c);
 }
 
 int dtfill_eval_totals(dtfill_t* h, double* sums_dev, int accumulate) {
@@ -1877,30 +1899,14 @@ int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_
     double* pf_d = (out_is_device && per_frame) ? per_frame : (double*)h->per_frame.p;
     double* sm_d = (out_is_device && sums) ? sums : (double*)h->sums.p;
     if (h->metrics_exact && npx < (1l << 31)) {
-        const double* g64 = (const double*)g_d;
-        const float* g32 = (const float*)g_d;
-        if (gt_is_f64)
-            rc = mode == 0 ? k4x_enqueue<double, 0>(h, p_d, g64, B, npx, pf_d, s) : k4x_enqueue<double, 1>(h, p_d, g64, B, npx, pf_d, s);
-        else
-            rc = mode == 0 ? k4x_enqueue<float, 0>(h, p_d, g32, B, npx, pf_d, s) : k4x_enqueue<float, 1>(h, p_d, g32, B, npx, pf_d, s);
+        rc = with_gt_mode(gt_is_f64, mode, [&](auto g, auto m) {
+            using GT = decltype(g);
+            return k4x_enqueue<GT, decltype(m)::value>(h, p_d, (const GT*)g_d, B, npx, pf_d, s);
+        });
         if (rc) return rc;
         k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, accumulate);
-    } else {
-    int chunks = (int)((npx + 16383) / 16384);     // chunk boundaries stay multiples of 4 pixels when npx is
-    if (chunks < 1) chunks = 1;
-    if (chunks > 64) chunks = 64;
-    while (chunks > 1 && (((npx + chunks - 1) / chunks) & 3)) --chunks;
-    if ((rc = ensure(h, h->partial, (size_t)B * chunks * ACC * 8))) return rc;
-    dim3 grid(chunks, B);
-    double* part = (double*)h->partial.p;
-    if (gt_is_f64) {
-        if (mode == 0) k4_metrics_partial<double, 0><<<grid, 256, 0, s>>>(p_d, (const double*)g_d, npx, chunks, part);
-        else k4_metrics_partial<double, 1><<<grid, 256, 0, s>>>(p_d, (const double*)g_d, npx, chunks, part);
-    } else {
-        if (mode == 0) k4_metrics_partial<float, 0><<<grid, 256, 0, s>>>(p_d, (const float*)g_d, npx, chunks, part);
-        else k4_metrics_partial<float, 1><<<grid, 256, 0, s>>>(p_d, (const float*)g_d, npx, chunks, part);
-    }
-    k4_metrics_final<<<1, 256, 0, s>>>(part, B, chunks, mode, pf_d, sm_d, accumulate);
+    } else if ((rc = metrics_onepass(h, h->partial, p_d, g_d, gt_is_f64, mode, B, npx, pf_d, sm_d, accumulate, s))) {
+        return rc;
     }
     CU(cudaGetLastError());
     if (!out_is_device) {
@@ -1942,14 +1948,11 @@ int eval_png_run(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets
     //    counts leave the device
     if ((rc = ensure(h, h->depth_dev, (size_t)B * npx * 4))) return rc;
     if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc;
-    float* depth = (float*)h->depth_dev.p;
-    int32_t* counts = (int32_t*)h->counts_out_dev.p;
-    {
-        InputScope scope(h, true, H_in, crop_top, nullptr);
-        if ((rc = enqueue(h, samples, B, H_in - crop_top, W, src_thr, val_thr, depth, nullptr, nullptr, nullptr, counts,
-                          nullptr, true)))
-            return rc;
-    }
+    FillCall fill;
+    fill.kind = FillCall::U16; fill.in = samples; fill.in_H = H_in; fill.crop = crop_top;
+    fill.B = B; fill.H = H_in - crop_top; fill.W = W; fill.src_thr = src_thr; fill.val_thr = val_thr;
+    fill.depth = (float*)h->depth_dev.p; fill.counts = (int32_t*)h->counts_out_dev.p;
+    if ((rc = enqueue(h, fill, nullptr, true))) return rc;
     // 3. Result.evaluate of the filled depth against the same rows of the ground-truth samples, in numpy's summation
     //    order whatever dtfill_set_metrics_exact says
     if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
@@ -1959,15 +1962,15 @@ int eval_png_run(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets
     const uint16_t* g_d = gt_dev ? gt_dev : samples + (size_t)B * npx_in;
     if (floor) {
         const K4xWindow rows{npx_in, W, crop_top, 0, W};
-        rc = k4x_enqueue<double, 0, uint16_t, false, true>(h, depth, g_d, B, npx, pf_d, s, rows);
+        rc = k4x_enqueue<double, 0, uint16_t, false, true>(h, fill.depth, g_d, B, npx, pf_d, s, rows);
     } else {
-        rc = k4x_enqueue<double, 0>(h, depth, g_d, B, npx, pf_d, s);
+        rc = k4x_enqueue<double, 0>(h, fill.depth, g_d, B, npx, pf_d, s);
     }
     if (rc) return rc;
     k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(st_host, status, (size_t)nfiles * 4, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(st_host + nfiles, counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(st_host + nfiles, fill.counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
     if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
     if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
     int fill_bad = -1;
@@ -1998,7 +2001,7 @@ int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offs
     if (!h || !lidar || !lidar_offsets || !gt || !gt_offsets)
         return fail(DTFILL_E_ARG, "dtfill_eval_png: NULL handle, files or offsets");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_eval_png: B, H, W must be positive");
-    if ((int64_t)H * (1 + 2 * (int64_t)W) >= (1ll << 28))
+    if (!png_frame_fits(H, W))
         return fail(DTFILL_E_ARG, "dtfill_eval_png: frame too large (H * (1 + 2 W) < 2^28 bytes)");
     return eval_png_run(h, lidar, lidar_offsets, gt, gt_offsets, nullptr, B, H, W, 0, false, src_thr,
                         val_thr, per_frame, sums, first_bad_frame);
@@ -2015,7 +2018,7 @@ int dtfill_eval_png_kitti(dtfill_t* h, const uint8_t* lidar, const int64_t* lida
         return fail(DTFILL_E_ARG, std::string(who) + ": give the ground truth either as files and offsets or as device samples");
     if (B <= 0 || H_in <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H_in, W must be positive");
     if (crop_top < 0 || crop_top >= H_in) return fail(DTFILL_E_ARG, std::string(who) + ": crop_top must lie in [0, H_in)");
-    if ((int64_t)H_in * (1 + 2 * (int64_t)W) >= (1ll << 28))
+    if (!png_frame_fits(H_in, W))
         return fail(DTFILL_E_ARG, std::string(who) + ": frame too large (H_in * (1 + 2 W) < 2^28 bytes)");
     return eval_png_run(h, lidar, lidar_offsets, gt, gt_offsets, gt_samples_dev, B, H_in, W, crop_top, true, src_thr,
                         val_thr, per_frame, sums, first_bad_frame);
@@ -2104,20 +2107,12 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
     // 4. the fill with K1's sampled input kind, strict order on the handle's stream; the filled depth stays on the device
     if ((rc = ensure(h, h->depth_dev, (size_t)B * npx * 4))) return rc;
     if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc;
-    float* lid_d = nullptr;
-    if (out_lidar) {
-        if ((rc = ensure(h, h->lidar_out_dev, (size_t)B * npx * 4))) return rc;
-        lid_d = (float*)h->lidar_out_dev.p;
-    }
-    float* depth = (float*)h->depth_dev.p;
-    int32_t* counts = (int32_t*)h->counts_out_dev.p;
-    {
-        InputScope scope(h, false, H, 0, lid_d);
-        h->in_sampled = true;
-        rc = enqueue(h, g_d, B, H, W, src_thr, val_thr, depth, nullptr, nullptr, nullptr, counts, nullptr, true);
-        h->in_sampled = false;
-        if (rc) return rc;
-    }
+    if (out_lidar && (rc = ensure(h, h->lidar_out_dev, (size_t)B * npx * 4))) return rc;
+    FillCall fill;
+    fill.kind = FillCall::SAMPLED; fill.in = g_d; fill.lidar = out_lidar ? (float*)h->lidar_out_dev.p : nullptr;
+    fill.B = B; fill.H = H; fill.W = W; fill.src_thr = src_thr; fill.val_thr = val_thr;
+    fill.depth = (float*)h->depth_dev.p; fill.counts = (int32_t*)h->counts_out_dev.p;
+    if ((rc = enqueue(h, fill, nullptr, true))) return rc;
     // 5. Result_NYU.evaluate of the window of the filled depth against the same window of the ground truth, in numpy's
     //    summation order whatever dtfill_set_metrics_exact says
     if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
@@ -2125,16 +2120,16 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
     double* pf_d = (double*)h->per_frame.p;
     double* sm_d = (double*)h->sums.p;
     const K4xWindow win{npx, W, r0, c0, c1 - c0};
-    if ((rc = k4x_enqueue<float, 1, float, true>(h, depth, g_d, B, (long)(r1 - r0) * (c1 - c0), pf_d, s, win))) return rc;
+    if ((rc = k4x_enqueue<float, 1, float, true>(h, fill.depth, g_d, B, (long)(r1 - r0) * (c1 - c0), pf_d, s, win))) return rc;
     k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
     CU(cudaGetLastError());
     if ((rc = ensure_pinned(h->pin_smp_out, (size_t)B * 8 + 4))) return rc;
     int32_t* out_h = (int32_t*)h->pin_smp_out.p;            // the fill's counts [B][2], then the flag word
-    CU(cudaMemcpyAsync(out_h, counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(out_h, fill.counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(out_h + 2 * B, h->smp_bad.p, 4, cudaMemcpyDeviceToHost, s));
     if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
     if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
-    if (out_lidar) CU(cudaMemcpyAsync(out_lidar, lid_d, (size_t)B * npx * 4, cudaMemcpyDeviceToHost, s));
+    if (out_lidar) CU(cudaMemcpyAsync(out_lidar, fill.lidar, (size_t)B * npx * 4, cudaMemcpyDeviceToHost, s));
     int fill_bad = -1;
     rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
     h->last_h2d_bytes = h2d;
