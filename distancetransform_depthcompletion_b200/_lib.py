@@ -103,8 +103,11 @@ def load() -> ctypes.CDLL:
                                           ctypes.POINTER(ci)]
         try:
             L.dtfill_eval_png_kitti.argtypes = [vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, cf, cf, vp, vp, ctypes.POINTER(ci)]
-        except AttributeError:      # an older build of the same ABI version
-            raise DTFillError(f"{LIB_PATH} lacks dtfill_eval_png_kitti: rebuild it with "
+            L.dtfill_eval_sampled_mt.argtypes = [vp, vp, ci, ci, ci, ci, ci, vp, ci, ci, ci, ci, ci, cf, cf, vp, vp, vp,
+                                                 vp, vp, vp, vp, vp, ctypes.POINTER(ci)]
+            L.dtfill_debug_mt_draw_host.argtypes = [vp, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp]
+        except AttributeError as e:      # an older build of the same ABI version
+            raise DTFillError(f"{LIB_PATH} lacks {str(e).split()[-1].strip(chr(39))}: rebuild it with "
                               "`python -m distancetransform_depthcompletion_b200.build`") from None
         L.dtfill_debug_depth_samples_host.argtypes = [vp, ctypes.c_long, vp]
         L.dtfill_debug_depth_samples_host.restype = ci
@@ -119,7 +122,8 @@ def load() -> ctypes.CDLL:
                      "dtfill_run_eval_async", "dtfill_eval_totals", "dtfill_edt", "dtfill_set_sparse_upload",
                      "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo", "dtfill_png_decode",
                      "dtfill_run_png", "dtfill_debug_png_decode_host", "dtfill_png_encode", "dtfill_png_encode_depth",
-                     "dtfill_run_png_to_png", "dtfill_eval_png", "dtfill_eval_sampled", "dtfill_eval_png_kitti"):
+                     "dtfill_run_png_to_png", "dtfill_eval_png", "dtfill_eval_sampled", "dtfill_eval_png_kitti",
+                     "dtfill_eval_sampled_mt", "dtfill_debug_mt_draw_host"):
             getattr(L, name).restype = ci
         _lib = L
         return L
@@ -397,6 +401,38 @@ class Handle:
                                            ctypes.byref(bad)), "dtfill_eval_sampled")
         return (per_frame, sums, lidar) if want_lidar else (per_frame, sums)
 
+    def eval_sampled_mt(self, gt, B: int, H: int, W: int, n: int, key: np.ndarray, pos: int, crop, src_thr: float,
+                        val_thr: float, gt_is_device: bool = False, want_coords: bool = False):
+        """eval_sampled with the coordinates drawn on the device from the MT19937 state (key uint32 [624], pos), as
+        n = RandomState.randint draws per frame, rows then columns -> dict(per_frame [B,9], sums [10], key, pos,
+        words int64 [B] (32-bit words each frame consumed), first_bad, and rows / cols int32 [B,n] with want_coords).
+        A frame Distance_Transform rejects is reported under "index_error" (the state outputs are still written); other
+        failures raise."""
+        r0, r1, c0, c1 = (int(v) for v in crop)
+        if not gt_is_device:
+            assert gt.dtype == np.float32 and gt.shape == (B, H, W) and gt.flags.c_contiguous
+        key = np.ascontiguousarray(key, np.uint32)
+        assert key.shape == (624,)
+        per_frame = np.empty((B, METRIC_COLS), np.float64)
+        sums = np.empty(METRIC_COLS + 1, np.float64)
+        out_key = np.empty(624, np.uint32)
+        out_pos = ctypes.c_int(-1)
+        words = np.empty(B, np.int64)
+        rows = np.empty((B, n), np.int32) if want_coords else None
+        cols = np.empty((B, n), np.int32) if want_coords else None
+        bad = ctypes.c_int(-1)
+        rc = self._L.dtfill_eval_sampled_mt(self._h, _ptr(gt), int(bool(gt_is_device)), int(B), int(H), int(W), int(n),
+                                            _ptr(key), int(pos), r0, r1, c0, c1, float(src_thr), float(val_thr), None,
+                                            _ptr(rows), _ptr(cols), _ptr(out_key), ctypes.byref(out_pos), _ptr(words),
+                                            _ptr(per_frame), _ptr(sums), ctypes.byref(bad))
+        res = dict(per_frame=per_frame, sums=sums, key=out_key, pos=out_pos.value, words=words, rows=rows, cols=cols,
+                   first_bad=bad.value)
+        if rc == E_INDEX:
+            res["index_error"] = last_error()
+            return res
+        _check(rc, "dtfill_eval_sampled_mt")
+        return res
+
     def png_encode_device_async(self, in_ptr: int, is_float: bool, B: int, H: int, W: int, out_ptr: int,
                                 capacity: int, offsets_ptr: int):
         """Device frames (uint16, or float32 depth when is_float) -> device files + offsets [B+1], enqueued on the
@@ -602,6 +638,20 @@ def png_decode_host(png: bytes, H: int, W: int):
     if st < 0:
         raise ValueError("dtfill_debug_png_decode_host: bad arguments")
     return st, out
+
+
+def mt_draw_host(key, pos: int, B: int, H: int, W: int, n: int):
+    """Test hook: the draw of Handle.eval_sampled_mt run serially on the CPU (no GPU) -> (rows int32 [B,n], cols int32
+    [B,n], key uint32 [624], pos, words int64 [B])."""
+    key = np.ascontiguousarray(key, np.uint32)
+    if key.shape != (624,):
+        raise ValueError("mt_draw_host: the key must hold 624 words")
+    rows, cols = np.empty((B, n), np.int32), np.empty((B, n), np.int32)
+    out_key, out_pos, words = np.empty(624, np.uint32), ctypes.c_int(-1), np.empty(B, np.int64)
+    if load().dtfill_debug_mt_draw_host(_ptr(key), int(pos), int(B), int(H), int(W), int(n), _ptr(rows), _ptr(cols),
+                                        _ptr(out_key), ctypes.byref(out_pos), _ptr(words)) != 0:
+        raise ValueError("dtfill_debug_mt_draw_host: bad arguments")
+    return rows, cols, out_key, out_pos.value, words
 
 
 def png_encode_bound(H: int, W: int) -> int:

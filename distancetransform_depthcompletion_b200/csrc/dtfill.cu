@@ -2024,14 +2024,11 @@ int dtfill_eval_png_kitti(dtfill_t* h, const uint8_t* lidar, const int64_t* lida
                         val_thr, per_frame, sums, first_bad_frame);
 }
 
-int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, const int32_t* rows,
-                        const int32_t* cols, const int64_t* sample_offsets, int coords_are_device, int r0, int r1, int c0,
-                        int c1, float src_thr, float val_thr, float* out_lidar, double* per_frame, double* sums,
-                        int* first_bad_frame) {
-    const char* who = "dtfill_eval_sampled";
-    if (first_bad_frame) *first_bad_frame = -1;
-    if (!h || !gt || !rows || !cols || !sample_offsets)
-        return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, ground truth, coordinates or offsets");
+namespace {
+
+// The checks dtfill_eval_sampled and dtfill_eval_sampled_mt share: frame size, window, alignment of a device ground truth.
+int sampled_frame_check(const char* who, const float* gt, int gt_is_device, int B, int H, int W, int r0, int r1, int c0,
+                        int c1) {
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": B, H, W must be positive");
     if ((long)H + W >= 60000 || (long)H * W >= (1l << 31) || W > 28000)
         return fail(DTFILL_E_ARG, std::string(who) + ": frame size not supported (H + W < 60000, W <= 28000)");
@@ -2041,52 +2038,21 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
                                       std::to_string(H) + " x " + std::to_string(W) + " frame");
     if (gt_is_device && (W & 3) == 0 && ((uintptr_t)gt & 15))
         return fail(DTFILL_E_ARG, std::string(who) + ": device ground truth must be 16-byte aligned");
-    CU(cudaSetDevice(h->device));
-    int rc = dtfill_flush(h);        // fills in flight (pipelined mode) may still use lane 0's workspace
-    if (rc) return rc;
+    return 0;
+}
+
+// Steps 2-6 of dtfill_eval_sampled and dtfill_eval_sampled_mt, after the device coordinates d_rows / d_cols / d_off are
+// enqueued on the handle's stream: the ground truth, the sample bitmap, the fill, the metrics of the window, the copies
+// back and the verdict.  h2d: bytes the caller sent up already; d2h: bytes of copies back the caller enqueued already
+// (they complete with this call's synchronisation).
+int eval_sampled_run(dtfill_t* h, const char* who, const float* gt, int gt_is_device, int B, int H, int W,
+                     const int32_t* d_rows, const int32_t* d_cols, const int64_t* d_off, size_t h2d, size_t d2h, int r0,
+                     int r1, int c0, int c1, float src_thr, float val_thr, float* out_lidar, double* per_frame,
+                     double* sums, int* first_bad_frame) {
     const long npx = (long)H * W;
     const int WW = (W + 31) / 32;
     cudaStream_t s = h->stream;
-    size_t h2d = 0;
-    // 1. coordinates: host ones are checked here and go up in one copy through the pinned staging buffer (rows, cols, then
-    //    the offsets rebased to 0); device ones are checked by k10_sample_bits
-    const int32_t* d_rows = rows;
-    const int32_t* d_cols = cols;
-    const int64_t* d_off = sample_offsets;
-    if (!coords_are_device) {
-        const int64_t* o = sample_offsets;
-        if (o[0] < 0) return fail(DTFILL_E_ARG, std::string(who) + ": sample_offsets[0] < 0");
-        for (int b = 0; b < B; ++b) {
-            if (o[b + 1] < o[b]) {
-                if (first_bad_frame) *first_bad_frame = b;
-                return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(b) + " has a negative sample count");
-            }
-            for (int64_t i = o[b]; i < o[b + 1]; ++i)
-                if ((unsigned)rows[i] >= (unsigned)H || (unsigned)cols[i] >= (unsigned)W) {
-                    if (first_bad_frame) *first_bad_frame = b;
-                    return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(b) + ": sample (" +
-                                                  std::to_string(rows[i]) + ", " + std::to_string(cols[i]) +
-                                                  ") outside the frame");
-                }
-        }
-        const size_t n = (size_t)(o[B] - o[0]);
-        const size_t off_at = (2 * n * 4 + 15) & ~(size_t)15;
-        const size_t total = off_at + (size_t)(B + 1) * 8;
-        if ((rc = ensure_pinned(h->pin_smp, total))) return rc;
-        if ((rc = ensure(h, h->smp_coords, total))) return rc;
-        uint8_t* pin = (uint8_t*)h->pin_smp.p;
-        if (n) {
-            memcpy(pin, rows + o[0], n * 4);
-            memcpy(pin + n * 4, cols + o[0], n * 4);
-        }
-        int64_t* po = (int64_t*)(pin + off_at);
-        for (int b = 0; b <= B; ++b) po[b] = o[b] - o[0];
-        CU(cudaMemcpyAsync(h->smp_coords.p, pin, total, cudaMemcpyHostToDevice, s));
-        h2d += total;
-        d_rows = (const int32_t*)h->smp_coords.p;
-        d_cols = d_rows + n;
-        d_off = (const int64_t*)((uint8_t*)h->smp_coords.p + off_at);
-    }
+    int rc;
     // 2. the ground truth, unless it is resident
     const float* g_d = gt;
     if (!gt_is_device) {
@@ -2133,7 +2099,7 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
     int fill_bad = -1;
     rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
     h->last_h2d_bytes = h2d;
-    h->last_d2h_bytes = (size_t)B * 8 + 4 + (per_frame ? (size_t)B * 9 * 8 : 0) + (sums ? 10 * 8 : 0) +
+    h->last_d2h_bytes = d2h + (size_t)B * 8 + 4 + (per_frame ? (size_t)B * 9 * 8 : 0) + (sums ? 10 * 8 : 0) +
                         (out_lidar ? (size_t)B * npx * 4 : 0);
     if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
     // 6. the verdict: device coordinates outside the frame, then Distance_Transform's frame by frame
@@ -2144,6 +2110,153 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
                                       ": a sample outside the frame, or a negative sample count");
     }
     return fill_verdict(rc, fill_bad, out_h, B, "frame ", first_bad_frame);
+}
+
+}  // namespace
+
+int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, const int32_t* rows,
+                        const int32_t* cols, const int64_t* sample_offsets, int coords_are_device, int r0, int r1, int c0,
+                        int c1, float src_thr, float val_thr, float* out_lidar, double* per_frame, double* sums,
+                        int* first_bad_frame) {
+    const char* who = "dtfill_eval_sampled";
+    if (first_bad_frame) *first_bad_frame = -1;
+    if (!h || !gt || !rows || !cols || !sample_offsets)
+        return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, ground truth, coordinates or offsets");
+    int rc = sampled_frame_check(who, gt, gt_is_device, B, H, W, r0, r1, c0, c1);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    rc = dtfill_flush(h);            // fills in flight (pipelined mode) may still use lane 0's workspace
+    if (rc) return rc;
+    cudaStream_t s = h->stream;
+    size_t h2d = 0;
+    // 1. coordinates: host ones are checked here and go up in one copy through the pinned staging buffer (rows, cols, then
+    //    the offsets rebased to 0); device ones are checked by k10_sample_bits
+    const int32_t* d_rows = rows;
+    const int32_t* d_cols = cols;
+    const int64_t* d_off = sample_offsets;
+    if (!coords_are_device) {
+        const int64_t* o = sample_offsets;
+        if (o[0] < 0) return fail(DTFILL_E_ARG, std::string(who) + ": sample_offsets[0] < 0");
+        for (int b = 0; b < B; ++b) {
+            if (o[b + 1] < o[b]) {
+                if (first_bad_frame) *first_bad_frame = b;
+                return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(b) + " has a negative sample count");
+            }
+            for (int64_t i = o[b]; i < o[b + 1]; ++i)
+                if ((unsigned)rows[i] >= (unsigned)H || (unsigned)cols[i] >= (unsigned)W) {
+                    if (first_bad_frame) *first_bad_frame = b;
+                    return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(b) + ": sample (" +
+                                                  std::to_string(rows[i]) + ", " + std::to_string(cols[i]) +
+                                                  ") outside the frame");
+                }
+        }
+        const size_t n = (size_t)(o[B] - o[0]);
+        const size_t off_at = (2 * n * 4 + 15) & ~(size_t)15;
+        const size_t total = off_at + (size_t)(B + 1) * 8;
+        if ((rc = ensure_pinned(h->pin_smp, total))) return rc;
+        if ((rc = ensure(h, h->smp_coords, total))) return rc;
+        uint8_t* pin = (uint8_t*)h->pin_smp.p;
+        if (n) {
+            memcpy(pin, rows + o[0], n * 4);
+            memcpy(pin + n * 4, cols + o[0], n * 4);
+        }
+        int64_t* po = (int64_t*)(pin + off_at);
+        for (int b = 0; b <= B; ++b) po[b] = o[b] - o[0];
+        CU(cudaMemcpyAsync(h->smp_coords.p, pin, total, cudaMemcpyHostToDevice, s));
+        h2d += total;
+        d_rows = (const int32_t*)h->smp_coords.p;
+        d_cols = d_rows + n;
+        d_off = (const int64_t*)((uint8_t*)h->smp_coords.p + off_at);
+    }
+    return eval_sampled_run(h, who, gt, gt_is_device, B, H, W, d_rows, d_cols, d_off, h2d, 0, r0, r1, c0, c1, src_thr,
+                            val_thr, out_lidar, per_frame, sums, first_bad_frame);
+}
+
+int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, int n,
+                           const uint32_t* mt_key, int mt_pos, int r0, int r1, int c0, int c1, float src_thr,
+                           float val_thr, float* out_lidar, int32_t* out_rows, int32_t* out_cols, uint32_t* out_key,
+                           int* out_pos, int64_t* out_words, double* per_frame, double* sums, int* first_bad_frame) {
+    const char* who = "dtfill_eval_sampled_mt";
+    if (first_bad_frame) *first_bad_frame = -1;
+    if (!h || !gt || !mt_key) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, ground truth or key");
+    if (n < 0) return fail(DTFILL_E_ARG, std::string(who) + ": negative sample count");
+    if (H < 13 || W < 17) return fail(DTFILL_E_ARG, std::string(who) + ": frames need H >= 13 and W >= 17 (randint(H - 12), randint(W - 16))");
+    if (mt_pos < 0 || mt_pos > MT_N) return fail(DTFILL_E_ARG, std::string(who) + ": pos outside [0, 624]");
+    int rc = sampled_frame_check(who, gt, gt_is_device, B, H, W, r0, r1, c0, c1);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    rc = dtfill_flush(h);            // fills in flight (pipelined mode) may still use lane 0's workspace
+    if (rc) return rc;
+    cudaStream_t s = h->stream;
+    // 1. the draw: the key goes up through the pinned staging buffer; k11_mt_draw writes the coordinates, the offsets, the
+    //    words per frame and the final state into one device buffer, whose state part comes back in one copy
+    const size_t npts = (size_t)B * n;
+    const size_t off_at = (2 * npts * 4 + 15) & ~(size_t)15;
+    const size_t key_at = (off_at + (size_t)(B + 1) * 8 + 15) & ~(size_t)15;
+    const size_t back_at = key_at + MT_N * 4;                 // final key, pos, then the words per frame
+    const size_t words_at = back_at + ((MT_N * 4 + 4 + 15) & ~(size_t)15);
+    const size_t back_bytes = words_at - back_at + (size_t)B * 8;
+    if ((rc = ensure_pinned(h->pin_smp, MT_N * 4 + back_bytes))) return rc;
+    if ((rc = ensure(h, h->smp_coords, words_at + (size_t)B * 8))) return rc;
+    uint8_t* pin = (uint8_t*)h->pin_smp.p;
+    uint8_t* dev = (uint8_t*)h->smp_coords.p;
+    memcpy(pin, mt_key, MT_N * 4);
+    CU(cudaMemcpyAsync(dev + key_at, pin, MT_N * 4, cudaMemcpyHostToDevice, s));
+    int32_t* d_rows = (int32_t*)dev;
+    int32_t* d_cols = d_rows + npts;
+    int64_t* d_off = (int64_t*)(dev + off_at);
+    CU(cudaFuncSetAttribute(k11_mt_draw, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K11_SMEM));
+    k11_mt_draw<<<1, K11_THREADS, K11_SMEM, s>>>((const uint32_t*)(dev + key_at), mt_pos, B, n, (uint32_t)(H - 13),
+                                                 (uint32_t)(W - 17), d_rows, d_cols, d_off, (int64_t*)(dev + words_at),
+                                                 (uint32_t*)(dev + back_at), (int*)(dev + back_at + MT_N * 4));
+    CU(cudaGetLastError());
+    uint8_t* back = pin + MT_N * 4;
+    CU(cudaMemcpyAsync(back, dev + back_at, back_bytes, cudaMemcpyDeviceToHost, s));
+    size_t d2h = back_bytes;
+    if (out_rows && npts) { CU(cudaMemcpyAsync(out_rows, d_rows, npts * 4, cudaMemcpyDeviceToHost, s)); d2h += npts * 4; }
+    if (out_cols && npts) { CU(cudaMemcpyAsync(out_cols, d_cols, npts * 4, cudaMemcpyDeviceToHost, s)); d2h += npts * 4; }
+    // 2-6. as dtfill_eval_sampled; the state is written whatever the verdict
+    rc = eval_sampled_run(h, who, gt, gt_is_device, B, H, W, d_rows, d_cols, d_off, MT_N * 4, d2h, r0, r1, c0, c1,
+                          src_thr, val_thr, out_lidar, per_frame, sums, first_bad_frame);
+    if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
+    if (out_key) memcpy(out_key, back, MT_N * 4);
+    if (out_pos) memcpy(out_pos, back + MT_N * 4, 4);
+    if (out_words) memcpy(out_words, back + (words_at - back_at), (size_t)B * 8);
+    return rc;
+}
+
+int dtfill_debug_mt_draw_host(const uint32_t* key, int pos, int B, int H, int W, int n, int32_t* rows, int32_t* cols,
+                              uint32_t* out_key, int* out_pos, int64_t* out_words) {
+    if (!key || pos < 0 || pos > MT_N || B < 0 || H < 13 || W < 17 || n < 0 || (n && B && (!rows || !cols)) || !out_key ||
+        !out_pos || (B && !out_words))
+        return -1;
+    uint32_t st[MT_N], nxt[MT_N];
+    memcpy(st, key, sizeof st);
+    int p = pos;
+    const uint32_t rng[2] = {(uint32_t)(H - 13), (uint32_t)(W - 17)};
+    int32_t* out[2] = {rows, cols};
+    const int add[2] = {6, 8};
+    for (int b = 0; b < B; ++b) {
+        int64_t used = 0;
+        for (int kind = 0; kind < 2; ++kind) {
+            const uint32_t m = mt_mask(rng[kind]);
+            for (int j = 0; j < n; ++j) {
+                uint32_t v = 0;
+                if (rng[kind]) {
+                    do {
+                        if (p == MT_N) { mt_twist_block(st, nxt); memcpy(st, nxt, sizeof st); p = 0; }
+                        v = mt_temper(st[p++]) & m;
+                        ++used;
+                    } while (v > rng[kind]);
+                }
+                out[kind][(size_t)b * n + j] = (int32_t)v + add[kind];
+            }
+        }
+        out_words[b] = used;
+    }
+    memcpy(out_key, st, sizeof st);
+    *out_pos = p;
+    return 0;
 }
 
 int dtfill_set_band_cap(dtfill_t* h, int cap) {

@@ -23,6 +23,8 @@
 //                         offsets, pack), so that filled maps leave the device compressed
 //   K10 k10_sample_bits   NYU sample coordinates -> a bitmap of 1 bit per pixel, read by K1's sampled input kind, which
 //                         forms `gt * Mask` from the dense ground truth in registers (dtfill_eval_sampled)
+//   K11 k11_mt_draw       numpy's RandomState (MT19937, masked rejection) run on the device from its state: the NYU sample
+//                         coordinates of a batch, the input of K10 (dtfill_eval_sampled_mt)
 // One header per kernel (dtfill_k*.cuh); dtfill_common.cuh holds the key format, the structs and the helpers.
 //
 // Key format of the fast path (SURVEY.md section 7 H1): dist:11 | order:4 | label:17.  "order" is the position
@@ -46,3 +48,4 @@
 #include "dtfill_k8_png.cuh"
 #include "dtfill_k9_png_encode.cuh"
 #include "dtfill_k10_sample.cuh"
+#include "dtfill_k11_draw.cuh"

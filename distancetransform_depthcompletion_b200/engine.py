@@ -205,6 +205,25 @@ class DTFillEngine:
         self._inflight = {}       # the call synchronised: every earlier call has finished
         return res
 
+    def eval_drawn(self, gt, n: int, rng=None, crop=None, src_thr: float | None = None, return_coords: bool = False):
+        """eval_nyu.evaluate_fill_drawn against the float32 CUDA tensor gt [B,H,W], used in place, on torch's current
+        stream: n samples per frame drawn on the device from rng's MT19937 state (a RandomState, or None for the np.random
+        module), rng advanced as the reference's loop advances it.  Synchronous: returns (per_frame [B,9], sums [10])
+        float64 numpy arrays (and the drawn rows, cols int64 [B,n] with return_coords).  Fills still in flight are joined
+        first."""
+        import numpy as np
+        from . import eval_nyu
+        torch = self.torch
+        assert gt.is_cuda and gt.dtype == torch.float32 and gt.dim() == 3
+        gt = eval_nyu._aligned(gt)
+        crop = eval_nyu.NYU_EVAL_CROP if crop is None else crop
+        src_thr = eval_nyu.NYU_SRC_THR if src_thr is None else src_thr
+        self._bind_stream()
+        res = eval_nyu._eval_drawn(lambda: self.handle, gt.data_ptr(), True, gt.shape, n, np.random if rng is None else rng,
+                                   crop, src_thr, return_coords)
+        self._inflight = {}       # the call synchronised: every earlier call has finished
+        return res
+
     def flush(self):
         """Pipelined mode: torch's current stream waits for every fill still in flight."""
         self._bind_stream()

@@ -5,6 +5,7 @@ script's evaluation loop on the GPU.
     Distance_Transform(lidar)      -> depth_map [H,W]    eval_NYU.py:120-133  (any size, dtype of the input)
     nyu_sample_coords(n)           -> (rows, cols)       data_read.py:360-364 (the random sample of one frame)
     evaluate_fill_sampled(gt, rows, cols) -> (per_frame [B,9], sums [10])   eval_NYU.py:138-254 from dense ground truth
+    evaluate_fill_drawn(gt, n, rng)       -> (per_frame [B,9], sums [10])   the same loop with its draws, from rng's state
     evaluate_fill_kitti_png_files(lidar_files, gt) -> (per_frame [B,9], sums [10])   the script's KITTI branch, from files
 """
 from __future__ import annotations
@@ -143,33 +144,122 @@ def evaluate_fill_sampled(gt, rows, cols, crop=NYU_EVAL_CROP, src_thr: float = N
     outside the frame -- all before the device is touched -- and IndexError for the first frame Distance_Transform rejects
     (no valid depth, exactly one valid depth, labels outside the list of valid depths)."""
     from .tools import VALID_THR
-    is_tensor = type(gt).__module__.startswith("torch")
-    if is_tensor:
-        import torch
-        if gt.dtype != torch.float32:
-            raise TypeError(f"evaluate_fill_sampled: ground truth dtype {gt.dtype} not supported (float32 only)")
-        if not gt.is_cuda:
-            gt = gt.numpy()
-            is_tensor = False
-    if is_tensor and device is not None and int(device) != gt.device.index:
-        raise ValueError(f"evaluate_fill_sampled: device={device} but the ground truth is on {gt.device}")
-    if not is_tensor:
-        gt = np.asarray(gt)
-        if gt.dtype != np.float32:
-            raise TypeError(f"evaluate_fill_sampled: ground truth dtype {gt.dtype} not supported (float32 only)")
-    if gt.ndim != 3:
-        raise ValueError(f"evaluate_fill_sampled: ground truth must be [B,H,W], got shape {tuple(gt.shape)}")
+    gt, is_tensor = _dense_gt(gt, device, "evaluate_fill_sampled")
     B, H, W = (int(v) for v in gt.shape)
-    if B == 0 or H == 0 or W == 0:
-        raise ValueError("evaluate_fill_sampled: empty batch")
     crop = _check_crop(crop, H, W)
     r, c, off = _sample_arrays(rows, cols, B, H, W)
     if is_tensor:
         gt = _aligned(gt)
-        torch.cuda.current_stream(gt.device).synchronize()      # the handle's stream reads gt
+        _torch_sync(gt)                 # the handle's stream reads gt
         h = _lib.get_handle(gt.device.index)
         return h.eval_sampled(gt.data_ptr(), B, H, W, r, c, off, crop, src_thr, VALID_THR, gt_is_device=True)
     return _lib.get_handle(device).eval_sampled(np.ascontiguousarray(gt), B, H, W, r, c, off, crop, src_thr, VALID_THR)
+
+
+def _dense_gt(gt, device, who):
+    """The dense float32 ground truth [B,H,W] of evaluate_fill_sampled / evaluate_fill_drawn: (a CUDA tensor or a numpy
+    array, whether it is a tensor).  TypeError / ValueError before the device is touched."""
+    is_tensor = type(gt).__module__.startswith("torch")
+    if is_tensor:
+        import torch
+        if gt.dtype != torch.float32:
+            raise TypeError(f"{who}: ground truth dtype {gt.dtype} not supported (float32 only)")
+        if not gt.is_cuda:
+            gt = gt.numpy()
+            is_tensor = False
+    if is_tensor and device is not None and int(device) != gt.device.index:
+        raise ValueError(f"{who}: device={device} but the ground truth is on {gt.device}")
+    if not is_tensor:
+        gt = np.asarray(gt)
+        if gt.dtype != np.float32:
+            raise TypeError(f"{who}: ground truth dtype {gt.dtype} not supported (float32 only)")
+    if gt.ndim != 3:
+        raise ValueError(f"{who}: ground truth must be [B,H,W], got shape {tuple(gt.shape)}")
+    if any(int(v) == 0 for v in gt.shape):
+        raise ValueError(f"{who}: empty batch")
+    return gt, is_tensor
+
+
+def _torch_sync(t):
+    import torch
+    torch.cuda.current_stream(t.device).synchronize()
+
+
+def evaluate_fill_drawn(gt, n: int, rng=np.random, crop=NYU_EVAL_CROP, src_thr: float = NYU_SRC_THR,
+                        device: int | None = None, return_coords: bool = False):
+    """evaluate_fill_sampled with the reference's draws made on the GPU from rng's state, that is this loop in one call:
+
+        for b in range(B):
+            rows = rng.randint(H - 12, size=n) + 6;  cols = rng.randint(W - 16, size=n) + 8   data_read.py:360-364
+            Mask = np.zeros((H, W)); Mask[rows, cols] = 1
+            pred = Distance_Transform(gt[b] * Mask)                                          eval_NYU.py:120-133
+            result.evaluate(crop(pred), crop(gt[b]))                                          eval_NYU.py:202-207
+
+    rng: a np.random.RandomState or the np.random module (its global state), MT19937 either way: only the generator's
+    state goes up (2.5 KB), and the device reproduces randint's masked rejection on numpy's stream bit for bit.  rng
+    ends where the loop leaves it, so after np.random.seed(s) this call draws the reference's masks, and the next host
+    draw or the next call continues the same stream.  gt, crop, src_thr, device and the result are those of
+    evaluate_fill_sampled; with return_coords the drawn (rows, cols) follow as int64 [B,n] arrays.
+
+    Raises TypeError for an rng that is not MT19937-based (a np.random.Generator among them) and what
+    evaluate_fill_sampled raises for gt and crop; ValueError with numpy's message for n < 0 ("negative dimensions are
+    not allowed") and for frames too small to draw from (H <= 12 or W <= 16 with n > 0: "high <= 0") -- all before the
+    device is touched and with rng untouched.  IndexError for the first frame Distance_Transform rejects (n = 0 and
+    n = 1 at frame 0), with rng left after that frame's draws, as the loop leaves it."""
+    gt, is_tensor = _dense_gt(gt, device, "evaluate_fill_drawn")
+    if is_tensor:
+        gt = _aligned(gt)
+        _torch_sync(gt)                 # the handle's stream reads gt
+        return _eval_drawn(lambda: _lib.get_handle(gt.device.index), gt.data_ptr(), True, gt.shape, n, rng, crop,
+                           src_thr, return_coords)
+    return _eval_drawn(lambda: _lib.get_handle(device), np.ascontiguousarray(gt), False, gt.shape, n, rng, crop, src_thr,
+                       return_coords)
+
+
+def _mt_state(rng):
+    get = getattr(rng, "get_state", None)
+    st = get(legacy=False) if callable(get) else None
+    if not isinstance(st, dict) or st.get("bit_generator") != "MT19937":
+        raise TypeError(f"evaluate_fill_drawn: rng must be a np.random.RandomState or the np.random module (MT19937), "
+                        f"got {rng!r}")
+    return st
+
+
+def _set_mt(rng, st, key, pos):
+    """rng.set_state with the MT19937 key and pos, keeping the state's cached Gaussian."""
+    rng.set_state({"bit_generator": "MT19937", "state": {"key": np.asarray(key, np.uint32), "pos": int(pos)},
+                   "has_gauss": st["has_gauss"], "gauss": st["gauss"]})
+
+
+def _eval_drawn(get_handle, gt, gt_is_device, shape, n, rng, crop, src_thr, return_coords):
+    """The body of evaluate_fill_drawn and DTFillEngine.eval_drawn; get_handle() gives the Handle once the arguments
+    are checked."""
+    import operator
+    from .tools import VALID_THR
+    B, H, W = (int(v) for v in shape)
+    crop = _check_crop(crop, H, W)
+    st = _mt_state(rng)
+    n = operator.index(n)
+    if n < 0:
+        raise ValueError("negative dimensions are not allowed")          # randint(size=n)
+    if n > 0 and (H - 12 <= 0 or W - 16 <= 0):
+        raise ValueError("high <= 0")
+    if n == 0 and (H < 13 or W < 17):     # randint draws nothing; an empty mask leaves no valid depth in frame 0
+        raise IndexError("frame 0: labels index outside the list of valid depths (numpy IndexError)")
+    key, pos = np.asarray(st["state"]["key"], np.uint32), int(st["state"]["pos"])
+    r = get_handle().eval_sampled_mt(gt, B, H, W, n, key, pos, crop, src_thr, VALID_THR, gt_is_device=gt_is_device,
+                          want_coords=return_coords)
+    if "index_error" in r:
+        # the loop stops after frame first_bad's draws: replay the words every frame up to it consumed
+        bg = np.random.MT19937()
+        bg.state = {"bit_generator": "MT19937", "state": {"key": key, "pos": pos}}
+        bg.random_raw(int(r["words"][:r["first_bad"] + 1].sum()))
+        _set_mt(rng, st, bg.state["state"]["key"], bg.state["state"]["pos"])
+        raise IndexError(r["index_error"])
+    _set_mt(rng, st, r["key"], r["pos"])
+    if return_coords:
+        return r["per_frame"], r["sums"], r["rows"].astype(np.int64), r["cols"].astype(np.int64)
+    return r["per_frame"], r["sums"]
 
 
 def _aligned(t):

@@ -285,6 +285,35 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
                         int* first_bad_frame);
 
 /*
+ * dtfill_eval_sampled with the coordinates drawn on the device, as the reference draws them with numpy's legacy generator
+ * (np.random / RandomState, MT19937):
+ *     for b in range(B):
+ *         rows_b = rng.randint(H - 12, size=n) + 6;  cols_b = rng.randint(W - 16, size=n) + 8    data_read.py:360-364
+ *         ... the loop body of dtfill_eval_sampled
+ * The generator's state goes in as mt_key [624] (host) and mt_pos in [0, 624], the `key` and `pos` of
+ * RandomState.get_state(); only the key goes up (dtfill_transfer_bytes: 2496 bytes with a resident ground truth).
+ * k11_mt_draw reproduces randint's masked rejection on the stream bit for bit and writes each frame's n rows and n columns
+ * in the layout k10_sample_bits reads; the rest is dtfill_eval_sampled's path.  Outputs (host, nullable): out_key [624] and
+ * *out_pos, the state the loop leaves behind (numpy twists lazily: the key of the block that holds the last consumed word,
+ * pos just past it, possibly 624; the input state when no word is consumed); out_words int64 [B], the 32-bit words frame b
+ * consumed (rows, then columns); out_rows / out_cols int32 [B*n], the drawn coordinates (for tests); out_lidar, per_frame,
+ * sums as for dtfill_eval_sampled.  Synchronous; strict order on the handle's stream.
+ * Errors: DTFILL_E_ARG before anything is enqueued for n < 0, H < 13, W < 17, mt_pos outside [0, 624] and what
+ * dtfill_eval_sampled refuses; then DTFILL_E_INDEX for the first frame Distance_Transform rejects (*first_bad_frame), in
+ * which case the state outputs are still written: the caller can rewind to the end of that frame's draw.
+ */
+int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, int n,
+                           const uint32_t* mt_key, int mt_pos, int r0, int r1, int c0, int c1, float src_thr,
+                           float val_thr, float* out_lidar, int32_t* out_rows, int32_t* out_cols, uint32_t* out_key,
+                           int* out_pos, int64_t* out_words, double* per_frame, double* sums, int* first_bad_frame);
+
+/* Host-only test hook (no handle, no GPU), like dtfill_debug_png_decode_host: the draw of dtfill_eval_sampled_mt from
+ * (key, pos) for B frames of H x W, run serially on the CPU with the kernel's MT19937 helpers.  rows / cols int32 [B*n],
+ * out_key [624], *out_pos, out_words int64 [B] as there.  Returns 0, or -1 for bad arguments. */
+int dtfill_debug_mt_draw_host(const uint32_t* key, int pos, int B, int H, int W, int n, int32_t* rows, int32_t* cols,
+                              uint32_t* out_key, int* out_pos, int64_t* out_words);
+
+/*
  * One step of an evaluation sweep, fused (BASELINE.json configs[4]; the loop body of eval.py:212-232: DT_complete_batch,
  * Result.evaluate per frame, running `+=` of the per-frame metrics): dtfill_run_async followed, on the same internal
  * stream, by the metric kernels on the filled depth against gt_dev (float64 when gt_is_f64, else float32, [B,H,W]).  The
