@@ -503,7 +503,9 @@ class Handle:
         _check(self._L.dtfill_set_sparse_upload(self._h, int(bool(enabled))), "dtfill_set_sparse_upload")
 
     def transfer_bytes(self):
-        """(host-to-device, device-to-host) bytes the last synchronous call with host buffers moved over the link."""
+        """(host-to-device, device-to-host) bytes the last synchronous call moved over the link: every call with an
+        in_is_device / out_is_device flag and every eval_* call starts both at 0 and counts each copy between host and
+        device it issues (the fills' 8-byte status words excepted); the *_async calls and eval_totals leave them alone."""
         a, b = ctypes.c_ulonglong(0), ctypes.c_ulonglong(0)
         _check(self._L.dtfill_transfer_bytes(self._h, ctypes.byref(a), ctypes.byref(b)), "dtfill_transfer_bytes")
         return int(a.value), int(b.value)

@@ -370,23 +370,25 @@ struct dtfill_ctx {
     Buf mx_terms, mx_counts, mx_leaf_start, mx_leaf_sum;     // dtfill_metrics in numpy's summation order (k4x_*)
     // PNG decode (k8_png_*): uploaded files + offsets, filtered bytes per frame, decoded samples (dtfill_run_png), status
     Buf png_data, png_scratch, png_samples, png_status;
-    PinBuf pin_png, pin_png_status;   // pinned staging of host file bytes / of the per-frame status
+    PinBuf pin_png;                   // pinned staging of host file bytes
+    PinBuf pin_png_status;            // pinned staging of small results on their way back: the decode status per frame
+                                      // (then the fill's counts of dtfill_eval_png*), or the counts and the flag word of
+                                      // dtfill_eval_sampled*
     // PNG encode (k9_png_*): uploaded input, filtered bytes, row Adler-32s, segment chunks and sizes, packed files and
     // their offsets (host outputs), filled depth of dtfill_run_png_to_png
     Buf enc_in, enc_filt, enc_adler, enc_slots, enc_seg, enc_out, enc_off, enc_depth;
     PinBuf pin_enc_off;
-    // dtfill_eval_sampled: uploaded host coordinates, the flag word of k10_sample_bits; pinned staging of host coordinates,
-    // and of the counts and the flag word on their way back
+    // dtfill_eval_sampled: uploaded host coordinates, the flag word of k10_sample_bits; pinned staging of host coordinates
     Buf smp_coords, smp_bad;
-    PinBuf pin_smp, pin_smp_out;
+    PinBuf pin_smp;
     bool metrics_exact = true;        // dtfill_metrics / _ex reproduce np.mean's pairwise sums bit for bit
     bool sparse_upload = true;        // pageable float32 inputs are compacted on the host instead of mirrored (see CopyPool)
-    size_t last_h2d_bytes = 0, last_d2h_bytes = 0;   // bytes the last synchronous host call moved over the link
+    size_t last_h2d_bytes = 0, last_d2h_bytes = 0;   // the link ledger of the last call (ledger_reset, copy_h2d, copy_d2h)
     CopyPool* pool_in = nullptr;
     CopyPool* pool_out = nullptr;
     int stage_threads = -1;           // threads per direction; -1: automatic; 0: never stage (driver-staged copies)
-    int32_t* counts_host = nullptr;   // pinned staging for out_counts (a pageable destination would serialise the
-    size_t counts_host_cap = 0;       // sliced copies: cudaMemcpyAsync to pageable memory blocks the host)
+    PinBuf counts_host;               // pinned staging for out_counts (a pageable destination would serialise the
+                                      // sliced copies: cudaMemcpyAsync to pageable memory blocks the host)
     bool profiling = false;
 #ifdef DTFILL_TRACE
     unsigned long long* trace_dev = nullptr;   // [TRACE_CALLS][4 kernels][4]
@@ -420,6 +422,36 @@ int ensure(dtfill_t* h, Buf& b, size_t bytes) {
     }
     b.cap = want;
     return 0;
+}
+
+// The link ledger (dtfill_transfer_bytes): every public entry point that can take host buffers starts it afresh on entry,
+// and every copy between host and device it issues goes through copy_h2d / copy_d2h, which count the bytes.  Only the
+// status ring's words (bookkeeping the asynchronous calls share) and the debug hooks copy outside the ledger.
+void ledger_reset(dtfill_t* h) {
+    if (h) h->last_h2d_bytes = h->last_d2h_bytes = 0;
+}
+
+int copy_h2d(dtfill_t* h, void* dst, const void* src, size_t bytes, cudaStream_t s) {
+    CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, s));
+    h->last_h2d_bytes += bytes;
+    return 0;
+}
+
+int copy_d2h(dtfill_t* h, void* dst, const void* src, size_t bytes, cudaStream_t s) {
+    CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s));
+    h->last_d2h_bytes += bytes;
+    return 0;
+}
+
+// An input of `bytes` bytes that may be on the host: p stays when it is on the device, else it becomes buf, to which
+// the host data is copied on the handle's stream.
+template <typename T>
+int device_input(dtfill_t* h, const T*& p, int on_device, Buf& buf, size_t bytes) {
+    if (on_device) return 0;
+    int rc = ensure(h, buf, bytes);
+    if (!rc) rc = copy_h2d(h, buf.p, p, bytes, h->stream);
+    if (!rc) p = (const T*)buf.p;
+    return rc;
 }
 
 // Host buffers of a dtfill_run call with host pointers: each sub-batch copies its own slices on its own stream, so
@@ -872,11 +904,10 @@ int enqueue(dtfill_t* h, const FillCall& c, const HostIO* hio = nullptr, bool fo
                 if (cnt) {
                     uint32_t* di = (uint32_t*)h->sparse_dev.p + ro;
                     uint32_t* dv = di + cap;
-                    CU(cudaMemcpyAsync(di, pi, cnt * 4, cudaMemcpyHostToDevice, st));
-                    CU(cudaMemcpyAsync(dv, pv, cnt * 4, cudaMemcpyHostToDevice, st));
+                    int r;
+                    if ((r = copy_h2d(h, di, pi, cnt * 4, st)) || (r = copy_h2d(h, dv, pv, cnt * 4, st))) return r;
                     k0_scatter_pairs<<<(unsigned)((cnt + 255) / 256), 256, 0, st>>>(di, dv, (unsigned)cnt, dst);
                 }
-                h->last_h2d_bytes += cnt * 8;
                 return 0;
             }
             // a slice denser than the pair buffer allows: the mirror after all
@@ -891,22 +922,18 @@ int enqueue(dtfill_t* h, const FillCall& c, const HostIO* hio = nullptr, bool fo
             h->pool_in->copy(pin, src, nb * frame_bytes);
             src = pin;
         }
-        CU(cudaMemcpyAsync((char*)const_cast<void*>(c.in) + b0 * frame_bytes, src, nb * frame_bytes, cudaMemcpyHostToDevice, st));
-        h->last_h2d_bytes += nb * frame_bytes;
-        return 0;
+        return copy_h2d(h, (char*)const_cast<void*>(c.in) + b0 * frame_bytes, src, nb * frame_bytes, st);
     };
     auto copy_out = [&](cudaStream_t st, int b0, int nb) -> int {
         if (!hio) return 0;
         const size_t o = (size_t)b0 * H * W, n = (size_t)nb * H * W;
-        CU(cudaMemcpyAsync((hio->depth_pin ? hio->depth_pin : hio->depth) + o, c.depth + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->lidar) CU(cudaMemcpyAsync((hio->lidar_pin ? hio->lidar_pin : hio->lidar) + o, c.lidar + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->dt) CU(cudaMemcpyAsync((hio->dt_pin ? hio->dt_pin : hio->dt) + o, c.dt + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->lbl) CU(cudaMemcpyAsync((hio->lbl_pin ? hio->lbl_pin : hio->lbl) + o, c.lbl + o, n * 4, cudaMemcpyDeviceToHost, st));
-        if (hio->mask) CU(cudaMemcpyAsync((hio->mask_pin ? hio->mask_pin : hio->mask) + o, c.mask + o, n, cudaMemcpyDeviceToHost, st));
-        if (hio->counts)
-            CU(cudaMemcpyAsync(hio->counts + 2 * (size_t)b0, c.counts + 2 * (size_t)b0, (size_t)nb * 8,
-                               cudaMemcpyDeviceToHost, st));
-        h->last_d2h_bytes += n * (4 + (hio->lidar ? 4 : 0) + (hio->dt ? 4 : 0) + (hio->lbl ? 4 : 0) + (hio->mask ? 1 : 0));
+        int r;
+        if ((r = copy_d2h(h, (hio->depth_pin ? hio->depth_pin : hio->depth) + o, c.depth + o, n * 4, st))) return r;
+        if (hio->lidar && (r = copy_d2h(h, (hio->lidar_pin ? hio->lidar_pin : hio->lidar) + o, c.lidar + o, n * 4, st))) return r;
+        if (hio->dt && (r = copy_d2h(h, (hio->dt_pin ? hio->dt_pin : hio->dt) + o, c.dt + o, n * 4, st))) return r;
+        if (hio->lbl && (r = copy_d2h(h, (hio->lbl_pin ? hio->lbl_pin : hio->lbl) + o, c.lbl + o, n * 4, st))) return r;
+        if (hio->mask && (r = copy_d2h(h, (hio->mask_pin ? hio->mask_pin : hio->mask) + o, c.mask + o, n, st))) return r;
+        if (hio->counts && (r = copy_d2h(h, hio->counts + 2 * (size_t)b0, c.counts + 2 * (size_t)b0, (size_t)nb * 8, st))) return r;
         return 0;
     };
     if (nsub == 1 && !(hio && hio->any_out_pin())) {
@@ -994,13 +1021,10 @@ int enqueue(dtfill_t* h, const FillCall& c, const HostIO* hio = nullptr, bool fo
 // Per-frame metrics in numpy's own summation order (k4x_*): per-pixel terms of the valid pixels compacted in raster order,
 // then the pairwise tree of np.add.reduce; groups of frames share a scratch of at most ~4 GiB (a batch of 256 KITTI frames
 // with a float64 ground truth needs 3.5 GB: one group, every frame's tree in flight at once).  GT: the arithmetic type,
-// GS: the ground truth as stored.  WIN: npx is the area of the crop window `win` of frames of win.frame_px pixels.
-// CROP_FLOOR: npx pixels per prediction frame against rows win.r0: of ground-truth frames of win.frame_px samples, the
-// prediction floored at 0.9 (k4x_compact).  Device pointers; enqueued on s.
-template <typename GT, int MODE, typename GS, bool WIN = false, bool CROP_FLOOR = false>
-int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, double* per_frame, cudaStream_t s,
-                const K4xWindow& win = K4xWindow{}) {
-    const long pstride = WIN ? win.frame_px : npx, gstride = WIN || CROP_FLOOR ? win.frame_px : npx;
+// GS: the ground truth as stored; npx pixels per frame lie in pred and gt as geom says (k4x_compact).  Device pointers;
+// enqueued on the handle's stream.
+template <typename GT, int MODE, typename GS, bool WIN, bool FLOOR>
+int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, const K4xGeom& geom, int B, long npx, double* per_frame) {
     const size_t gsz = sizeof(GT);
     const long maxl = npx / 64 + 2;
     long G = (long)((1ull << 32) / ((size_t)4 * npx * gsz));
@@ -1014,11 +1038,31 @@ int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, int B, long npx, d
         const int ng = (int)(B - g0 < G ? B - g0 : G);
         GT* tm = (GT*)h->mx_terms.p;
         int* cn = (int*)h->mx_counts.p;
-        k4x_compact<GT, MODE, GS, WIN, CROP_FLOOR><<<ng, K4X_THREADS, 0, s>>>(pred + g0 * pstride, gt + g0 * gstride, npx, tm,
-                                                                                cn, win);
-        k4x_reduce<GT><<<ng, K4X_RTHREADS, 0, s>>>(tm, cn, npx, MODE, (int*)h->mx_leaf_start.p, (GT*)h->mx_leaf_sum.p,
-                                                   per_frame + g0 * 9);
+        k4x_compact<GT, MODE, GS, WIN, FLOOR><<<ng, K4X_THREADS, 0, h->stream>>>(pred, gt, geom, g0, npx, tm, cn);
+        k4x_reduce<GT><<<ng, K4X_RTHREADS, 0, h->stream>>>(tm, cn, npx, MODE, (int*)h->mx_leaf_start.p,
+                                                           (GT*)h->mx_leaf_sum.p, per_frame + g0 * 9);
     }
+    return 0;
+}
+
+// Result.evaluate / Result_NYU.evaluate of B frames in numpy's summation order, on the handle's stream: the per-frame
+// metrics [B,9] and their column sums [10] (added to when accumulate).  out_is_device: per_frame / sums are device
+// vectors the kernels write, the handle's buffers standing in for a null one; otherwise the results are copied from the
+// handle's buffers to whichever of the host pointers per_frame / sums is non-null (the caller synchronises).
+template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool FLOOR = false>
+int k4x_score(dtfill_t* h, const float* pred, const GS* gt, const K4xGeom& geom, int B, long npx, double* per_frame,
+              double* sums, int out_is_device = 0, int accumulate = 0) {
+    int rc;
+    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
+    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
+    double* pf_d = (out_is_device && per_frame) ? per_frame : (double*)h->per_frame.p;
+    double* sm_d = (out_is_device && sums) ? sums : (double*)h->sums.p;
+    if ((rc = k4x_enqueue<GT, MODE, GS, WIN, FLOOR>(h, pred, gt, geom, B, npx, pf_d))) return rc;
+    k4x_sums<<<1, 32, 0, h->stream>>>(pf_d, B, sm_d, accumulate);
+    CU(cudaGetLastError());
+    if (out_is_device) return 0;
+    if (per_frame && (rc = copy_d2h(h, per_frame, pf_d, (size_t)B * 9 * 8, h->stream))) return rc;
+    if (sums && (rc = copy_d2h(h, sums, sm_d, 10 * 8, h->stream))) return rc;
     return 0;
 }
 
@@ -1110,7 +1154,6 @@ void dtfill_destroy(dtfill_t* h) {
         }
     }
     for (void* q : h->retired) cudaFree(q);
-    if (h->counts_host) cudaFreeHost(h->counts_host);
     delete h->pool_in;
     delete h->pool_out;
     if (h->status_ring) cudaFreeHost(h->status_ring);
@@ -1217,7 +1260,7 @@ int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, 
     const bool pipelined = !out_is_device && (!in_is_device || in_resident);
     if (!in_is_device) {
         if ((rc = ensure(h, h->in_dev, in_bytes))) return rc;
-        if (!pipelined) CU(cudaMemcpyAsync(h->in_dev.p, in, in_bytes, cudaMemcpyHostToDevice, h->stream));
+        if (!pipelined && (rc = copy_h2d(h, h->in_dev.p, in, in_bytes, h->stream))) return rc;
         c.in = h->in_dev.p;
     }
     if (!out_is_device) {
@@ -1229,7 +1272,6 @@ int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, 
         if (out_mask) { if ((rc = ensure(h, h->mask_dev, npx))) return rc; c.mask = (uint8_t*)h->mask_dev.p; }
         if (out_counts) { if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc; c.counts = (int32_t*)h->counts_out_dev.p; }
     }
-    h->last_h2d_bytes = h->last_d2h_bytes = 0;
     if (pipelined) {
         HostIO hio;
         hio.in = in_resident ? nullptr : in; hio.lidar = out_lidar; hio.depth = out_depth; hio.dt = out_dt; hio.lbl = out_lbl; hio.mask = out_mask;
@@ -1272,28 +1314,23 @@ int run_sync(dtfill_t* h, const void* in, int in_is_device, bool u16, int in_H, 
             }
         }
         if (out_counts) {
-            if (h->counts_host_cap < (size_t)B * 2) {
-                if (h->counts_host) cudaFreeHost(h->counts_host);
-                h->counts_host = nullptr;
-                h->counts_host_cap = 0;
-                CU(cudaHostAlloc((void**)&h->counts_host, (size_t)B * 8 + 64, cudaHostAllocDefault));
-                h->counts_host_cap = (size_t)B * 2 + 16;
-            }
-            hio.counts = h->counts_host;
+            if ((rc = ensure_pinned(h->counts_host, (size_t)B * 8))) return rc;
+            hio.counts = (int32_t*)h->counts_host.p;
         }
         if ((rc = enqueue(h, c, &hio, true))) return rc;
         rc = dtfill_status(h, first_bad_frame, nullptr);
-        if (out_counts && (rc == 0 || rc == DTFILL_E_INDEX)) memcpy(out_counts, h->counts_host, (size_t)B * 8);
+        if (out_counts && (rc == 0 || rc == DTFILL_E_INDEX)) memcpy(out_counts, h->counts_host.p, (size_t)B * 8);
         return rc;
     }
     if ((rc = enqueue(h, c, nullptr, true))) return rc;
     if (!out_is_device) {
-        CU(cudaMemcpyAsync(out_depth, c.depth, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_lidar) CU(cudaMemcpyAsync(out_lidar, c.lidar, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_dt) CU(cudaMemcpyAsync(out_dt, c.dt, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_lbl) CU(cudaMemcpyAsync(out_lbl, c.lbl, npx * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (out_mask) CU(cudaMemcpyAsync(out_mask, c.mask, npx, cudaMemcpyDeviceToHost, h->stream));
-        if (out_counts) CU(cudaMemcpyAsync(out_counts, c.counts, (size_t)B * 8, cudaMemcpyDeviceToHost, h->stream));
+        cudaStream_t s = h->stream;
+        if ((rc = copy_d2h(h, out_depth, c.depth, npx * 4, s))) return rc;
+        if (out_lidar && (rc = copy_d2h(h, out_lidar, c.lidar, npx * 4, s))) return rc;
+        if (out_dt && (rc = copy_d2h(h, out_dt, c.dt, npx * 4, s))) return rc;
+        if (out_lbl && (rc = copy_d2h(h, out_lbl, c.lbl, npx * 4, s))) return rc;
+        if (out_mask && (rc = copy_d2h(h, out_mask, c.mask, npx, s))) return rc;
+        if (out_counts && (rc = copy_d2h(h, out_counts, c.counts, (size_t)B * 8, s))) return rc;
     }
     return dtfill_status(h, first_bad_frame, nullptr);
 }
@@ -1311,6 +1348,7 @@ int dtfill_run(dtfill_t* h, const float* in, int in_is_device, int B, int H, int
                float* out_depth, float* out_dt, int32_t* out_lbl, uint8_t* out_mask, int32_t* out_counts,
                int out_is_device, int* first_bad_frame) {
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     if (!h || !in || !out_depth) return fail(DTFILL_E_ARG, "dtfill_run: NULL handle, input or out_depth");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_run: B, H, W must be positive");
     return run_sync(h, in, in_is_device, false, H, 0, B, H, W, src_thr, val_thr, nullptr, out_depth, out_dt, out_lbl,
@@ -1321,6 +1359,7 @@ int dtfill_run_u16(dtfill_t* h, const uint16_t* in, int in_is_device, int B, int
                    float val_thr, float* out_lidar, float* out_depth, float* out_dt, int32_t* out_lbl, uint8_t* out_mask,
                    int32_t* out_counts, int out_is_device, int* first_bad_frame) {
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     int rc = check_u16_args("dtfill_run_u16", h, in, out_depth, B, H_in, W, crop_top);
     if (rc) return rc;
     return run_sync(h, in, in_is_device, true, H_in, crop_top, B, H_in - crop_top, W, src_thr, val_thr, out_lidar, out_depth,
@@ -1416,8 +1455,7 @@ int png_stage(dtfill_t* h, const PngFiles* sets, int nsets, const uint8_t** d_da
         pos += f.offsets[f.B] - o0;
     }
     po[i] = pos;
-    CU(cudaMemcpyAsync(h->png_data.p, pin, total, cudaMemcpyHostToDevice, h->stream));
-    h->last_h2d_bytes = total;
+    if ((rc = copy_h2d(h, h->png_data.p, pin, total, h->stream))) return rc;
     *d_data = (const uint8_t*)h->png_data.p;
     *d_off = (const int64_t*)((uint8_t*)h->png_data.p + off_at);
     return 0;
@@ -1456,6 +1494,7 @@ int png_status_host(dtfill_t* h, int B, int32_t** out) {
 int dtfill_png_decode(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int in_is_device, int B, int H, int W,
                       uint16_t* out, int32_t* out_status, int out_is_device, int* first_bad_frame) {
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     int rc = png_args("dtfill_png_decode", h, data, offsets, out, B, H, W);
     if (rc) return rc;
     if (out_is_device && !out_status) return fail(DTFILL_E_ARG, "dtfill_png_decode: out_status is required with device outputs");
@@ -1472,8 +1511,8 @@ int dtfill_png_decode(dtfill_t* h, const uint8_t* data, const int64_t* offsets, 
     if (in_is_device && out_is_device) return 0;
     int32_t* st_host = nullptr;
     if ((rc = png_status_host(h, B, &st_host))) return rc;
-    if (!out_is_device) CU(cudaMemcpyAsync(out, od, (size_t)B * H * W * 2, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaMemcpyAsync(st_host, os, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream));
+    if (!out_is_device && (rc = copy_d2h(h, out, od, (size_t)B * H * W * 2, h->stream))) return rc;
+    if ((rc = copy_d2h(h, st_host, os, (size_t)B * 4, h->stream))) return rc;
     CU(cudaStreamSynchronize(h->stream));
     if (!out_is_device && out_status) memcpy(out_status, st_host, (size_t)B * 4);
     return png_verdict(st_host, B, first_bad_frame);
@@ -1483,6 +1522,7 @@ int dtfill_run_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int
                    int crop_top, float src_thr, float val_thr, float* out_lidar, float* out_depth, float* out_dt,
                    int32_t* out_lbl, uint8_t* out_mask, int32_t* out_counts, int out_is_device, int* first_bad_frame) {
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     int rc = png_args("dtfill_run_png", h, data, offsets, out_depth, B, H_in, W);
     if (rc) return rc;
     if ((rc = check_u16_args("dtfill_run_png", h, data, out_depth, B, H_in, W, crop_top))) return rc;
@@ -1493,12 +1533,10 @@ int dtfill_run_png(dtfill_t* h, const uint8_t* data, const int64_t* offsets, int
     if ((rc = png_status_host(h, B, &st_host))) return rc;
     uint16_t* samples = (uint16_t*)h->png_samples.p;
     if ((rc = png_enqueue(h, data, offsets, in_is_device, B, H_in, W, samples, (int32_t*)h->png_status.p))) return rc;
-    CU(cudaMemcpyAsync(st_host, h->png_status.p, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream));
-    const size_t h2d = in_is_device ? 0 : h->last_h2d_bytes;
+    if ((rc = copy_d2h(h, st_host, h->png_status.p, (size_t)B * 4, h->stream))) return rc;
     // the fill of dtfill_run_u16 on the decoded samples; it ends with a synchronisation, so st_host is final afterwards
     rc = run_sync(h, samples, 1, true, H_in, crop_top, B, H_in - crop_top, W, src_thr, val_thr, out_lidar, out_depth, out_dt,
                   out_lbl, out_mask, out_counts, out_is_device, first_bad_frame, true);
-    h->last_h2d_bytes += h2d;
     if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
     const int rd = png_verdict(st_host, B, first_bad_frame);     // a decode failure wins over IndexError
     return rd ? rd : rc;
@@ -1620,15 +1658,8 @@ int png_encode_call(const char* who, dtfill_t* h, const void* in, bool is_float,
     int rc = png_encode_args(who, h, in, out, out_offsets, B, H, W, out_capacity);
     if (rc) return rc;
     CU(cudaSetDevice(h->device));
-    h->last_h2d_bytes = h->last_d2h_bytes = 0;
     const void* in_d = in;
-    if (!in_is_device) {
-        const size_t in_bytes = (size_t)B * H * W * (is_float ? 4 : 2);
-        if ((rc = ensure(h, h->enc_in, in_bytes))) return rc;
-        CU(cudaMemcpyAsync(h->enc_in.p, in, in_bytes, cudaMemcpyHostToDevice, h->stream));
-        h->last_h2d_bytes = in_bytes;
-        in_d = h->enc_in.p;
-    }
+    if ((rc = device_input(h, in_d, in_is_device, h->enc_in, (size_t)B * H * W * (is_float ? 4 : 2)))) return rc;
     uint8_t* out_d = out;
     int64_t* off_d = out_offsets;
     if (!out_is_device) {
@@ -1646,12 +1677,11 @@ int png_encode_call(const char* who, dtfill_t* h, const void* in, bool is_float,
     // offsets first, then exactly offsets[B] bytes of files
     if ((rc = ensure_pinned(h->pin_enc_off, (size_t)(B + 1) * 8))) return rc;
     int64_t* off_h = (int64_t*)h->pin_enc_off.p;
-    CU(cudaMemcpyAsync(off_h, off_d, (size_t)(B + 1) * 8, cudaMemcpyDeviceToHost, h->stream));
+    if ((rc = copy_d2h(h, off_h, off_d, (size_t)(B + 1) * 8, h->stream))) return rc;
     CU(cudaStreamSynchronize(h->stream));
     memcpy(out_offsets, off_h, (size_t)(B + 1) * 8);
-    CU(cudaMemcpyAsync(out, out_d, (size_t)off_h[B], cudaMemcpyDeviceToHost, h->stream));
+    if ((rc = copy_d2h(h, out, out_d, (size_t)off_h[B], h->stream))) return rc;
     CU(cudaStreamSynchronize(h->stream));
-    h->last_d2h_bytes = (size_t)(B + 1) * 8 + (size_t)off_h[B];
     return 0;
 }
 
@@ -1708,12 +1738,14 @@ int64_t dtfill_png_encode_bound(int H, int W) {
 
 int dtfill_png_encode(dtfill_t* h, const uint16_t* in, int in_is_device, int B, int H, int W, uint8_t* out,
                       int64_t out_capacity, int64_t* out_offsets, int out_is_device) {
+    ledger_reset(h);
     return png_encode_call("dtfill_png_encode", h, in, false, in_is_device, B, H, W, out, out_capacity, out_offsets,
                            out_is_device);
 }
 
 int dtfill_png_encode_depth(dtfill_t* h, const float* in, int in_is_device, int B, int H, int W, uint8_t* out,
                             int64_t out_capacity, int64_t* out_offsets, int out_is_device) {
+    ledger_reset(h);
     return png_encode_call("dtfill_png_encode_depth", h, in, true, in_is_device, B, H, W, out, out_capacity, out_offsets,
                            out_is_device);
 }
@@ -1731,16 +1763,15 @@ int dtfill_run_png_to_png(dtfill_t* h, const uint8_t* data, const int64_t* offse
     CU(cudaSetDevice(h->device));
     if ((rc = ensure(h, h->enc_depth, (size_t)B * H * W * 4))) return rc;
     float* depth = (float*)h->enc_depth.p;
+    // (dtfill_run_png starts the link ledger: nothing has crossed the link before it)
     const int run = dtfill_run_png(h, data, offsets, in_is_device, B, H_in, W, crop_top, src_thr, val_thr, nullptr, depth,
                                    nullptr, nullptr, nullptr, nullptr, 1, first_bad_frame);
     if (run != 0 && run != DTFILL_E_INDEX && run != DTFILL_E_DATA) return run;
     const std::string verdict = g_err;
-    const size_t h2d = h->last_h2d_bytes;
     if ((rc = png_encode_call("dtfill_run_png_to_png", h, depth, true, 1, B, H, W, out, out_capacity, out_offsets,
                               out_is_device)))
         return rc;
     if (out_is_device) CU(cudaStreamSynchronize(h->stream));
-    h->last_h2d_bytes = h2d;
     if (run) g_err = verdict;
     return run;
 }
@@ -1872,6 +1903,7 @@ int dtfill_metrics(dtfill_t* h, const float* pred, const void* gt, int gt_is_f64
 
 int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_f64, int in_is_device, int B, int H, int W,
                       int mode, double* per_frame, double* sums, int out_is_device, int accumulate) {
+    ledger_reset(h);
     if (!h || !pred || !gt) return fail(DTFILL_E_ARG, "dtfill_metrics: NULL handle or input");
     if (accumulate && !(out_is_device && sums))
         return fail(DTFILL_E_ARG, "dtfill_metrics_ex: accumulate needs a device-resident sums vector");
@@ -1881,39 +1913,30 @@ int dtfill_metrics_ex(dtfill_t* h, const float* pred, const void* gt, int gt_is_
     { int frc = dtfill_flush(h); if (frc) return frc; }      // pipelined fills feeding this evaluation
     const long npx = (long)H * W;
     const size_t tot = (size_t)B * npx;
-    const size_t gsz = gt_is_f64 ? 8 : 4;
+    cudaStream_t s = h->stream;
     int rc;
     const float* p_d = pred;
     const void* g_d = gt;
-    cudaStream_t s = h->stream;
-    if (!in_is_device) {
-        if ((rc = ensure(h, h->in_dev, tot * 4))) return rc;
-        if ((rc = ensure(h, h->gt_dev, tot * gsz))) return rc;
-        CU(cudaMemcpyAsync(h->in_dev.p, pred, tot * 4, cudaMemcpyHostToDevice, s));
-        CU(cudaMemcpyAsync(h->gt_dev.p, gt, tot * gsz, cudaMemcpyHostToDevice, s));
-        p_d = (const float*)h->in_dev.p;
-        g_d = h->gt_dev.p;
-    }
-    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
-    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
-    double* pf_d = (out_is_device && per_frame) ? per_frame : (double*)h->per_frame.p;
-    double* sm_d = (out_is_device && sums) ? sums : (double*)h->sums.p;
+    if ((rc = device_input(h, p_d, in_is_device, h->in_dev, tot * 4))) return rc;
+    if ((rc = device_input(h, g_d, in_is_device, h->gt_dev, tot * (gt_is_f64 ? 8 : 4)))) return rc;
     if (h->metrics_exact && npx < (1l << 31)) {
         rc = with_gt_mode(gt_is_f64, mode, [&](auto g, auto m) {
             using GT = decltype(g);
-            return k4x_enqueue<GT, decltype(m)::value>(h, p_d, (const GT*)g_d, B, npx, pf_d, s);
+            return k4x_score<GT, decltype(m)::value>(h, p_d, (const GT*)g_d, K4xGeom{npx, 0, npx, 0, W, W}, B, npx,
+                                                     per_frame, sums, out_is_device, accumulate);
         });
         if (rc) return rc;
-        k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, accumulate);
-    } else if ((rc = metrics_onepass(h, h->partial, p_d, g_d, gt_is_f64, mode, B, npx, pf_d, sm_d, accumulate, s))) {
-        return rc;
+    } else {
+        if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
+        if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
+        double* pf_d = (out_is_device && per_frame) ? per_frame : (double*)h->per_frame.p;
+        double* sm_d = (out_is_device && sums) ? sums : (double*)h->sums.p;
+        if ((rc = metrics_onepass(h, h->partial, p_d, g_d, gt_is_f64, mode, B, npx, pf_d, sm_d, accumulate, s))) return rc;
+        CU(cudaGetLastError());
+        if (!out_is_device && per_frame && (rc = copy_d2h(h, per_frame, pf_d, (size_t)B * 9 * 8, s))) return rc;
+        if (!out_is_device && sums && (rc = copy_d2h(h, sums, sm_d, 10 * 8, s))) return rc;
     }
-    CU(cudaGetLastError());
-    if (!out_is_device) {
-        if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
-        if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
-        CU(cudaStreamSynchronize(s));
-    }
+    if (!out_is_device) CU(cudaStreamSynchronize(s));
     return 0;
 }
 
@@ -1942,7 +1965,6 @@ int eval_png_run(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets
     const uint8_t* d_data;
     const int64_t* d_off;
     if ((rc = png_stage(h, sets, gt_dev ? 1 : 2, &d_data, &d_off))) return rc;
-    const size_t h2d = h->last_h2d_bytes;
     if ((rc = png_enqueue(h, d_data, d_off, 1, nfiles, H_in, W, samples, status))) return rc;
     // 2. the fill of dtfill_run_u16 on rows crop_top: of the LiDAR samples, strict order on the handle's stream; only the
     //    counts leave the device
@@ -1955,28 +1977,15 @@ int eval_png_run(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets
     if ((rc = enqueue(h, fill, nullptr, true))) return rc;
     // 3. Result.evaluate of the filled depth against the same rows of the ground-truth samples, in numpy's summation
     //    order whatever dtfill_set_metrics_exact says
-    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
-    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
-    double* pf_d = (double*)h->per_frame.p;
-    double* sm_d = (double*)h->sums.p;
     const uint16_t* g_d = gt_dev ? gt_dev : samples + (size_t)B * npx_in;
-    if (floor) {
-        const K4xWindow rows{npx_in, W, crop_top, 0, W};
-        rc = k4x_enqueue<double, 0, uint16_t, false, true>(h, fill.depth, g_d, B, npx, pf_d, s, rows);
-    } else {
-        rc = k4x_enqueue<double, 0>(h, fill.depth, g_d, B, npx, pf_d, s);
-    }
+    const K4xGeom rows{npx, 0, npx_in, (long)crop_top * W, W, W};
+    rc = floor ? k4x_score<double, 0, uint16_t, false, true>(h, fill.depth, g_d, rows, B, npx, per_frame, sums)
+               : k4x_score<double, 0, uint16_t>(h, fill.depth, g_d, rows, B, npx, per_frame, sums);
     if (rc) return rc;
-    k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(st_host, status, (size_t)nfiles * 4, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(st_host + nfiles, fill.counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
-    if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
+    if ((rc = copy_d2h(h, st_host, status, (size_t)nfiles * 4, s))) return rc;
+    if ((rc = copy_d2h(h, st_host + nfiles, fill.counts, (size_t)B * 8, s))) return rc;
     int fill_bad = -1;
     rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
-    h->last_h2d_bytes = h2d;
-    h->last_d2h_bytes = (size_t)nfiles * 4 + (size_t)B * (8 + (per_frame ? 9 * 8 : 0)) + (sums ? 10 * 8 : 0);
     if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
     // 4. the verdict, frame by frame as the loop meets it: a decode failure (LiDAR before ground truth) wins over an
     //    IndexError of Distance_Transform
@@ -1998,6 +2007,7 @@ int dtfill_eval_png(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offs
                     const int64_t* gt_offsets, int B, int H, int W, float src_thr, float val_thr, double* per_frame,
                     double* sums, int* first_bad_frame) {
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     if (!h || !lidar || !lidar_offsets || !gt || !gt_offsets)
         return fail(DTFILL_E_ARG, "dtfill_eval_png: NULL handle, files or offsets");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_eval_png: B, H, W must be positive");
@@ -2012,6 +2022,7 @@ int dtfill_eval_png_kitti(dtfill_t* h, const uint8_t* lidar, const int64_t* lida
                           float src_thr, float val_thr, double* per_frame, double* sums, int* first_bad_frame) {
     const char* who = "dtfill_eval_png_kitti";
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     if (!h || !lidar || !lidar_offsets) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, LiDAR files or offsets");
     const bool files = gt || gt_offsets;
     if (files == (gt_samples_dev != nullptr) || (files && !(gt && gt_offsets)))
@@ -2043,24 +2054,18 @@ int sampled_frame_check(const char* who, const float* gt, int gt_is_device, int 
 
 // Steps 2-6 of dtfill_eval_sampled and dtfill_eval_sampled_mt, after the device coordinates d_rows / d_cols / d_off are
 // enqueued on the handle's stream: the ground truth, the sample bitmap, the fill, the metrics of the window, the copies
-// back and the verdict.  h2d: bytes the caller sent up already; d2h: bytes of copies back the caller enqueued already
-// (they complete with this call's synchronisation).
+// back and the verdict (copies back the caller enqueued already complete with this call's synchronisation).
 int eval_sampled_run(dtfill_t* h, const char* who, const float* gt, int gt_is_device, int B, int H, int W,
-                     const int32_t* d_rows, const int32_t* d_cols, const int64_t* d_off, size_t h2d, size_t d2h, int r0,
-                     int r1, int c0, int c1, float src_thr, float val_thr, float* out_lidar, double* per_frame,
-                     double* sums, int* first_bad_frame) {
+                     const int32_t* d_rows, const int32_t* d_cols, const int64_t* d_off, int r0, int r1, int c0, int c1,
+                     float src_thr, float val_thr, float* out_lidar, double* per_frame, double* sums,
+                     int* first_bad_frame) {
     const long npx = (long)H * W;
     const int WW = (W + 31) / 32;
     cudaStream_t s = h->stream;
     int rc;
     // 2. the ground truth, unless it is resident
     const float* g_d = gt;
-    if (!gt_is_device) {
-        if ((rc = ensure(h, h->gt_dev, (size_t)B * npx * 4))) return rc;
-        CU(cudaMemcpyAsync(h->gt_dev.p, gt, (size_t)B * npx * 4, cudaMemcpyHostToDevice, s));
-        h2d += (size_t)B * npx * 4;
-        g_d = (const float*)h->gt_dev.p;
-    }
+    if ((rc = device_input(h, g_d, gt_is_device, h->gt_dev, (size_t)B * npx * 4))) return rc;
     // 3. the sample bitmap in lane 0's srcbits (the lane of a strict-order fill), sized as the fill sizes it so that the
     //    fill does not reallocate it
     Lane* L = &h->lanes[0];
@@ -2081,26 +2086,17 @@ int eval_sampled_run(dtfill_t* h, const char* who, const float* gt, int gt_is_de
     if ((rc = enqueue(h, fill, nullptr, true))) return rc;
     // 5. Result_NYU.evaluate of the window of the filled depth against the same window of the ground truth, in numpy's
     //    summation order whatever dtfill_set_metrics_exact says
-    if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
-    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
-    double* pf_d = (double*)h->per_frame.p;
-    double* sm_d = (double*)h->sums.p;
-    const K4xWindow win{npx, W, r0, c0, c1 - c0};
-    if ((rc = k4x_enqueue<float, 1, float, true>(h, fill.depth, g_d, B, (long)(r1 - r0) * (c1 - c0), pf_d, s, win))) return rc;
-    k4x_sums<<<1, 32, 0, s>>>(pf_d, B, sm_d, 0);
-    CU(cudaGetLastError());
-    if ((rc = ensure_pinned(h->pin_smp_out, (size_t)B * 8 + 4))) return rc;
-    int32_t* out_h = (int32_t*)h->pin_smp_out.p;            // the fill's counts [B][2], then the flag word
-    CU(cudaMemcpyAsync(out_h, fill.counts, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(out_h + 2 * B, h->smp_bad.p, 4, cudaMemcpyDeviceToHost, s));
-    if (per_frame) CU(cudaMemcpyAsync(per_frame, pf_d, (size_t)B * 9 * 8, cudaMemcpyDeviceToHost, s));
-    if (sums) CU(cudaMemcpyAsync(sums, sm_d, 10 * 8, cudaMemcpyDeviceToHost, s));
-    if (out_lidar) CU(cudaMemcpyAsync(out_lidar, fill.lidar, (size_t)B * npx * 4, cudaMemcpyDeviceToHost, s));
+    const long at = (long)r0 * W + c0;
+    const K4xGeom win{npx, at, npx, at, W, c1 - c0};
+    if ((rc = k4x_score<float, 1, float, true>(h, fill.depth, g_d, win, B, (long)(r1 - r0) * (c1 - c0), per_frame, sums)))
+        return rc;
+    if ((rc = ensure_pinned(h->pin_png_status, (size_t)B * 8 + 4))) return rc;
+    int32_t* out_h = (int32_t*)h->pin_png_status.p;          // the fill's counts [B][2], then the flag word
+    if ((rc = copy_d2h(h, out_h, fill.counts, (size_t)B * 8, s))) return rc;
+    if ((rc = copy_d2h(h, out_h + 2 * B, h->smp_bad.p, 4, s))) return rc;
+    if (out_lidar && (rc = copy_d2h(h, out_lidar, fill.lidar, (size_t)B * npx * 4, s))) return rc;
     int fill_bad = -1;
     rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
-    h->last_h2d_bytes = h2d;
-    h->last_d2h_bytes = d2h + (size_t)B * 8 + 4 + (per_frame ? (size_t)B * 9 * 8 : 0) + (sums ? 10 * 8 : 0) +
-                        (out_lidar ? (size_t)B * npx * 4 : 0);
     if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
     // 6. the verdict: device coordinates outside the frame, then Distance_Transform's frame by frame
     const int bad = out_h[2 * B];
@@ -2120,6 +2116,7 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
                         int* first_bad_frame) {
     const char* who = "dtfill_eval_sampled";
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     if (!h || !gt || !rows || !cols || !sample_offsets)
         return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, ground truth, coordinates or offsets");
     int rc = sampled_frame_check(who, gt, gt_is_device, B, H, W, r0, r1, c0, c1);
@@ -2127,8 +2124,6 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
     CU(cudaSetDevice(h->device));
     rc = dtfill_flush(h);            // fills in flight (pipelined mode) may still use lane 0's workspace
     if (rc) return rc;
-    cudaStream_t s = h->stream;
-    size_t h2d = 0;
     // 1. coordinates: host ones are checked here and go up in one copy through the pinned staging buffer (rows, cols, then
     //    the offsets rebased to 0); device ones are checked by k10_sample_bits
     const int32_t* d_rows = rows;
@@ -2162,14 +2157,13 @@ int dtfill_eval_sampled(dtfill_t* h, const float* gt, int gt_is_device, int B, i
         }
         int64_t* po = (int64_t*)(pin + off_at);
         for (int b = 0; b <= B; ++b) po[b] = o[b] - o[0];
-        CU(cudaMemcpyAsync(h->smp_coords.p, pin, total, cudaMemcpyHostToDevice, s));
-        h2d += total;
+        if ((rc = copy_h2d(h, h->smp_coords.p, pin, total, h->stream))) return rc;
         d_rows = (const int32_t*)h->smp_coords.p;
         d_cols = d_rows + n;
         d_off = (const int64_t*)((uint8_t*)h->smp_coords.p + off_at);
     }
-    return eval_sampled_run(h, who, gt, gt_is_device, B, H, W, d_rows, d_cols, d_off, h2d, 0, r0, r1, c0, c1, src_thr,
-                            val_thr, out_lidar, per_frame, sums, first_bad_frame);
+    return eval_sampled_run(h, who, gt, gt_is_device, B, H, W, d_rows, d_cols, d_off, r0, r1, c0, c1, src_thr, val_thr,
+                            out_lidar, per_frame, sums, first_bad_frame);
 }
 
 int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, int n,
@@ -2178,6 +2172,7 @@ int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B
                            int* out_pos, int64_t* out_words, double* per_frame, double* sums, int* first_bad_frame) {
     const char* who = "dtfill_eval_sampled_mt";
     if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
     if (!h || !gt || !mt_key) return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, ground truth or key");
     if (n < 0) return fail(DTFILL_E_ARG, std::string(who) + ": negative sample count");
     if (H < 13 || W < 17) return fail(DTFILL_E_ARG, std::string(who) + ": frames need H >= 13 and W >= 17 (randint(H - 12), randint(W - 16))");
@@ -2201,7 +2196,7 @@ int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B
     uint8_t* pin = (uint8_t*)h->pin_smp.p;
     uint8_t* dev = (uint8_t*)h->smp_coords.p;
     memcpy(pin, mt_key, MT_N * 4);
-    CU(cudaMemcpyAsync(dev + key_at, pin, MT_N * 4, cudaMemcpyHostToDevice, s));
+    if ((rc = copy_h2d(h, dev + key_at, pin, MT_N * 4, s))) return rc;
     int32_t* d_rows = (int32_t*)dev;
     int32_t* d_cols = d_rows + npts;
     int64_t* d_off = (int64_t*)(dev + off_at);
@@ -2211,13 +2206,12 @@ int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B
                                                  (uint32_t*)(dev + back_at), (int*)(dev + back_at + MT_N * 4));
     CU(cudaGetLastError());
     uint8_t* back = pin + MT_N * 4;
-    CU(cudaMemcpyAsync(back, dev + back_at, back_bytes, cudaMemcpyDeviceToHost, s));
-    size_t d2h = back_bytes;
-    if (out_rows && npts) { CU(cudaMemcpyAsync(out_rows, d_rows, npts * 4, cudaMemcpyDeviceToHost, s)); d2h += npts * 4; }
-    if (out_cols && npts) { CU(cudaMemcpyAsync(out_cols, d_cols, npts * 4, cudaMemcpyDeviceToHost, s)); d2h += npts * 4; }
+    if ((rc = copy_d2h(h, back, dev + back_at, back_bytes, s))) return rc;
+    if (out_rows && npts && (rc = copy_d2h(h, out_rows, d_rows, npts * 4, s))) return rc;
+    if (out_cols && npts && (rc = copy_d2h(h, out_cols, d_cols, npts * 4, s))) return rc;
     // 2-6. as dtfill_eval_sampled; the state is written whatever the verdict
-    rc = eval_sampled_run(h, who, gt, gt_is_device, B, H, W, d_rows, d_cols, d_off, MT_N * 4, d2h, r0, r1, c0, c1,
-                          src_thr, val_thr, out_lidar, per_frame, sums, first_bad_frame);
+    rc = eval_sampled_run(h, who, gt, gt_is_device, B, H, W, d_rows, d_cols, d_off, r0, r1, c0, c1, src_thr, val_thr,
+                          out_lidar, per_frame, sums, first_bad_frame);
     if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
     if (out_key) memcpy(out_key, back, MT_N * 4);
     if (out_pos) memcpy(out_pos, back + MT_N * 4, 4);
@@ -2376,6 +2370,7 @@ int dtfill_kernel_times(dtfill_t* h, float* ms) {
 
 int dtfill_dt_pool_ex(dtfill_t* h, const float* data, const float* mask, int in_is_device, int B, int H, int W,
                       int table_size, int scale_num, float* out, uint8_t* out_masks, int out_is_device) {
+    ledger_reset(h);
     if (!h || !data || !mask) return fail(DTFILL_E_ARG, "dtfill_dt_pool: NULL handle, data or mask");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_dt_pool: B, H, W must be positive");
     if (table_size < 1 || (table_size & 1) == 0 || table_size > 2 * K5_MAXR + 1)
@@ -2390,13 +2385,8 @@ int dtfill_dt_pool_ex(dtfill_t* h, const float* data, const float* mask, int in_
     cudaStream_t s = h->stream;
     int rc;
     const float* d_d = data; const float* m_d = mask; float* o_d = out;
-    if (!in_is_device) {
-        if ((rc = ensure(h, h->in_dev, npx * 4))) return rc;
-        if ((rc = ensure(h, h->gt_dev, npx * 4))) return rc;
-        CU(cudaMemcpyAsync(h->in_dev.p, data, npx * 4, cudaMemcpyHostToDevice, s));
-        CU(cudaMemcpyAsync(h->gt_dev.p, mask, npx * 4, cudaMemcpyHostToDevice, s));
-        d_d = (const float*)h->in_dev.p; m_d = (const float*)h->gt_dev.p;
-    }
+    if ((rc = device_input(h, d_d, in_is_device, h->in_dev, npx * 4))) return rc;
+    if ((rc = device_input(h, m_d, in_is_device, h->gt_dev, npx * 4))) return rc;
     uint8_t* k_d = out_masks;
     if (!out_is_device) {
         if ((rc = ensure(h, h->depth_dev, npx * 4 * nl))) return rc;
@@ -2422,8 +2412,8 @@ int dtfill_dt_pool_ex(dtfill_t* h, const float* data, const float* mask, int in_
     }
     CU(cudaGetLastError());
     if (!out_is_device) {
-        CU(cudaMemcpyAsync(out, o_d, npx * 4 * nl, cudaMemcpyDeviceToHost, s));
-        if (out_masks) CU(cudaMemcpyAsync(out_masks, k_d, npx * nl, cudaMemcpyDeviceToHost, s));
+        if ((rc = copy_d2h(h, out, o_d, npx * 4 * nl, s))) return rc;
+        if (out_masks && (rc = copy_d2h(h, out_masks, k_d, npx * nl, s))) return rc;
         CU(cudaStreamSynchronize(s));
     }
     return 0;
@@ -2431,6 +2421,7 @@ int dtfill_dt_pool_ex(dtfill_t* h, const float* data, const float* mask, int in_
 
 int dtfill_dt_pool_demo(dtfill_t* h, const float* data, int in_is_device, int B, int H, int W, int table_size, int scale_num,
                         float* out, int out_is_device) {
+    ledger_reset(h);
     if (!h || !data) return fail(DTFILL_E_ARG, "dtfill_dt_pool_demo: NULL handle or data");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_dt_pool_demo: B, H, W must be positive");
     if (table_size < 1 || (table_size & 1) == 0 || table_size > 2 * K5_MAXR + 1)
@@ -2445,11 +2436,7 @@ int dtfill_dt_pool_demo(dtfill_t* h, const float* data, int in_is_device, int B,
     cudaStream_t s = h->stream;
     int rc;
     const float* d_d = data; float* o_d = out;
-    if (!in_is_device) {
-        if ((rc = ensure(h, h->in_dev, npx * 4))) return rc;
-        CU(cudaMemcpyAsync(h->in_dev.p, data, npx * 4, cudaMemcpyHostToDevice, s));
-        d_d = (const float*)h->in_dev.p;
-    }
+    if ((rc = device_input(h, d_d, in_is_device, h->in_dev, npx * 4))) return rc;
     if (!out_is_device) {
         if ((rc = ensure(h, h->depth_dev, npx * 4 * nl))) return rc;
         o_d = (float*)h->depth_dev.p;
@@ -2464,7 +2451,7 @@ int dtfill_dt_pool_demo(dtfill_t* h, const float* data, int in_is_device, int B,
             w[i * table_size + j] = (float)p;
         }
     if ((rc = ensure(h, h->sums, 1024))) return rc;
-    CU(cudaMemcpyAsync(h->sums.p, w, sizeof(float) * table_size * table_size, cudaMemcpyHostToDevice, s));
+    if ((rc = copy_h2d(h, h->sums.p, w, sizeof(float) * table_size * table_size, s))) return rc;
     CU(cudaStreamSynchronize(s));                     // w lives on this stack frame
     dim3 grid((W + K5_TW - 1) / K5_TW, (H + K5_TH - 1) / K5_TH, B);
     for (int l = 0; l < nl; ++l) {
@@ -2473,7 +2460,7 @@ int dtfill_dt_pool_demo(dtfill_t* h, const float* data, int in_is_device, int B,
     }
     CU(cudaGetLastError());
     if (!out_is_device) {
-        CU(cudaMemcpyAsync(out, o_d, npx * 4 * nl, cudaMemcpyDeviceToHost, s));
+        if ((rc = copy_d2h(h, out, o_d, npx * 4 * nl, s))) return rc;
         CU(cudaStreamSynchronize(s));
     }
     return 0;
@@ -2486,6 +2473,7 @@ int dtfill_dt_pool(dtfill_t* h, const float* data, const float* mask, int in_is_
 
 int dtfill_outlier_removal(dtfill_t* h, const float* in, int in_is_device, int B, int H, int W, float* out,
                            int out_is_device) {
+    ledger_reset(h);
     if (!h || !in || !out) return fail(DTFILL_E_ARG, "dtfill_outlier_removal: NULL argument");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_outlier_removal: B, H, W must be positive");
     CU(cudaSetDevice(h->device));
@@ -2494,11 +2482,7 @@ int dtfill_outlier_removal(dtfill_t* h, const float* in, int in_is_device, int B
     cudaStream_t s = h->stream;
     int rc;
     const float* i_d = in; float* o_d = out;
-    if (!in_is_device) {
-        if ((rc = ensure(h, h->in_dev, npx * 4))) return rc;
-        CU(cudaMemcpyAsync(h->in_dev.p, in, npx * 4, cudaMemcpyHostToDevice, s));
-        i_d = (const float*)h->in_dev.p;
-    }
+    if ((rc = device_input(h, i_d, in_is_device, h->in_dev, npx * 4))) return rc;
     if (!out_is_device) {
         if ((rc = ensure(h, h->depth_dev, npx * 4))) return rc;
         o_d = (float*)h->depth_dev.p;
@@ -2511,7 +2495,7 @@ int dtfill_outlier_removal(dtfill_t* h, const float* in, int in_is_device, int B
     else k6_outlier_removal<false><<<grid, 256, 0, s>>>(i_d, H, W, ngroups, o_d);
     CU(cudaGetLastError());
     if (!out_is_device) {
-        CU(cudaMemcpyAsync(out, o_d, npx * 4, cudaMemcpyDeviceToHost, s));
+        if ((rc = copy_d2h(h, out, o_d, npx * 4, s))) return rc;
         CU(cudaStreamSynchronize(s));
     }
     return 0;
@@ -2519,6 +2503,7 @@ int dtfill_outlier_removal(dtfill_t* h, const float* in, int in_is_device, int B
 
 int dtfill_edt(dtfill_t* h, const float* in, int in_is_device, int B, int H, int W, float src_thr, int32_t* out_d2,
                int32_t* out_idx, int out_is_device) {
+    ledger_reset(h);
     if (!h || !in || !out_d2) return fail(DTFILL_E_ARG, "dtfill_edt: NULL handle, input or out_d2");
     if (B <= 0 || H <= 0 || W <= 0) return fail(DTFILL_E_ARG, "dtfill_edt: B, H, W must be positive");
     if (H > 4096 || W > 25600)
@@ -2529,11 +2514,7 @@ int dtfill_edt(dtfill_t* h, const float* in, int in_is_device, int B, int H, int
     cudaStream_t s = h->stream;
     int rc;
     const float* i_d = in;
-    if (!in_is_device) {
-        if ((rc = ensure(h, h->in_dev, npx * 4))) return rc;
-        CU(cudaMemcpyAsync(h->in_dev.p, in, npx * 4, cudaMemcpyHostToDevice, s));
-        i_d = (const float*)h->in_dev.p;
-    }
+    if ((rc = device_input(h, i_d, in_is_device, h->in_dev, npx * 4))) return rc;
     int32_t* d2 = out_d2; int32_t* ix = out_idx;
     if (!out_is_device) {
         if ((rc = ensure(h, h->depth_dev, npx * 4))) return rc;
@@ -2553,8 +2534,8 @@ int dtfill_edt(dtfill_t* h, const float* in, int in_is_device, int B, int H, int
     else k7_edt_columns<1><<<dim3((W + 127) / 128, B), 128, 0, s>>>((const uint16_t*)h->edt_rows.p, B, H, W, (uint2*)h->edt_stack.p, d2, ix);
     CU(cudaGetLastError());
     if (!out_is_device) {
-        CU(cudaMemcpyAsync(out_d2, d2, npx * 4, cudaMemcpyDeviceToHost, s));
-        if (out_idx) CU(cudaMemcpyAsync(out_idx, ix, npx * 4, cudaMemcpyDeviceToHost, s));
+        if ((rc = copy_d2h(h, out_d2, d2, npx * 4, s))) return rc;
+        if (out_idx && (rc = copy_d2h(h, out_idx, ix, npx * 4, s))) return rc;
         CU(cudaStreamSynchronize(s));
     }
     return 0;

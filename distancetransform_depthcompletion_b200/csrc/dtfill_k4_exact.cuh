@@ -19,9 +19,8 @@ namespace dtfill {
 // reproduce exactly that tree, so the metrics are the reference's bit for bit -- the fixed-order float64 sums of
 // k4_metrics_partial agree with numpy's float32 pairwise sums only to ~1e-5.
 //   k4x_compact  one block per frame: the terms of the valid pixels, compacted in raster order (ballots + warp ranks);
-//                the ground truth is stored as the arithmetic type or, in KITTI mode, as 16-bit PNG samples; the WIN
-//                instance (NYU mode, float32) scores a crop window of the frames, the CROP_FLOOR instance (KITTI mode,
-//                u16 samples) the rows crop_top: of the ground truth against a floored prediction of those rows
+//                the ground truth is stored as the arithmetic type or, in KITTI mode, as 16-bit PNG samples; where
+//                the scored pixels lie in either operand is a K4xGeom
 //   k4x_reduce   one block per frame: the leaves (<= 128 elements) of the tree in parallel, then the tree itself
 // Terms: 0 |d|^2, 1 |d| (KITTI) or |d| / t (NYU), 2 |dinv|^2, 3 |dinv|; counts: valid, delta1..3.
 // ------------------------------------------------------------------------------------------------------
@@ -77,39 +76,46 @@ __device__ __forceinline__ GT gt_value(GS s)
     }
 }
 
-// A crop window of the frames (WIN instances, dtfill_eval_sampled: eval_NYU.py:202-207 scores pred[6:234, 8:312]): pixel i
-// of the window in its raster order is pixel (r0 + i / cw) * W + c0 + i % cw of a frame of frame_px pixels.  The terms of
-// the window's valid pixels are then compacted in the order numpy's boolean index of the cropped view gives them.
-struct K4xWindow {
-    long frame_px;
-    int W, r0, c0, cw;
-    __device__ __forceinline__ long at(long i) const
-    {
-        const int y = (int)i / cw;
-        return (long)(r0 + y) * W + c0 + ((int)i - y * cw);
-    }
+// Where the scored pixels lie.  Frame f of the prediction starts at pred_origin + f * pred_stride, frame f of the ground
+// truth at gt_origin + f * gt_stride; pixel i of a frame, in the raster order of a region `width` pixels wide, is row
+// i / width and column i % width of it, at row * pitch + column from the frame's start.  The descriptions in use:
+//   whole frames (dtfill_metrics, dtfill_eval_png): both strides H * W, origins 0, width == pitch
+//   a crop window (dtfill_eval_sampled: eval_NYU.py:202-207 scores pred[6:234, 8:312]): both strides H * W, both origins
+//     r0 * W + c0, pitch W, width c1 - c0; the terms of the window's valid pixels are then compacted in the order numpy's
+//     boolean index of the cropped view gives them
+//   rows crop_top: of the ground truth against a prediction of only those rows (the KITTI branch of eval_NYU.py,
+//     dtfill_eval_png_kitti): prediction stride (H_in - crop_top) * W, ground-truth stride H_in * W and origin
+//     crop_top * W, width == pitch
+struct K4xGeom {
+    long pred_stride, pred_origin, gt_stride, gt_origin;
+    int pitch, width;
 };
 
-// The KITTI branch of eval_NYU.py (CROP_FLOOR instances, dtfill_eval_png_kitti): the prediction holds only rows
-// win.r0: of the ground truth's frames of win.frame_px = H_in * W samples, so prediction frame b is the npx pixels from
-// b * npx and ground-truth frame b the npx samples from b * win.frame_px + win.r0 * win.W (the rows are a contiguous
-// suffix of the frame).  The prediction is floored in registers, before the validity test and the terms:
-// relu(pred - 0.9) + 0.9 (eval_NYU.py:202-206, float32) equals fmaxf(pred, 0.9f) on every value the fill gives from PNG
-// samples (s / 256, s in 0..65535; pinned by tests/test_eval_kitti_png.py).
-// npx: pixels per frame, or per window (WIN); the term arrays hold npx entries per frame either way
-template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool CROP_FLOOR = false>
-__global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restrict__ pred, const GS* __restrict__ gt, long npx,
+// npx: the scored pixels per frame; the term arrays hold npx entries per frame.  Block b scores frame f0 + b.
+// WIN: width < pitch (a region with width == pitch is contiguous, and pixel i is element i: no division per pixel).
+// FLOOR: the prediction is floored in registers, before the validity test and the terms: relu(pred - 0.9) + 0.9
+// (eval_NYU.py:202-206, float32) equals fmaxf(pred, 0.9f) on every value the fill gives from PNG samples (s / 256,
+// s in 0..65535; pinned by tests/test_eval_kitti_png.py).
+template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool FLOOR = false>
+__global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restrict__ pred, const GS* __restrict__ gt,
+                                                            const K4xGeom geom, long f0, long npx,
                                                             GT* __restrict__ terms /*[frames][4][npx]*/,
-                                                            int* __restrict__ counts /*[frames][4]*/, const K4xWindow win)
+                                                            int* __restrict__ counts /*[frames][4]*/)
 {
-    static_assert(!(WIN && CROP_FLOOR), "a window or the KITTI branch's crop, not both");
     __shared__ int wtot[K4X_THREADS / 32], wbase[K4X_THREADS / 32];
     __shared__ int hits[3];
     const int b = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    auto px = [&](long i) -> long { if constexpr (WIN) return win.at(i); else return i; };
-    const float* p = pred + (long)b * (WIN ? win.frame_px : npx);
-    const GS* g = gt + (CROP_FLOOR ? (long)b * win.frame_px + (long)win.r0 * win.W : (long)b * (WIN ? win.frame_px : npx));
-    auto out = [&](long i) -> float { if constexpr (CROP_FLOOR) return fmaxf(p[i], 0.9f); else return p[px(i)]; };
+    const float* p = pred + geom.pred_origin + (f0 + b) * geom.pred_stride;
+    const GS* g = gt + geom.gt_origin + (f0 + b) * geom.gt_stride;
+    auto px = [&](long i) -> long {
+        if constexpr (WIN) {
+            const int y = (int)i / geom.width;
+            return (long)y * geom.pitch + ((int)i - y * geom.width);
+        } else {
+            return i;
+        }
+    };
+    auto out = [&](long i) -> float { if constexpr (FLOOR) return fmaxf(p[px(i)], 0.9f); else return p[px(i)]; };
     GT* tb = terms + (long)b * 4 * npx;
     const long seg = ((npx + K4X_THREADS - 1) / K4X_THREADS) * 32;     // pixels per warp, a multiple of 32
     const long i0 = min(npx, wid * seg), i1 = min(npx, i0 + seg);

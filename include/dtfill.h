@@ -448,9 +448,13 @@ int dtfill_set_stage_threads(dtfill_t* h, int threads);
  * are a source (tools.py:8) or valid (tools.py:22) -- the only pixels whose value the path ever reads -- and the device
  * rebuilds the dense slice from zeros + pairs in front of the first kernel.  Results are bit-identical; it applies when
  * 0.0f is neither a source nor valid (true for the reference's thresholds 0.1 / 0.001 and 0.1) and falls back to the
- * dense copy for a slice with more than 25 % such pixels.  dtfill_transfer_bytes reports what the last synchronous call
- * with host buffers moved over the link in each direction. */
+ * dense copy for a slice with more than 25 % such pixels. */
 int dtfill_set_sparse_upload(dtfill_t* h, int enabled);
+/* The bytes the last synchronous call moved over the link, host to device and device to host.  Every call that takes an
+ * in_is_device or out_is_device flag, and every dtfill_eval_* call but dtfill_eval_totals, starts both counts at 0 and
+ * adds every copy between host and device it issues (0 when all its buffers are on the device); the status words that
+ * every fill reports are not counted.  The *_async calls, dtfill_eval_totals and dtfill_allreduce_sums leave the counts
+ * as they are. */
 int dtfill_transfer_bytes(dtfill_t* h, unsigned long long* h2d_bytes, unsigned long long* d2h_bytes);
 /* Host-only test hook (needs neither a handle nor a GPU): the compaction of the sparse upload on src[0..n): indices and
  * value bits of the pixels that are a source or valid for the given thresholds, in order; returns their number, or -1 on

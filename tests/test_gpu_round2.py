@@ -284,11 +284,12 @@ def test_allreduce_sums_two_ranks_equal_one_rank(handle, torch_mod):
 
 
 @pytest.mark.gpu
-def test_sparse_upload_matches_dense_upload(handle):
+def test_sparse_upload_matches_dense_upload_and_link_bytes(handle):
     """dtfill_run with a pageable float32 input compacts it on the host to (pixel, value) pairs (include/dtfill.h, sparse
     upload): same outputs as the dense copy and as the oracle, for sparse frames, for frames too dense for the pair
     buffer (fallback inside one call), for NaN / negative / denormal / signed-zero pixels and for the valid-but-not-source
-    band of tools.py:8 vs :22; thresholds that make 0.0 a source switch it off."""
+    band of tools.py:8 vs :22; thresholds that make 0.0 a source switch it off.  The bytes each call moved over the link:
+    the whole array or the pairs up, every output and the counts down."""
     rng = np.random.default_rng(11)
     H, W, B = 96, 256, 20
     x = np.zeros((B, H, W), np.float32)
@@ -311,7 +312,7 @@ def test_sparse_upload_matches_dense_upload(handle):
             assert np.array_equal(r[k], want[k], equal_nan=True), (sparse, k)
     assert outs[False][1][0] == x.nbytes                                # dense: the whole array crossed the link
     assert outs[True][1][0] < x.nbytes                                  # sparse: pairs, plus the slices that fell back
-    assert outs[True][1][1] == outs[False][1][1] == B * H * W * 13
+    assert outs[True][1][1] == outs[False][1][1] == B * H * W * 13 + B * 8     # outputs and counts
     # a source threshold >= 1 makes 0.0 a source: the dense copy must be taken (every pixel valid, so no IndexError)
     xd = (np.round(rng.uniform(1.0, 50.0, (2, H, W)) * 256) / 256).astype(np.float32)
     r = handle.run_host(xd, 1.0, 0.1, want_dt=True)
