@@ -106,6 +106,8 @@ def load() -> ctypes.CDLL:
             L.dtfill_eval_sampled_mt.argtypes = [vp, vp, ci, ci, ci, ci, ci, vp, ci, ci, ci, ci, ci, cf, cf, vp, vp, vp,
                                                  vp, vp, vp, vp, vp, ctypes.POINTER(ci)]
             L.dtfill_debug_mt_draw_host.argtypes = [vp, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp]
+            L.dtfill_eval_sampled_mt_many.argtypes = [vp, vp, ci, ci, ci, ci, ci, vp, vp, vp, ci, ci, ci, ci, cf, cf, vp,
+                                                      vp, vp, vp, vp, ctypes.POINTER(ci), ctypes.POINTER(ci)]
         except AttributeError as e:      # an older build of the same ABI version
             raise DTFillError(f"{LIB_PATH} lacks {str(e).split()[-1].strip(chr(39))}: rebuild it with "
                               "`python -m distancetransform_depthcompletion_b200.build`") from None
@@ -123,7 +125,7 @@ def load() -> ctypes.CDLL:
                      "dtfill_transfer_bytes", "dtfill_set_metrics_exact", "dtfill_dt_pool_demo", "dtfill_png_decode",
                      "dtfill_run_png", "dtfill_debug_png_decode_host", "dtfill_png_encode", "dtfill_png_encode_depth",
                      "dtfill_run_png_to_png", "dtfill_eval_png", "dtfill_eval_sampled", "dtfill_eval_png_kitti",
-                     "dtfill_eval_sampled_mt", "dtfill_debug_mt_draw_host"):
+                     "dtfill_eval_sampled_mt", "dtfill_debug_mt_draw_host", "dtfill_eval_sampled_mt_many"):
             getattr(L, name).restype = ci
         _lib = L
         return L
@@ -431,6 +433,39 @@ class Handle:
             res["index_error"] = last_error()
             return res
         _check(rc, "dtfill_eval_sampled_mt")
+        return res
+
+    def eval_sampled_mt_many(self, gt, B: int, H: int, W: int, n, keys: np.ndarray, pos, crop, src_thr: float,
+                             val_thr: float, gt_is_device: bool = False):
+        """eval_sampled_mt for D generators at once over the same ground truth: n int [D], keys uint32 [D,624], pos int [D]
+        -> dict(per_frame [D,B,9], sums [D,10], keys [D,624], pos int [D], words int64 [D,B], first_bad_draw,
+        first_bad_frame).  A frame Distance_Transform rejects is reported under "index_error" (the state outputs are still
+        written for every draw); other failures raise."""
+        r0, r1, c0, c1 = (int(v) for v in crop)
+        if not gt_is_device:
+            assert gt.dtype == np.float32 and gt.shape == (B, H, W) and gt.flags.c_contiguous
+        keys = np.ascontiguousarray(keys, np.uint32)
+        D = keys.shape[0]
+        assert keys.shape == (D, 624) and D > 0
+        n = np.ascontiguousarray(n, np.int32)
+        pos = np.ascontiguousarray(pos, np.int32)
+        assert n.shape == (D,) and pos.shape == (D,)
+        per_frame = np.empty((D, B, METRIC_COLS), np.float64)
+        sums = np.empty((D, METRIC_COLS + 1), np.float64)
+        out_keys = np.empty((D, 624), np.uint32)
+        out_pos = np.empty(D, np.int32)
+        words = np.empty((D, B), np.int64)
+        bad_d, bad_f = ctypes.c_int(-1), ctypes.c_int(-1)
+        rc = self._L.dtfill_eval_sampled_mt_many(self._h, _ptr(gt), int(bool(gt_is_device)), int(B), int(H), int(W), D,
+                                                 _ptr(n), _ptr(keys), _ptr(pos), r0, r1, c0, c1, float(src_thr),
+                                                 float(val_thr), _ptr(out_keys), _ptr(out_pos), _ptr(words),
+                                                 _ptr(per_frame), _ptr(sums), ctypes.byref(bad_d), ctypes.byref(bad_f))
+        res = dict(per_frame=per_frame, sums=sums, keys=out_keys, pos=out_pos, words=words, first_bad_draw=bad_d.value,
+                   first_bad_frame=bad_f.value)
+        if rc == E_INDEX:
+            res["index_error"] = last_error()
+            return res
+        _check(rc, "dtfill_eval_sampled_mt_many")
         return res
 
     def png_encode_device_async(self, in_ptr: int, is_float: bool, B: int, H: int, W: int, out_ptr: int,

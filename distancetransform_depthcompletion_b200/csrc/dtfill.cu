@@ -586,6 +586,7 @@ struct FillCall {
     int32_t* lbl = nullptr;
     uint8_t* mask = nullptr;
     int32_t* counts = nullptr;
+    int gt_frames = 0;                // SAMPLED: frame f reads ground-truth frame f mod gt_frames (0: B, one frame each)
     // optional evaluation fused behind the fill (dtfill_run_eval_async): ground truth [B,H,W], float64 or float32, mode
     const void* eval_gt = nullptr;
     int eval_gt_f64 = 0, eval_mode = 0;
@@ -603,11 +604,12 @@ struct EnqueueState {
 
 // K1 on input of type T, one warp per row: the 128-bit-load kernel where rows start 16-byte aligned (W % 4 for 4-byte
 // pixels, W % 8 for uint16 samples), in its whole-group form when W % 16 == 0; the scalar kernel otherwise.  Frame
-// fp.frame0 starts fp.in_H rows into the input (in_H = H but for uint16 samples with a crop).
+// fp.frame0 starts fp.in_H rows into the input (in_H = H but for uint16 samples with a crop); the sampled kind finds its
+// ground-truth frames itself (frame f reads frame f mod fp.gt_frames) and takes the input as it is.
 template <typename T>
 void launch_k1(const void* in, int grid, int threads, cudaStream_t s, const FrameParams& fp, const Workspace& ws, uint8_t* om,
                float* olid) {
-    const T* in_s = (const T*)in + (size_t)fp.frame0 * fp.in_H * fp.W;
+    const T* in_s = std::is_same<T, SampledGt>::value ? (const T*)in : (const T*)in + (size_t)fp.frame0 * fp.in_H * fp.W;
     if ((fp.W & 15) == 0) k1_mask_rows_v16<T, true><<<grid, threads, 0, s>>>(in_s, fp, ws, om, olid);
     else if (fp.W % (int)(16 / sizeof(T)) == 0) k1_mask_rows_v16<T, false><<<grid, threads, 0, s>>>(in_s, fp, ws, om, olid);
     else k1_mask_rows<T><<<grid, threads, 0, s>>>(in_s, fp, ws, om, olid);
@@ -643,6 +645,7 @@ int enqueue_range(dtfill_t* h, Lane* L, cudaStream_t s, const FillCall& c, const
     fp.mul_dist = 1u << (32 - DSH);
     fp.four = 4u;
     fp.one = 1u;
+    if (c.kind == FillCall::SAMPLED) fp.gt_frames = c.gt_frames > 0 ? c.gt_frames : c.B;
 #ifdef DTFILL_TRACE
     fp.trace = h->trace_dev ? h->trace_dev + (size_t)(h->ncalls % dtfill_ctx::TRACE_CALLS) * 16 : nullptr;
 #endif
@@ -1023,8 +1026,9 @@ int enqueue(dtfill_t* h, const FillCall& c, const HostIO* hio = nullptr, bool fo
 // with a float64 ground truth needs 3.5 GB: one group, every frame's tree in flight at once).  GT: the arithmetic type,
 // GS: the ground truth as stored; npx pixels per frame lie in pred and gt as geom says (k4x_compact).  Device pointers;
 // enqueued on the handle's stream.
-template <typename GT, int MODE, typename GS, bool WIN, bool FLOOR>
-int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, const K4xGeom& geom, int B, long npx, double* per_frame) {
+template <typename GT, int MODE, typename GS, bool WIN, bool FLOOR, bool WRAP>
+int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, const K4xGeomOf<WRAP>& geom, int B, long npx,
+                double* per_frame) {
     const size_t gsz = sizeof(GT);
     const long maxl = npx / 64 + 2;
     long G = (long)((1ull << 32) / ((size_t)4 * npx * gsz));
@@ -1038,7 +1042,7 @@ int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, const K4xGeom& geo
         const int ng = (int)(B - g0 < G ? B - g0 : G);
         GT* tm = (GT*)h->mx_terms.p;
         int* cn = (int*)h->mx_counts.p;
-        k4x_compact<GT, MODE, GS, WIN, FLOOR><<<ng, K4X_THREADS, 0, h->stream>>>(pred, gt, geom, g0, npx, tm, cn);
+        k4x_compact<GT, MODE, GS, WIN, FLOOR, WRAP><<<ng, K4X_THREADS, 0, h->stream>>>(pred, gt, geom, g0, npx, tm, cn);
         k4x_reduce<GT><<<ng, K4X_RTHREADS, 0, h->stream>>>(tm, cn, npx, MODE, (int*)h->mx_leaf_start.p,
                                                            (GT*)h->mx_leaf_sum.p, per_frame + g0 * 9);
     }
@@ -1049,20 +1053,23 @@ int k4x_enqueue(dtfill_t* h, const float* pred, const GS* gt, const K4xGeom& geo
 // metrics [B,9] and their column sums [10] (added to when accumulate).  out_is_device: per_frame / sums are device
 // vectors the kernels write, the handle's buffers standing in for a null one; otherwise the results are copied from the
 // handle's buffers to whichever of the host pointers per_frame / sums is non-null (the caller synchronises).
-template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool FLOOR = false>
-int k4x_score(dtfill_t* h, const float* pred, const GS* gt, const K4xGeom& geom, int B, long npx, double* per_frame,
-              double* sums, int out_is_device = 0, int accumulate = 0) {
+// WRAP: the B frames are B / geom.gt_frames draws over gt_frames ground-truth frames, and sums holds one row [10] per draw.
+template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool FLOOR = false, bool WRAP = false>
+int k4x_score(dtfill_t* h, const float* pred, const GS* gt, const K4xGeomOf<WRAP>& geom, int B, long npx,
+              double* per_frame, double* sums, int out_is_device = 0, int accumulate = 0) {
+    int nsums = 1;
+    if constexpr (WRAP) nsums = (int)(B / geom.gt_frames);
     int rc;
     if ((rc = ensure(h, h->per_frame, (size_t)B * 9 * 8))) return rc;
-    if ((rc = ensure(h, h->sums, 10 * 8))) return rc;
+    if ((rc = ensure(h, h->sums, (size_t)nsums * 10 * 8))) return rc;
     double* pf_d = (out_is_device && per_frame) ? per_frame : (double*)h->per_frame.p;
     double* sm_d = (out_is_device && sums) ? sums : (double*)h->sums.p;
-    if ((rc = k4x_enqueue<GT, MODE, GS, WIN, FLOOR>(h, pred, gt, geom, B, npx, pf_d))) return rc;
-    k4x_sums<<<1, 32, 0, h->stream>>>(pf_d, B, sm_d, accumulate);
+    if ((rc = k4x_enqueue<GT, MODE, GS, WIN, FLOOR, WRAP>(h, pred, gt, geom, B, npx, pf_d))) return rc;
+    k4x_sums<<<nsums, 32, 0, h->stream>>>(pf_d, B / nsums, sm_d, accumulate);
     CU(cudaGetLastError());
     if (out_is_device) return 0;
     if (per_frame && (rc = copy_d2h(h, per_frame, pf_d, (size_t)B * 9 * 8, h->stream))) return rc;
-    if (sums && (rc = copy_d2h(h, sums, sm_d, 10 * 8, h->stream))) return rc;
+    if (sums && (rc = copy_d2h(h, sums, sm_d, (size_t)nsums * 10 * 8, h->stream))) return rc;
     return 0;
 }
 
@@ -1848,21 +1855,21 @@ __global__ void k4_fold_totals(LaneTotals lanes, double* __restrict__ sums, int 
 }
 
 // Distance_Transform's verdict on the frames of a synchronous fill, frame by frame as the evaluation loop meets them: rc and
-// fill_bad are what dtfill_status reported, cnt the fill's counts [B][2].  `what` names a frame in the message.
-int fill_verdict(int rc, int fill_bad, const int32_t* cnt, int B, const char* what, int* first_bad_frame) {
+// fill_bad are what dtfill_status reported, cnt the fill's counts [B][2].  name(b) names frame b in the message.
+int fill_verdict(int rc, int fill_bad, const int32_t* cnt, int B, const std::function<std::string(int)>& name,
+                 int* first_bad_frame) {
     const int lim = rc == DTFILL_E_INDEX ? fill_bad : B;
     for (int b = 0; b < lim; ++b)
         if (cnt[2 * b + 1] == 1) {
             // eval_NYU.py:126 np.squeeze(lidar[with_value]) makes a single valid depth 0-dimensional; :128 then fails
             if (first_bad_frame) *first_bad_frame = b;
-            return fail(DTFILL_E_INDEX, what + std::to_string(b) +
+            return fail(DTFILL_E_INDEX, name(b) +
                                             ": one valid depth (numpy IndexError: too many indices for array: array is "
                                             "0-dimensional, but 1 were indexed)");
         }
     if (rc == DTFILL_E_INDEX) {
         if (first_bad_frame) *first_bad_frame = fill_bad;
-        return fail(DTFILL_E_INDEX, what + std::to_string(fill_bad) +
-                                        ": labels index outside the list of valid depths (numpy IndexError)");
+        return fail(DTFILL_E_INDEX, name(fill_bad) + ": labels index outside the list of valid depths (numpy IndexError)");
     }
     return 0;
 }
@@ -1998,7 +2005,8 @@ int eval_png_run(dtfill_t* h, const uint8_t* lidar, const int64_t* lidar_offsets
                                            png_reason(st) + " (status " + std::to_string(st) + ")");
         }
     }
-    return fill_verdict(rc, fill_bad, st_host + nfiles, B, "LiDAR file ", first_bad_frame);
+    return fill_verdict(rc, fill_bad, st_host + nfiles, B, [](int b) { return "LiDAR file " + std::to_string(b); },
+                        first_bad_frame);
 }
 
 }  // namespace
@@ -2055,12 +2063,16 @@ int sampled_frame_check(const char* who, const float* gt, int gt_is_device, int 
 // Steps 2-6 of dtfill_eval_sampled and dtfill_eval_sampled_mt, after the device coordinates d_rows / d_cols / d_off are
 // enqueued on the handle's stream: the ground truth, the sample bitmap, the fill, the metrics of the window, the copies
 // back and the verdict (copies back the caller enqueued already complete with this call's synchronisation).
+// draw0 >= 0 (dtfill_eval_sampled_mt_many): the call runs `draws` draws of B frames each over the B ground-truth frames,
+// draws * B filled frames in all, frame f of which is frame f % B of draw draw0 + f / B (named so in the messages);
+// per_frame holds draws * B rows, sums one row per draw.  Otherwise draws == 1.
 int eval_sampled_run(dtfill_t* h, const char* who, const float* gt, int gt_is_device, int B, int H, int W,
                      const int32_t* d_rows, const int32_t* d_cols, const int64_t* d_off, int r0, int r1, int c0, int c1,
                      float src_thr, float val_thr, float* out_lidar, double* per_frame, double* sums,
-                     int* first_bad_frame) {
+                     int* first_bad_frame, int draws = 1, int draw0 = -1) {
     const long npx = (long)H * W;
     const int WW = (W + 31) / 32;
+    const int F = draws * B;                                  // frames filled
     cudaStream_t s = h->stream;
     int rc;
     // 2. the ground truth, unless it is resident
@@ -2069,43 +2081,50 @@ int eval_sampled_run(dtfill_t* h, const char* who, const float* gt, int gt_is_de
     // 3. the sample bitmap in lane 0's srcbits (the lane of a strict-order fill), sized as the fill sizes it so that the
     //    fill does not reallocate it
     Lane* L = &h->lanes[0];
-    if ((rc = ensure(h, L->srcbits, (size_t)B * H * WW * 4))) return rc;
+    if ((rc = ensure(h, L->srcbits, (size_t)F * H * WW * 4))) return rc;
     if ((rc = ensure(h, h->smp_bad, 4))) return rc;
-    CU(cudaMemsetAsync(L->srcbits.p, 0, (size_t)B * H * WW * 4, s));
+    CU(cudaMemsetAsync(L->srcbits.p, 0, (size_t)F * H * WW * 4, s));
     CU(cudaMemsetAsync(h->smp_bad.p, 0x7F, 4, s));           // 0x7F7F7F7F: above every frame index
-    k10_sample_bits<<<B, K10_THREADS, 0, s>>>(d_rows, d_cols, d_off, H, W, WW, (uint32_t*)L->srcbits.p, (int*)h->smp_bad.p);
+    k10_sample_bits<<<F, K10_THREADS, 0, s>>>(d_rows, d_cols, d_off, H, W, WW, (uint32_t*)L->srcbits.p, (int*)h->smp_bad.p);
     CU(cudaGetLastError());
     // 4. the fill with K1's sampled input kind, strict order on the handle's stream; the filled depth stays on the device
-    if ((rc = ensure(h, h->depth_dev, (size_t)B * npx * 4))) return rc;
-    if ((rc = ensure(h, h->counts_out_dev, (size_t)B * 8))) return rc;
-    if (out_lidar && (rc = ensure(h, h->lidar_out_dev, (size_t)B * npx * 4))) return rc;
+    if ((rc = ensure(h, h->depth_dev, (size_t)F * npx * 4))) return rc;
+    if ((rc = ensure(h, h->counts_out_dev, (size_t)F * 8))) return rc;
+    if (out_lidar && (rc = ensure(h, h->lidar_out_dev, (size_t)F * npx * 4))) return rc;
     FillCall fill;
     fill.kind = FillCall::SAMPLED; fill.in = g_d; fill.lidar = out_lidar ? (float*)h->lidar_out_dev.p : nullptr;
-    fill.B = B; fill.H = H; fill.W = W; fill.src_thr = src_thr; fill.val_thr = val_thr;
+    fill.B = F; fill.H = H; fill.W = W; fill.src_thr = src_thr; fill.val_thr = val_thr; fill.gt_frames = B;
     fill.depth = (float*)h->depth_dev.p; fill.counts = (int32_t*)h->counts_out_dev.p;
     if ((rc = enqueue(h, fill, nullptr, true))) return rc;
     // 5. Result_NYU.evaluate of the window of the filled depth against the same window of the ground truth, in numpy's
     //    summation order whatever dtfill_set_metrics_exact says
     const long at = (long)r0 * W + c0;
     const K4xGeom win{npx, at, npx, at, W, c1 - c0};
-    if ((rc = k4x_score<float, 1, float, true>(h, fill.depth, g_d, win, B, (long)(r1 - r0) * (c1 - c0), per_frame, sums)))
-        return rc;
-    if ((rc = ensure_pinned(h->pin_png_status, (size_t)B * 8 + 4))) return rc;
-    int32_t* out_h = (int32_t*)h->pin_png_status.p;          // the fill's counts [B][2], then the flag word
-    if ((rc = copy_d2h(h, out_h, fill.counts, (size_t)B * 8, s))) return rc;
-    if ((rc = copy_d2h(h, out_h + 2 * B, h->smp_bad.p, 4, s))) return rc;
-    if (out_lidar && (rc = copy_d2h(h, out_lidar, fill.lidar, (size_t)B * npx * 4, s))) return rc;
+    const long wpx = (long)(r1 - r0) * (c1 - c0);
+    rc = draw0 < 0 ? k4x_score<float, 1, float, true>(h, fill.depth, g_d, win, F, wpx, per_frame, sums)
+                   : k4x_score<float, 1, float, true, false, true>(h, fill.depth, g_d, K4xWrapGeom{win, B}, F, wpx,
+                                                                   per_frame, sums);
+    if (rc) return rc;
+    if ((rc = ensure_pinned(h->pin_png_status, (size_t)F * 8 + 4))) return rc;
+    int32_t* out_h = (int32_t*)h->pin_png_status.p;          // the fill's counts [F][2], then the flag word
+    if ((rc = copy_d2h(h, out_h, fill.counts, (size_t)F * 8, s))) return rc;
+    if ((rc = copy_d2h(h, out_h + 2 * F, h->smp_bad.p, 4, s))) return rc;
+    if (out_lidar && (rc = copy_d2h(h, out_lidar, fill.lidar, (size_t)F * npx * 4, s))) return rc;
     int fill_bad = -1;
     rc = dtfill_status(h, &fill_bad, nullptr);       // synchronises
     if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
     // 6. the verdict: device coordinates outside the frame, then Distance_Transform's frame by frame
-    const int bad = out_h[2 * B];
-    if (bad < B) {
+    auto name = [&](int f) {
+        return draw0 < 0 ? "frame " + std::to_string(f)
+                         : "draw " + std::to_string(draw0 + f / B) + ", frame " + std::to_string(f % B);
+    };
+    const int bad = out_h[2 * F];
+    if (bad < F) {
         if (first_bad_frame) *first_bad_frame = bad;
-        return fail(DTFILL_E_ARG, std::string(who) + ": frame " + std::to_string(bad) +
+        return fail(DTFILL_E_ARG, std::string(who) + ": " + name(bad) +
                                       ": a sample outside the frame, or a negative sample count");
     }
-    return fill_verdict(rc, fill_bad, out_h, B, "frame ", first_bad_frame);
+    return fill_verdict(rc, fill_bad, out_h, F, name, first_bad_frame);
 }
 
 }  // namespace
@@ -2216,6 +2235,93 @@ int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B
     if (out_key) memcpy(out_key, back, MT_N * 4);
     if (out_pos) memcpy(out_pos, back + MT_N * 4, 4);
     if (out_words) memcpy(out_words, back + (words_at - back_at), (size_t)B * 8);
+    return rc;
+}
+
+// dtfill_eval_sampled_mt_many fills whole draws at a time, at most this many pixels per fill (and always one draw at
+// least): the workspace of a fill grows with its pixels, and 2^28 pixels keep it near the size that a call of 1024 KITTI
+// frames uses already.  654 NYU frames of 240 x 320: 5 draws per fill.
+constexpr long EVAL_MANY_FILL_PX = 1l << 28;
+
+int dtfill_eval_sampled_mt_many(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, int D, const int* n,
+                                const uint32_t* mt_keys, const int* mt_pos, int r0, int r1, int c0, int c1, float src_thr,
+                                float val_thr, uint32_t* out_keys, int* out_pos, int64_t* out_words, double* per_frame,
+                                double* sums, int* first_bad_draw, int* first_bad_frame) {
+    const char* who = "dtfill_eval_sampled_mt_many";
+    if (first_bad_draw) *first_bad_draw = -1;
+    if (first_bad_frame) *first_bad_frame = -1;
+    ledger_reset(h);
+    if (!h || !gt || !n || !mt_keys || !mt_pos || !per_frame || !sums)
+        return fail(DTFILL_E_ARG, std::string(who) + ": NULL handle, ground truth, counts, keys, positions or results");
+    if (D <= 0) return fail(DTFILL_E_ARG, std::string(who) + ": D must be positive");
+    if (H < 13 || W < 17) return fail(DTFILL_E_ARG, std::string(who) + ": frames need H >= 13 and W >= 17 (randint(H - 12), randint(W - 16))");
+    for (int d = 0; d < D; ++d) {
+        if (n[d] < 0) return fail(DTFILL_E_ARG, std::string(who) + ": draw " + std::to_string(d) + ": negative sample count");
+        if (mt_pos[d] < 0 || mt_pos[d] > MT_N)
+            return fail(DTFILL_E_ARG, std::string(who) + ": draw " + std::to_string(d) + ": pos outside [0, 624]");
+    }
+    int rc = sampled_frame_check(who, gt, gt_is_device, B, H, W, r0, r1, c0, c1);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    rc = dtfill_flush(h);            // fills in flight (pipelined mode) may still use lane 0's workspace
+    if (rc) return rc;
+    cudaStream_t s = h->stream;
+    const long npx = (long)H * W;
+    // 1. every draw at once: the keys and {pos, n} per draw go up in one copy through the pinned staging buffer;
+    //    k11_mt_draw_many (one block per generator) writes the coordinates of the D * B frames, their offsets, the words
+    //    per frame and the final states into one device buffer, whose state part comes back in one copy:
+    //    words [D][B] int64, keys [D][624], pos [D]
+    size_t npts = 0;
+    for (int d = 0; d < D; ++d) npts += (size_t)B * n[d];
+    const size_t off_at = (2 * npts * 4 + 15) & ~(size_t)15;
+    const size_t in_at = (off_at + ((size_t)D * B + 1) * 8 + 15) & ~(size_t)15;
+    const size_t in_bytes = (size_t)D * MT_N * 4 + (size_t)D * 8;
+    const size_t back_at = (in_at + in_bytes + 15) & ~(size_t)15;
+    const size_t back_bytes = (size_t)D * B * 8 + (size_t)D * MT_N * 4 + (size_t)D * 4;
+    const size_t pin_back = (in_bytes + 15) & ~(size_t)15;
+    if ((rc = ensure_pinned(h->pin_smp, pin_back + back_bytes))) return rc;
+    if ((rc = ensure(h, h->smp_coords, back_at + back_bytes))) return rc;
+    uint8_t* pin = (uint8_t*)h->pin_smp.p;
+    uint8_t* dev = (uint8_t*)h->smp_coords.p;
+    memcpy(pin, mt_keys, (size_t)D * MT_N * 4);
+    int32_t* pin_draws = (int32_t*)(pin + (size_t)D * MT_N * 4);
+    for (int d = 0; d < D; ++d) { pin_draws[2 * d] = mt_pos[d]; pin_draws[2 * d + 1] = n[d]; }
+    if ((rc = copy_h2d(h, dev + in_at, pin, in_bytes, s))) return rc;
+    int32_t* d_rows = (int32_t*)dev;
+    int32_t* d_cols = d_rows + npts;
+    int64_t* d_off = (int64_t*)(dev + off_at);
+    int64_t* d_words = (int64_t*)(dev + back_at);
+    uint32_t* d_keys_out = (uint32_t*)(d_words + (size_t)D * B);
+    CU(cudaFuncSetAttribute(k11_mt_draw_many, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K11_SMEM));
+    k11_mt_draw_many<<<D, K11_THREADS, K11_SMEM, s>>>((const uint32_t*)(dev + in_at),
+                                                      (const int32_t*)(dev + in_at + (size_t)D * MT_N * 4), D, B,
+                                                      (uint32_t)(H - 13), (uint32_t)(W - 17), d_rows, d_cols, d_off, d_words,
+                                                      d_keys_out, (int*)(d_keys_out + (size_t)D * MT_N));
+    CU(cudaGetLastError());
+    uint8_t* back = pin + pin_back;
+    if ((rc = copy_d2h(h, back, d_words, back_bytes, s))) return rc;
+    // 2-6. whole draws per fill; the ground truth goes up once (unless it is resident), and a fill that meets a frame
+    //    Distance_Transform rejects ends the call
+    const float* g_d = gt;
+    if ((rc = device_input(h, g_d, gt_is_device, h->gt_dev, (size_t)B * npx * 4))) return rc;
+    long per_fill = EVAL_MANY_FILL_PX / ((long)B * npx);
+    if (per_fill < 1) per_fill = 1;
+    for (int d0 = 0; d0 < D; d0 += (int)per_fill) {
+        const int nd = (int)(D - d0 < per_fill ? D - d0 : per_fill);
+        int bad = -1;
+        rc = eval_sampled_run(h, who, g_d, 1, B, H, W, d_rows, d_cols, d_off + (size_t)d0 * B, r0, r1, c0, c1, src_thr,
+                              val_thr, nullptr, per_frame + (size_t)d0 * B * 9, sums + (size_t)d0 * 10, &bad, nd, d0);
+        if (rc && bad >= 0) {
+            if (first_bad_draw) *first_bad_draw = d0 + bad / B;
+            if (first_bad_frame) *first_bad_frame = bad % B;
+        }
+        if (rc) break;
+    }
+    if (rc != 0 && rc != DTFILL_E_INDEX) return rc;
+    // the states, whatever the verdict (the first fill's synchronisation completed their copy)
+    if (out_words) memcpy(out_words, back, (size_t)D * B * 8);
+    if (out_keys) memcpy(out_keys, back + (size_t)D * B * 8, (size_t)D * MT_N * 4);
+    if (out_pos) memcpy(out_pos, back + (size_t)D * B * 8 + (size_t)D * MT_N * 4, (size_t)D * 4);
     return rc;
 }
 

@@ -46,7 +46,12 @@ constexpr int MAX_CELLS = 15360;   // planner grid limit (30 KB of shared memory
 
 struct FrameParams {
     int B, H, W, WW;           // WW = 32-bit words per bit row
-    int in_H, in_crop;         // input frames hold in_H rows; rows [in_crop, in_crop + H) are the frame (uint16 input)
+    int in_H;                  // input frames hold in_H rows
+    union {
+        int in_crop;           // uint16 input: rows [in_crop, in_crop + H) of an input frame are the frame
+        int gt_frames;         // sampled input: frame f of the call reads ground-truth frame f mod gt_frames (several
+                               // draws over one ground truth, dtfill_eval_sampled_mt_many; B otherwise)
+    };
     float src_thr, val_thr;
     float src_cut;             // smallest float x (in the total order) with !(float32(1 - x) > src_thr)
     int init_dist;             // "unreached" distance of the fast path: H + W + 8

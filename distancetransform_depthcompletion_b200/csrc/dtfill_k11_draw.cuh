@@ -80,11 +80,12 @@ __device__ __forceinline__ void k11_bar(int id, int count) {
     asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(count) : "memory");
 }
 
-__global__ void __launch_bounds__(K11_THREADS) k11_mt_draw(const uint32_t* __restrict__ key_in, int pos, int B, int n,
-                                                          uint32_t rng_r, uint32_t rng_c, int32_t* __restrict__ rows,
-                                                          int32_t* __restrict__ cols, int64_t* __restrict__ offsets,
-                                                          int64_t* __restrict__ words, uint32_t* __restrict__ key_out,
-                                                          int* __restrict__ pos_out)
+// The draws of one generator by one block: the body of k11_mt_draw and of each block of k11_mt_draw_many.  rows / cols
+// point at the generator's first slot; offsets[b] = off_base + b * n for b < B, and for b == B too when write_end.
+__device__ __forceinline__ void k11_draw(const uint32_t* __restrict__ key_in, int pos, int B, int n, uint32_t rng_r,
+                                         uint32_t rng_c, int32_t* __restrict__ rows, int32_t* __restrict__ cols,
+                                         int64_t* __restrict__ offsets, long long off_base, bool write_end,
+                                         int64_t* __restrict__ words, uint32_t* __restrict__ key_out, int* __restrict__ pos_out)
 {
     extern __shared__ __align__(16) uint8_t k11_smem[];
     uint32_t* raw = (uint32_t*)k11_smem;                      // [2][K11_S]
@@ -98,7 +99,7 @@ __global__ void __launch_bounds__(K11_THREADS) k11_mt_draw(const uint32_t* __res
     const int tid = threadIdx.x;
     const int nr = rng_r ? n : 0, nc = rng_c ? n : 0;        // words-consuming accepts per row / column phase
     const long long total = (long long)B * n;
-    for (int b = tid; b <= B; b += K11_THREADS) offsets[b] = (long long)b * n;
+    for (int b = tid; b < B + (int)write_end; b += K11_THREADS) offsets[b] = off_base + (long long)b * n;
     if (!rng_r) for (long long i = tid; i < total; i += K11_THREADS) rows[i] = 6;
     if (!rng_c) for (long long i = tid; i < total; i += K11_THREADS) cols[i] = 8;
     if (nr + nc == 0) {                                       // no word is consumed: the state comes back unchanged
@@ -263,6 +264,33 @@ __global__ void __launch_bounds__(K11_THREADS) k11_mt_draw(const uint32_t* __res
         __syncthreads();
         if (done_s) break;
     }
+}
+
+__global__ void __launch_bounds__(K11_THREADS) k11_mt_draw(const uint32_t* __restrict__ key_in, int pos, int B, int n,
+                                                          uint32_t rng_r, uint32_t rng_c, int32_t* __restrict__ rows,
+                                                          int32_t* __restrict__ cols, int64_t* __restrict__ offsets,
+                                                          int64_t* __restrict__ words, uint32_t* __restrict__ key_out,
+                                                          int* __restrict__ pos_out)
+{
+    k11_draw(key_in, pos, B, n, rng_r, rng_c, rows, cols, offsets, 0, true, words, key_out, pos_out);
+}
+
+// D independent generators, one block each (dtfill_eval_sampled_mt_many): block d draws B frames of n_d samples from
+// keys[d] / draws[d] = {pos_d, n_d}.  Its coordinates start at slot B * (n_0 + ... + n_{d-1}), its offsets are those of
+// frames d*B .. d*B + B - 1 of the whole run (so k10_sample_bits reads the D*B frames as one batch; the last block writes
+// offsets[D*B]), and its words, final key and pos go to row d of words [D][B], keys_out [D][624] and pos_out [D].
+__global__ void __launch_bounds__(K11_THREADS) k11_mt_draw_many(const uint32_t* __restrict__ keys,
+                                                               const int32_t* __restrict__ draws, int D, int B,
+                                                               uint32_t rng_r, uint32_t rng_c, int32_t* __restrict__ rows,
+                                                               int32_t* __restrict__ cols, int64_t* __restrict__ offsets,
+                                                               int64_t* __restrict__ words, uint32_t* __restrict__ keys_out,
+                                                               int* __restrict__ pos_out)
+{
+    const int d = blockIdx.x;
+    long long base = 0;
+    for (int e = 0; e < d; ++e) base += (long long)B * draws[2 * e + 1];
+    k11_draw(keys + (size_t)d * MT_N, draws[2 * d], B, draws[2 * d + 1], rng_r, rng_c, rows + base, cols + base,
+             offsets + (size_t)d * B, base, d == D - 1, words + (size_t)d * B, keys_out + (size_t)d * MT_N, pos_out + d);
 }
 
 }  // namespace dtfill

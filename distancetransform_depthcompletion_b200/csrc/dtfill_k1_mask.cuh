@@ -32,7 +32,9 @@ __device__ __forceinline__ uint32_t sign_nibble_bytes(float t0, float t1, float 
     return (w * 0x00204081u) >> 28;
 }
 
-// Sampled input (T = SampledGt, dtfill_eval_sampled): the sample bitmap of k10_sample_bits lies in ws.srcbits, in the layout
+// Sampled input (T = SampledGt, dtfill_eval_sampled): `in` is the whole ground truth, not offset to the sub-batch, and frame
+// frame0 + f of the call reads ground-truth frame (frame0 + f) mod fp.gt_frames, so that the frames of several draws share
+// one ground truth.  The sample bitmap of k10_sample_bits lies in ws.srcbits, in the layout
 // K1 writes its source bits in.  A word is read by the two lanes (or, in the scalar kernel, the warp) that later overwrite
 // it, and every read value is consumed before the warp's shuffles / ballots that precede the write.  A pixel keeps its
 // ground-truth value when its bit is set and becomes g * 0 otherwise, as `gt * Mask` does (data_read.py:364): -0 for a
@@ -61,7 +63,11 @@ __global__ void __launch_bounds__(256) k1_mask_rows_v16(const T* __restrict__ in
     float* rowvals = reinterpret_cast<float*>(ws.scratch);
     for (long row = warp; row < nrows; row += nwarps) {
         const T* rp = in + row * W;
-        if (fp.in_H != fp.H) {                       // cropped input frames (uint16 entry): row -> (frame, y)
+        if constexpr (std::is_same<T, SampledGt>::value) {   // row -> (frame, y), y of ground-truth frame f mod gt_frames
+            const long frame = rows32 ? (long)((uint32_t)row / (uint32_t)fp.H) : row / fp.H;
+            const long g = (long)((uint32_t)(fp.frame0 + frame) % (uint32_t)fp.gt_frames);
+            rp = in + (g * fp.H + (row - frame * fp.H)) * W;
+        } else if (fp.in_H != fp.H) {                // cropped input frames (uint16 entry): row -> (frame, y)
             const long frame = rows32 ? (long)((uint32_t)row / (uint32_t)fp.H) : row / fp.H;
             rp = in + (frame * fp.in_H + fp.in_crop + (row - frame * fp.H)) * W;
         }
@@ -205,7 +211,11 @@ __global__ void __launch_bounds__(256) k1_mask_rows(const T* __restrict__ in, Fr
     float* rowvals = reinterpret_cast<float*>(ws.scratch);
     for (long row = warp; row < nrows; row += nwarps) {
         const T* rp = in + row * W;
-        if (fp.in_H != fp.H) {                       // cropped input frames (uint16 entry): row -> (frame, y)
+        if constexpr (std::is_same<T, SampledGt>::value) {   // row -> (frame, y), y of ground-truth frame f mod gt_frames
+            const long frame = rows32 ? (long)((uint32_t)row / (uint32_t)fp.H) : row / fp.H;
+            const long g = (long)((uint32_t)(fp.frame0 + frame) % (uint32_t)fp.gt_frames);
+            rp = in + (g * fp.H + (row - frame * fp.H)) * W;
+        } else if (fp.in_H != fp.H) {                // cropped input frames (uint16 entry): row -> (frame, y)
             const long frame = rows32 ? (long)((uint32_t)row / (uint32_t)fp.H) : row / fp.H;
             rp = in + (frame * fp.in_H + fp.in_crop + (row - frame * fp.H)) * W;
         }

@@ -90,15 +90,22 @@ struct K4xGeom {
     long pred_stride, pred_origin, gt_stride, gt_origin;
     int pitch, width;
 };
+// The geometry of the WRAP instances: prediction frame f is scored against ground-truth frame f mod gt_frames (the D
+// draws of dtfill_eval_sampled_mt_many, D * gt_frames filled frames over one ground truth).
+struct K4xWrapGeom : K4xGeom {
+    long gt_frames;
+};
+template <bool WRAP> using K4xGeomOf = typename std::conditional<WRAP, K4xWrapGeom, K4xGeom>::type;
 
 // npx: the scored pixels per frame; the term arrays hold npx entries per frame.  Block b scores frame f0 + b.
 // WIN: width < pitch (a region with width == pitch is contiguous, and pixel i is element i: no division per pixel).
 // FLOOR: the prediction is floored in registers, before the validity test and the terms: relu(pred - 0.9) + 0.9
 // (eval_NYU.py:202-206, float32) equals fmaxf(pred, 0.9f) on every value the fill gives from PNG samples (s / 256,
 // s in 0..65535; pinned by tests/test_eval_kitti_png.py).
-template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool FLOOR = false>
+// WRAP: the ground-truth frame of prediction frame f is f mod geom.gt_frames.
+template <typename GT, int MODE, typename GS = GT, bool WIN = false, bool FLOOR = false, bool WRAP = false>
 __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restrict__ pred, const GS* __restrict__ gt,
-                                                            const K4xGeom geom, long f0, long npx,
+                                                            const K4xGeomOf<WRAP> geom, long f0, long npx,
                                                             GT* __restrict__ terms /*[frames][4][npx]*/,
                                                             int* __restrict__ counts /*[frames][4]*/)
 {
@@ -106,7 +113,9 @@ __global__ void __launch_bounds__(K4X_THREADS) k4x_compact(const float* __restri
     __shared__ int hits[3];
     const int b = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const float* p = pred + geom.pred_origin + (f0 + b) * geom.pred_stride;
-    const GS* g = gt + geom.gt_origin + (f0 + b) * geom.gt_stride;
+    long fg = f0 + b;
+    if constexpr (WRAP) fg = (long)((uint32_t)fg % (uint32_t)geom.gt_frames);     // frames of a call < 2^31
+    const GS* g = gt + geom.gt_origin + fg * geom.gt_stride;
     auto px = [&](long i) -> long {
         if constexpr (WIN) {
             const int y = (int)i / geom.width;
@@ -268,9 +277,12 @@ __global__ void __launch_bounds__(K4X_RTHREADS) k4x_reduce(const GT* __restrict_
     }
 }
 
-// column sums of per_frame over the batch (the running totals of eval.py:212-232), as k4_metrics_final computes them
+// column sums of per_frame over the batch (the running totals of eval.py:212-232), as k4_metrics_final computes them;
+// block k sums rows [k*B, k*B + B) into sums[k] (one block per draw of dtfill_eval_sampled_mt_many, one block elsewhere)
 __global__ void __launch_bounds__(32) k4x_sums(const double* __restrict__ per_frame, int B, double* __restrict__ sums, int accumulate)
 {
+    per_frame += (long)blockIdx.x * B * 9;
+    sums += blockIdx.x * 10;
     if (threadIdx.x < 10) {
         double s = 0.0;
         if (threadIdx.x < 9)

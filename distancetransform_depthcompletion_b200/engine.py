@@ -224,6 +224,22 @@ class DTFillEngine:
         self._inflight = {}       # the call synchronised: every earlier call has finished
         return res
 
+    def eval_drawn_many(self, gt, n, rngs, crop=None, src_thr: float | None = None):
+        """eval_nyu.evaluate_fill_drawn_many against the float32 CUDA tensor gt [B,H,W], used in place, on torch's current
+        stream: D draws, draw d of n (or n[d]) samples per frame from rngs[d]'s MT19937 state, each generator advanced as
+        eval_drawn advances it.  Synchronous: returns (per_frame [D,B,9], sums [D,10]) float64 numpy arrays.  Fills still
+        in flight are joined first."""
+        from . import eval_nyu
+        torch = self.torch
+        assert gt.is_cuda and gt.dtype == torch.float32 and gt.dim() == 3
+        gt = eval_nyu._aligned(gt)
+        crop = eval_nyu.NYU_EVAL_CROP if crop is None else crop
+        src_thr = eval_nyu.NYU_SRC_THR if src_thr is None else src_thr
+        self._bind_stream()
+        res = eval_nyu._eval_drawn_many(lambda: self.handle, gt.data_ptr(), True, gt.shape, n, rngs, crop, src_thr)
+        self._inflight = {}       # the call synchronised: every earlier call has finished
+        return res
+
     def flush(self):
         """Pipelined mode: torch's current stream waits for every fill still in flight."""
         self._bind_stream()

@@ -6,6 +6,7 @@ script's evaluation loop on the GPU.
     nyu_sample_coords(n)           -> (rows, cols)       data_read.py:360-364 (the random sample of one frame)
     evaluate_fill_sampled(gt, rows, cols) -> (per_frame [B,9], sums [10])   eval_NYU.py:138-254 from dense ground truth
     evaluate_fill_drawn(gt, n, rng)       -> (per_frame [B,9], sums [10])   the same loop with its draws, from rng's state
+    evaluate_fill_drawn_many(gt, n, rngs) -> (per_frame [D,B,9], sums [D,10])   D such draws, each from its own generator
     evaluate_fill_kitti_png_files(lidar_files, gt) -> (per_frame [B,9], sums [10])   the script's KITTI branch, from files
 """
 from __future__ import annotations
@@ -216,12 +217,11 @@ def evaluate_fill_drawn(gt, n: int, rng=np.random, crop=NYU_EVAL_CROP, src_thr: 
                        return_coords)
 
 
-def _mt_state(rng):
+def _mt_state(rng, who="evaluate_fill_drawn"):
     get = getattr(rng, "get_state", None)
     st = get(legacy=False) if callable(get) else None
     if not isinstance(st, dict) or st.get("bit_generator") != "MT19937":
-        raise TypeError(f"evaluate_fill_drawn: rng must be a np.random.RandomState or the np.random module (MT19937), "
-                        f"got {rng!r}")
+        raise TypeError(f"{who}: rng must be a np.random.RandomState or the np.random module (MT19937), got {rng!r}")
     return st
 
 
@@ -259,6 +259,100 @@ def _eval_drawn(get_handle, gt, gt_is_device, shape, n, rng, crop, src_thr, retu
     _set_mt(rng, st, r["key"], r["pos"])
     if return_coords:
         return r["per_frame"], r["sums"], r["rows"].astype(np.int64), r["cols"].astype(np.int64)
+    return r["per_frame"], r["sums"]
+
+
+def evaluate_fill_drawn_many(gt, n, rngs, crop=NYU_EVAL_CROP, src_thr: float = NYU_SRC_THR, device: int | None = None):
+    """D calls of evaluate_fill_drawn over the same ground truth in one call on the GPU, that is this loop:
+
+        for d in range(D):
+            per_frame[d], sums[d] = evaluate_fill_drawn(gt, n[d], rngs[d], crop, src_thr)
+
+    with its results bit for bit and every generator left where the loop leaves it (its cached Gaussian kept).  NYU
+    numbers are reported per sample count and averaged over several random draws; a list n covers that whole grid in one
+    call.  The generators are independent, so the device draws them side by side, one block each, and fills and scores
+    the frames of several draws together.
+
+    rngs: a sequence of D >= 1 MT19937 generators (np.random.RandomState, or the np.random module), no generator twice --
+    the draws would then depend on each other; evaluate_fill_drawn already continues one stream over many calls.  n: one
+    sample count for every draw, or a sequence of D counts.  gt, crop, src_thr, device: those of evaluate_fill_drawn.
+    Returns (per_frame float64 [D,B,9], sums float64 [D,10]).
+
+    Raises, before the device is touched and with every generator untouched: what evaluate_fill_drawn raises for any
+    draw's arguments, TypeError for an n that is not an integer or a sequence, ValueError for a sequence n whose length
+    is not D, for D = 0 and for a generator that appears twice.  IndexError ("draw d, frame b: ...") for the first frame
+    Distance_Transform rejects, in loop order: the generators of draws before d end where their draws end, generator d
+    after frame b's draws, and the generators after d stay untouched."""
+    gt, is_tensor = _dense_gt(gt, device, "evaluate_fill_drawn_many")
+    if is_tensor:
+        gt = _aligned(gt)
+        _torch_sync(gt)                 # the handle's stream reads gt
+        return _eval_drawn_many(lambda: _lib.get_handle(gt.device.index), gt.data_ptr(), True, gt.shape, n, rngs, crop,
+                                src_thr)
+    return _eval_drawn_many(lambda: _lib.get_handle(device), np.ascontiguousarray(gt), False, gt.shape, n, rngs, crop,
+                            src_thr)
+
+
+def _bit_generator(rng):
+    """What a generator draws from: the np.random module and the RandomState behind it are one stream, and so are
+    RandomStates built on one bit generator."""
+    if rng is np.random:
+        rng = np.random.mtrand._rand
+    return getattr(rng, "_bit_generator", rng)
+
+
+def _eval_drawn_many(get_handle, gt, gt_is_device, shape, n, rngs, crop, src_thr):
+    """The body of evaluate_fill_drawn_many and DTFillEngine.eval_drawn_many; get_handle() gives the Handle once the
+    arguments are checked."""
+    import operator
+    from .tools import VALID_THR
+    who = "evaluate_fill_drawn_many"
+    B, H, W = (int(v) for v in shape)
+    crop = _check_crop(crop, H, W)
+    rngs = list(rngs)
+    D = len(rngs)
+    if D == 0:
+        raise ValueError(f"{who}: no generators")
+    states = [_mt_state(r, who) for r in rngs]
+    seen = {}
+    for d, r in enumerate(rngs):
+        e = seen.setdefault(id(_bit_generator(r)), d)
+        if e != d:
+            raise ValueError(f"{who}: draws {e} and {d} share one generator; give each draw its own RandomState")
+    if isinstance(n, (str, bytes)):
+        raise TypeError(f"{who}: n must be an integer or a sequence of D integers, got {n!r}")
+    try:
+        ns = [operator.index(n)] * D
+    except TypeError:
+        try:
+            ns = [operator.index(v) for v in n]
+        except TypeError:
+            raise TypeError(f"{who}: n must be an integer or a sequence of D integers, got {n!r}") from None
+        if len(ns) != D:
+            raise ValueError(f"{who}: {len(ns)} sample counts for {D} generators")
+    for v in ns:                          # the checks of _eval_drawn, draw by draw
+        if v < 0:
+            raise ValueError("negative dimensions are not allowed")          # randint(size=n)
+        if v > 0 and (H - 12 <= 0 or W - 16 <= 0):
+            raise ValueError("high <= 0")
+        if v == 0 and (H < 13 or W < 17):     # randint draws nothing; an empty mask leaves no valid depth in frame 0
+            raise IndexError("draw 0, frame 0: labels index outside the list of valid depths (numpy IndexError)")
+    keys = np.stack([np.asarray(st["state"]["key"], np.uint32) for st in states])
+    pos = np.array([int(st["state"]["pos"]) for st in states], np.int32)
+    r = get_handle().eval_sampled_mt_many(gt, B, H, W, np.array(ns, np.int32), keys, pos, crop, src_thr, VALID_THR,
+                                          gt_is_device=gt_is_device)
+    last = D
+    if "index_error" in r:
+        last = r["first_bad_draw"]
+        # draw `last` stops after frame first_bad_frame's draws: replay the words every frame up to it consumed
+        bg = np.random.MT19937()
+        bg.state = {"bit_generator": "MT19937", "state": {"key": keys[last], "pos": int(pos[last])}}
+        bg.random_raw(int(r["words"][last, :r["first_bad_frame"] + 1].sum()))
+        _set_mt(rngs[last], states[last], bg.state["state"]["key"], bg.state["state"]["pos"])
+    for d in range(last):
+        _set_mt(rngs[d], states[d], r["keys"][d], r["pos"][d])
+    if "index_error" in r:
+        raise IndexError(r["index_error"])
     return r["per_frame"], r["sums"]
 
 

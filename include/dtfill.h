@@ -307,6 +307,26 @@ int dtfill_eval_sampled_mt(dtfill_t* h, const float* gt, int gt_is_device, int B
                            float val_thr, float* out_lidar, int32_t* out_rows, int32_t* out_cols, uint32_t* out_key,
                            int* out_pos, int64_t* out_words, double* per_frame, double* sums, int* first_bad_frame);
 
+/*
+ * D draws of dtfill_eval_sampled_mt over the same ground truth in one call, each from its own generator:
+ *     for d in range(D):  dtfill_eval_sampled_mt(gt, n[d], mt_keys[d], mt_pos[d]) -> rows d*B .. d*B + B - 1, sums[d]
+ * with the same results bit for bit.  The generators are independent: k11_mt_draw_many draws them side by side, one block
+ * each, and the D * B frames go through the fill and the scoring together, whole draws per fill (at most 2^28 pixels per
+ * fill, at least one draw), frame f of a fill reading ground-truth frame f mod B.  Inputs (host): n [D] >= 0, mt_keys
+ * [D][624], mt_pos [D] in [0, 624].  Only the keys and {pos, n} per draw go up (dtfill_transfer_bytes: D * 2504 bytes
+ * with a resident ground truth).  Outputs (host): per_frame [D*B][9], sums [D][10] (column sums of draw d's rows, then
+ * B), and, nullable, out_keys [D][624], out_pos [D], out_words int64 [D][B] as dtfill_eval_sampled_mt writes them per
+ * draw.  Synchronous; strict order on the handle's stream.
+ * Errors: DTFILL_E_ARG before anything is enqueued for D <= 0, a negative n[d], an mt_pos[d] outside [0, 624] and what
+ * dtfill_eval_sampled_mt refuses; then DTFILL_E_INDEX for the first frame Distance_Transform rejects, in loop order:
+ * draw *first_bad_draw, frame *first_bad_frame.  Fills after the one holding it do not run; the state outputs are still
+ * written for every draw, so the caller can rewind the failing draw to the end of that frame's draws.
+ */
+int dtfill_eval_sampled_mt_many(dtfill_t* h, const float* gt, int gt_is_device, int B, int H, int W, int D, const int* n,
+                                const uint32_t* mt_keys, const int* mt_pos, int r0, int r1, int c0, int c1, float src_thr,
+                                float val_thr, uint32_t* out_keys, int* out_pos, int64_t* out_words, double* per_frame,
+                                double* sums, int* first_bad_draw, int* first_bad_frame);
+
 /* Host-only test hook (no handle, no GPU), like dtfill_debug_png_decode_host: the draw of dtfill_eval_sampled_mt from
  * (key, pos) for B frames of H x W, run serially on the CPU with the kernel's MT19937 helpers.  rows / cols int32 [B*n],
  * out_key [624], *out_pos, out_words int64 [B] as there.  Returns 0, or -1 for bad arguments. */
